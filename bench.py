@@ -9,6 +9,7 @@ so scaling is weak (per-GPU work fixed).
   python bench.py [--gpus N --steps K --warmup W]            # our arm (libarapb200.so), batched API
   python bench.py --path opt_h [...]                          # our arm through the reference's own Opt.h call sequence
   python bench.py --impl reference [...]                      # the reference arm: CPU oracle port
+  python bench.py --dump-outputs DIR [...]                    # also write the last timed step's outputs (rank 0)
 Prints ONE JSON line (rank 0).
 """
 from __future__ import annotations
@@ -49,6 +50,37 @@ def workload_config(workload: str, pairs):
     return {"workload": f"{workload} {W}x{H}, {nseg} segment(s) per pair, fd={fd}, synth seeds {seed0}+",
             "schedule": f"{NCONT}x{NGN}x{NPCG}", "active_px_per_pair": float(np.mean(act)),
             "matches_per_pair": float(np.mean([len(p.matches) for p in pairs])), "warp": "forward warp of RGB + mask per segment"}
+
+
+DUMP_BYTES = 64_000_000     # --dump-outputs budget: all files together
+DUMP_SEED = 0               # seeds the pixel sample taken when the full outputs exceed the budget
+
+
+def dump_outputs(out_dir: str, outs, flats):
+    """Write what the timed path returned in its last step as float32 .npy files, one array per output field with the
+    problems stacked on axis 0: flow, rgb, mask (and costs) per problem, plus flat_flow, flat_rgb, flat_mask per pair
+    when a pair has several segments.  If the per-pixel arrays exceed DUMP_BYTES, every one of them keeps the same fixed,
+    seeded sample of pixels (row-major indices in pixel_index.npy) instead of the full image: the two pixel axes
+    [H, W] become one axis [n], e.g. flow.npy [problems, n, 2] and mask.npy [problems, n]."""
+    fields = {k: [o[k] for o in outs] for k in ("flow", "rgb", "mask")}
+    if flats:
+        fields.update({"flat_" + k: [f[i] for f in flats] for i, k in enumerate(("flow", "rgb", "mask"))})
+    H, W = outs[0]["mask"].shape
+    # float32 bytes of one pixel in every array; 1 MB is left for costs.npy and the .npy headers
+    px_bytes = sum(4 * len(v) * v[0][0, 0].size for v in fields.values())
+    budget = DUMP_BYTES - 1_000_000
+    n = H * W if px_bytes * H * W <= budget else budget // (px_bytes + 8)   # + 8: the float64 pixel_index entry
+    idx = None if n == H * W else np.sort(np.random.default_rng(DUMP_SEED).choice(H * W, n, replace=False))
+    os.makedirs(out_dir, exist_ok=True)
+    for k, v in fields.items():
+        a = np.stack([np.asarray(x).reshape(H * W, -1) for x in v]).astype(np.float32)
+        pixels = (H, W) if idx is None else (n,)
+        a = (a if idx is None else a[:, idx]).reshape((len(v),) + pixels + np.shape(v[0])[2:])
+        np.save(os.path.join(out_dir, k + ".npy"), a)
+    if idx is not None:
+        np.save(os.path.join(out_dir, "pixel_index.npy"), idx.astype(np.float64))
+    if all("costs" in o for o in outs):
+        np.save(os.path.join(out_dir, "costs.npy"), np.stack([o["costs"] for o in outs]).astype(np.float32))
 
 
 def measured_traffic(problems_per_launch: int):
@@ -284,7 +316,14 @@ def main():
     ap.add_argument("--batch", type=int, default=0, help="pairs per GPU per step (0 = backend default)")
     ap.add_argument("--backend", default="auto", choices=["auto", "stream", "resident"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the outputs of the last one to DIR/<name>.npy (float32, at most "
+                         "64 MB; rank 0's pairs)")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
@@ -348,16 +387,17 @@ def main():
                 opt_h_stage_log.append({k: round(v, 4) for k, v in cs.seconds.items()})
                 io_bytes[0] += cs.h2d_bytes
                 io_bytes[1] += cs.d2h_bytes
-                outs.append({"flow": cs.warp_field(), "rgb": cs.warped_rgb, "mask": cs.warped_mask})
+                outs.append({"flow": cs.warp_field(), "rgb": cs.warped_rgb, "mask": cs.warped_mask, "costs": cs.costs})
         else:
             outs = [batch.submit(i, p.rgb, m, p.matches, out=out_bufs[i]) for i, (p, m) in enumerate(problems)]
             out_bufs[:] = outs
             batch.run()
+        flats = []
         if nseg > 1:  # layer flatten of every pair (para_gen.py:136-175) belongs to the pair's end-to-end time
             for k in range(len(pairs)):
                 o = outs[k * nseg:(k + 1) * nseg]
-                lib.flatten([x["flow"] for x in o], [x["rgb"] for x in o], [x["mask"] for x in o])
-        return outs
+                flats.append(lib.flatten([x["flow"] for x in o], [x["rgb"] for x in o], [x["mask"] for x in o]))
+        return outs, flats
 
     flush = torch.empty(256 << 20, dtype=torch.uint8, device="cuda")  # > the 126 MiB L2
 
@@ -377,14 +417,14 @@ def main():
         flush_l2()
         if opt_h:
             ev[0].record()
-            one_step()
+            last = one_step()
             ev[1].record()
             ev[1].synchronize()
             ms = ev[0].elapsed_time(ev[1])
             dev_ms += ms
             solve_ms += ms
         else:
-            one_step()
+            last = one_step()
             tm = batch.timing_ms()
             dev_ms += tm["solve"] + tm["warp"]
             solve_ms += tm["solve"]
@@ -394,6 +434,8 @@ def main():
     barrier()
     wall = time.perf_counter() - t0
     clocks = sampler.stop()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, *last)
     # max over ranks (device-timed region and end-to-end wall)
     t = torch.tensor([dev_ms, wall * 1000.0, solve_ms], dtype=torch.float64, device="cuda")
     lt = torch.tensor([launches], dtype=torch.int64, device="cuda")

@@ -1,7 +1,22 @@
 """Shared problem builders for the parity tests (seeded, small enough for the oracle to finish in seconds)."""
+import lzma
+import os
+import shutil
+
 import numpy as np
 
 from arap_flow_b200 import synth
+
+GOLD = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+
+
+def cat512_flo(tmp_dir):
+    """Path of the reference's shipped cat512_iFlo.flo, restored byte for byte into tmp_dir from the xz-compressed copy
+    under tests/golden (the raw file is 2 MB)."""
+    path = os.path.join(str(tmp_dir), "cat512_iFlo.flo")
+    with lzma.open(os.path.join(GOLD, "cat512_iFlo.flo.xz")) as src, open(path, "wb") as dst:
+        shutil.copyfileobj(src, dst)
+    return path
 
 
 def random_problem(W, H, seed, p_inactive=0.25, n_cstr=10, angle_amp=0.3, x_amp=0.5):

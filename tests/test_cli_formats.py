@@ -7,6 +7,7 @@ import numpy as np
 import pytest
 
 from arap_flow_b200 import flowio
+from tests.helpers import cat512_flo
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 BIN = os.path.join(ROOT, "arap_flow_b200", "bin")
@@ -61,8 +62,9 @@ def test_png_encoder_round_trip(tmp_path):
 
 def test_flo_and_constraint_readers(gold, tmp_path):
     out = str(tmp_path / "copy.flo")
-    subprocess.check_call([TOOL, "flocopy", os.path.join(gold, "cat512_iFlo.flo"), out])
-    assert open(out, "rb").read() == open(os.path.join(gold, "cat512_iFlo.flo"), "rb").read()
+    flo = cat512_flo(tmp_path)
+    subprocess.check_call([TOOL, "flocopy", flo, out])
+    assert open(out, "rb").read() == open(flo, "rb").read()
     bad = tmp_path / "bad.flo"
     bad.write_bytes(b"XXXX" + b"\0" * 20)
     assert subprocess.call([TOOL, "flocopy", str(bad), out], stderr=subprocess.DEVNULL) != 0
@@ -70,9 +72,9 @@ def test_flo_and_constraint_readers(gold, tmp_path):
     c = flowio.read_constraints(os.path.join(gold, "cat512_iCstr.txt"))
     assert int(got[0]) == len(c) == 9 and int(got[1]) == int(c.sum())
     # python-side .flo round trip
-    fl = flowio.read_flo(os.path.join(gold, "cat512_iFlo.flo"))
+    fl = flowio.read_flo(flo)
     flowio.write_flo(out, fl)
-    assert open(out, "rb").read() == open(os.path.join(gold, "cat512_iFlo.flo"), "rb").read()
+    assert open(out, "rb").read() == open(flo, "rb").read()
 
 
 def test_argv_contracts_without_gpu(tmp_path):

@@ -5,7 +5,7 @@ import numpy as np
 import pytest
 
 from arap_flow_b200 import flowio, lib, synth
-from tests.helpers import epe, random_problem, synth_gn_problem
+from tests.helpers import cat512_flo, epe, random_problem, synth_gn_problem
 
 pytestmark = pytest.mark.gpu
 
@@ -173,10 +173,10 @@ def test_deform_edge_cases(oracle):
 
 
 # ------------------------------------------------------------------------------------- forward warp
-def test_warp_golden_cat512(oracle, gold):
+def test_warp_golden_cat512(oracle, gold, tmp_path):
     rgb = flowio.read_png_rgb(os.path.join(gold, "cat512_iRGB.png"))
     msk = flowio.read_png_mask_red(os.path.join(gold, "cat512_iMsk.png"))
-    flo = flowio.read_flo(os.path.join(gold, "cat512_iFlo.flo"))
+    flo = flowio.read_flo(cat512_flo(tmp_path))
     r, m, sp = lib.warp_flow(flo, rgb, msk)
     assert _eq(m, flowio.read_png_rgb(os.path.join(gold, "cat512_wMsk.png"))[..., 0])          # shipped golden
     assert _eq(r, flowio.read_png_rgb(os.path.join(gold, "cat512_reftool_wRGB.png")))          # reference tool

@@ -7,16 +7,18 @@ import pytest
 
 from arap_flow_b200 import flowio
 
+from .helpers import cat512_flo
 
-def _cat(gold):
+
+def _cat(gold, tmp_path):
     rgb = flowio.read_png_rgb(os.path.join(gold, "cat512_iRGB.png"))
     msk = flowio.read_png_mask_red(os.path.join(gold, "cat512_iMsk.png"))
-    flo = flowio.read_flo(os.path.join(gold, "cat512_iFlo.flo"))
+    flo = flowio.read_flo(cat512_flo(tmp_path))
     return rgb, msk, flo
 
 
-def test_warp_oracle_matches_shipped_golden_mask(oracle, gold):
-    rgb, msk, flo = _cat(gold)
+def test_warp_oracle_matches_shipped_golden_mask(oracle, gold, tmp_path):
+    rgb, msk, flo = _cat(gold, tmp_path)
     o_rgb, o_m, sp = oracle.warp(oracle.flow_to_pos(flo), rgb, msk)
     g_m = flowio.read_png_rgb(os.path.join(gold, "cat512_wMsk.png"))
     assert np.array_equal(o_m, g_m[..., 0]) and np.array_equal(g_m[..., 0], g_m[..., 2])
@@ -27,10 +29,10 @@ def test_warp_oracle_matches_shipped_golden_mask(oracle, gold):
     assert d.max() <= 1 and (d.max(-1) > 0).mean() < 0.005
 
 
-def test_warp_oracle_bit_exact_vs_reference_tool(oracle, gold):
+def test_warp_oracle_bit_exact_vs_reference_tool(oracle, gold, tmp_path):
     """cat512 RGB and three synthetic cases (folds, out-of-frame motion, ragged masks, identity) produced by the
     reference's own warp_image binary (tools/make_golden.py)."""
-    rgb, msk, flo = _cat(gold)
+    rgb, msk, flo = _cat(gold, tmp_path)
     o_rgb, _, _ = oracle.warp(oracle.flow_to_pos(flo), rgb, msk)
     assert np.array_equal(o_rgb, flowio.read_png_rgb(os.path.join(gold, "cat512_reftool_wRGB.png")))
     z = np.load(os.path.join(gold, "warp_reftool_cases.npz"))
@@ -71,13 +73,13 @@ def test_solve_pin_record(gold):
     assert pin["median_epe_px"] < 0.12
 
 
-def test_solve_energy_pin_vs_shipped_golden(oracle, gold):
+def test_solve_energy_pin_vs_shipped_golden(oracle, gold, tmp_path):
     """Energy-level anchor for the solve (the trajectory-level one is chaotic, see test_solve_pin_record): evaluate the
     ARAP energy AS DEFINED (arap_plan.t:13-23; float64 residuals, angles at their closed-form optimum for the given
     positions) at the reference's shipped result cat512_iFlo.flo and at the oracle's recorded full-schedule result.  Both
     must have minimised the same energy to the same level."""
     from .helpers import optimal_angles
-    rgb, msk, flo_gold = _cat(gold)
+    rgb, msk, flo_gold = _cat(gold, tmp_path)
     flo_ours = np.load(os.path.join(gold, "cat512_oracle_flow.npz"))["flow"]
     cstr = flowio.read_constraints(os.path.join(gold, "cat512_iCstr.txt"))
     H, W = msk.shape
@@ -98,8 +100,8 @@ def test_solve_energy_pin_vs_shipped_golden(oracle, gold):
 
 
 @pytest.mark.slow
-def test_solve_cat512_full(oracle, gold):
-    rgb, msk, flo = _cat(gold)
+def test_solve_cat512_full(oracle, gold, tmp_path):
+    rgb, msk, flo = _cat(gold, tmp_path)
     cstr = flowio.read_constraints(os.path.join(gold, "cat512_iCstr.txt"))
     X, A, costs = oracle.solve(msk, cstr)
     fl = oracle.flow(X)

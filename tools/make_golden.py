@@ -12,6 +12,7 @@ from __future__ import annotations
 
 import argparse
 import json
+import lzma
 import os
 import shutil
 import subprocess
@@ -132,18 +133,22 @@ def main():
         ("deformation/cat512_iRGB.png", "cat512_iRGB.png"),
         ("deformation/cat512_iMsk.png", "cat512_iMsk.png"),
         ("deformation/cat512_iCstr.txt", "cat512_iCstr.txt"),
-        ("warping/cat512_iFlo.flo", "cat512_iFlo.flo"),
         ("warping/cat512_wRGB.png", "cat512_wRGB.png"),
         ("warping/cat512_wMsk.png", "cat512_wMsk.png"),
     ):
         shutil.copyfile(os.path.join(REF, src), os.path.join(GOLD, dst))
         os.chmod(os.path.join(GOLD, dst), 0o644)
+    # the shipped flow is 2 MB raw: stored xz-compressed, byte for byte (tests/helpers.py cat512_flo restores it)
+    with open(os.path.join(REF, "warping/cat512_iFlo.flo"), "rb") as f:
+        flo_bytes = f.read()
+    with open(os.path.join(GOLD, "cat512_iFlo.flo.xz"), "wb") as f:
+        f.write(lzma.compress(flo_bytes, preset=9 | lzma.PRESET_EXTREME))
     # 2. reference warp tool outputs: cat512 (its RGB differs from the shipped golden by +-1 on 978 px,
     #    SURVEY.md 4) and synthetic cases with folds / out-of-frame motion / ragged masks.
     with tempfile.TemporaryDirectory() as tmp:
         rgb = flowio.read_png_rgb(os.path.join(GOLD, "cat512_iRGB.png"))
         msk = flowio.read_png_mask_red(os.path.join(GOLD, "cat512_iMsk.png"))
-        flo = flowio.read_flo(os.path.join(GOLD, "cat512_iFlo.flo"))
+        flo = flowio.read_flo(os.path.join(REF, "warping/cat512_iFlo.flo"))
         wr, wm = ref_warp(rgb, msk, flo, tmp)
         flowio.write_png(os.path.join(GOLD, "cat512_reftool_wRGB.png"), wr)
         cases = {}
@@ -179,7 +184,11 @@ def main():
         epe = np.hypot(*(np.moveaxis(fl - flo, -1, 0)))
         cerr = [float(np.hypot(*(fl[y1, x1] - (x2 - x1, y2 - y1)))) for x1, y1, x2, y2 in cstr]
         gcerr = [float(np.hypot(*(flo[y1, x1] - (x2 - x1, y2 - y1)))) for x1, y1, x2, y2 in cstr]
-        np.savez_compressed(os.path.join(GOLD, "cat512_oracle_flow.npz"), flow=fl, angle=A, costs=costs)
+        np.savez_compressed(os.path.join(GOLD, "cat512_oracle_flow.npz"), flow=fl, costs=costs)
+        # the rasteriser on the solved positions themselves (positions rebuilt from the float32 flow can differ)
+        wr, wm, _ = O.warp(X, rgb, msk)
+        flowio.write_png(os.path.join(GOLD, "cat512_oracle_wRGB.png"), wr)
+        flowio.write_png(os.path.join(GOLD, "cat512_oracle_wMsk.png"), wm)
         out = dict(
             what="oracle full solve (19x8x400) on cat512 vs the shipped golden cat512_iFlo.flo",
             threads=O.num_threads(), seconds=dt,
