@@ -64,13 +64,17 @@ WarpArena& warp_arena()
 }
 
 int warp_common(int W, int H, const float* pos_or_flow, bool is_flow, const uint8_t* rgb, const uint8_t* mask_red,
-                uint8_t* out_rgb, uint8_t* out_mask, uint32_t* out_splat)
+                uint8_t* out_rgb, uint8_t* out_mask, uint32_t* out_splat, float* out_bflow = nullptr,
+                uint8_t* out_occ = nullptr)
 {
     if (W <= 0 || H <= 0 || !pos_or_flow || !rgb || !mask_red || !out_rgb || !out_mask) return 1;
     const size_t N = (size_t)W * H;
+    const bool ex = out_bflow || out_occ; // the occlusion needs the backward flow
     auto up256 = [](size_t b) { return (b + 255) & ~(size_t)255; };
     const size_t o_in = 0, o_pos = o_in + up256(8 * N), o_z = o_pos + up256(8 * N), o_rgb = o_z + up256(4 * N),
-                 o_orgb = o_rgb + up256(3 * N), o_m = o_orgb + up256(3 * N), o_om = o_m + up256(N), total = o_om + up256(N);
+                 o_orgb = o_rgb + up256(3 * N), o_m = o_orgb + up256(3 * N), o_om = o_m + up256(N),
+                 o_bf = o_om + up256(N), o_fl = o_bf + (ex ? up256(8 * N) : 0), o_occ = o_fl + (out_occ ? up256(8 * N) : 0),
+                 total = o_occ + (out_occ ? up256(N) : 0);
     WarpArena& ar = warp_arena();
     std::lock_guard<std::mutex> g(ar.mu);
     unsigned char* b = ar.reserve(total);
@@ -78,6 +82,7 @@ int warp_common(int W, int H, const float* pos_or_flow, bool is_flow, const uint
     float2* d_in = (float2*)(b + o_in);
     float2* d_pos = (float2*)(b + o_pos);
     unsigned* d_z = (unsigned*)(b + o_z);
+    float2* d_bf = ex ? (float2*)(b + o_bf) : nullptr;
     ARAP_CUDA_CHECK(cudaMemcpyAsync(d_in, pos_or_flow, 8 * N, cudaMemcpyHostToDevice, s));
     ARAP_CUDA_CHECK(cudaMemcpyAsync(b + o_rgb, rgb, 3 * N, cudaMemcpyHostToDevice, s));
     ARAP_CUDA_CHECK(cudaMemcpyAsync(b + o_m, mask_red, N, cudaMemcpyHostToDevice, s));
@@ -86,10 +91,20 @@ int warp_common(int W, int H, const float* pos_or_flow, bool is_flow, const uint
         enqueue_flow_to_pos(W, H, d_in, d_pos, s);
         pos = d_pos;
     }
-    enqueue_warp(W, H, pos, b + o_rgb, b + o_m, d_z, b + o_orgb, b + o_om, s);
+    enqueue_warp(W, H, pos, b + o_rgb, b + o_m, d_z, b + o_orgb, b + o_om, s, d_bf);
+    if (out_occ) {
+        const float2* flow = d_in; // forward flow: given, or X - grid exactly as the batch path extracts it
+        if (!is_flow) {
+            enqueue_pos_to_flow(W, H, d_in, (float2*)(b + o_fl), s);
+            flow = (const float2*)(b + o_fl);
+        }
+        enqueue_occlusion(W, H, b + o_m, flow, d_z, d_bf, b + o_occ, s);
+        ARAP_CUDA_CHECK(cudaMemcpyAsync(out_occ, b + o_occ, N, cudaMemcpyDeviceToHost, s));
+    }
     ARAP_CUDA_CHECK(cudaMemcpyAsync(out_rgb, b + o_orgb, 3 * N, cudaMemcpyDeviceToHost, s));
     ARAP_CUDA_CHECK(cudaMemcpyAsync(out_mask, b + o_om, N, cudaMemcpyDeviceToHost, s));
     if (out_splat) ARAP_CUDA_CHECK(cudaMemcpyAsync(out_splat, d_z, 4 * N, cudaMemcpyDeviceToHost, s));
+    if (out_bflow) ARAP_CUDA_CHECK(cudaMemcpyAsync(out_bflow, d_bf, 8 * N, cudaMemcpyDeviceToHost, s));
     ARAP_CUDA_OR_RETURN(cudaStreamSynchronize(s));
     return 0;
 }
@@ -158,6 +173,15 @@ int arapb200_warp_flow(int W, int H, const float* flow, const uint8_t* rgb, cons
     });
 }
 
+int arapb200_warp_ex(int W, int H, const float* pos_or_flow, int is_flow, const uint8_t* rgb, const uint8_t* mask_red,
+                     uint8_t* out_rgb, uint8_t* out_mask, uint32_t* out_splat, float* out_bflow, uint8_t* out_occ)
+{
+    return guarded([&]() -> int {
+        return warp_common(W, H, pos_or_flow, is_flow != 0, rgb, mask_red, out_rgb, out_mask, out_splat, out_bflow,
+                           out_occ);
+    });
+}
+
 int arapb200_deform(int W, int H, const uint8_t* rgb, const uint8_t* mask_red, const int32_t* matches, int n_matches,
                     int nCont, int nGN, int nPCG, int backend, float* out_flow, uint8_t* out_rgb, uint8_t* out_mask,
                     float* out_costs)
@@ -196,6 +220,14 @@ int arapb200_batch_submit(arapb200_batch* b, int slot, int W, int H, const uint8
                           const int32_t* matches, int n_matches, float* out_flow, uint8_t* out_rgb,
                           uint8_t* out_mask, float* out_costs)
 {
+    return arapb200_batch_submit_ex(b, slot, W, H, rgb, mask_red, matches, n_matches, out_flow, out_rgb, out_mask,
+                                    out_costs, nullptr, nullptr);
+}
+
+int arapb200_batch_submit_ex(arapb200_batch* b, int slot, int W, int H, const uint8_t* rgb, const uint8_t* mask_red,
+                             const int32_t* matches, int n_matches, float* out_flow, uint8_t* out_rgb,
+                             uint8_t* out_mask, float* out_costs, float* out_bflow, uint8_t* out_occ)
+{
     return guarded([&]() -> int {
         if (!b || slot < 0 || slot >= b->max_problems) return 1;
         // everything run() will dereference is checked here, while the caller can still be told
@@ -208,6 +240,7 @@ int arapb200_batch_submit(arapb200_batch* b, int slot, int W, int H, const uint8
         HostProblem& hp = b->slots[slot];
         hp.W = W; hp.H = H; hp.rgb = rgb; hp.mask_red = mask_red; hp.matches = matches; hp.n_matches = n_matches;
         hp.out_flow = out_flow; hp.out_rgb = out_rgb; hp.out_mask = out_mask; hp.out_costs = out_costs;
+        hp.out_bflow = out_bflow; hp.out_occ = out_occ;
         b->pending[slot] = 1;
         return 0;
     });

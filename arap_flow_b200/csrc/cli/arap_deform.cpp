@@ -1,6 +1,8 @@
 // arap_deform -- command-line front end with the argv / list-file / environment contract of the reference's
 // ARAP/deformation/src/main.cpp:162-241, as driven by para_gen.py:178-214, run_arap.py:10-15 and generate.py:
-//   arap_deform RGB MASK CSTR FLO_out WRGB_out WMASK_out      or      arap_deform LISTFILE
+//   arap_deform RGB MASK CSTR FLO_out WRGB_out WMASK_out [BFLO_out OCC_out]      or      arap_deform LISTFILE
+// The two optional outputs (8 tokens instead of 6, in argv or on a list line) are the backward flow (.flo) and the
+// occlusion of frame 1 (PNG, 255 = occluded; DESIGN.md 4.3); lines of 6 tokens run and write exactly what they always did.
 // Differences from the reference are on the inside only: consecutive list entries of one image size are
 // solved together (several problems per cooperative launch), nothing is interpreted from $ARAP_PLAN.
 //
@@ -12,10 +14,10 @@
 //                                    one long-lived process per GPU: keeps the context, the plan and the
 //                                    device buffers, and runs every list file dropped into SPOOLDIR; --warm
 //                                    builds plan + buffers for that image size at start-up
-//   ARAP_SERVER=SPOOLDIR arap_deform LISTFILE | RGB MASK CSTR FLO WRGB WMASK
+//   ARAP_SERVER=SPOOLDIR arap_deform LISTFILE | RGB MASK CSTR FLO WRGB WMASK [BFLO OCC]
 //                                    thin client: same argv contract, same "Saved" lines, same exit code;
 //                                    the work is done by the server that watches SPOOLDIR
-// Protocol: the client writes SPOOLDIR/<id>.job.tmp (the 6-tuples, one per line), renames it to <id>.job and
+// Protocol: the client writes SPOOLDIR/<id>.job.tmp (the 6- or 8-tuples, one per line), renames it to <id>.job and
 // waits for <id>.done (first line = exit code); the server renames <id>.job to <id>.run while it works.
 // SPOOLDIR/stop makes the server exit.
 #include "../../../include/Opt.h"
@@ -44,6 +46,8 @@ using namespace arapcli;
 
 struct InputPaths {
     std::string rgb, mask, cstr, flo, wrgb, wmask;
+    std::string bflo, occ; // both empty = a 6-token line: no backward flow / occlusion
+    bool extras() const { return !bflo.empty(); }
 };
 
 static void usage()
@@ -58,7 +62,11 @@ static void usage()
     puts("Flow \t\t [output] path to optical flow (.flo only)");
     puts("warped_RGB \t [output] path to output warped image (.png), all intermediate directories must exist");
     puts("warped_Mask \t [output] path to output warped mask (.png), all intermediate directories must exist");
-    puts("\n./arap_deform LISTFILE   (one such 6-tuple per line)");
+    puts("\n./arap_deform RGB Mask Constraint Flow warped_RGB warped_Mask Backward_Flow Occlusion\n");
+    puts("also writes, from the same solve and warp:");
+    puts("Backward_Flow \t [output] path to the backward flow (.flo): from each frame-2 pixel to its frame-1 source point, 0 where nothing landed");
+    puts("Occlusion \t [output] path to the occlusion of frame 1 (.png): 255 where a pixel is not visible in frame 2, else 0");
+    puts("\n./arap_deform LISTFILE   (one such 6- or 8-tuple per line, both kinds may be mixed; further tokens are ignored)");
     puts("./arap_deform --serve SPOOLDIR [--warm WxH]   (resident worker: runs the list files that clients with ARAP_SERVER=SPOOLDIR");
     puts("                                               submit; --warm pre-builds the plan and buffers for that image size)");
     puts("Environment: ARAP_PLAN = path of the ARAP energy file (default ./arap_plan.t); CUDA_VISIBLE_DEVICES selects the GPU;");
@@ -75,6 +83,8 @@ struct Loaded {
     std::vector<int32_t> cstr;
     std::vector<float> flow;
     std::vector<uint8_t> wrgb, wmask;
+    std::vector<float> bflow;  // only for 8-token lines
+    std::vector<uint8_t> occ;
 };
 
 // the GPU context that outlives a list file (and, in --serve mode, every client request)
@@ -93,7 +103,11 @@ static bool read_list(const char* path, std::vector<InputPaths>& lines)
     while (getline(infile, line)) {
         std::stringstream s(line);
         InputPaths p;
-        if (s >> p.rgb >> p.mask >> p.cstr >> p.flo >> p.wrgb >> p.wmask) lines.push_back(p);
+        if (s >> p.rgb >> p.mask >> p.cstr >> p.flo >> p.wrgb >> p.wmask) {
+            std::string b, o;
+            if (s >> b >> o) { p.bflo = b; p.occ = o; }
+            lines.push_back(p);
+        }
     }
     return true;
 }
@@ -177,8 +191,10 @@ static int process(const std::vector<InputPaths>& lines, Context& C)
         }
         for (size_t k = 0; k < g->items.size(); ++k) {
             Loaded& L = g->items[k];
-            if (arapb200_batch_submit(C.ctx, (int)k, g->W, g->H, L.rgb.px.data(), L.mask_red.data(), L.cstr.data(),
-                                      (int)(L.cstr.size() / 4), L.flow.data(), L.wrgb.data(), L.wmask.data(), NULL))
+            const bool ex = !L.occ.empty();
+            if (arapb200_batch_submit_ex(C.ctx, (int)k, g->W, g->H, L.rgb.px.data(), L.mask_red.data(), L.cstr.data(),
+                                         (int)(L.cstr.size() / 4), L.flow.data(), L.wrgb.data(), L.wmask.data(), NULL,
+                                         ex ? L.bflow.data() : NULL, ex ? L.occ.data() : NULL))
                 return 1;
         }
         return arapb200_batch_run(C.ctx);
@@ -187,10 +203,16 @@ static int process(const std::vector<InputPaths>& lines, Context& C)
     auto save_one = [&](const Group& g, size_t k) -> bool {
         const Loaded& L = g.items[k];
         const InputPaths& p = lines[g.first + k];
-        std::vector<uint8_t> m3((size_t)3 * g.W * g.H); // warped mask as an RGB image, 255 = object (README.md:25-32)
-        for (size_t q = 0; q < L.wmask.size(); ++q) m3[3 * q] = m3[3 * q + 1] = m3[3 * q + 2] = L.wmask[q];
-        return save_png_rgb(p.wrgb, g.W, g.H, L.wrgb.data()) && save_png_rgb(p.wmask, g.W, g.H, m3.data()) &&
-               write_flo(p.flo, g.W, g.H, L.flow.data());
+        auto gray3 = [](const std::vector<uint8_t>& m) { // a mask as an RGB image (README.md:25-32)
+            std::vector<uint8_t> m3(3 * m.size());
+            for (size_t q = 0; q < m.size(); ++q) m3[3 * q] = m3[3 * q + 1] = m3[3 * q + 2] = m[q];
+            return m3;
+        };
+        if (!save_png_rgb(p.wrgb, g.W, g.H, L.wrgb.data()) || !save_png_rgb(p.wmask, g.W, g.H, gray3(L.wmask).data()) ||
+            !write_flo(p.flo, g.W, g.H, L.flow.data()))
+            return false;
+        return !p.extras() ||
+               (write_flo(p.bflo, g.W, g.H, L.bflow.data()) && save_png_rgb(p.occ, g.W, g.H, gray3(L.occ).data()));
     };
     auto save_stage = [&](const Group& g) -> bool {
         std::vector<std::future<bool>> jobs;
@@ -217,6 +239,10 @@ static int process(const std::vector<InputPaths>& lines, Context& C)
         L.flow.resize(2 * N);
         L.wrgb.resize(3 * N);
         L.wmask.resize(N);
+        if (lines[idx].extras()) {
+            L.bflow.resize(2 * N);
+            L.occ.resize(N);
+        }
         return true;
     };
 
@@ -383,8 +409,11 @@ static int submit(const std::string& dir, const std::vector<InputPaths>& lines)
     const std::string base = dir + "/" + id;
     {
         std::ofstream o(base + ".job.tmp");
-        for (const InputPaths& p : lines)
-            o << p.rgb << " " << p.mask << " " << p.cstr << " " << p.flo << " " << p.wrgb << " " << p.wmask << "\n";
+        for (const InputPaths& p : lines) {
+            o << p.rgb << " " << p.mask << " " << p.cstr << " " << p.flo << " " << p.wrgb << " " << p.wmask;
+            if (p.extras()) o << " " << p.bflo << " " << p.occ;
+            o << "\n";
+        }
         if (!o) return 1;
     }
     if (rename((base + ".job.tmp").c_str(), (base + ".job").c_str()) != 0) return 1;
@@ -426,8 +455,9 @@ int main(int argc, const char* argv[])
         return serve(argv[2], ww, wh);
     }
     std::vector<InputPaths> lines;
-    if (argc == 7) {
-        lines.push_back({argv[1], argv[2], argv[3], argv[4], argv[5], argv[6]});
+    if (argc == 7 || argc == 9) {
+        lines.push_back({argv[1], argv[2], argv[3], argv[4], argv[5], argv[6], argc == 9 ? argv[7] : "",
+                         argc == 9 ? argv[8] : ""});
     } else if (argc == 2) { // a list file: main.cpp:182-193
         read_list(argv[1], lines);
     } else {

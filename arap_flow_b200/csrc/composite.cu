@@ -5,8 +5,11 @@
 //   match filter + segment masks (para_gen.py:216-223, 468-482, 513-537): "next" row N3, the step right before the solve.
 // One thread per pixel; the winning layer is the LAST segment whose mask is non-zero (else segment 0), so the result
 // does not depend on any ordering between threads.  Pure select arithmetic: bit-identical to the numpy original.
+// Opt-in (arapb200_flatten_ex): the flattened backward flow and the occlusion of frame 1 across the layers, with the
+// same occlusion rule as the per-problem warp (warp.cuh occlusion_of, DESIGN.md 4.3).
 #include "../../include/arapb200.h"
 #include "common.cuh"
+#include "warp.cuh"
 
 #include <mutex>
 #include <vector>
@@ -19,18 +22,30 @@ struct Layers {
     const float2* flow[MAX_LAYERS];
     const unsigned char* rgb[MAX_LAYERS];
     const unsigned char* mask[MAX_LAYERS];
+    const float2* bflow[MAX_LAYERS];      // backward flow of each layer (only read for out_bflow / out_occ)
+    const unsigned char* src[MAX_LAYERS]; // frame-1 input mask of each layer, 0 = object (only read for out_occ)
     int n;
 };
 
-__global__ void __launch_bounds__(256) k_flatten(size_t N, Layers L, const unsigned char* __restrict__ bg,
-                                                  float2* __restrict__ out_flow, unsigned char* __restrict__ out_rgb,
-                                                  unsigned char* __restrict__ out_mask)
+// the layer in front at pixel i: the last one whose warped mask is non-zero, -1 = none
+__device__ __forceinline__ int front_layer(const Layers& L, size_t i)
 {
+    for (int s = L.n - 1; s >= 0; --s)
+        if (L.mask[s][i] != 0) return s;
+    return -1;
+}
+
+// out_bflow / out_occ may be null (arapb200_flatten passes null for both)
+__global__ void __launch_bounds__(256) k_flatten(int W, int H, Layers L, const unsigned char* __restrict__ bg,
+                                                  float2* __restrict__ out_flow, unsigned char* __restrict__ out_rgb,
+                                                  unsigned char* __restrict__ out_mask, float2* __restrict__ out_bflow,
+                                                  unsigned char* __restrict__ out_occ)
+{
+    const size_t N = (size_t)W * H;
     const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (i >= N) return;
-    int win = 0;
-    for (int s = L.n - 1; s >= 1; --s)
-        if (L.mask[s][i] != 0) { win = s; break; }
+    const int front = front_layer(L, i);
+    const int win = front < 0 ? 0 : front; // segment 0 is the base of the flow / colour / mask layering
     const unsigned char m = L.mask[win][i];
     out_flow[i] = L.flow[win][i];
     out_mask[i] = m;
@@ -38,6 +53,15 @@ __global__ void __launch_bounds__(256) k_flatten(size_t N, Layers L, const unsig
     out_rgb[3 * i] = src[3 * i];
     out_rgb[3 * i + 1] = src[3 * i + 1];
     out_rgb[3 * i + 2] = src[3 * i + 2];
+    if (out_bflow) out_bflow[i] = front < 0 ? make_float2(0.f, 0.f) : L.bflow[front][i];
+    if (out_occ) {
+        int seg = -1; // p's surface: the (last) layer whose input mask has p on the object
+        for (int s = L.n - 1; s >= 0; --s)
+            if (L.src[s][i] == 0) { seg = s; break; }
+        const float2 f = seg >= 0 ? L.flow[seg][i] : make_float2(0.f, 0.f);
+        out_occ[i] = occlusion_of(W, H, (int)(i % W), (int)(i / W), seg, f, seg >= 0 ? L.bflow[seg] : nullptr,
+                                  [&L](size_t q) { return front_layer(L, q); });
+    }
 }
 
 // ---- N3: match filter (para_gen.py:216-223) and per-segment masks (:513-537) ----
@@ -168,23 +192,28 @@ extern "C" int arapb200_segment_mask(int W, int H, const uint8_t* labels, int se
     return 0;
 }
 
-extern "C" int arapb200_flatten(int W, int H, int n_layers, const float* const* flows, const uint8_t* const* rgbs,
-                                const uint8_t* const* masks, const uint8_t* background, float* out_flow,
-                                uint8_t* out_rgb, uint8_t* out_mask)
+namespace {
+int flatten_common(int W, int H, int n_layers, const float* const* flows, const uint8_t* const* rgbs,
+                   const uint8_t* const* masks, const uint8_t* background, const uint8_t* const* src_masks,
+                   const float* const* bflows, float* out_flow, uint8_t* out_rgb, uint8_t* out_mask, float* out_bflow,
+                   uint8_t* out_occ)
 {
     if (W <= 0 || H <= 0 || n_layers < 1 || n_layers > MAX_LAYERS || !flows || !rgbs || !masks) return 1;
+    if ((out_bflow || out_occ) && !bflows) return 1;
+    if (out_occ && !src_masks) return 1;
+    const bool ex = out_bflow || out_occ;
     const size_t N = (size_t)W * H;
     Layers L{};
     L.n = n_layers;
     // One grow-only device arena per process (cudaMalloc / cudaFree of 15 multi-megabyte blocks per call cost far more
-    // than the kernel): [layers: flow, rgb, mask][background][outputs], every block 256-byte aligned.
+    // than the kernel): [layers: flow, rgb, mask (, bflow, src mask)][background][outputs], every block 256-byte aligned.
     static std::mutex mu;
     static unsigned char* arena = nullptr;
     static size_t arena_bytes = 0;
     static int arena_dev = -1;
     std::lock_guard<std::mutex> lock(mu);
     auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
-    const size_t per_layer = al(N * sizeof(float2)) + al(3 * N) + al(N);
+    const size_t per_layer = al(N * sizeof(float2)) + al(3 * N) + al(N) + (ex ? al(N * sizeof(float2)) + al(N) : 0);
     const size_t need = (size_t)(n_layers + 1) * per_layer + al(3 * N);
     int dev = 0;
     int rc = 0;
@@ -205,6 +234,8 @@ extern "C" int arapb200_flatten(int W, int H, int n_layers, const float* const* 
         L.flow[s] = (const float2*)up(flows[s], N * sizeof(float2));
         L.rgb[s] = (const unsigned char*)up(rgbs[s], 3 * N);
         L.mask[s] = (const unsigned char*)up(masks[s], N);
+        if (ex) L.bflow[s] = (const float2*)up(bflows[s], N * sizeof(float2));
+        if (out_occ) L.src[s] = (const unsigned char*)up(src_masks[s], N);
     }
     const unsigned char* d_bg = nullptr;
     if (!rc && background) d_bg = (const unsigned char*)up(background, 3 * N);
@@ -212,11 +243,33 @@ extern "C" int arapb200_flatten(int W, int H, int n_layers, const float* const* 
         float2* d_of = (float2*)take(N * sizeof(float2));
         unsigned char* d_or = take(3 * N);
         unsigned char* d_om = take(N);
-        k_flatten<<<(unsigned)((N + 255) / 256), 256>>>(N, L, d_bg, d_of, d_or, d_om);
+        float2* d_ob = out_bflow ? (float2*)take(N * sizeof(float2)) : nullptr;
+        unsigned char* d_oo = out_occ ? take(N) : nullptr;
+        k_flatten<<<(unsigned)((N + 255) / 256), 256>>>(W, H, L, d_bg, d_of, d_or, d_om, d_ob, d_oo);
         if (cudaMemcpy(out_flow, d_of, N * sizeof(float2), cudaMemcpyDeviceToHost) ||
-            cudaMemcpy(out_rgb, d_or, 3 * N, cudaMemcpyDeviceToHost) || cudaMemcpy(out_mask, d_om, N, cudaMemcpyDeviceToHost))
+            cudaMemcpy(out_rgb, d_or, 3 * N, cudaMemcpyDeviceToHost) || cudaMemcpy(out_mask, d_om, N, cudaMemcpyDeviceToHost) ||
+            (d_ob && cudaMemcpy(out_bflow, d_ob, N * sizeof(float2), cudaMemcpyDeviceToHost)) ||
+            (d_oo && cudaMemcpy(out_occ, d_oo, N, cudaMemcpyDeviceToHost)))
             rc = 3;
     }
     if (rc) fprintf(stderr, "arapb200_flatten: CUDA failure (%s)\n", cudaGetErrorString(cudaGetLastError()));
     return rc;
+}
+} // namespace
+
+extern "C" int arapb200_flatten(int W, int H, int n_layers, const float* const* flows, const uint8_t* const* rgbs,
+                                const uint8_t* const* masks, const uint8_t* background, float* out_flow,
+                                uint8_t* out_rgb, uint8_t* out_mask)
+{
+    return flatten_common(W, H, n_layers, flows, rgbs, masks, background, nullptr, nullptr, out_flow, out_rgb, out_mask,
+                          nullptr, nullptr);
+}
+
+extern "C" int arapb200_flatten_ex(int W, int H, int n_layers, const float* const* flows, const uint8_t* const* rgbs,
+                                   const uint8_t* const* masks, const uint8_t* background, const uint8_t* const* src_masks,
+                                   const float* const* bflows, float* out_flow, uint8_t* out_rgb, uint8_t* out_mask,
+                                   float* out_bflow, uint8_t* out_occ)
+{
+    return flatten_common(W, H, n_layers, flows, rgbs, masks, background, src_masks, bflows, out_flow, out_rgb, out_mask,
+                          out_bflow, out_occ);
 }

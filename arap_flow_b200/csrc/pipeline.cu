@@ -147,8 +147,8 @@ BatchPipeline::~BatchPipeline()
     for (Dev& d : dev_) {
         cudaFree(d.X); cudaFree(d.U); cudaFree(d.C); cudaFree(d.flow); cudaFree(d.A); cudaFree(d.M);
         cudaFree(d.costs); cudaFree(d.rgb); cudaFree(d.mask); cudaFree(d.orgb); cudaFree(d.omask);
-        cudaFree(d.z); cudaFree(d.matches);
-        cudaFreeHost(d.h_in); cudaFreeHost(d.h_out);
+        cudaFree(d.z); cudaFree(d.matches); cudaFree(d.bflow); cudaFree(d.occ);
+        cudaFreeHost(d.h_in); cudaFreeHost(d.h_out); cudaFreeHost(d.h_extra);
     }
     for (auto& e : ev_) cudaEventDestroy(e);
     cudaStreamDestroy(stream_);
@@ -260,6 +260,12 @@ int BatchPipeline::run(const HostProblem* problems, int count)
             d.matches_cap = d.recs.size() * 2 + 1024;
             ARAP_CUDA_OR_RETURN(cudaMalloc(&d.matches, d.matches_cap * sizeof(MatchRec)));
         }
+        if ((hp.out_bflow || hp.out_occ) && !d.h_extra) {
+            const size_t Nmax = (size_t)maxW_ * maxH_;
+            ARAP_CUDA_OR_RETURN(cudaMalloc(&d.bflow, Nmax * sizeof(float2)));
+            ARAP_CUDA_OR_RETURN(cudaMalloc(&d.occ, Nmax));
+            ARAP_CUDA_OR_RETURN(cudaMallocHost(&d.h_extra, 9 * Nmax));
+        }
         memcpy(d.h_in, hp.rgb, 3 * N);
         memcpy(d.h_in + 3 * N, hp.mask_red, N);
     }
@@ -348,8 +354,13 @@ int BatchPipeline::run(const HostProblem* problems, int count)
         const HostProblem& hp = problems[i];
         Dev& d = dev_[i];
         enqueue_pos_to_flow(hp.W, hp.H, d.X, d.flow, stream_);
-        enqueue_warp(hp.W, hp.H, d.X, d.rgb, d.mask, d.z, d.orgb, d.omask, stream_);
+        const bool extras = hp.out_bflow || hp.out_occ;
+        enqueue_warp(hp.W, hp.H, d.X, d.rgb, d.mask, d.z, d.orgb, d.omask, stream_, extras ? d.bflow : nullptr);
         launches_ += 1 + warp_launches_per_call();
+        if (extras) {
+            enqueue_occlusion(hp.W, hp.H, d.mask, d.flow, d.z, d.bflow, d.occ, stream_);
+            launches_ += 1;
+        }
     }
     ARAP_CUDA_OR_RETURN(cudaEventRecord(ev_[3], stream_));
     for (int i = 0; i < count; ++i) {
@@ -361,6 +372,10 @@ int BatchPipeline::run(const HostProblem* problems, int count)
         ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(o + 8 * N, d.orgb, 3 * N, cudaMemcpyDeviceToHost, stream_));
         ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(o + 11 * N, d.omask, N, cudaMemcpyDeviceToHost, stream_));
         ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(o + 12 * N, d.costs, cbytes, cudaMemcpyDeviceToHost, stream_));
+        if (hp.out_bflow || hp.out_occ) {
+            ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(d.h_extra, d.bflow, N * sizeof(float2), cudaMemcpyDeviceToHost, stream_));
+            ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(d.h_extra + 8 * N, d.occ, N, cudaMemcpyDeviceToHost, stream_));
+        }
     }
     ARAP_CUDA_OR_RETURN(cudaStreamSynchronize(stream_));
     if (resident_ && n_resident_ > 0) {
@@ -386,6 +401,8 @@ int BatchPipeline::run(const HostProblem* problems, int count)
         if (hp.out_rgb) memcpy(hp.out_rgb, o + 8 * N, 3 * N);
         if (hp.out_mask) memcpy(hp.out_mask, o + 11 * N, N);
         if (hp.out_costs) memcpy(hp.out_costs, o + 12 * N, cbytes);
+        if (hp.out_bflow) memcpy(hp.out_bflow, d.h_extra, N * sizeof(float2));
+        if (hp.out_occ) memcpy(hp.out_occ, d.h_extra + 8 * N, N);
     }
     if (resident_) launches_ += resident_->launches() - r0;
     cudaEventElapsedTime(&ms_total_, ev_[0], ev_[3]);

@@ -19,6 +19,8 @@ struct HostProblem {
     unsigned char* out_rgb = nullptr;        // uint8x3[N]
     unsigned char* out_mask = nullptr;       // uint8[N]
     float* out_costs = nullptr;              // float[nCont*(nGN+1)] or null
+    float* out_bflow = nullptr;              // float2[N] backward flow or null (opt-in, DESIGN.md 4.3)
+    unsigned char* out_occ = nullptr;        // uint8[N] occlusion of frame 1 or null (opt-in)
 };
 
 // compact constraint record: source pixel index and the match, after the reference's filtering
@@ -75,6 +77,9 @@ private:
         MatchRec* matches = nullptr;
         size_t matches_cap = 0;
         unsigned char *h_in = nullptr, *h_out = nullptr;
+        // opt-in extras, allocated the first time the slot asks for them: backward flow, occlusion, pinned [bflow | occ]
+        float2* bflow = nullptr;
+        unsigned char *occ = nullptr, *h_extra = nullptr;
         std::vector<MatchRec> recs;
         bool resident = false;
     };

@@ -75,17 +75,20 @@ __global__ void __launch_bounds__(256) k_splat(int W, int H, const float2* __res
     splat_tri(W, H, p10, p01, p11, id + 1, z); // (pos10, pos01, pos11)  main.cpp:200-202
 }
 
-// pass 2: one thread per output pixel
+// pass 2: one thread per output pixel.  BFLOW: also the backward flow -- the winning triangle's barycentrics applied to
+// its undeformed vertex coordinates give the exact frame-1 source point of the pixel (DESIGN.md 4.3).
+template <bool BFLOW>
 __global__ void __launch_bounds__(256) k_resolve(int W, int H, const float2* __restrict__ pos,
                                                   const unsigned char* __restrict__ rgb,
                                                   const unsigned* __restrict__ z, unsigned char* __restrict__ out_rgb,
-                                                  unsigned char* __restrict__ out_mask)
+                                                  unsigned char* __restrict__ out_mask, float2* __restrict__ out_bflow)
 {
     const size_t N = (size_t)W * H;
     const size_t o = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (o >= N) return;
     const unsigned id = z[o];
     unsigned char c0 = 0, c1 = 0, c2 = 0, m = 0;
+    float2 bf = make_float2(0.f, 0.f); // nothing landed: the background is static
     if (id) {
         const unsigned t = (id - 1) & 1u;
         const size_t i00 = (id - 1) >> 1, i01 = i00 + 1, i10 = i00 + W, i11 = i10 + 1;
@@ -104,11 +107,34 @@ __global__ void __launch_bounds__(256) k_resolve(int W, int H, const float2* __r
         c1 = (unsigned char)__float2int_rz(v[1]);
         c2 = (unsigned char)__float2int_rz(v[2]);
         m = 255;
+        if (BFLOW) { // vertices (x0, y0 + t), (x0 + 1, y0), (x0 + t, y0 + 1); the colour's operation order
+            const int x0 = (int)(i00 % W), y0 = (int)(i00 / W);
+            const float xa = (float)x0, xb = (float)(x0 + 1), xc = (float)(x0 + (int)t);
+            const float ya = (float)(y0 + (int)t), yb = (float)y0, yc = (float)(y0 + 1);
+            const float sx = __fadd_rn(__fadd_rn(__fmul_rn(xa, w.b0), __fmul_rn(xb, w.b1)), __fmul_rn(xc, w.b2));
+            const float sy = __fadd_rn(__fadd_rn(__fmul_rn(ya, w.b0), __fmul_rn(yb, w.b1)), __fmul_rn(yc, w.b2));
+            bf = make_float2(__fsub_rn(sx, (float)x), __fsub_rn(sy, (float)y));
+        }
     }
     out_rgb[3 * o] = c0;
     out_rgb[3 * o + 1] = c1;
     out_rgb[3 * o + 2] = c2;
     out_mask[o] = m;
+    if (BFLOW) out_bflow[o] = bf;
+}
+
+// occlusion of frame 1: one thread per frame-1 pixel, gathering z, bflow and the forward flow (DESIGN.md 4.3)
+__global__ void __launch_bounds__(256) k_occlusion(int W, int H, const unsigned char* __restrict__ mask_red,
+                                                    const float2* __restrict__ flow, const unsigned* __restrict__ z,
+                                                    const float2* __restrict__ bflow, unsigned char* __restrict__ occ)
+{
+    const size_t N = (size_t)W * H;
+    const size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= N) return;
+    const int seg = mask_red[p] == 0 ? 0 : -1;
+    const float2 f = seg == 0 ? flow[p] : make_float2(0.f, 0.f);
+    occ[p] = occlusion_of(W, H, (int)(p % W), (int)(p / W), seg, f, bflow,
+                          [z](size_t q) { return z[q] != 0 ? 0 : -1; });
 }
 
 // positions from a flow field (main.cpp:160-166); also used for flow extraction X - grid
@@ -137,13 +163,26 @@ __global__ void __launch_bounds__(256) k_grid_add(int W, int H, const float2* __
 int warp_launches_per_call() { return 2; }
 
 void enqueue_warp(int W, int H, const float2* d_pos, const unsigned char* d_rgb, const unsigned char* d_mask_red,
-                  unsigned* d_z, unsigned char* d_out_rgb, unsigned char* d_out_mask, cudaStream_t stream)
+                  unsigned* d_z, unsigned char* d_out_rgb, unsigned char* d_out_mask, cudaStream_t stream,
+                  float2* d_out_bflow)
 {
     const size_t N = (size_t)W * H;
     ARAP_CUDA_CHECK(cudaMemsetAsync(d_z, 0, N * sizeof(unsigned), stream));
     dim3 g1((W + 31) / 32, (H + 7) / 8);
     k_splat<<<g1, 256, 0, stream>>>(W, H, d_pos, d_mask_red, d_z);
-    k_resolve<<<(unsigned)((N + 255) / 256), 256, 0, stream>>>(W, H, d_pos, d_rgb, d_z, d_out_rgb, d_out_mask);
+    const unsigned g2 = (unsigned)((N + 255) / 256);
+    if (d_out_bflow)
+        k_resolve<true><<<g2, 256, 0, stream>>>(W, H, d_pos, d_rgb, d_z, d_out_rgb, d_out_mask, d_out_bflow);
+    else
+        k_resolve<false><<<g2, 256, 0, stream>>>(W, H, d_pos, d_rgb, d_z, d_out_rgb, d_out_mask, nullptr);
+    ARAP_CUDA_CHECK(cudaGetLastError());
+}
+
+void enqueue_occlusion(int W, int H, const unsigned char* d_mask_red, const float2* d_flow, const unsigned* d_z,
+                       const float2* d_bflow, unsigned char* d_occ, cudaStream_t stream)
+{
+    const size_t N = (size_t)W * H;
+    k_occlusion<<<(unsigned)((N + 255) / 256), 256, 0, stream>>>(W, H, d_mask_red, d_flow, d_z, d_bflow, d_occ);
     ARAP_CUDA_CHECK(cudaGetLastError());
 }
 

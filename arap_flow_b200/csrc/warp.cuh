@@ -4,11 +4,37 @@
 
 namespace arapb200 {
 
-// z: uint32[W*H] scratch that ends up holding the splat index (1 + 2*(y*W+x) + t, 0 = empty)
+// z: uint32[W*H] scratch that ends up holding the splat index (1 + 2*(y*W+x) + t, 0 = empty).
+// d_out_bflow (may be null): float2[W*H] backward flow, source point of every frame-2 pixel minus the pixel (DESIGN.md 4.3)
 void enqueue_warp(int W, int H, const float2* d_pos, const unsigned char* d_rgb, const unsigned char* d_mask_red,
-                  unsigned* d_z, unsigned char* d_out_rgb, unsigned char* d_out_mask, cudaStream_t stream);
+                  unsigned* d_z, unsigned char* d_out_rgb, unsigned char* d_out_mask, cudaStream_t stream,
+                  float2* d_out_bflow = nullptr);
+// occlusion of frame 1 (0 = visible in frame 2, 255 = not), from the z-buffer and backward flow enqueue_warp left and the
+// forward flow d_flow = X - grid
+void enqueue_occlusion(int W, int H, const unsigned char* d_mask_red, const float2* d_flow, const unsigned* d_z,
+                       const float2* d_bflow, unsigned char* d_occ, cudaStream_t stream);
 void enqueue_flow_to_pos(int W, int H, const float2* d_flow, float2* d_pos, cudaStream_t stream);
 void enqueue_pos_to_flow(int W, int H, const float2* d_pos, float2* d_flow, cudaStream_t stream);
 int warp_launches_per_call();
+
+#ifdef __CUDACC__
+// The occlusion rule of DESIGN.md 4.3 for frame-1 pixel p = (px, py), shared by the per-problem kernel and the layer
+// flatten.  seg: p's surface (-1 = background); f: p's forward flow; bflow: backward flow of p's surface;
+// owner(q): the surface that is in front at frame-2 pixel q (-1 = nothing landed).  Returns 0 (visible) or 255.
+template <class Owner>
+__device__ __forceinline__ unsigned char occlusion_of(int W, int H, int px, int py, int seg, float2 f,
+                                                      const float2* __restrict__ bflow, Owner owner)
+{
+    if (seg < 0) return owner((size_t)py * W + px) < 0 ? 0 : 255; // static background: visible unless covered
+    const float tx = __fadd_rn(__fadd_rn((float)px, f.x), 0.5f), ty = __fadd_rn(__fadd_rn((float)py, f.y), 0.5f);
+    if (!(tx >= 0.f && tx < (float)W && ty >= 0.f && ty < (float)H)) return 255; // left the frame (or NaN)
+    const int qx = (int)floorf(tx), qy = (int)floorf(ty);
+    const size_t q = (size_t)qy * W + qx;
+    if (owner(q) != seg) return 255;
+    const float2 b = bflow[q];
+    const float ex = __fadd_rn(b.x, (float)(qx - px)), ey = __fadd_rn(b.y, (float)(qy - py));
+    return (fabsf(ex) < 1.f && fabsf(ey) < 1.f) ? 0 : 255;
+}
+#endif
 
 } // namespace arapb200

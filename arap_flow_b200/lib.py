@@ -28,7 +28,7 @@ ARAP_SYMBOLS = [
     "arapb200_debug_apply_jtj", "arapb200_debug_cost", "arapb200_debug_sincos", "arapb200_debug_exact_sum",
     "arapb200_debug_resident_profile", "arapb200_debug_resident_profile_group", "arapb200_flatten", "arapb200_filter_matches", "arapb200_segment_mask",
     "arapb200_batch_set_option", "arapb200_batch_resident_count", "arapb200_debug_wide_sum", "arapb200_plan_error", "arapb200_plan_lm_info", "arapb200_plan_timing_report",
-    "arapb200_batch_launch_info",
+    "arapb200_batch_launch_info", "arapb200_warp_ex", "arapb200_batch_submit_ex", "arapb200_flatten_ex",
 ]
 
 
@@ -139,6 +139,22 @@ def warp_flow(flow, rgb, mask_red, want_splat=True):
     return o_rgb, o_m, sp
 
 
+def warp_ex(pos_or_flow, rgb, mask_red, is_flow=False):
+    """The warp with its extra outputs (include/arapb200.h arapb200_warp_ex, DESIGN.md 4.3): absolute positions, or a
+    forward flow with is_flow=True.  Returns a dict: rgb, mask, splat as warp(); bflow[H,W,2] f32, the backward flow on
+    the frame-2 grid; occ[H,W] u8, the occlusion of frame 1 (0 visible in frame 2, 255 not)."""
+    H, W = mask_red.shape
+    out = dict(rgb=np.zeros((H, W, 3), np.uint8), mask=np.zeros((H, W), np.uint8), splat=np.zeros((H, W), np.uint32),
+               bflow=np.zeros((H, W, 2), np.float32), occ=np.zeros((H, W), np.uint8))
+    L = load()
+    L.arapb200_warp_ex.argtypes = [C.c_int, C.c_int, _f32p, C.c_int, _u8p, _u8p, _u8p, _u8p, C.c_void_p, C.c_void_p,
+                                   C.c_void_p]
+    _check(L.arapb200_warp_ex(W, H, _c(pos_or_flow, np.float32), int(bool(is_flow)), _c(rgb, np.uint8),
+                              _c(mask_red, np.uint8), out["rgb"], out["mask"], out["splat"].ctypes.data,
+                              out["bflow"].ctypes.data, out["occ"].ctypes.data), "arapb200_warp_ex")
+    return out
+
+
 def deform(rgb, mask_red, matches, nCont=19, nGN=8, nPCG=400, backend=BACKEND_AUTO):
     """arap_deform for one image/segment: returns (flow[H,W,2], warped_rgb, warped_mask, costs[nCont,nGN+1])."""
     H, W = mask_red.shape
@@ -171,6 +187,29 @@ def flatten(flows, rgbs, masks, background=None):
                               P(*[a.ctypes.data for a in mk]), bg.ctypes.data if bg is not None else None,
                               o_f.ctypes.data, o_r.ctypes.data, o_m.ctypes.data), "arapb200_flatten")
     return o_f, o_r, o_m
+
+
+def flatten_ex(flows, rgbs, masks, src_masks=None, bflows=None, background=None, extras=True):
+    """flatten() plus, with extras, the flattened backward flow and the occlusion of frame 1 across the layers
+    (arapb200_flatten_ex).  src_masks: each segment's frame-1 input mask (0 = object); bflows: each segment's backward
+    flow; both are needed with extras.  Returns a dict flow, rgb, mask (+ bflow[H,W,2] f32, occ[H,W] u8 with extras)."""
+    n = len(flows)
+    H, W = masks[0].shape
+    arrs = [None if group is None else [_c(a, dt) for a in group] for group, dt in
+            ((flows, np.float32), (rgbs, np.uint8), (masks, np.uint8), (src_masks, np.uint8), (bflows, np.float32))]
+    P = C.c_void_p * n
+    ptrs = [None if group is None else P(*[a.ctypes.data for a in group]) for group in arrs]
+    bg = _c(background, np.uint8) if background is not None else None
+    out = dict(flow=np.zeros((H, W, 2), np.float32), rgb=np.zeros((H, W, 3), np.uint8), mask=np.zeros((H, W), np.uint8))
+    if extras:
+        out.update(bflow=np.zeros((H, W, 2), np.float32), occ=np.zeros((H, W), np.uint8))
+    L = load()
+    L.arapb200_flatten_ex.argtypes = [C.c_int] * 3 + [C.c_void_p] * 11
+    _check(L.arapb200_flatten_ex(W, H, n, ptrs[0], ptrs[1], ptrs[2], bg.ctypes.data if bg is not None else None, ptrs[3],
+                                 ptrs[4], out["flow"].ctypes.data, out["rgb"].ctypes.data, out["mask"].ctypes.data,
+                                 out["bflow"].ctypes.data if extras else None, out["occ"].ctypes.data if extras else None),
+           "arapb200_flatten_ex")
+    return out
 
 
 def filter_matches(matches, labels1, labels2):
@@ -218,9 +257,11 @@ class Batch:
         self.L.arapb200_batch_set_option.argtypes = [C.c_void_p, C.c_char_p, C.c_double]
         _check(self.L.arapb200_batch_set_option(self.h, name.encode(), float(value)), "arapb200_batch_set_option")
 
-    def submit(self, slot, rgb, mask_red, matches, out=None):
+    def submit(self, slot, rgb, mask_red, matches, out=None, extras=False):
         """Queue one problem.  `out` may be the dict a previous submit() of the same image size returned: its arrays are
-        then written in place instead of allocating fresh ones (what a caller looping over many pairs does)."""
+        then written in place instead of allocating fresh ones (what a caller looping over many pairs does).
+        extras=True: the dict also gets bflow[H,W,2] f32 (backward flow) and occ[H,W] u8 (occlusion of frame 1, 0 visible,
+        255 not), as lib.warp_ex computes them on the solved positions (arapb200_batch_submit_ex)."""
         H, W = mask_red.shape
         rgb = _c(rgb, np.uint8)
         mask_red = _c(mask_red, np.uint8)
@@ -228,10 +269,17 @@ class Batch:
         if out is None or out["flow"].shape != (H, W, 2):
             out = dict(flow=np.zeros((H, W, 2), np.float32), rgb=np.zeros((H, W, 3), np.uint8),
                        mask=np.zeros((H, W), np.uint8), costs=np.zeros((self.nCont, self.nGN + 1), np.float32))
+        if extras and "bflow" not in out:
+            out.update(bflow=np.zeros((H, W, 2), np.float32), occ=np.zeros((H, W), np.uint8))
         self._keep[slot] = (rgb, mask_red, m, out)
-        _check(self.L.arapb200_batch_submit(self.h, slot, W, H, rgb.ctypes.data, mask_red.ctypes.data, m.ctypes.data,
-                                            len(m), out["flow"].ctypes.data, out["rgb"].ctypes.data,
-                                            out["mask"].ctypes.data, out["costs"].ctypes.data), "arapb200_batch_submit")
+        args = (self.h, slot, W, H, rgb.ctypes.data, mask_red.ctypes.data, m.ctypes.data, len(m), out["flow"].ctypes.data,
+                out["rgb"].ctypes.data, out["mask"].ctypes.data, out["costs"].ctypes.data)
+        if extras:
+            self.L.arapb200_batch_submit_ex.argtypes = self.L.arapb200_batch_submit.argtypes + [C.c_void_p, C.c_void_p]
+            _check(self.L.arapb200_batch_submit_ex(*args, out["bflow"].ctypes.data, out["occ"].ctypes.data),
+                   "arapb200_batch_submit_ex")
+        else:
+            _check(self.L.arapb200_batch_submit(*args), "arapb200_batch_submit")
         return out
 
     def run(self):

@@ -38,6 +38,15 @@ ARAPB200_API int arapb200_warp(int W, int H, const float* pos, const uint8_t* rg
 /* warp tool front half (warping/src/main.cpp:160-166): positions = grid + flow, then warp */
 ARAPB200_API int arapb200_warp_flow(int W, int H, const float* flow, const uint8_t* rgb, const uint8_t* mask_red,
                        uint8_t* out_rgb, uint8_t* out_mask, uint32_t* out_splat);
+/* The warp with its opt-in extra outputs (DESIGN.md 4.3).  pos_or_flow: absolute positions (is_flow = 0, as
+ * arapb200_warp; forward flow = pos - grid) or a forward flow (is_flow = 1, as arapb200_warp_flow; positions = grid + flow).
+ * out_rgb, out_mask, out_splat as arapb200_warp; out_rgb and out_mask are required, every other output may be NULL.
+ * out_bflow float2[W*H]: backward flow on the frame-2 grid, the exact frame-1 source point of every pixel something
+ * landed on minus the pixel, (0, 0) elsewhere.  out_occ uint8[W*H]: occlusion of frame 1, 0 = the pixel is visible in
+ * frame 2, 255 = it is not (covered, folded, never rasterised or out of the frame). */
+ARAPB200_API int arapb200_warp_ex(int W, int H, const float* pos_or_flow, int is_flow, const uint8_t* rgb,
+                                  const uint8_t* mask_red, uint8_t* out_rgb, uint8_t* out_mask, uint32_t* out_splat,
+                                  float* out_bflow, uint8_t* out_occ);
 
 /* ---- one image / segment, end to end (replaces deformSingle, deformation/src/main.cpp:140-160:
  * border pins :130-136, resetGPU + continuation CombinedSolver.h:172-242, solve, warp, flow :352-366).
@@ -55,6 +64,15 @@ ARAPB200_API int arapb200_deform(int W, int H, const uint8_t* rgb, const uint8_t
 ARAPB200_API int arapb200_flatten(int W, int H, int n_layers, const float* const* flows, const uint8_t* const* rgbs,
                                   const uint8_t* const* masks, const uint8_t* background, float* out_flow,
                                   uint8_t* out_rgb, uint8_t* out_mask);
+/* arapb200_flatten with the extra outputs of the layers (DESIGN.md 4.3).  src_masks[s] uint8[W*H]: segment s's frame-1
+ * input mask (0 = object); bflows[s] float2[W*H]: its backward flow (arapb200_warp_ex / arapb200_batch_submit_ex).
+ * out_bflow float2[W*H]: the backward flow of the front layer (the last one whose warped mask is non-zero), (0, 0) where
+ * there is none.  out_occ uint8[W*H]: occlusion of frame 1 across the layers (0 visible, 255 not).  out_bflow and out_occ
+ * may be NULL; out_bflow needs bflows, out_occ needs bflows and src_masks.  With both NULL this is arapb200_flatten. */
+ARAPB200_API int arapb200_flatten_ex(int W, int H, int n_layers, const float* const* flows, const uint8_t* const* rgbs,
+                                     const uint8_t* const* masks, const uint8_t* background,
+                                     const uint8_t* const* src_masks, const float* const* bflows, float* out_flow,
+                                     uint8_t* out_rgb, uint8_t* out_mask, float* out_bflow, uint8_t* out_occ);
 
 /* ---- "next" row N3: match ingestion on the device (replaces the Python loops of para_gen.py:216-223 valid_cnstr,
  * :468-482 filter, :513-537 per-segment masks).
@@ -80,6 +98,13 @@ ARAPB200_API void arapb200_batch_destroy(arapb200_batch* b);
 ARAPB200_API int arapb200_batch_submit(arapb200_batch* b, int slot, int W, int H, const uint8_t* rgb,
                           const uint8_t* mask_red, const int32_t* matches, int n_matches, float* out_flow,
                           uint8_t* out_rgb, uint8_t* out_mask, float* out_costs);
+/* arapb200_batch_submit plus the extra outputs of arapb200_warp_ex for this problem: out_bflow float2[W*H], out_occ
+ * uint8[W*H] (either may be NULL).  Buffers for them are allocated for a slot the first time it asks; with both NULL
+ * this is exactly arapb200_batch_submit. */
+ARAPB200_API int arapb200_batch_submit_ex(arapb200_batch* b, int slot, int W, int H, const uint8_t* rgb,
+                                          const uint8_t* mask_red, const int32_t* matches, int n_matches,
+                                          float* out_flow, uint8_t* out_rgb, uint8_t* out_mask, float* out_costs,
+                                          float* out_bflow, uint8_t* out_occ);
 /* run everything submitted since the last run; returns after all outputs are in host memory */
 ARAPB200_API int arapb200_batch_run(arapb200_batch* b);
 /* device milliseconds of the last run: [0] total, [1] solve kernels only, [2] warp kernels only */
