@@ -182,6 +182,32 @@ int arapb200_warp_ex(int W, int H, const float* pos_or_flow, int is_flow, const 
     });
 }
 
+int arapb200_warp_seq(int W, int H, int K, const float* pos, const uint8_t* rgb, const uint8_t* mask_red,
+                      uint8_t* out_rgb, uint8_t* out_mask, float* out_flow, float* out_bflow, uint8_t* out_occ,
+                      float* out_flow0)
+{
+    return guarded([&]() -> int {
+        if (W <= 0 || H <= 0 || K <= 0 || !pos || !rgb || !mask_red || !out_rgb || !out_mask) return 1;
+        const size_t N = (size_t)W * H, F = N * K;
+        DevBuf<float2> d_pos(F), d_flow(F), d_bflow(F), d_flow0(F);
+        DevBuf<unsigned char> d_rgb(3 * N), d_mask(N), d_orgb(3 * F), d_omask(F), d_occ(F);
+        DevBuf<unsigned> d_z(2 * N);
+        d_pos.up((const float2*)pos);
+        d_rgb.up(rgb);
+        d_mask.up(mask_red);
+        const SeqOut o{d_orgb.p, d_omask.p, d_flow.p, d_bflow.p, d_occ.p, d_flow0.p};
+        enqueue_warp_seq(W, H, K, d_pos.p, d_rgb.p, d_mask.p, d_z.p, o, nullptr);
+        d_orgb.down(out_rgb);
+        d_omask.down(out_mask);
+        if (out_flow) d_flow.down((float2*)out_flow);
+        if (out_bflow) d_bflow.down((float2*)out_bflow);
+        if (out_occ) d_occ.down(out_occ);
+        if (out_flow0) d_flow0.down((float2*)out_flow0);
+        ARAP_CUDA_OR_RETURN(cudaDeviceSynchronize());
+        return 0;
+    });
+}
+
 int arapb200_deform(int W, int H, const uint8_t* rgb, const uint8_t* mask_red, const int32_t* matches, int n_matches,
                     int nCont, int nGN, int nPCG, int backend, float* out_flow, uint8_t* out_rgb, uint8_t* out_mask,
                     float* out_costs)
@@ -228,6 +254,17 @@ int arapb200_batch_submit_ex(arapb200_batch* b, int slot, int W, int H, const ui
                              const int32_t* matches, int n_matches, float* out_flow, uint8_t* out_rgb,
                              uint8_t* out_mask, float* out_costs, float* out_bflow, uint8_t* out_occ)
 {
+    return arapb200_batch_submit_seq(b, slot, W, H, rgb, mask_red, matches, n_matches, out_flow, out_rgb, out_mask,
+                                     out_costs, out_bflow, out_occ, 0, nullptr, nullptr, nullptr, nullptr, nullptr,
+                                     nullptr, nullptr);
+}
+
+int arapb200_batch_submit_seq(arapb200_batch* b, int slot, int W, int H, const uint8_t* rgb, const uint8_t* mask_red,
+                              const int32_t* matches, int n_matches, float* out_flow, uint8_t* out_rgb,
+                              uint8_t* out_mask, float* out_costs, float* out_bflow, uint8_t* out_occ, int n_frames,
+                              const int* steps, uint8_t* seq_rgb, uint8_t* seq_mask, float* seq_flow,
+                              float* seq_bflow, uint8_t* seq_occ, float* seq_flow0)
+{
     return guarded([&]() -> int {
         if (!b || slot < 0 || slot >= b->max_problems) return 1;
         // everything run() will dereference is checked here, while the caller can still be told
@@ -237,10 +274,25 @@ int arapb200_batch_submit_ex(arapb200_batch* b, int slot, int W, int H, const ui
                     b->maxW, b->maxH, n_matches);
             return 1;
         }
+        const bool any_out = seq_rgb || seq_mask || seq_flow || seq_bflow || seq_occ || seq_flow0;
+        if (n_frames < 0 || (n_frames == 0 && any_out) || (n_frames > 0 && (!steps || !seq_rgb || !seq_mask))) {
+            fprintf(stderr, "arapb200: batch_submit_seq: %d frames with%s step list and%s outputs (rgb and mask required)\n",
+                    n_frames, steps ? "" : " no", any_out ? "" : " no");
+            return 1;
+        }
+        for (int k = 0; k < n_frames; ++k)
+            if (steps[k] < 0 || steps[k] >= b->nCont || (k > 0 && steps[k] <= steps[k - 1])) {
+                fprintf(stderr, "arapb200: batch_submit_seq: steps must increase strictly within [0, %d]; step %d is %d\n",
+                        b->nCont - 1, k, steps[k]);
+                return 1;
+            }
         HostProblem& hp = b->slots[slot];
         hp.W = W; hp.H = H; hp.rgb = rgb; hp.mask_red = mask_red; hp.matches = matches; hp.n_matches = n_matches;
         hp.out_flow = out_flow; hp.out_rgb = out_rgb; hp.out_mask = out_mask; hp.out_costs = out_costs;
         hp.out_bflow = out_bflow; hp.out_occ = out_occ;
+        hp.steps.assign(steps, steps + n_frames);
+        hp.seq_rgb = seq_rgb; hp.seq_mask = seq_mask; hp.seq_flow = seq_flow; hp.seq_bflow = seq_bflow;
+        hp.seq_occ = seq_occ; hp.seq_flow0 = seq_flow0;
         b->pending[slot] = 1;
         return 0;
     });

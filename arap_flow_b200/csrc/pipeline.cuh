@@ -21,6 +21,11 @@ struct HostProblem {
     float* out_costs = nullptr;              // float[nCont*(nGN+1)] or null
     float* out_bflow = nullptr;              // float2[N] backward flow or null (opt-in, DESIGN.md 4.3)
     unsigned char* out_occ = nullptr;        // uint8[N] occlusion of frame 1 or null (opt-in)
+    // opt-in frame sequence (DESIGN.md 4.4): continuation steps t_1 < ... < t_K, and per frame k the outputs of
+    // enqueue_warp_seq, each [K][N][...] or null; out_rgb / out_mask are required when steps is not empty
+    std::vector<int> steps;
+    unsigned char *seq_rgb = nullptr, *seq_mask = nullptr, *seq_occ = nullptr;
+    float *seq_flow = nullptr, *seq_bflow = nullptr, *seq_flow0 = nullptr;
 };
 
 // compact constraint record: source pixel index and the match, after the reference's filtering
@@ -80,11 +85,22 @@ private:
         // opt-in extras, allocated the first time the slot asks for them: backward flow, occlusion, pinned [bflow | occ]
         float2* bflow = nullptr;
         unsigned char *occ = nullptr, *h_extra = nullptr;
+        // opt-in frame sequence, allocated the first time the slot asks and regrown for a longer list: X after each
+        // requested continuation step, two z-buffers, the frames' outputs; seq_cap frames of maxW x maxH each
+        int seq_cap = 0;
+        float2* seq_pos = nullptr;
+        unsigned* seq_z = nullptr;
+        SeqOut seq{};
         std::vector<MatchRec> recs;
         bool resident = false;
     };
     void solve_streaming(const HostProblem& hp, Dev& d);
     void solve_lm(const HostProblem& hp, Dev& d);
+    // the resident problems first .. first + count - 1 in one cooperative (or cluster) launch per schedule, or per
+    // continuation step when one of them asks for frames
+    void solve_resident(const HostProblem* problems, int first, int count, bool cluster);
+    void snapshot(const HostProblem& hp, Dev& d, int t); // X -> frame buffer if step t is one hp asks for
+    static void free_seq(Dev& d);
     LmSolver* lm_ = nullptr;
     int lmW_ = 0, lmH_ = 0;
     bool lm_on_ = false;

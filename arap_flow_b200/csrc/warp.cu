@@ -75,6 +75,29 @@ __global__ void __launch_bounds__(256) k_splat(int W, int H, const float2* __res
     splat_tri(W, H, p10, p01, p11, id + 1, z); // (pos10, pos01, pos11)  main.cpp:200-202
 }
 
+// vertices of the triangle a splat index names: (x0, y0 + t), (x0 + 1, y0), (x0 + t, y0 + 1) as pixel indices
+struct Tri {
+    size_t ia, ib, ic;
+};
+__device__ __forceinline__ Tri tri_of(int W, unsigned id)
+{
+    const unsigned t = (id - 1) & 1u;
+    const size_t i00 = (id - 1) >> 1, i01 = i00 + 1, i10 = i00 + W, i11 = i10 + 1;
+    return Tri{t ? i10 : i00, i01, t ? i11 : i10};
+}
+
+// The weights w applied to the triangle's vertices as vert(i) gives them: (Va*b0 + Vb*b1) + Vc*b2, the colour's operation
+// order, minus the pixel (qx, qy).  vert is the pixel grid for the backward flow of k_resolve<true>, a position array
+// for the frame-to-frame flows of k_interp (DESIGN.md 4.3, 4.4).
+template <class Vert>
+__device__ __forceinline__ float2 interp_minus_q(const Bary& w, const Tri& tr, Vert vert, int qx, int qy)
+{
+    const float2 a = vert(tr.ia), b = vert(tr.ib), c = vert(tr.ic);
+    const float sx = __fadd_rn(__fadd_rn(__fmul_rn(a.x, w.b0), __fmul_rn(b.x, w.b1)), __fmul_rn(c.x, w.b2));
+    const float sy = __fadd_rn(__fadd_rn(__fmul_rn(a.y, w.b0), __fmul_rn(b.y, w.b1)), __fmul_rn(c.y, w.b2));
+    return make_float2(__fsub_rn(sx, (float)qx), __fsub_rn(sy, (float)qy));
+}
+
 // pass 2: one thread per output pixel.  BFLOW: also the backward flow -- the winning triangle's barycentrics applied to
 // its undeformed vertex coordinates give the exact frame-1 source point of the pixel (DESIGN.md 4.3).
 template <bool BFLOW>
@@ -107,14 +130,10 @@ __global__ void __launch_bounds__(256) k_resolve(int W, int H, const float2* __r
         c1 = (unsigned char)__float2int_rz(v[1]);
         c2 = (unsigned char)__float2int_rz(v[2]);
         m = 255;
-        if (BFLOW) { // vertices (x0, y0 + t), (x0 + 1, y0), (x0 + t, y0 + 1); the colour's operation order
-            const int x0 = (int)(i00 % W), y0 = (int)(i00 / W);
-            const float xa = (float)x0, xb = (float)(x0 + 1), xc = (float)(x0 + (int)t);
-            const float ya = (float)(y0 + (int)t), yb = (float)y0, yc = (float)(y0 + 1);
-            const float sx = __fadd_rn(__fadd_rn(__fmul_rn(xa, w.b0), __fmul_rn(xb, w.b1)), __fmul_rn(xc, w.b2));
-            const float sy = __fadd_rn(__fadd_rn(__fmul_rn(ya, w.b0), __fmul_rn(yb, w.b1)), __fmul_rn(yc, w.b2));
-            bf = make_float2(__fsub_rn(sx, (float)x), __fsub_rn(sy, (float)y));
-        }
+        if (BFLOW)
+            bf = interp_minus_q(w, Tri{ia, ib, ic}, [W](size_t i) {
+                return make_float2((float)(int)(i % W), (float)(int)(i / W));
+            }, x, y);
     }
     out_rgb[3 * o] = c0;
     out_rgb[3 * o + 1] = c1;
@@ -132,6 +151,43 @@ __global__ void __launch_bounds__(256) k_occlusion(int W, int H, const unsigned 
     const size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
     if (p >= N) return;
     const int seg = mask_red[p] == 0 ? 0 : -1;
+    const float2 f = seg == 0 ? flow[p] : make_float2(0.f, 0.f);
+    occ[p] = occlusion_of(W, H, (int)(p % W), (int)(p / W), seg, f, bflow,
+                          [z](size_t q) { return z[q] != 0 ? 0 : -1; });
+}
+
+// interp(z_a, P_a, V)[q] = the weights of q's winning triangle in frame a (lk against P_a) applied to that triangle's
+// vertices in V, minus q; (0, 0) where nothing landed (z_a[q] == 0).  (z_{k-1}, P_{k-1}, P_k) is the flow from frame
+// k - 1 to frame k, (z_k, P_k, P_{k-1}) the backward flow from frame k to frame k - 1 (DESIGN.md 4.4).
+__global__ void __launch_bounds__(256) k_interp(int W, int H, const unsigned* __restrict__ z_a,
+                                                 const float2* __restrict__ P_a, const float2* __restrict__ V,
+                                                 float2* __restrict__ out)
+{
+    const size_t N = (size_t)W * H;
+    const size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= N) return;
+    const unsigned id = z_a[q];
+    float2 r = make_float2(0.f, 0.f);
+    if (id) {
+        const Tri tr = tri_of(W, id);
+        const float2 a = P_a[tr.ia], b = P_a[tr.ib], c = P_a[tr.ic];
+        const int x = (int)(q % W), y = (int)(q / W);
+        const Bary w = lk(a.x, a.y, b.x, b.y, c.x, c.y, (float)x, (float)y);
+        r = interp_minus_q(w, tr, [V](size_t i) { return V[i]; }, x, y);
+    }
+    out[q] = r;
+}
+
+// occlusion of frame k - 1 >= 1 in frame k: k_occlusion with p's surface taken from frame k - 1's z-buffer instead of
+// the input mask (DESIGN.md 4.4)
+__global__ void __launch_bounds__(256) k_occlusion_z(int W, int H, const unsigned* __restrict__ z_prev,
+                                                      const float2* __restrict__ flow, const unsigned* __restrict__ z,
+                                                      const float2* __restrict__ bflow, unsigned char* __restrict__ occ)
+{
+    const size_t N = (size_t)W * H;
+    const size_t p = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (p >= N) return;
+    const int seg = z_prev[p] != 0 ? 0 : -1;
     const float2 f = seg == 0 ? flow[p] : make_float2(0.f, 0.f);
     occ[p] = occlusion_of(W, H, (int)(p % W), (int)(p / W), seg, f, bflow,
                           [z](size_t q) { return z[q] != 0 ? 0 : -1; });
@@ -184,6 +240,34 @@ void enqueue_occlusion(int W, int H, const unsigned char* d_mask_red, const floa
     const size_t N = (size_t)W * H;
     k_occlusion<<<(unsigned)((N + 255) / 256), 256, 0, stream>>>(W, H, d_mask_red, d_flow, d_z, d_bflow, d_occ);
     ARAP_CUDA_CHECK(cudaGetLastError());
+}
+
+int enqueue_warp_seq(int W, int H, int K, const float2* d_pos, const unsigned char* d_rgb,
+                     const unsigned char* d_mask_red, unsigned* d_z2, const SeqOut& o, cudaStream_t stream)
+{
+    const size_t N = (size_t)W * H;
+    const unsigned g = (unsigned)((N + 255) / 256);
+    int launches = 0;
+    for (int k = 0; k < K; ++k) { // frame k + 1
+        const float2* P = d_pos + (size_t)k * N;
+        unsigned* z = d_z2 + (size_t)(k & 1) * N;
+        const unsigned* zp = d_z2 + (size_t)((k + 1) & 1) * N; // frame k's z-buffer (k >= 1)
+        float2 *flow = o.flow + (size_t)k * N, *bflow = o.bflow + (size_t)k * N;
+        // frame 1 is the single warp of DESIGN.md 4.3: its backward flow comes from k_resolve<true>, against the grid
+        enqueue_warp(W, H, P, d_rgb, d_mask_red, z, o.rgb + 3 * N * k, o.mask + N * k, stream, k == 0 ? bflow : nullptr);
+        enqueue_pos_to_flow(W, H, P, o.flow0 + (size_t)k * N, stream);
+        if (k == 0) {
+            enqueue_pos_to_flow(W, H, P, flow, stream);
+            enqueue_occlusion(W, H, d_mask_red, flow, z, bflow, o.occ, stream);
+        } else {
+            k_interp<<<g, 256, 0, stream>>>(W, H, zp, P - N, P, flow);
+            k_interp<<<g, 256, 0, stream>>>(W, H, z, P, P - N, bflow);
+            k_occlusion_z<<<g, 256, 0, stream>>>(W, H, zp, flow, z, bflow, o.occ + N * k);
+        }
+        ARAP_CUDA_CHECK(cudaGetLastError());
+        launches += warp_launches_per_call() + (k == 0 ? 3 : 4);
+    }
+    return launches;
 }
 
 void enqueue_flow_to_pos(int W, int H, const float2* d_flow, float2* d_pos, cudaStream_t stream)

@@ -13,6 +13,17 @@ void enqueue_warp(int W, int H, const float2* d_pos, const unsigned char* d_rgb,
 // forward flow d_flow = X - grid
 void enqueue_occlusion(int W, int H, const unsigned char* d_mask_red, const float2* d_flow, const unsigned* d_z,
                        const float2* d_bflow, unsigned char* d_occ, cudaStream_t stream);
+// Frame sequences (DESIGN.md 4.4).  Every buffer is [K][W*H][...] on the device; frame k (1-based) sits at index k - 1.
+struct SeqOut {
+    unsigned char *rgb, *mask; // warp of P_k (uint8x3, uint8)
+    float2 *flow, *bflow;      // frame k - 1 -> k on the frame k - 1 grid; frame k -> k - 1 on the frame k grid
+    unsigned char* occ;        // occlusion of frame k - 1 in frame k (0 visible, 255 not)
+    float2* flow0;             // P_k - grid
+};
+// d_pos: the K position fields P_1 .. P_K (frame 0 is the grid); d_z2: uint32[2][W*H] scratch (the z-buffers of two
+// consecutive frames).  Frames are rendered in order.  Returns the number of kernels launched.
+int enqueue_warp_seq(int W, int H, int K, const float2* d_pos, const unsigned char* d_rgb,
+                     const unsigned char* d_mask_red, unsigned* d_z2, const SeqOut& out, cudaStream_t stream);
 void enqueue_flow_to_pos(int W, int H, const float2* d_flow, float2* d_pos, cudaStream_t stream);
 void enqueue_pos_to_flow(int W, int H, const float2* d_pos, float2* d_flow, cudaStream_t stream);
 int warp_launches_per_call();

@@ -29,6 +29,7 @@ ARAP_SYMBOLS = [
     "arapb200_debug_resident_profile", "arapb200_debug_resident_profile_group", "arapb200_flatten", "arapb200_filter_matches", "arapb200_segment_mask",
     "arapb200_batch_set_option", "arapb200_batch_resident_count", "arapb200_debug_wide_sum", "arapb200_plan_error", "arapb200_plan_lm_info", "arapb200_plan_timing_report",
     "arapb200_batch_launch_info", "arapb200_warp_ex", "arapb200_batch_submit_ex", "arapb200_flatten_ex",
+    "arapb200_warp_seq", "arapb200_batch_submit_seq",
 ]
 
 
@@ -155,6 +156,32 @@ def warp_ex(pos_or_flow, rgb, mask_red, is_flow=False):
     return out
 
 
+SEQ_KEYS = ("rgb", "mask", "flow", "bflow", "occ", "flow0")
+
+
+def _seq_arrays(K, H, W):
+    return dict(rgb=np.zeros((K, H, W, 3), np.uint8), mask=np.zeros((K, H, W), np.uint8),
+                flow=np.zeros((K, H, W, 2), np.float32), bflow=np.zeros((K, H, W, 2), np.float32),
+                occ=np.zeros((K, H, W), np.uint8), flow0=np.zeros((K, H, W, 2), np.float32))
+
+
+def warp_seq(positions, rgb, mask_red):
+    """A frame sequence from position fields (include/arapb200.h arapb200_warp_seq, DESIGN.md 4.4): positions[K,H,W,2]
+    are P_1 .. P_K, frame 0 is the input image on the pixel grid.  Returns a dict of arrays with a leading K axis, index
+    k - 1 holding frame k: rgb, mask (the warp of P_k), flow (frame k-1 -> k on the frame k-1 grid), bflow (frame k ->
+    k-1 on the frame k grid), occ (occlusion of frame k-1 in frame k, 0 visible, 255 not), flow0 (P_k - grid)."""
+    H, W = mask_red.shape
+    pos = _c(positions, np.float32)
+    K = pos.shape[0]
+    assert pos.shape == (K, H, W, 2), pos.shape
+    out = _seq_arrays(K, H, W)
+    L = load()
+    L.arapb200_warp_seq.argtypes = [C.c_int, C.c_int, C.c_int, _f32p, _u8p, _u8p] + [C.c_void_p] * 6
+    _check(L.arapb200_warp_seq(W, H, K, pos, _c(rgb, np.uint8), _c(mask_red, np.uint8),
+                               *[out[k].ctypes.data for k in SEQ_KEYS]), "arapb200_warp_seq")
+    return out
+
+
 def deform(rgb, mask_red, matches, nCont=19, nGN=8, nPCG=400, backend=BACKEND_AUTO):
     """arap_deform for one image/segment: returns (flow[H,W,2], warped_rgb, warped_mask, costs[nCont,nGN+1])."""
     H, W = mask_red.shape
@@ -257,11 +284,13 @@ class Batch:
         self.L.arapb200_batch_set_option.argtypes = [C.c_void_p, C.c_char_p, C.c_double]
         _check(self.L.arapb200_batch_set_option(self.h, name.encode(), float(value)), "arapb200_batch_set_option")
 
-    def submit(self, slot, rgb, mask_red, matches, out=None, extras=False):
+    def submit(self, slot, rgb, mask_red, matches, out=None, extras=False, frames=None):
         """Queue one problem.  `out` may be the dict a previous submit() of the same image size returned: its arrays are
         then written in place instead of allocating fresh ones (what a caller looping over many pairs does).
         extras=True: the dict also gets bflow[H,W,2] f32 (backward flow) and occ[H,W] u8 (occlusion of frame 1, 0 visible,
-        255 not), as lib.warp_ex computes them on the solved positions (arapb200_batch_submit_ex)."""
+        255 not), as lib.warp_ex computes them on the solved positions (arapb200_batch_submit_ex).
+        frames: a strictly increasing list of continuation steps in [0, nCont-1]; the dict then also gets "seq", the
+        dict lib.warp_seq returns for the solver's states after those steps (arapb200_batch_submit_seq)."""
         H, W = mask_red.shape
         rgb = _c(rgb, np.uint8)
         mask_red = _c(mask_red, np.uint8)
@@ -271,10 +300,22 @@ class Batch:
                        mask=np.zeros((H, W), np.uint8), costs=np.zeros((self.nCont, self.nGN + 1), np.float32))
         if extras and "bflow" not in out:
             out.update(bflow=np.zeros((H, W, 2), np.float32), occ=np.zeros((H, W), np.uint8))
+        steps = None
+        if frames is not None:
+            steps = np.ascontiguousarray(frames, np.int32).reshape(-1)
+            if "seq" not in out or out["seq"]["mask"].shape[0] != len(steps):
+                out["seq"] = _seq_arrays(len(steps), H, W)
         self._keep[slot] = (rgb, mask_red, m, out)
         args = (self.h, slot, W, H, rgb.ctypes.data, mask_red.ctypes.data, m.ctypes.data, len(m), out["flow"].ctypes.data,
                 out["rgb"].ctypes.data, out["mask"].ctypes.data, out["costs"].ctypes.data)
-        if extras:
+        if steps is not None:
+            self.L.arapb200_batch_submit_seq.argtypes = (self.L.arapb200_batch_submit.argtypes +
+                                                         [C.c_void_p, C.c_void_p, C.c_int] + [C.c_void_p] * 7)
+            seq = out["seq"]
+            _check(self.L.arapb200_batch_submit_seq(
+                *args, out["bflow"].ctypes.data if extras else None, out["occ"].ctypes.data if extras else None,
+                len(steps), steps.ctypes.data, *[seq[k].ctypes.data for k in SEQ_KEYS]), "arapb200_batch_submit_seq")
+        elif extras:
             self.L.arapb200_batch_submit_ex.argtypes = self.L.arapb200_batch_submit.argtypes + [C.c_void_p, C.c_void_p]
             _check(self.L.arapb200_batch_submit_ex(*args, out["bflow"].ctypes.data, out["occ"].ctypes.data),
                    "arapb200_batch_submit_ex")

@@ -47,6 +47,18 @@ ARAPB200_API int arapb200_warp_flow(int W, int H, const float* flow, const uint8
 ARAPB200_API int arapb200_warp_ex(int W, int H, const float* pos_or_flow, int is_flow, const uint8_t* rgb,
                                   const uint8_t* mask_red, uint8_t* out_rgb, uint8_t* out_mask, uint32_t* out_splat,
                                   float* out_bflow, uint8_t* out_occ);
+/* A frame sequence from position fields the caller holds (DESIGN.md 4.4), e.g. X after each of several Opt_ProblemSolve
+ * calls.  pos float2[K][W*H]: P_1 .. P_K, absolute positions; frame 0 is the input image on the pixel grid.  Every output
+ * is [K][W*H][...] contiguous, index k - 1 holding frame k.  out_rgb uint8x3 / out_mask uint8: arapb200_warp of P_k
+ * (required).  out_flow float2: frame k - 1 -> k on the frame k - 1 grid (k = 1: P_1 - grid; k >= 2: at every pixel
+ * something landed on in frame k - 1, the weights of its winning triangle applied to that triangle's vertices in P_k,
+ * minus the pixel; (0, 0) elsewhere).  out_bflow float2: frame k -> k - 1 on the frame k grid, the same with the roles
+ * of the frames swapped (k = 1: arapb200_warp_ex's out_bflow).  out_occ uint8: occlusion of frame k - 1 in frame k
+ * (0 visible, 255 not; k = 1: arapb200_warp_ex's out_occ).  out_flow0 float2: P_k - grid.  Every output but out_rgb and
+ * out_mask may be NULL.  Colours are always sampled from the frame-0 image. */
+ARAPB200_API int arapb200_warp_seq(int W, int H, int K, const float* pos, const uint8_t* rgb, const uint8_t* mask_red,
+                                   uint8_t* out_rgb, uint8_t* out_mask, float* out_flow, float* out_bflow,
+                                   uint8_t* out_occ, float* out_flow0);
 
 /* ---- one image / segment, end to end (replaces deformSingle, deformation/src/main.cpp:140-160:
  * border pins :130-136, resetGPU + continuation CombinedSolver.h:172-242, solve, warp, flow :352-366).
@@ -105,6 +117,22 @@ ARAPB200_API int arapb200_batch_submit_ex(arapb200_batch* b, int slot, int W, in
                                           const uint8_t* mask_red, const int32_t* matches, int n_matches,
                                           float* out_flow, uint8_t* out_rgb, uint8_t* out_mask, float* out_costs,
                                           float* out_bflow, uint8_t* out_occ);
+/* arapb200_batch_submit_ex plus a frame sequence taken from the continuation schedule (DESIGN.md 4.4): steps int[n_frames]
+ * lists continuation steps, strictly increasing, each in [0, nCont - 1]; frame k is the solver's state after step
+ * steps[k - 1], rendered as arapb200_warp_seq renders P_k, with seq_rgb .. seq_flow0 its outputs ([n_frames][W*H][...]).
+ * seq_rgb and seq_mask are required, the others may be NULL.  The step list is copied: it need not outlive the call.
+ * Returns non-zero, and queues nothing, for n_frames < 0, outputs without frames, a missing seq_rgb / seq_mask or a
+ * step list that is not strictly increasing within [0, nCont - 1].  With n_frames == 0 and NULL sequence outputs this is
+ * exactly arapb200_batch_submit_ex.  A slot allocates its sequence buffers (37 B/px per frame on the device) the first
+ * time it asks and grows them for a longer list.  Frames are copied straight into the caller's buffers; pinned
+ * buffers make that copy faster.  A resident group in which any problem asks for frames runs one launch per
+ * continuation step (same results bit for bit). */
+ARAPB200_API int arapb200_batch_submit_seq(arapb200_batch* b, int slot, int W, int H, const uint8_t* rgb,
+                                           const uint8_t* mask_red, const int32_t* matches, int n_matches,
+                                           float* out_flow, uint8_t* out_rgb, uint8_t* out_mask, float* out_costs,
+                                           float* out_bflow, uint8_t* out_occ, int n_frames, const int* steps,
+                                           uint8_t* seq_rgb, uint8_t* seq_mask, float* seq_flow, float* seq_bflow,
+                                           uint8_t* seq_occ, float* seq_flow0);
 /* run everything submitted since the last run; returns after all outputs are in host memory */
 ARAPB200_API int arapb200_batch_run(arapb200_batch* b);
 /* device milliseconds of the last run: [0] total, [1] solve kernels only, [2] warp kernels only */
