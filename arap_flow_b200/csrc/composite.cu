@@ -7,10 +7,14 @@
 // does not depend on any ordering between threads.  Pure select arithmetic: bit-identical to the numpy original.
 // Opt-in (arapb200_flatten_ex): the flattened backward flow and the occlusion of frame 1 across the layers, with the
 // same occlusion rule as the per-problem warp (warp.cuh occlusion_of, DESIGN.md 4.3).
+// arapb200_composite: the same layers over a background that moves by its own affine map, with the forward flow,
+// backward flow and occlusion of both (DESIGN.md 4.5).
 #include "../../include/arapb200.h"
 #include "common.cuh"
 #include "warp.cuh"
 
+#include <algorithm>
+#include <cmath>
 #include <mutex>
 #include <vector>
 
@@ -23,7 +27,7 @@ struct Layers {
     const unsigned char* rgb[MAX_LAYERS];
     const unsigned char* mask[MAX_LAYERS];
     const float2* bflow[MAX_LAYERS];      // backward flow of each layer (only read for out_bflow / out_occ)
-    const unsigned char* src[MAX_LAYERS]; // frame-1 input mask of each layer, 0 = object (only read for out_occ)
+    const unsigned char* src[MAX_LAYERS]; // frame-a input mask of each layer, 0 = object (flatten: only read for out_occ)
     int n;
 };
 
@@ -62,6 +66,95 @@ __global__ void __launch_bounds__(256) k_flatten(int W, int H, Layers L, const u
         out_occ[i] = occlusion_of(W, H, (int)(i % W), (int)(i / W), seg, f, seg >= 0 ? L.bflow[seg] : nullptr,
                                   [&L](size_t q) { return front_layer(L, q); });
     }
+}
+
+// ---- background motion (DESIGN.md 4.5): the composite of the layers over an affinely moving background ----
+struct Affine {
+    float m00, m01, m02, m10, m11, m12;
+};
+
+__device__ __forceinline__ float2 affine_at(const Affine& M, int x, int y)
+{
+    const float fx = (float)x, fy = (float)y;
+    return make_float2(__fadd_rn(__fadd_rn(__fmul_rn(M.m00, fx), __fmul_rn(M.m01, fy)), M.m02),
+                       __fadd_rn(__fadd_rn(__fmul_rn(M.m10, fx), __fmul_rn(M.m11, fy)), M.m12));
+}
+
+// bilinear sample of the uint8x3 background at s, coordinates clamped to the image (NaN -> 0)
+__device__ __forceinline__ void sample_bg(const unsigned char* __restrict__ bg, int bgW, int bgH, float2 s,
+                                          unsigned char* __restrict__ out)
+{
+    const float sx = fminf(fmaxf(s.x, 0.f), (float)(bgW - 1)), sy = fminf(fmaxf(s.y, 0.f), (float)(bgH - 1));
+    const int x0 = (int)floorf(sx), y0 = (int)floorf(sy);
+    const int x1 = min(x0 + 1, bgW - 1), y1 = min(y0 + 1, bgH - 1);
+    const float fx = __fsub_rn(sx, (float)x0), fy = __fsub_rn(sy, (float)y0);
+    const float gx = __fsub_rn(1.f, fx), gy = __fsub_rn(1.f, fy);
+    const unsigned char* r0 = bg + 3 * (size_t)y0 * bgW;
+    const unsigned char* r1 = bg + 3 * (size_t)y1 * bgW;
+    for (int c = 0; c < 3; ++c) {
+        const float top = __fadd_rn(__fmul_rn((float)r0[3 * x0 + c], gx), __fmul_rn((float)r0[3 * x1 + c], fx));
+        const float bot = __fadd_rn(__fmul_rn((float)r1[3 * x0 + c], gx), __fmul_rn((float)r1[3 * x1 + c], fx));
+        out[c] = (unsigned char)min(255, __float2int_rn(__fadd_rn(__fmul_rn(top, gy), __fmul_rn(bot, fy))));
+    }
+}
+
+// frame-b pass: colour, mask and backward flow of the composite.  S: frame-b pixel -> background plane, B: frame-b
+// pixel -> frame a.  out_bflow may be null (no extras).
+__global__ void __launch_bounds__(256) k_composite_b(int W, int H, Layers L, const unsigned char* __restrict__ bg,
+                                                      int bgW, int bgH, int bg_x, int bg_y, Affine S, Affine B,
+                                                      unsigned char* __restrict__ out_rgb,
+                                                      unsigned char* __restrict__ out_mask, float2* __restrict__ out_bflow)
+{
+    const size_t N = (size_t)W * H;
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= N) return;
+    const int qx = (int)(i % W), qy = (int)(i / W);
+    const int front = front_layer(L, i);
+    if (front >= 0) {
+        out_mask[i] = L.mask[front][i];
+        out_rgb[3 * i] = L.rgb[front][3 * i];
+        out_rgb[3 * i + 1] = L.rgb[front][3 * i + 1];
+        out_rgb[3 * i + 2] = L.rgb[front][3 * i + 2];
+        if (out_bflow) out_bflow[i] = L.bflow[front][i];
+        return;
+    }
+    out_mask[i] = 0;
+    const float2 s = affine_at(S, qx, qy);
+    sample_bg(bg, bgW, bgH, make_float2(__fadd_rn(s.x, (float)bg_x), __fadd_rn(s.y, (float)bg_y)), out_rgb + 3 * i);
+    if (out_bflow) {
+        const float2 b = affine_at(B, qx, qy);
+        out_bflow[i] = make_float2(__fsub_rn(b.x, (float)qx), __fsub_rn(b.y, (float)qy));
+    }
+}
+
+// frame-a pass: forward flow and (out_occ non-null) occlusion, the background being surface L.n.  F: frame-a pixel ->
+// frame b; bflow_b: the frame-b backward flow k_composite_b wrote (read only for out_occ).
+__global__ void __launch_bounds__(256) k_composite_a(int W, int H, Layers L, Affine F,
+                                                      const float2* __restrict__ bflow_b, float2* __restrict__ out_flow,
+                                                      unsigned char* __restrict__ out_occ)
+{
+    const size_t N = (size_t)W * H;
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= N) return;
+    const int px = (int)(i % W), py = (int)(i / W);
+    int seg = L.n; // p's surface: the (last) layer whose input mask has p on the object, else the background
+    for (int s = L.n - 1; s >= 0; --s)
+        if (L.src[s][i] == 0) { seg = s; break; }
+    float2 f;
+    if (seg < L.n) {
+        const int front = front_layer(L, i);
+        out_flow[i] = L.flow[front < 0 ? 0 : front][i]; // the flatten's own selection
+        f = L.flow[seg][i];
+    } else {
+        const float2 a = affine_at(F, px, py);
+        f = make_float2(__fsub_rn(a.x, (float)px), __fsub_rn(a.y, (float)py));
+        out_flow[i] = f;
+    }
+    if (out_occ)
+        out_occ[i] = occlusion_of(W, H, px, py, seg, f, bflow_b, [&L](size_t q) {
+            const int s = front_layer(L, q);
+            return s < 0 ? L.n : s;
+        });
 }
 
 // ---- N3: match filter (para_gen.py:216-223) and per-segment masks (:513-537) ----
@@ -193,6 +286,30 @@ extern "C" int arapb200_segment_mask(int W, int H, const uint8_t* labels, int se
 }
 
 namespace {
+// One grow-only device arena per process, shared by the flatten and the composite (cudaMalloc / cudaFree of 15
+// multi-megabyte blocks per call cost far more than the kernel).  Callers hold arena_mu from arena_reserve until their
+// last copy out of it has returned.
+std::mutex arena_mu;
+unsigned char* arena = nullptr;
+size_t arena_bytes = 0;
+int arena_dev = -1;
+
+size_t al(size_t b) { return (b + 255) & ~(size_t)255; } // every block of the arena is 256-byte aligned
+
+// 0, or 2 on a CUDA failure
+int arena_reserve(size_t need)
+{
+    int dev = 0;
+    if (cudaGetDevice(&dev) != cudaSuccess) return 2;
+    if (need > arena_bytes || dev != arena_dev) {
+        if (arena) { cudaFree(arena); arena = nullptr; arena_bytes = 0; }
+        if (cudaMalloc(&arena, need) != cudaSuccess) return 2;
+        arena_bytes = need;
+        arena_dev = dev;
+    }
+    return 0;
+}
+
 int flatten_common(int W, int H, int n_layers, const float* const* flows, const uint8_t* const* rgbs,
                    const uint8_t* const* masks, const uint8_t* background, const uint8_t* const* src_masks,
                    const float* const* bflows, float* out_flow, uint8_t* out_rgb, uint8_t* out_mask, float* out_bflow,
@@ -205,24 +322,11 @@ int flatten_common(int W, int H, int n_layers, const float* const* flows, const 
     const size_t N = (size_t)W * H;
     Layers L{};
     L.n = n_layers;
-    // One grow-only device arena per process (cudaMalloc / cudaFree of 15 multi-megabyte blocks per call cost far more
-    // than the kernel): [layers: flow, rgb, mask (, bflow, src mask)][background][outputs], every block 256-byte aligned.
-    static std::mutex mu;
-    static unsigned char* arena = nullptr;
-    static size_t arena_bytes = 0;
-    static int arena_dev = -1;
-    std::lock_guard<std::mutex> lock(mu);
-    auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+    // arena: [layers: flow, rgb, mask (, bflow, src mask)][background][outputs]
+    std::lock_guard<std::mutex> lock(arena_mu);
     const size_t per_layer = al(N * sizeof(float2)) + al(3 * N) + al(N) + (ex ? al(N * sizeof(float2)) + al(N) : 0);
     const size_t need = (size_t)(n_layers + 1) * per_layer + al(3 * N);
-    int dev = 0;
-    int rc = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) rc = 2;
-    if (!rc && (need > arena_bytes || dev != arena_dev)) {
-        if (arena) { cudaFree(arena); arena = nullptr; arena_bytes = 0; }
-        if (cudaMalloc(&arena, need) != cudaSuccess) rc = 2;
-        else { arena_bytes = need; arena_dev = dev; }
-    }
+    int rc = arena_reserve(need);
     unsigned char* cur = arena;
     auto take = [&](size_t bytes) { unsigned char* p = cur; cur += al(bytes); return p; };
     auto up = [&](const void* h, size_t bytes) -> void* {
@@ -272,4 +376,143 @@ extern "C" int arapb200_flatten_ex(int W, int H, int n_layers, const float* cons
 {
     return flatten_common(W, H, n_layers, flows, rgbs, masks, background, src_masks, bflows, out_flow, out_rgb, out_mask,
                           out_bflow, out_occ);
+}
+
+namespace {
+// 2x3 affine maps in binary64, row-major: (a00 a01 a02; a10 a11 a12).  The derivation of DESIGN.md 4.5, in its order;
+// fp-contract=off keeps a host compiler from fusing a product and a sum where the target has FMA.
+struct Aff64 {
+    double a[6];
+};
+
+#if defined(__GNUC__) && !defined(__clang__)
+#define ARAP_NO_CONTRACT __attribute__((optimize("fp-contract=off")))
+#else
+#define ARAP_NO_CONTRACT
+#endif
+
+ARAP_NO_CONTRACT Aff64 aff_inverse(const Aff64& A, double* det)
+{
+    const double* a = A.a;
+    *det = a[0] * a[4] - a[1] * a[3];
+    Aff64 r;
+    r.a[0] = a[4] / *det;
+    r.a[1] = -a[1] / *det;
+    r.a[3] = -a[3] / *det;
+    r.a[4] = a[0] / *det;
+    r.a[2] = -(r.a[0] * a[2] + r.a[1] * a[5]);
+    r.a[5] = -(r.a[3] * a[2] + r.a[4] * a[5]);
+    return r;
+}
+
+ARAP_NO_CONTRACT Aff64 aff_compose(const Aff64& P, const Aff64& Q) // P o Q
+{
+    const double* p = P.a;
+    const double* q = Q.a;
+    Aff64 r;
+    for (int row = 0; row < 2; ++row) {
+        const double* pr = p + 3 * row;
+        r.a[3 * row] = pr[0] * q[0] + pr[1] * q[3];
+        r.a[3 * row + 1] = pr[0] * q[1] + pr[1] * q[4];
+        r.a[3 * row + 2] = (pr[0] * q[2] + pr[1] * q[5]) + pr[2];
+    }
+    return r;
+}
+
+bool aff_finite(const double* a)
+{
+    for (int k = 0; k < 6; ++k)
+        if (!std::isfinite(a[k])) return false;
+    return true;
+}
+
+// F, B, S rounded to binary32 (c[3][2][3]); false for a non-finite or singular motion or a non-finite coefficient
+bool composite_coeffs(const double* motion_from, const double* motion_to, float c[18])
+{
+    Aff64 Af{{1.0, 0.0, 0.0, 0.0, 1.0, 0.0}}, At;
+    if (motion_from) std::copy(motion_from, motion_from + 6, Af.a);
+    std::copy(motion_to, motion_to + 6, At.a);
+    if (!aff_finite(Af.a) || !aff_finite(At.a)) return false;
+    double det_f = 0.0, det_t = 0.0;
+    const Aff64 If = aff_inverse(Af, &det_f), It = aff_inverse(At, &det_t);
+    if (det_f == 0.0 || det_t == 0.0) return false;
+    const Aff64 m[3] = {aff_compose(At, If), aff_compose(Af, It), It}; // F, B, S
+    for (int k = 0; k < 18; ++k) {
+        c[k] = (float)m[k / 6].a[k % 6];
+        if (!std::isfinite(c[k])) return false;
+    }
+    return true;
+}
+
+Affine affine_of(const float* c) { return Affine{c[0], c[1], c[2], c[3], c[4], c[5]}; }
+
+template <class T> bool all_set(const T* const* p, int n)
+{
+    if (!p) return false;
+    for (int s = 0; s < n; ++s)
+        if (!p[s]) return false;
+    return true;
+}
+} // namespace
+
+extern "C" int arapb200_composite(int W, int H, int n_layers, const float* const* flows, const uint8_t* const* rgbs,
+                                  const uint8_t* const* masks, const uint8_t* const* src_masks,
+                                  const float* const* bflows, int bgW, int bgH, const uint8_t* background, int bg_x,
+                                  int bg_y, const double* motion_from, const double* motion_to, float* out_flow,
+                                  uint8_t* out_rgb, uint8_t* out_mask, float* out_bflow, uint8_t* out_occ,
+                                  float* out_coeffs)
+{
+    // every rejection comes before any CUDA call and any write
+    if (W <= 0 || H <= 0 || n_layers < 0 || n_layers > MAX_LAYERS) return 1;
+    const bool ex = out_bflow || out_occ;
+    if (n_layers > 0 && (!all_set(flows, n_layers) || !all_set(rgbs, n_layers) || !all_set(masks, n_layers) ||
+                         !all_set(src_masks, n_layers) || (ex && !all_set(bflows, n_layers))))
+        return 1;
+    if (!background || bgW <= 0 || bgH <= 0 || !motion_to || !out_flow || !out_rgb || !out_mask) return 1;
+    float cf[18];
+    if (!composite_coeffs(motion_from, motion_to, cf)) return 1;
+    if (out_coeffs) std::copy(cf, cf + 18, out_coeffs);
+
+    const size_t N = (size_t)W * H, NB = (size_t)bgW * bgH;
+    Layers L{};
+    L.n = n_layers;
+    // arena: [layers: flow, rgb, mask, src mask (, bflow)][background][outputs: flow, rgb, mask (, bflow)(, occ)]
+    std::lock_guard<std::mutex> lock(arena_mu);
+    const size_t per_layer = al(N * sizeof(float2)) + al(3 * N) + 2 * al(N) + (ex ? al(N * sizeof(float2)) : 0);
+    const size_t need = (size_t)n_layers * per_layer + al(3 * NB) + al(N * sizeof(float2)) + al(3 * N) + al(N) +
+                        (ex ? al(N * sizeof(float2)) : 0) + (out_occ ? al(N) : 0);
+    int rc = arena_reserve(need);
+    unsigned char* cur = arena;
+    auto take = [&](size_t bytes) { unsigned char* p = cur; cur += al(bytes); return p; };
+    auto up = [&](const void* h, size_t bytes) -> void* {
+        void* d = take(bytes);
+        if (cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, nullptr) != cudaSuccess) rc = 2;
+        return d;
+    };
+    for (int s = 0; s < n_layers && !rc; ++s) {
+        L.flow[s] = (const float2*)up(flows[s], N * sizeof(float2));
+        L.rgb[s] = (const unsigned char*)up(rgbs[s], 3 * N);
+        L.mask[s] = (const unsigned char*)up(masks[s], N);
+        L.src[s] = (const unsigned char*)up(src_masks[s], N);
+        if (ex) L.bflow[s] = (const float2*)up(bflows[s], N * sizeof(float2));
+    }
+    const unsigned char* d_bg = rc ? nullptr : (const unsigned char*)up(background, 3 * NB);
+    if (!rc) {
+        float2* d_of = (float2*)take(N * sizeof(float2));
+        unsigned char* d_or = take(3 * N);
+        unsigned char* d_om = take(N);
+        float2* d_ob = ex ? (float2*)take(N * sizeof(float2)) : nullptr; // out_occ reads the whole frame-b bflow
+        unsigned char* d_oo = out_occ ? take(N) : nullptr;
+        const unsigned blocks = (unsigned)((N + 255) / 256);
+        k_composite_b<<<blocks, 256>>>(W, H, L, d_bg, bgW, bgH, bg_x, bg_y, affine_of(cf + 12), affine_of(cf + 6), d_or,
+                                        d_om, d_ob);
+        k_composite_a<<<blocks, 256>>>(W, H, L, affine_of(cf), d_ob, d_of, d_oo);
+        if (cudaMemcpy(out_flow, d_of, N * sizeof(float2), cudaMemcpyDeviceToHost) ||
+            cudaMemcpy(out_rgb, d_or, 3 * N, cudaMemcpyDeviceToHost) || cudaMemcpy(out_mask, d_om, N, cudaMemcpyDeviceToHost) ||
+            (out_bflow && cudaMemcpy(out_bflow, d_ob, N * sizeof(float2), cudaMemcpyDeviceToHost)) ||
+            (d_oo && cudaMemcpy(out_occ, d_oo, N, cudaMemcpyDeviceToHost)))
+            rc = 3;
+    }
+    if (rc) fprintf(stderr, "arapb200_composite: CUDA failure (%s)\n", cudaGetErrorString(cudaGetLastError()));
+    return rc;
 }

@@ -29,7 +29,7 @@ ARAP_SYMBOLS = [
     "arapb200_debug_resident_profile", "arapb200_debug_resident_profile_group", "arapb200_flatten", "arapb200_filter_matches", "arapb200_segment_mask",
     "arapb200_batch_set_option", "arapb200_batch_resident_count", "arapb200_debug_wide_sum", "arapb200_plan_error", "arapb200_plan_lm_info", "arapb200_plan_timing_report",
     "arapb200_batch_launch_info", "arapb200_warp_ex", "arapb200_batch_submit_ex", "arapb200_flatten_ex",
-    "arapb200_warp_seq", "arapb200_batch_submit_seq",
+    "arapb200_warp_seq", "arapb200_batch_submit_seq", "arapb200_composite",
 ]
 
 
@@ -237,6 +237,66 @@ def flatten_ex(flows, rgbs, masks, src_masks=None, bflows=None, background=None,
                                  out["bflow"].ctypes.data if extras else None, out["occ"].ctypes.data if extras else None),
            "arapb200_flatten_ex")
     return out
+
+
+COMPOSITE_ARGTYPES = [C.c_int] * 3 + [C.c_void_p] * 5 + [C.c_int] * 2 + [C.c_void_p] + [C.c_int] * 2 + [C.c_void_p] * 8
+
+
+def _motion(m):
+    m = np.ascontiguousarray(m, np.float64)
+    if m.shape != (2, 3):
+        raise ValueError(f"a motion is a 2x3 affine matrix, got shape {m.shape}")
+    return m
+
+
+def composite(flows, rgbs, masks, src_masks, bflows, background, motion, motion_from=None, origin=(0, 0), extras=True,
+              shape=None):
+    """The layers of flatten_ex over a background that moves by its own affine map (arapb200_composite, DESIGN.md 4.5):
+    frame b rendered from frame a.  motion / motion_from: 2x3 float64 maps from the background plane to frames b / a
+    (motion_from None = identity, the pair case).  background uint8[bgH,bgW,3]; frame pixel q of a still background shows
+    background[q + origin].  src_masks: each layer's frame-a input mask (0 = object); bflows: each layer's backward flow,
+    needed with extras.  shape=(H, W) is needed only with no layers.  Returns a dict flow (frame a), rgb, mask (frame b),
+    coeffs[3,2,3] f32 (the maps F: a -> b, B: b -> a, S: b -> background plane, as the kernels used them), and with
+    extras bflow[H,W,2] (frame b) and occ[H,W] (frame a, 0 visible in frame b, 255 not)."""
+    n = len(masks)
+    H, W = masks[0].shape if n else shape
+    groups = [None if g is None else [_c(a, dt) for a in g] for g, dt in
+              ((flows, np.float32), (rgbs, np.uint8), (masks, np.uint8), (src_masks, np.uint8), (bflows, np.float32))]
+    P = C.c_void_p * n
+    ptrs = [None if g is None or n == 0 else P(*[a.ctypes.data for a in g]) for g in groups]
+    bg = _c(background, np.uint8)
+    mt = _motion(motion)
+    mf = None if motion_from is None else _motion(motion_from)
+    out = dict(flow=np.zeros((H, W, 2), np.float32), rgb=np.zeros((H, W, 3), np.uint8), mask=np.zeros((H, W), np.uint8),
+               coeffs=np.zeros((3, 2, 3), np.float32))
+    if extras:
+        out.update(bflow=np.zeros((H, W, 2), np.float32), occ=np.zeros((H, W), np.uint8))
+    L = load()
+    L.arapb200_composite.argtypes = COMPOSITE_ARGTYPES
+    _check(L.arapb200_composite(W, H, n, *ptrs, bg.shape[1], bg.shape[0], bg.ctypes.data, int(origin[0]), int(origin[1]),
+                                None if mf is None else mf.ctypes.data, mt.ctypes.data, out["flow"].ctypes.data,
+                                out["rgb"].ctypes.data, out["mask"].ctypes.data,
+                                out["bflow"].ctypes.data if extras else None, out["occ"].ctypes.data if extras else None,
+                                out["coeffs"].ctypes.data), "arapb200_composite")
+    return out
+
+
+def composite_seq(seqs, src_masks, background, motions, origin=(0, 0)):
+    """A layered frame sequence over a moving background (DESIGN.md 4.5).  seqs: per layer, the out["seq"] dict of
+    Batch.submit(..., frames=...) (K frames each); src_masks: the layers' input masks; motions[K] the background's
+    motions A_1 .. A_K (frame 0 has the identity; synth.motion_path gives the chord path).  Frame k is composite() of the
+    layers' frame k with motion_from = A_{k-1}, motion = A_k and as source masks the input masks for k = 1 and
+    255 - mask[k-1] for k >= 2.  Frame 0 is the caller's: it must show the background crop
+    background[oy:oy+H, ox:ox+W] where no layer is.  Returns composite()'s keys (with extras) stacked on a leading K axis."""
+    K = len(motions)
+    assert seqs and all(len(q["mask"]) == K for q in seqs), "one seq per layer, K frames each, K = len(motions)"
+    frames = []
+    for k in range(K):
+        src = list(src_masks) if k == 0 else [255 - q["mask"][k - 1] for q in seqs]
+        frames.append(composite([q["flow"][k] for q in seqs], [q["rgb"][k] for q in seqs], [q["mask"][k] for q in seqs],
+                                src, [q["bflow"][k] for q in seqs], background, motions[k],
+                                motion_from=None if k == 0 else motions[k - 1], origin=origin))
+    return {key: np.stack([f[key] for f in frames]) for key in frames[0]}
 
 
 def filter_matches(matches, labels1, labels2):

@@ -121,3 +121,47 @@ def config(name: str, index: int = 0) -> SynthPair:
     if name == "C4":
         return synth(1920, 1080, 1, 1, 4000 + index, axes=(0.46, 0.46))
     raise ValueError(name)
+
+
+# ---- background motion (DESIGN.md 4.5): own generators, so that synth()'s draws stay as they are -------------------
+def background(W: int, H: int, seed: int = 0) -> np.ndarray:
+    """A background image (uint8 [H, W, 3]) textured as synth()'s images are."""
+    return _texture(np.random.default_rng(seed), W, H)
+
+
+SHIFT_FRAC = 0.05   # translation: uniform in +-5 % of W (x) and of H (y)
+ROT_DEG = 5.0       # rotation: uniform in +-5 degrees
+SCALE = 0.05        # scale: uniform in [0.95, 1.05]
+
+
+def background_margin(A, W: int, H: int) -> int:
+    """The smallest integer m such that a (W+2m) x (H+2m) background at origin (m, m) covers inv(A) of the whole frame
+    with 0.01 px to spare for binary32 evaluation, i.e. such that the composite never clamps a sample."""
+    A = np.asarray(A, np.float64)
+    Ai = np.linalg.inv(np.vstack([A, [0.0, 0.0, 1.0]]))[:2]
+    corners = np.array([[0, 0, 1], [W - 1, 0, 1], [0, H - 1, 1], [W - 1, H - 1, 1]], np.float64)
+    u = corners @ Ai.T          # the preimage of the frame is the parallelogram of its corners' preimages
+    over = max(0.0, -u[:, 0].min(), -u[:, 1].min(), u[:, 0].max() - (W - 1), u[:, 1].max() - (H - 1))
+    return int(math.ceil(over + 0.01)) if over > 0 else 0
+
+
+def background_motion(W: int, H: int, seed: int = 0):
+    """A random affine background motion about the frame centre, FlyingChairs-style: A(u) = c + s R(th) (u - c) + t with
+    t uniform in +-SHIFT_FRAC (W, H), th in +-ROT_DEG degrees, s in [1 - SCALE, 1 + SCALE].  Returns (A float64 [2, 3],
+    m = background_margin(A, W, H))."""
+    rng = np.random.default_rng(seed)
+    t = rng.uniform(-SHIFT_FRAC, SHIFT_FRAC, 2) * (W, H)
+    th = math.radians(rng.uniform(-ROT_DEG, ROT_DEG))
+    s = rng.uniform(1.0 - SCALE, 1.0 + SCALE)
+    c = np.array([(W - 1) / 2.0, (H - 1) / 2.0])
+    R = s * np.array([[math.cos(th), -math.sin(th)], [math.sin(th), math.cos(th)]])
+    A = np.hstack([R, (c - R @ c + t)[:, None]])
+    return A, background_margin(A, W, H)
+
+
+def motion_path(A, steps, nCont: int) -> list:
+    """The chord path of a pair motion A for the frames of a sequence (DESIGN.md 4.4): A_k = (1 - a_k) I + a_k A with
+    a_k = (t_k + 1) / nCont for the continuation steps t_k, as the match constraints move.  Returns [A_1 .. A_K]."""
+    A = np.asarray(A, np.float64)
+    I = np.array([[1.0, 0.0, 0.0], [0.0, 1.0, 0.0]])
+    return [(1.0 - (t + 1) / nCont) * I + ((t + 1) / nCont) * A for t in steps]

@@ -85,6 +85,28 @@ ARAPB200_API int arapb200_flatten_ex(int W, int H, int n_layers, const float* co
                                      const uint8_t* const* masks, const uint8_t* background,
                                      const uint8_t* const* src_masks, const float* const* bflows, float* out_flow,
                                      uint8_t* out_rgb, uint8_t* out_mask, float* out_bflow, uint8_t* out_occ);
+/* The layers of arapb200_flatten_ex over a background that moves by its own affine map (DESIGN.md 4.5): renders frame b
+ * from frame a.  A motion is a row-major 2x3 binary64 matrix mapping background-plane points to frame pixels; the plane
+ * has frame 0's coordinates.  motion_from is frame a's motion (NULL = identity, the pair case), motion_to frame b's.
+ * n_layers (0 .. 32) layers as arapb200_flatten_ex: flows, rgbs, masks (warped), src_masks (frame-a input masks, 0 =
+ * object; required, they decide which frame-a pixels are background) and bflows (required for out_bflow / out_occ).
+ * n_layers == 0 is a pure background-motion pair.  background uint8x3[bgW*bgH], sampled bilinearly at
+ * inv(motion_to)(q) + (bg_x, bg_y) where no layer is in front, coordinates clamped to the image.
+ * out_flow float2[W*H] (frame a: the flatten's flow on object pixels, the background's motion elsewhere), out_rgb,
+ * out_mask (objects only, as the flatten) and out_bflow float2[W*H] (frame b), out_occ uint8[W*H] (frame a, 0 visible
+ * in frame b, 255 not).  out_bflow, out_occ and out_coeffs may be NULL; out_coeffs float[3][2][3] receives the binary32
+ * maps the kernels use: F (frame a -> b), B (frame b -> a), S (frame b -> background plane).  Returns non-zero before
+ * any CUDA call and without writing anything for: W or H <= 0, n_layers outside [0, 32], a missing layer array or
+ * entry (src_masks included) when n_layers > 0, out_bflow / out_occ without bflows when n_layers > 0, a NULL
+ * background or bgW / bgH <= 0, a NULL motion_to, a non-finite or singular motion or non-finite derived maps, and a
+ * NULL out_flow, out_rgb or out_mask.  With both motions the identity and a W x H background at (0, 0), rgb, mask,
+ * bflow and occ are arapb200_flatten_ex's with that background bit for bit. */
+ARAPB200_API int arapb200_composite(int W, int H, int n_layers, const float* const* flows, const uint8_t* const* rgbs,
+                                    const uint8_t* const* masks, const uint8_t* const* src_masks,
+                                    const float* const* bflows, int bgW, int bgH, const uint8_t* background, int bg_x,
+                                    int bg_y, const double* motion_from, const double* motion_to, float* out_flow,
+                                    uint8_t* out_rgb, uint8_t* out_mask, float* out_bflow, uint8_t* out_occ,
+                                    float* out_coeffs);
 
 /* ---- "next" row N3: match ingestion on the device (replaces the Python loops of para_gen.py:216-223 valid_cnstr,
  * :468-482 filter, :513-537 per-segment masks).
