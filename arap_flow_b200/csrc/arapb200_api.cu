@@ -1,5 +1,6 @@
 // arapb200_api.cu -- the flat C ABI of include/arapb200.h (host buffers in, host buffers out).
 #include "../../include/arapb200.h"
+#include "composite.cuh"
 #include "pipeline.cuh"
 
 #include <cmath>
@@ -134,6 +135,10 @@ struct arapb200_batch {
     std::vector<HostProblem> slots;
     std::vector<char> pending;
     std::vector<HostProblem> todo;
+    // scenes queued for the next run (HostScene::first holds the first slot until run() maps it into todo) and, per
+    // slot, the queued scene that owns it (-1 = none)
+    std::vector<HostScene> scenes;
+    std::vector<int> scene_of;
     float ms[3] = {0, 0, 0};
     long long launches = 0;
 };
@@ -234,6 +239,7 @@ arapb200_batch* arapb200_batch_create(int maxW, int maxH, int max_problems, int 
         b->pipe.reset(new BatchPipeline(maxW, maxH, max_problems, nCont, nGN, nPCG, backend));
         b->slots.resize(max_problems);
         b->pending.assign(max_problems, 0);
+        b->scene_of.assign(max_problems, -1);
         return 0;
     });
     if (rc) { delete b; return nullptr; }
@@ -267,6 +273,10 @@ int arapb200_batch_submit_seq(arapb200_batch* b, int slot, int W, int H, const u
 {
     return guarded([&]() -> int {
         if (!b || slot < 0 || slot >= b->max_problems) return 1;
+        if (b->scene_of[slot] >= 0) {
+            fprintf(stderr, "arapb200: batch_submit: slot %d belongs to a scene queued for the next run\n", slot);
+            return 1;
+        }
         // everything run() will dereference is checked here, while the caller can still be told
         if (W <= 0 || H <= 0 || (size_t)W * H > (size_t)b->maxW * b->maxH || !rgb || !mask_red || n_matches < 0 ||
             (n_matches > 0 && !matches)) {
@@ -293,7 +303,87 @@ int arapb200_batch_submit_seq(arapb200_batch* b, int slot, int W, int H, const u
         hp.steps.assign(steps, steps + n_frames);
         hp.seq_rgb = seq_rgb; hp.seq_mask = seq_mask; hp.seq_flow = seq_flow; hp.seq_bflow = seq_bflow;
         hp.seq_occ = seq_occ; hp.seq_flow0 = seq_flow0;
+        hp.scene = false; // the slot may have been a scene layer in an earlier run
         b->pending[slot] = 1;
+        return 0;
+    });
+}
+
+int arapb200_batch_submit_scene(arapb200_batch* b, int slot, int n_layers, int W, int H, const uint8_t* rgb,
+                                const uint8_t* const* masks_red, const int32_t* const* matches, const int* n_matches,
+                                int bgW, int bgH, const uint8_t* background, int bg_x, int bg_y, const double* motion,
+                                int n_frames, const int* steps, const double* frame_motions, float* out_flow,
+                                uint8_t* out_rgb, uint8_t* out_mask, float* out_bflow, uint8_t* out_occ, uint8_t* out_rgb0,
+                                float* out_costs, uint8_t* seq_rgb, uint8_t* seq_mask, float* seq_flow, float* seq_bflow,
+                                uint8_t* seq_occ)
+{
+    return guarded([&]() -> int {
+        // every rejection comes before anything is queued
+        if (!b || n_layers < 1 || n_layers > MAX_LAYERS || slot < 0 || slot > b->max_problems - n_layers) return 1;
+        for (int s = slot; s < slot + n_layers; ++s)
+            if (b->scene_of[s] >= 0) {
+                fprintf(stderr, "arapb200: batch_submit_scene: slot %d belongs to another queued scene\n", s);
+                return 1;
+            }
+        if (W <= 0 || H <= 0 || (size_t)W * H > (size_t)b->maxW * b->maxH || !rgb || !masks_red || !matches ||
+            !n_matches) {
+            fprintf(stderr, "arapb200: batch_submit_scene: bad scene (%dx%d in a %dx%d batch, null input?)\n", W, H,
+                    b->maxW, b->maxH);
+            return 1;
+        }
+        for (int s = 0; s < n_layers; ++s)
+            if (!masks_red[s] || n_matches[s] < 0 || (n_matches[s] > 0 && !matches[s])) {
+                fprintf(stderr, "arapb200: batch_submit_scene: layer %d: null mask or bad match list\n", s);
+                return 1;
+            }
+        if (!background || bgW <= 0 || bgH <= 0 || !motion || !out_flow || !out_rgb || !out_mask) {
+            fprintf(stderr, "arapb200: batch_submit_scene: null background, motion or pair output, or bad background size\n");
+            return 1;
+        }
+        const bool any_out = seq_rgb || seq_mask || seq_flow || seq_bflow || seq_occ;
+        if (n_frames < 0 || (n_frames == 0 && any_out) ||
+            (n_frames > 0 && (!steps || !frame_motions || !seq_rgb || !seq_mask))) {
+            fprintf(stderr, "arapb200: batch_submit_scene: %d frames with%s step list,%s motions and%s outputs (rgb and "
+                    "mask required)\n", n_frames, steps ? "" : " no", frame_motions ? "" : " no", any_out ? "" : " no");
+            return 1;
+        }
+        for (int k = 0; k < n_frames; ++k)
+            if (steps[k] < 0 || steps[k] >= b->nCont || (k > 0 && steps[k] <= steps[k - 1])) {
+                fprintf(stderr, "arapb200: batch_submit_scene: steps must increase strictly within [0, %d]; step %d is %d\n",
+                        b->nCont - 1, k, steps[k]);
+                return 1;
+            }
+        HostScene sc;
+        sc.maps.resize(18 * (size_t)(1 + n_frames));
+        bool ok = composite_coeffs(nullptr, motion, sc.maps.data());
+        for (int k = 0; k < n_frames && ok; ++k) // frame k + 1: A_k -> A_{k+1}, A_0 = identity
+            ok = composite_coeffs(k == 0 ? nullptr : frame_motions + 6 * (k - 1), frame_motions + 6 * k,
+                                  sc.maps.data() + 18 * (k + 1));
+        if (!ok) {
+            fprintf(stderr, "arapb200: batch_submit_scene: non-finite or singular motion\n");
+            return 1;
+        }
+        sc.first = slot;
+        sc.n = n_layers;
+        sc.W = W; sc.H = H;
+        sc.background = background; sc.bgW = bgW; sc.bgH = bgH; sc.bg_x = bg_x; sc.bg_y = bg_y;
+        sc.out_flow = out_flow; sc.out_rgb = out_rgb; sc.out_mask = out_mask; sc.out_bflow = out_bflow;
+        sc.out_occ = out_occ; sc.out_rgb0 = out_rgb0;
+        sc.seq_rgb = seq_rgb; sc.seq_mask = seq_mask; sc.seq_flow = seq_flow; sc.seq_bflow = seq_bflow;
+        sc.seq_occ = seq_occ;
+        const size_t cn = (size_t)b->nCont * (b->nGN + 1);
+        for (int s = 0; s < n_layers; ++s) {
+            HostProblem& hp = b->slots[slot + s];
+            hp = HostProblem{};
+            hp.W = W; hp.H = H; hp.rgb = rgb; hp.mask_red = masks_red[s]; hp.matches = matches[s];
+            hp.n_matches = n_matches[s];
+            hp.out_costs = out_costs ? out_costs + cn * s : nullptr;
+            hp.steps.assign(steps, steps + n_frames);
+            hp.scene = true;
+            b->pending[slot + s] = 1;
+            b->scene_of[slot + s] = (int)b->scenes.size();
+        }
+        b->scenes.push_back(std::move(sc));
         return 0;
     });
 }
@@ -305,12 +395,18 @@ int arapb200_batch_run(arapb200_batch* b)
         b->ms[0] = b->ms[1] = b->ms[2] = 0.f;
         const long long l0 = b->pipe->launches();
         b->todo.clear();
+        std::vector<int> at(b->max_problems, -1); // slot -> index in todo
         for (int s = 0; s < b->max_problems; ++s)
             if (b->pending[s]) {
+                at[s] = (int)b->todo.size();
                 b->todo.push_back(b->slots[s]);
                 b->pending[s] = 0;
             }
-        const int rc = b->pipe->run(b->todo.data(), (int)b->todo.size());
+        std::vector<HostScene> scenes;
+        scenes.swap(b->scenes);
+        b->scene_of.assign(b->max_problems, -1);
+        for (HostScene& sc : scenes) sc.first = at[sc.first]; // a scene's slots are consecutive and all pending
+        const int rc = b->pipe->run(b->todo.data(), (int)b->todo.size(), scenes.data(), (int)scenes.size());
         if (rc) return rc;
         b->ms[0] = b->pipe->last_ms_total();
         b->ms[1] = b->pipe->last_ms_solve();

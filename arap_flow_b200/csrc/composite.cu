@@ -9,8 +9,10 @@
 // same occlusion rule as the per-problem warp (warp.cuh occlusion_of, DESIGN.md 4.3).
 // arapb200_composite: the same layers over a background that moves by its own affine map, with the forward flow,
 // backward flow and occlusion of both (DESIGN.md 4.5).
+// The batch's scenes (DESIGN.md 4.6) launch the same composite on layers that stay on the device (composite.cuh).
 #include "../../include/arapb200.h"
 #include "common.cuh"
+#include "composite.cuh"
 #include "warp.cuh"
 
 #include <algorithm>
@@ -20,16 +22,6 @@
 
 namespace arapb200 {
 namespace {
-
-constexpr int MAX_LAYERS = 32;
-struct Layers {
-    const float2* flow[MAX_LAYERS];
-    const unsigned char* rgb[MAX_LAYERS];
-    const unsigned char* mask[MAX_LAYERS];
-    const float2* bflow[MAX_LAYERS];      // backward flow of each layer (only read for out_bflow / out_occ)
-    const unsigned char* src[MAX_LAYERS]; // frame-a input mask of each layer, 0 = object (flatten: only read for out_occ)
-    int n;
-};
 
 // the layer in front at pixel i: the last one whose warped mask is non-zero, -1 = none
 __device__ __forceinline__ int front_layer(const Layers& L, size_t i)
@@ -128,7 +120,10 @@ __global__ void __launch_bounds__(256) k_composite_b(int W, int H, Layers L, con
 }
 
 // frame-a pass: forward flow and (out_occ non-null) occlusion, the background being surface L.n.  F: frame-a pixel ->
-// frame b; bflow_b: the frame-b backward flow k_composite_b wrote (read only for out_occ).
+// frame b; bflow_b: the frame-b backward flow k_composite_b wrote (read only for out_occ).  kSrcPrev: L.src are the
+// warped masks of frame k-1 of a sequence, p being on layer s where one is 255 -- the "255 - mask" of the flatten recipe
+// (DESIGN.md 4.4) read in place.
+template <bool kSrcPrev>
 __global__ void __launch_bounds__(256) k_composite_a(int W, int H, Layers L, Affine F,
                                                       const float2* __restrict__ bflow_b, float2* __restrict__ out_flow,
                                                       unsigned char* __restrict__ out_occ)
@@ -139,7 +134,7 @@ __global__ void __launch_bounds__(256) k_composite_a(int W, int H, Layers L, Aff
     const int px = (int)(i % W), py = (int)(i / W);
     int seg = L.n; // p's surface: the (last) layer whose input mask has p on the object, else the background
     for (int s = L.n - 1; s >= 0; --s)
-        if (L.src[s][i] == 0) { seg = s; break; }
+        if (kSrcPrev ? L.src[s][i] == 255 : L.src[s][i] == 0) { seg = s; break; }
     float2 f;
     if (seg < L.n) {
         const int front = front_layer(L, i);
@@ -155,6 +150,26 @@ __global__ void __launch_bounds__(256) k_composite_a(int W, int H, Layers L, Aff
             const int s = front_layer(L, q);
             return s < 0 ? L.n : s;
         });
+}
+
+// frame 0 of a scene: the input image where any layer's input mask is 0 (the object), the background crop elsewhere
+__global__ void __launch_bounds__(256) k_scene_input(int W, int H, Layers L, const unsigned char* __restrict__ rgb,
+                                                      const unsigned char* __restrict__ bg, int bgW, int bgH, int bg_x,
+                                                      int bg_y, unsigned char* __restrict__ out)
+{
+    const size_t N = (size_t)W * H;
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= N) return;
+    bool object = false;
+    for (int s = 0; s < L.n; ++s) object = object || L.src[s][i] == 0;
+    const unsigned char* c = rgb + 3 * i;
+    if (!object) {
+        const int x = min(max((int)(i % W) + bg_x, 0), bgW - 1), y = min(max((int)(i / W) + bg_y, 0), bgH - 1);
+        c = bg + 3 * ((size_t)y * bgW + x);
+    }
+    out[3 * i] = c[0];
+    out[3 * i + 1] = c[1];
+    out[3 * i + 2] = c[2];
 }
 
 // ---- N3: match filter (para_gen.py:216-223) and per-segment masks (:513-537) ----
@@ -378,6 +393,7 @@ extern "C" int arapb200_flatten_ex(int W, int H, int n_layers, const float* cons
                           out_bflow, out_occ);
 }
 
+namespace arapb200 {
 namespace {
 // 2x3 affine maps in binary64, row-major: (a00 a01 a02; a10 a11 a12).  The derivation of DESIGN.md 4.5, in its order;
 // fp-contract=off keeps a host compiler from fusing a product and a sum where the target has FMA.
@@ -426,7 +442,9 @@ bool aff_finite(const double* a)
     return true;
 }
 
-// F, B, S rounded to binary32 (c[3][2][3]); false for a non-finite or singular motion or a non-finite coefficient
+Affine affine_of(const float* c) { return Affine{c[0], c[1], c[2], c[3], c[4], c[5]}; }
+} // namespace
+
 bool composite_coeffs(const double* motion_from, const double* motion_to, float c[18])
 {
     Aff64 Af{{1.0, 0.0, 0.0, 0.0, 1.0, 0.0}}, At;
@@ -444,8 +462,26 @@ bool composite_coeffs(const double* motion_from, const double* motion_to, float 
     return true;
 }
 
-Affine affine_of(const float* c) { return Affine{c[0], c[1], c[2], c[3], c[4], c[5]}; }
+void enqueue_composite(int W, int H, const Layers& L, bool src_prev, const unsigned char* d_bg, int bgW, int bgH,
+                       int bg_x, int bg_y, const float c[18], float2* d_flow, unsigned char* d_rgb,
+                       unsigned char* d_mask, float2* d_bflow, unsigned char* d_occ, cudaStream_t stream)
+{
+    const unsigned blocks = (unsigned)(((size_t)W * H + 255) / 256);
+    k_composite_b<<<blocks, 256, 0, stream>>>(W, H, L, d_bg, bgW, bgH, bg_x, bg_y, affine_of(c + 12), affine_of(c + 6),
+                                              d_rgb, d_mask, d_bflow);
+    if (src_prev) k_composite_a<true><<<blocks, 256, 0, stream>>>(W, H, L, affine_of(c), d_bflow, d_flow, d_occ);
+    else k_composite_a<false><<<blocks, 256, 0, stream>>>(W, H, L, affine_of(c), d_bflow, d_flow, d_occ);
+}
 
+void enqueue_scene_input(int W, int H, const Layers& L, const unsigned char* d_rgb, const unsigned char* d_bg, int bgW,
+                         int bgH, int bg_x, int bg_y, unsigned char* d_out, cudaStream_t stream)
+{
+    const unsigned blocks = (unsigned)(((size_t)W * H + 255) / 256);
+    k_scene_input<<<blocks, 256, 0, stream>>>(W, H, L, d_rgb, d_bg, bgW, bgH, bg_x, bg_y, d_out);
+}
+} // namespace arapb200
+
+namespace {
 template <class T> bool all_set(const T* const* p, int n)
 {
     if (!p) return false;
@@ -503,10 +539,7 @@ extern "C" int arapb200_composite(int W, int H, int n_layers, const float* const
         unsigned char* d_om = take(N);
         float2* d_ob = ex ? (float2*)take(N * sizeof(float2)) : nullptr; // out_occ reads the whole frame-b bflow
         unsigned char* d_oo = out_occ ? take(N) : nullptr;
-        const unsigned blocks = (unsigned)((N + 255) / 256);
-        k_composite_b<<<blocks, 256>>>(W, H, L, d_bg, bgW, bgH, bg_x, bg_y, affine_of(cf + 12), affine_of(cf + 6), d_or,
-                                        d_om, d_ob);
-        k_composite_a<<<blocks, 256>>>(W, H, L, affine_of(cf), d_ob, d_of, d_oo);
+        enqueue_composite(W, H, L, false, d_bg, bgW, bgH, bg_x, bg_y, cf, d_of, d_or, d_om, d_ob, d_oo, nullptr);
         if (cudaMemcpy(out_flow, d_of, N * sizeof(float2), cudaMemcpyDeviceToHost) ||
             cudaMemcpy(out_rgb, d_or, 3 * N, cudaMemcpyDeviceToHost) || cudaMemcpy(out_mask, d_om, N, cudaMemcpyDeviceToHost) ||
             (out_bflow && cudaMemcpy(out_bflow, d_ob, N * sizeof(float2), cudaMemcpyDeviceToHost)) ||

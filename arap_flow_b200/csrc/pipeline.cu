@@ -1,5 +1,6 @@
 // pipeline.cu -- see pipeline.cuh
 #include "pipeline.cuh"
+#include "composite.cuh"
 #include <algorithm>
 #include <cmath>
 #include <cstring>
@@ -87,6 +88,25 @@ __global__ void __launch_bounds__(256) k_scatter_t(const MatchRec* __restrict__ 
 
 __global__ void k_copy_cost(const StreamScalars* __restrict__ sc, float* __restrict__ dst) { *dst = sc->cost; }
 
+// a scene's device buffer: [background][rgb0][flow][rgb][mask][bflow][occ], the last five holding the pair (index 0) and
+// frames 1 .. K, so that each frame output leaves in one copy
+struct SceneLayout {
+    size_t bg, rgb0, flow, rgb, mask, bflow, occ, bytes;
+    SceneLayout(const HostScene& sc)
+    {
+        auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
+        const size_t N = (size_t)sc.W * sc.H, F = N * (sc.maps.size() / 18);
+        bg = 0;
+        rgb0 = bg + al(3 * (size_t)sc.bgW * sc.bgH);
+        flow = rgb0 + (sc.out_rgb0 ? al(3 * N) : 0);
+        rgb = flow + al(8 * F);
+        mask = rgb + al(3 * F);
+        bflow = mask + al(F);
+        occ = bflow + al(8 * F);
+        bytes = occ + al(F);
+    }
+};
+
 } // namespace
 
 void enqueue_reset_state(int W, int H, const unsigned char* d_mask_red, float2* d_X, float2* d_U, float* d_A,
@@ -151,6 +171,7 @@ BatchPipeline::~BatchPipeline()
         cudaFreeHost(d.h_in); cudaFreeHost(d.h_out); cudaFreeHost(d.h_extra);
         free_seq(d);
     }
+    for (SceneDev& sd : scene_dev_) cudaFree(sd.buf);
     for (auto& e : ev_) cudaEventDestroy(e);
     cudaStreamDestroy(stream_);
 }
@@ -276,6 +297,47 @@ void BatchPipeline::solve_resident(const HostProblem* problems, int first, int c
     }
 }
 
+// frame 0, the pair, then frame k = 1 .. K with the layers' frame k and as source masks the input masks (k = 1) or the
+// warped masks of frame k - 1 (DESIGN.md 4.6)
+void BatchPipeline::enqueue_scene(const HostScene& sc, unsigned char* buf)
+{
+    const SceneLayout o(sc);
+    const size_t N = (size_t)sc.W * sc.H;
+    const int K = (int)(sc.maps.size() / 18) - 1;
+    const unsigned char* bg = buf + o.bg;
+    Layers L{};
+    L.n = sc.n;
+    for (int s = 0; s < sc.n; ++s) {
+        const Dev& d = dev_[sc.first + s];
+        L.flow[s] = d.flow;
+        L.rgb[s] = d.orgb;
+        L.mask[s] = d.omask;
+        L.bflow[s] = d.bflow;
+        L.src[s] = d.mask;
+    }
+    if (sc.out_rgb0) {
+        enqueue_scene_input(sc.W, sc.H, L, dev_[sc.first].rgb, bg, sc.bgW, sc.bgH, sc.bg_x, sc.bg_y, buf + o.rgb0, stream_);
+        launches_ += 1;
+    }
+    for (int k = 0; k <= K; ++k) {
+        if (k > 0)
+            for (int s = 0; s < sc.n; ++s) {
+                const SeqOut& q = dev_[sc.first + s].seq;
+                const size_t f = (size_t)(k - 1) * N;
+                L.flow[s] = q.flow + f;
+                L.rgb[s] = q.rgb + 3 * f;
+                L.mask[s] = q.mask + f;
+                L.bflow[s] = q.bflow + f;
+                L.src[s] = k == 1 ? dev_[sc.first + s].mask : q.mask + f - N;
+            }
+        const size_t f = (size_t)k * N;
+        enqueue_composite(sc.W, sc.H, L, k >= 2, bg, sc.bgW, sc.bgH, sc.bg_x, sc.bg_y, sc.maps.data() + 18 * k,
+                          (float2*)(buf + o.flow) + f, buf + o.rgb + 3 * f, buf + o.mask + f,
+                          (float2*)(buf + o.bflow) + f, buf + o.occ + f, stream_);
+        launches_ += 2;
+    }
+}
+
 void BatchPipeline::set_pcg_rtol(float rtol)
 {
     pcg_rtol_ = rtol > 0.0f ? rtol : 0.0f;
@@ -288,7 +350,7 @@ void BatchPipeline::set_gn_rtol(float rtol)
     if (resident_) resident_->set_gn_rtol(rtol);
 }
 
-int BatchPipeline::run(const HostProblem* problems, int count)
+int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* scenes, int n_scenes)
 {
     if (count <= 0) return 0;
     if (count > (int)dev_.size()) {
@@ -312,12 +374,12 @@ int BatchPipeline::run(const HostProblem* problems, int count)
             d.matches_cap = d.recs.size() * 2 + 1024;
             ARAP_CUDA_OR_RETURN(cudaMalloc(&d.matches, d.matches_cap * sizeof(MatchRec)));
         }
-        if ((hp.out_bflow || hp.out_occ) && !d.h_extra) {
-            const size_t Nmax = (size_t)maxW_ * maxH_;
+        const size_t Nmax = (size_t)maxW_ * maxH_;
+        if ((hp.out_bflow || hp.out_occ || hp.scene) && !d.bflow) {
             ARAP_CUDA_OR_RETURN(cudaMalloc(&d.bflow, Nmax * sizeof(float2)));
             ARAP_CUDA_OR_RETURN(cudaMalloc(&d.occ, Nmax));
-            ARAP_CUDA_OR_RETURN(cudaMallocHost(&d.h_extra, 9 * Nmax));
         }
+        if ((hp.out_bflow || hp.out_occ) && !d.h_extra) ARAP_CUDA_OR_RETURN(cudaMallocHost(&d.h_extra, 9 * Nmax));
         if ((int)hp.steps.size() > d.seq_cap) {
             free_seq(d);
             const size_t F = (size_t)maxW_ * maxH_ * hp.steps.size(); // pixels of all frames
@@ -334,6 +396,18 @@ int BatchPipeline::run(const HostProblem* problems, int count)
         memcpy(d.h_in, hp.rgb, 3 * N);
         memcpy(d.h_in + 3 * N, hp.mask_red, N);
     }
+    if (n_scenes > (int)scene_dev_.size()) scene_dev_.resize(n_scenes);
+    for (int j = 0; j < n_scenes; ++j) {
+        SceneDev& sd = scene_dev_[j];
+        const size_t need = SceneLayout(scenes[j]).bytes;
+        if (need > sd.cap) {
+            ARAP_CUDA_OR_RETURN(cudaFree(sd.buf));
+            sd.buf = nullptr;
+            sd.cap = 0;
+            ARAP_CUDA_OR_RETURN(cudaMalloc(&sd.buf, need));
+            sd.cap = need;
+        }
+    }
     ARAP_CUDA_OR_RETURN(cudaEventRecord(ev_[0], stream_));
     for (int i = 0; i < count; ++i) {
         const HostProblem& hp = problems[i];
@@ -348,6 +422,11 @@ int BatchPipeline::run(const HostProblem* problems, int count)
         launches_ += 1;
         d.resident = false;
         if (resident_ && !lm_on_) resident_->prepare_enqueue(i, hp.W, hp.H, d.M, stream_);
+    }
+    for (int j = 0; j < n_scenes; ++j) {
+        const HostScene& sc = scenes[j];
+        ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(scene_dev_[j].buf, sc.background, 3 * (size_t)sc.bgW * sc.bgH,
+                                            cudaMemcpyHostToDevice, stream_));
     }
     n_resident_ = 0;
     if (resident_ && !lm_on_) {
@@ -405,7 +484,7 @@ int BatchPipeline::run(const HostProblem* problems, int count)
         const HostProblem& hp = problems[i];
         Dev& d = dev_[i];
         enqueue_pos_to_flow(hp.W, hp.H, d.X, d.flow, stream_);
-        const bool extras = hp.out_bflow || hp.out_occ;
+        const bool extras = hp.out_bflow || hp.out_occ || hp.scene;
         enqueue_warp(hp.W, hp.H, d.X, d.rgb, d.mask, d.z, d.orgb, d.omask, stream_, extras ? d.bflow : nullptr);
         launches_ += 1 + warp_launches_per_call();
         if (extras) {
@@ -415,16 +494,20 @@ int BatchPipeline::run(const HostProblem* problems, int count)
         if (!hp.steps.empty())
             launches_ += enqueue_warp_seq(hp.W, hp.H, (int)hp.steps.size(), d.seq_pos, d.rgb, d.mask, d.seq_z, d.seq, stream_);
     }
+    for (int j = 0; j < n_scenes; ++j) enqueue_scene(scenes[j], scene_dev_[j].buf);
     ARAP_CUDA_OR_RETURN(cudaEventRecord(ev_[3], stream_));
     for (int i = 0; i < count; ++i) {
         const HostProblem& hp = problems[i];
         Dev& d = dev_[i];
         const size_t N = (size_t)hp.W * hp.H;
         unsigned char* o = d.h_out;
-        ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(o, d.flow, N * sizeof(float2), cudaMemcpyDeviceToHost, stream_));
-        ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(o + 8 * N, d.orgb, 3 * N, cudaMemcpyDeviceToHost, stream_));
-        ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(o + 11 * N, d.omask, N, cudaMemcpyDeviceToHost, stream_));
-        ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(o + 12 * N, d.costs, cbytes, cudaMemcpyDeviceToHost, stream_));
+        if (!hp.scene) {
+            ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(o, d.flow, N * sizeof(float2), cudaMemcpyDeviceToHost, stream_));
+            ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(o + 8 * N, d.orgb, 3 * N, cudaMemcpyDeviceToHost, stream_));
+            ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(o + 11 * N, d.omask, N, cudaMemcpyDeviceToHost, stream_));
+        }
+        if (!hp.scene || hp.out_costs)
+            ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(o + 12 * N, d.costs, cbytes, cudaMemcpyDeviceToHost, stream_));
         if (hp.out_bflow || hp.out_occ) {
             ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(d.h_extra, d.bflow, N * sizeof(float2), cudaMemcpyDeviceToHost, stream_));
             ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(d.h_extra + 8 * N, d.occ, N, cudaMemcpyDeviceToHost, stream_));
@@ -436,6 +519,21 @@ int BatchPipeline::run(const HostProblem* problems, int count)
             {hp.seq_bflow, d.seq.bflow, 8 * F}, {hp.seq_occ, d.seq.occ, F}, {hp.seq_flow0, d.seq.flow0, 8 * F}};
         for (const auto& c : seq)
             if (c.dst && F) ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(c.dst, c.src, c.bytes, cudaMemcpyDeviceToHost, stream_));
+    }
+    // scene outputs go straight to the caller's buffers: the pair is frame index 0 of each block, frames 1 .. K follow
+    for (int j = 0; j < n_scenes; ++j) {
+        const HostScene& sc = scenes[j];
+        const SceneLayout l(sc);
+        const unsigned char* b = scene_dev_[j].buf;
+        const size_t N = (size_t)sc.W * sc.H, F = N * (sc.maps.size() / 18 - 1);
+        const struct { void* dst; size_t off, bytes; } out[] = {
+            {sc.out_flow, l.flow, 8 * N}, {sc.out_rgb, l.rgb, 3 * N}, {sc.out_mask, l.mask, N},
+            {sc.out_bflow, l.bflow, 8 * N}, {sc.out_occ, l.occ, N}, {sc.out_rgb0, l.rgb0, 3 * N},
+            {sc.seq_flow, l.flow + 8 * N, 8 * F}, {sc.seq_rgb, l.rgb + 3 * N, 3 * F}, {sc.seq_mask, l.mask + N, F},
+            {sc.seq_bflow, l.bflow + 8 * N, 8 * F}, {sc.seq_occ, l.occ + N, F}};
+        for (const auto& c : out)
+            if (c.dst && c.bytes)
+                ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(c.dst, b + c.off, c.bytes, cudaMemcpyDeviceToHost, stream_));
     }
     ARAP_CUDA_OR_RETURN(cudaStreamSynchronize(stream_));
     if (resident_ && n_resident_ > 0) {

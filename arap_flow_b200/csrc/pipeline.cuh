@@ -26,6 +26,25 @@ struct HostProblem {
     std::vector<int> steps;
     unsigned char *seq_rgb = nullptr, *seq_mask = nullptr, *seq_occ = nullptr;
     float *seq_flow = nullptr, *seq_bflow = nullptr, *seq_flow0 = nullptr;
+    // a layer of a HostScene: backward flow, occlusion and frames are computed and stay on the device; of the outputs
+    // above only out_costs is copied out
+    bool scene = false;
+};
+
+// A scene (DESIGN.md 4.6): problems first .. first + n - 1 of a run are its layers in segment order (same W x H and rgb),
+// composited on the device over a moving background.  maps: the composite_coeffs of the pair (motion_from = identity),
+// then of frame k = 1 .. K (A_{k-1} -> A_k), K = the layers' step count.  Host buffers; outputs as
+// arapb200_batch_submit_scene describes them.
+struct HostScene {
+    int first = 0, n = 0, W = 0, H = 0;
+    const unsigned char* background = nullptr; // uint8x3[bgW*bgH]
+    int bgW = 0, bgH = 0, bg_x = 0, bg_y = 0;
+    std::vector<float> maps;                   // [1 + K][18]
+    float* out_flow = nullptr;
+    unsigned char *out_rgb = nullptr, *out_mask = nullptr, *out_occ = nullptr, *out_rgb0 = nullptr;
+    float* out_bflow = nullptr;
+    unsigned char *seq_rgb = nullptr, *seq_mask = nullptr, *seq_occ = nullptr;
+    float *seq_flow = nullptr, *seq_bflow = nullptr;
 };
 
 // compact constraint record: source pixel index and the match, after the reference's filtering
@@ -47,8 +66,9 @@ public:
     ~BatchPipeline();
     BatchPipeline(const BatchPipeline&) = delete;
     BatchPipeline& operator=(const BatchPipeline&) = delete;
-    // upload, solve (all continuation steps), flow, warp, download -- for every problem given.  Blocking.
-    int run(const HostProblem* problems, int count);
+    // upload, solve (all continuation steps), flow, warp, download -- for every problem given; then the composite of every
+    // scene, whose layers are among the problems.  Blocking.
+    int run(const HostProblem* problems, int count, const HostScene* scenes = nullptr, int n_scenes = 0);
     long long launches() const { return launches_; }
     float last_ms_total() const { return ms_total_; }
     float last_ms_solve() const { return ms_solve_; }
@@ -101,6 +121,14 @@ private:
     void solve_resident(const HostProblem* problems, int first, int count, bool cluster);
     void snapshot(const HostProblem& hp, Dev& d, int t); // X -> frame buffer if step t is one hp asks for
     static void free_seq(Dev& d);
+    // device buffer of the j-th scene of a run, allocated the first time and grown for a larger scene: the background,
+    // frame 0 and the composited pair and frames (21 B/px each), laid out by SceneLayout (pipeline.cu)
+    struct SceneDev {
+        unsigned char* buf = nullptr;
+        size_t cap = 0;
+    };
+    std::vector<SceneDev> scene_dev_;
+    void enqueue_scene(const HostScene& sc, unsigned char* buf); // the scene's kernels (DESIGN.md 4.6)
     LmSolver* lm_ = nullptr;
     int lmW_ = 0, lmH_ = 0;
     bool lm_on_ = false;

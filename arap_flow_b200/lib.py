@@ -29,7 +29,7 @@ ARAP_SYMBOLS = [
     "arapb200_debug_resident_profile", "arapb200_debug_resident_profile_group", "arapb200_flatten", "arapb200_filter_matches", "arapb200_segment_mask",
     "arapb200_batch_set_option", "arapb200_batch_resident_count", "arapb200_debug_wide_sum", "arapb200_plan_error", "arapb200_plan_lm_info", "arapb200_plan_timing_report",
     "arapb200_batch_launch_info", "arapb200_warp_ex", "arapb200_batch_submit_ex", "arapb200_flatten_ex",
-    "arapb200_warp_seq", "arapb200_batch_submit_seq", "arapb200_composite",
+    "arapb200_warp_seq", "arapb200_batch_submit_seq", "arapb200_composite", "arapb200_batch_submit_scene",
 ]
 
 
@@ -381,6 +381,68 @@ class Batch:
                    "arapb200_batch_submit_ex")
         else:
             _check(self.L.arapb200_batch_submit(*args), "arapb200_batch_submit")
+        return out
+
+    SCENE_KEYS = ("flow", "rgb", "mask", "bflow", "occ")
+
+    def submit_scene(self, slot, rgb, masks, matches, background, motion, origin=(0, 0), frames=None, frame_motions=None,
+                     input_frame=False, out=None):
+        """Queue a scene (arapb200_batch_submit_scene, DESIGN.md 4.6): one image rgb, its segments' masks (0 = object, in
+        segment order) with one match list each, and a background uint8[bgH,bgW,3] that moves by the 2x3 float64 map
+        `motion` (frame pixel q of a still background shows background[q + origin]).  The layers take slots
+        slot .. slot + len(masks) - 1, are solved and warped like submit(..., extras=True) problems and composited on the
+        device; only the composite is copied out.  Returns a dict with composite()'s image keys (flow, rgb, mask, bflow,
+        occ: what composite() gives for those layers with motion_from=None), costs[n_layers, nCont, nGN+1], with
+        input_frame=True rgb0[H,W,3] (frame 0: rgb on the objects, the background crop elsewhere), and with frames (a
+        strictly increasing list of continuation steps) and frame_motions (A_1 .. A_K, e.g. synth.motion_path) "seq",
+        stacked like composite_seq()'s result.  `out` may be the dict a previous submit_scene() of the same shape returned:
+        its arrays are then written in place."""
+        n = len(masks)
+        H, W = masks[0].shape
+        rgb = _c(rgb, np.uint8)
+        mk = [_c(m, np.uint8) for m in masks]
+        mt = [_c(m, np.int32).reshape(-1, 4) for m in matches]
+        if len(mt) != n:
+            raise ValueError(f"{n} masks but {len(mt)} match lists")
+        bg = _c(background, np.uint8)
+        A = _motion(motion)
+        steps = fm = None
+        K = 0
+        if frames is not None:
+            steps = np.ascontiguousarray(frames, np.int32).reshape(-1)
+            K = len(steps)
+        if frame_motions is not None:
+            fm = np.ascontiguousarray(np.asarray(frame_motions, np.float64).reshape(-1, 2, 3))
+            if len(fm) != K:   # the library reads one motion per frame
+                raise ValueError(f"{len(fm)} frame motions for {K} frames")
+        if out is None or out["flow"].shape != (H, W, 2) or out["costs"].shape[0] != n:
+            out = dict(flow=np.zeros((H, W, 2), np.float32), rgb=np.zeros((H, W, 3), np.uint8),
+                       mask=np.zeros((H, W), np.uint8), bflow=np.zeros((H, W, 2), np.float32),
+                       occ=np.zeros((H, W), np.uint8), costs=np.zeros((n, self.nCont, self.nGN + 1), np.float32))
+        if input_frame and "rgb0" not in out:
+            out["rgb0"] = np.zeros((H, W, 3), np.uint8)
+        elif not input_frame:
+            out.pop("rgb0", None)
+        if K and ("seq" not in out or out["seq"]["mask"].shape[0] != K):
+            out["seq"] = dict(flow=np.zeros((K, H, W, 2), np.float32), rgb=np.zeros((K, H, W, 3), np.uint8),
+                              mask=np.zeros((K, H, W), np.uint8), bflow=np.zeros((K, H, W, 2), np.float32),
+                              occ=np.zeros((K, H, W), np.uint8))
+        elif not K:
+            out.pop("seq", None)
+        P = C.c_void_p * n
+        ptrs = (P(*[m.ctypes.data for m in mk]), P(*[m.ctypes.data for m in mt]), (C.c_int * n)(*[len(m) for m in mt]))
+        self._keep[slot] = (rgb, mk, mt, bg, A, steps, fm, ptrs, out)
+        seq = out.get("seq")
+        self.L.arapb200_batch_submit_scene.argtypes = ([C.c_void_p] + [C.c_int] * 4 + [C.c_void_p] * 4 + [C.c_int] * 2 +
+                                                       [C.c_void_p] + [C.c_int] * 2 + [C.c_void_p, C.c_int] +
+                                                       [C.c_void_p] * 14)
+        _check(self.L.arapb200_batch_submit_scene(
+            self.h, slot, n, W, H, rgb.ctypes.data, *ptrs, bg.shape[1], bg.shape[0], bg.ctypes.data, int(origin[0]),
+            int(origin[1]), A.ctypes.data, K, None if steps is None else steps.ctypes.data,
+            None if fm is None else fm.ctypes.data, *[out[k].ctypes.data for k in self.SCENE_KEYS],
+            out["rgb0"].ctypes.data if input_frame else None, out["costs"].ctypes.data,
+            *[None if seq is None else seq[k].ctypes.data for k in ("rgb", "mask", "flow", "bflow", "occ")]),
+            "arapb200_batch_submit_scene")
         return out
 
     def run(self):

@@ -155,11 +155,50 @@ ARAPB200_API int arapb200_batch_submit_seq(arapb200_batch* b, int slot, int W, i
                                            float* out_bflow, uint8_t* out_occ, int n_frames, const int* steps,
                                            uint8_t* seq_rgb, uint8_t* seq_mask, float* seq_flow, float* seq_bflow,
                                            uint8_t* seq_occ, float* seq_flow0);
+/* A scene (DESIGN.md 4.6): one image, its n_layers segments and a background with its own motion, solved, warped and
+ * composited in the batch without the layers leaving the device.  Slots slot .. slot + n_layers - 1 take one layer each,
+ * in segment order (later layers are in front, as in arapb200_flatten); layer s is an ordinary problem with the shared
+ * W x H and rgb, its own masks_red[s] (0 = object) and its own matches[s] / n_matches[s], grouped and launched as run()
+ * groups any problems.  The solve and the warp read rgb only on the object, so rgb may be the raw image.
+ * The pair: out_flow, out_rgb, out_mask, out_bflow, out_occ are exactly arapb200_composite of the layers' ordinary
+ * outputs (flow, rgb, mask, backward flow, input mask) with motion_from = NULL and motion_to = motion (row-major 2x3
+ * binary64, required; the identity gives a still background), over background uint8x3[bgW*bgH] at origin (bg_x, bg_y).
+ * out_flow, out_rgb and out_mask are required; out_bflow, out_occ, out_rgb0 and out_costs may be NULL.
+ * out_costs float[n_layers][nCont][nGN+1]: the layers' cost logs.
+ * out_rgb0 uint8x3[W*H], frame 0: rgb where any masks_red[s] is 0, else background[q + (bg_x, bg_y)] (coordinates clamped
+ * to the image, as the composite clamps them).
+ * Frames: n_frames > 0 asks every layer for the frames of steps (as arapb200_batch_submit_seq) and frame_motions
+ * double[n_frames][2][3] gives A_1 .. A_K.  Frame k is arapb200_composite of the layers' frame k with motion_from =
+ * A_{k-1} (A_0 = identity) and motion_to = A_k, and as source masks the input masks for k = 1 and 255 - (the layers'
+ * warped masks of frame k - 1) for k >= 2 (lib.composite_seq).  seq_rgb uint8x3, seq_mask uint8, seq_flow float2,
+ * seq_bflow float2, seq_occ uint8, each [n_frames][W*H][...]; seq_rgb and seq_mask are required with frames, the others
+ * may be NULL.  Steps and motions are copied: they need not outlive the call; every other buffer must stay valid until
+ * the run.
+ * Only the composited outputs (and out_costs) are copied to the host; the scene keeps a device buffer of its own for the
+ * background, frame 0 and 21 B/px per composited frame (the pair and each frame), allocated the first time and grown for
+ * a larger scene.  Its kernels count in arapb200_batch_launches and in the total and warp spans of arapb200_batch_timing.
+ * Returns non-zero, and queues nothing, for: a NULL batch; n_layers outside [1, 32]; slots outside the batch; slots that
+ * belong to another scene queued for the same run; W or H <= 0, or W * H above the batch's maxW * maxH; a NULL rgb,
+ * masks_red, matches or n_matches array, a NULL mask, a negative n_matches[s], or a NULL matches[s] with
+ * n_matches[s] > 0; a NULL background, bgW or bgH <= 0, a NULL motion, a NULL out_flow, out_rgb or out_mask; n_frames
+ * < 0, frame outputs without frames, frames without steps, frame_motions, seq_rgb or seq_mask, a step list that is not
+ * strictly increasing within [0, nCont - 1]; and a non-finite or singular motion (or non-finite derived maps) among
+ * motion and frame_motions.  Until the next arapb200_batch_run, an ordinary submit into a slot of a queued scene is
+ * refused too. */
+ARAPB200_API int arapb200_batch_submit_scene(arapb200_batch* b, int slot, int n_layers, int W, int H, const uint8_t* rgb,
+                                             const uint8_t* const* masks_red, const int32_t* const* matches,
+                                             const int* n_matches, int bgW, int bgH, const uint8_t* background,
+                                             int bg_x, int bg_y, const double* motion, int n_frames, const int* steps,
+                                             const double* frame_motions, float* out_flow, uint8_t* out_rgb,
+                                             uint8_t* out_mask, float* out_bflow, uint8_t* out_occ, uint8_t* out_rgb0,
+                                             float* out_costs, uint8_t* seq_rgb, uint8_t* seq_mask, float* seq_flow,
+                                             float* seq_bflow, uint8_t* seq_occ);
 /* run everything submitted since the last run; returns after all outputs are in host memory */
 ARAPB200_API int arapb200_batch_run(arapb200_batch* b);
-/* device milliseconds of the last run: [0] total, [1] solve kernels only, [2] warp kernels only */
+/* device milliseconds of the last run: [0] total, [1] solve kernels only, [2] warp kernels only (with the scenes'
+ * composite kernels) */
 ARAPB200_API int arapb200_batch_timing(arapb200_batch* b, float* ms3);
-/* number of kernel launches issued by the last run */
+/* number of kernel launches issued by the last run (the scenes' composite kernels included) */
 ARAPB200_API long long arapb200_batch_launches(arapb200_batch* b);
 
 /* how many problems of the last run were solved by the resident (on-chip) back-end; the rest took the streaming one */
