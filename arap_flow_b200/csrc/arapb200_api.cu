@@ -1,6 +1,7 @@
 // arapb200_api.cu -- the flat C ABI of include/arapb200.h (host buffers in, host buffers out).
 #include "../../include/arapb200.h"
 #include "composite.cuh"
+#include "devmem.cuh"
 #include "pipeline.cuh"
 
 #include <cmath>
@@ -13,56 +14,8 @@ using namespace arapb200;
 
 namespace {
 
-template <class T>
-struct DevBuf {
-    T* p = nullptr;
-    size_t n = 0;
-    explicit DevBuf(size_t count) : n(count) { ARAP_CUDA_CHECK(cudaMalloc(&p, (count ? count : 1) * sizeof(T))); }
-    ~DevBuf() { cudaFree(p); }
-    DevBuf(const DevBuf&) = delete;
-    DevBuf& operator=(const DevBuf&) = delete;
-    void up(const T* h, cudaStream_t s = nullptr)
-    {
-        ARAP_CUDA_CHECK(cudaMemcpyAsync(p, h, n * sizeof(T), cudaMemcpyHostToDevice, s));
-    }
-    void down(T* h, cudaStream_t s = nullptr)
-    {
-        ARAP_CUDA_CHECK(cudaMemcpyAsync(h, p, n * sizeof(T), cudaMemcpyDeviceToHost, s));
-    }
-};
-
-// Device workspace of the stand-alone warp calls (warp_image, the Opt.h mirror's copyResultToCPU): grown on demand, kept
-// for the life of the process -- seven cudaMalloc/cudaFree pairs per call cost more than the warp itself (and cudaFree
-// synchronises the device).  One per device; the mutex also serialises concurrent callers on it.
-struct WarpArena {
-    std::mutex mu;
-    unsigned char* base = nullptr;
-    size_t cap = 0;
-    cudaStream_t stream = nullptr;
-    unsigned char* reserve(size_t bytes)
-    {
-        if (bytes > cap) {
-            if (base) ARAP_CUDA_CHECK(cudaFree(base));
-            base = nullptr; cap = 0;
-            ARAP_CUDA_CHECK(cudaMalloc(&base, bytes));
-            cap = bytes;
-        }
-        if (!stream) ARAP_CUDA_CHECK(cudaStreamCreateWithFlags(&stream, cudaStreamNonBlocking));
-        return base;
-    }
-};
-
-WarpArena& warp_arena()
-{
-    static std::mutex table_mu;
-    static WarpArena* table[64] = {};          // never freed: outlives the CUDA context teardown at exit
-    int dev = 0;
-    ARAP_CUDA_CHECK(cudaGetDevice(&dev));
-    if (dev < 0 || dev >= 64) arap_fail(1, "warp: device ordinal %d out of range", dev);
-    std::lock_guard<std::mutex> g(table_mu);
-    if (!table[dev]) table[dev] = new WarpArena;
-    return *table[dev];
-}
+// the stand-alone warp calls (warp_image, the Opt.h mirror's copyResultToCPU), each on its device's non-blocking stream
+WorkspaceTable warp_workspaces;
 
 int warp_common(int W, int H, const float* pos_or_flow, bool is_flow, const uint8_t* rgb, const uint8_t* mask_red,
                 uint8_t* out_rgb, uint8_t* out_mask, uint32_t* out_splat, float* out_bflow = nullptr,
@@ -71,15 +24,15 @@ int warp_common(int W, int H, const float* pos_or_flow, bool is_flow, const uint
     if (W <= 0 || H <= 0 || !pos_or_flow || !rgb || !mask_red || !out_rgb || !out_mask) return 1;
     const size_t N = (size_t)W * H;
     const bool ex = out_bflow || out_occ; // the occlusion needs the backward flow
-    auto up256 = [](size_t b) { return (b + 255) & ~(size_t)255; };
-    const size_t o_in = 0, o_pos = o_in + up256(8 * N), o_z = o_pos + up256(8 * N), o_rgb = o_z + up256(4 * N),
-                 o_orgb = o_rgb + up256(3 * N), o_m = o_orgb + up256(3 * N), o_om = o_m + up256(N),
-                 o_bf = o_om + up256(N), o_fl = o_bf + (ex ? up256(8 * N) : 0), o_occ = o_fl + (out_occ ? up256(8 * N) : 0),
-                 total = o_occ + (out_occ ? up256(N) : 0);
-    WarpArena& ar = warp_arena();
-    std::lock_guard<std::mutex> g(ar.mu);
-    unsigned char* b = ar.reserve(total);
-    cudaStream_t s = ar.stream;
+    Layout l;
+    const size_t o_in = l.take(8 * N), o_pos = l.take(8 * N), o_z = l.take(4 * N), o_rgb = l.take(3 * N),
+                 o_orgb = l.take(3 * N), o_m = l.take(N), o_om = l.take(N), o_bf = l.take(ex ? 8 * N : 0),
+                 o_fl = l.take(out_occ ? 8 * N : 0), o_occ = l.take(out_occ ? N : 0);
+    Workspace& ws = warp_workspaces.current();
+    std::lock_guard<std::mutex> g(ws.mu);
+    unsigned char* b = ws.buf.reserve(l.bytes());
+    if (!ws.stream) ARAP_CUDA_CHECK(cudaStreamCreateWithFlags(&ws.stream, cudaStreamNonBlocking));
+    cudaStream_t s = ws.stream;
     float2* d_in = (float2*)(b + o_in);
     float2* d_pos = (float2*)(b + o_pos);
     unsigned* d_z = (unsigned*)(b + o_z);
@@ -108,23 +61,6 @@ int warp_common(int W, int H, const float* pos_or_flow, bool is_flow, const uint
     if (out_bflow) ARAP_CUDA_CHECK(cudaMemcpyAsync(out_bflow, d_bf, 8 * N, cudaMemcpyDeviceToHost, s));
     ARAP_CUDA_OR_RETURN(cudaStreamSynchronize(s));
     return 0;
-}
-
-// every extern "C" entry point runs its body through this: an ArapError (CUDA failure, watchdog, capacity) becomes the
-// function's non-zero return code instead of taking the host process down
-template <class F>
-int guarded(F&& f)
-{
-    try {
-        return f();
-    } catch (const ArapError& e) {
-        return e.code;
-    } catch (const std::exception& e) {
-        fprintf(stderr, "arapb200: %s\n", e.what());
-        return 2;
-    } catch (...) {
-        return 2;
-    }
 }
 
 } // namespace
@@ -658,25 +594,25 @@ int arapb200_debug_resident_profile_group(int W, int H, const uint8_t* mask_red,
         DevBuf<float> dM(N);
         DevBuf<MatchRec> dm(recs.size());
         DevBuf<unsigned long long> dprof(RS_MAX_CTAS * RS_PROF_SLOTS);
-        std::vector<std::unique_ptr<DevBuf<float2>>> dX, dC;
-        std::vector<std::unique_ptr<DevBuf<float>>> dA, dcost;
+        std::vector<DevBuf<float2>> dX, dC;
+        std::vector<DevBuf<float>> dA, dcost;
         dmask.up(mask_red);
         if (!recs.empty()) dm.up(recs.data());
         ARAP_CUDA_OR_RETURN(cudaMemset(dprof.p, 0, RS_MAX_CTAS * RS_PROF_SLOTS * sizeof(unsigned long long)));
         ResidentSolver rs(W, H, copies);
         for (int i = 0; i < copies; ++i) {
-            dX.emplace_back(new DevBuf<float2>(N));
-            dC.emplace_back(new DevBuf<float2>(N));
-            dA.emplace_back(new DevBuf<float>(N));
-            dcost.emplace_back(new DevBuf<float>((size_t)nCont * (nGN + 1)));
-            enqueue_reset_state(W, H, dmask.p, dX[i]->p, dU.p, dA[i]->p, dM.p, nullptr);
-            enqueue_target_image(W, H, dm.p, (int)recs.size(), dC[i]->p, nullptr);
+            dX.emplace_back(N);
+            dC.emplace_back(N);
+            dA.emplace_back(N);
+            dcost.emplace_back((size_t)nCont * (nGN + 1));
+            enqueue_reset_state(W, H, dmask.p, dX[i].p, dU.p, dA[i].p, dM.p, nullptr);
+            enqueue_target_image(W, H, dm.p, (int)recs.size(), dC[i].p, nullptr);
             rs.prepare_enqueue(i, W, H, dM.p, nullptr);
         }
         ARAP_CUDA_OR_RETURN(cudaDeviceSynchronize());
         for (int i = 0; i < copies; ++i) {
             if (!rs.prepare_finish(i)) return 3;
-            rs.set_problem(i, dX[i]->p, dA[i]->p, dC[i]->p, 1, sqrtf(100.f), sqrtf(0.01f), dcost[i]->p, nullptr);
+            rs.set_problem(i, dX[i].p, dA[i].p, dC[i].p, 1, sqrtf(100.f), sqrtf(0.01f), dcost[i].p, nullptr);
         }
         if (rs.group_size(0, copies) < copies) return 4; // they must share ONE launch
         rs.set_profile(dprof.p);

@@ -13,12 +13,12 @@
 #include "../../include/arapb200.h"
 #include "common.cuh"
 #include "composite.cuh"
+#include "devmem.cuh"
 #include "warp.cuh"
 
 #include <algorithm>
 #include <cmath>
 #include <mutex>
-#include <vector>
 
 namespace arapb200 {
 namespace {
@@ -239,20 +239,6 @@ __global__ void __launch_bounds__(256) k_segment_mask(size_t N, const unsigned c
 
 using namespace arapb200;
 
-namespace {
-struct Scratch { // RAII device allocations of one call
-    std::vector<void*> p;
-    ~Scratch() { for (void* d : p) cudaFree(d); }
-    template <class T> T* get(size_t n)
-    {
-        void* d = nullptr;
-        if (cudaMalloc(&d, (n ? n : 1) * sizeof(T)) != cudaSuccess) return nullptr;
-        p.push_back(d);
-        return (T*)d;
-    }
-};
-} // namespace
-
 extern "C" int arapb200_filter_matches(int W1, int H1, const uint8_t* labels1, int W2, int H2, const uint8_t* labels2,
                                        const int32_t* matches, int n, int32_t* out_matches, uint8_t* out_labels,
                                        int* n_out)
@@ -261,69 +247,43 @@ extern "C" int arapb200_filter_matches(int W1, int H1, const uint8_t* labels1, i
         return 1;
     *n_out = 0;
     if (n == 0) return 0;
-    Scratch s;
-    const size_t N1 = (size_t)W1 * H1, N2 = (size_t)W2 * H2;
-    unsigned char* d_l1 = s.get<unsigned char>(N1);
-    unsigned char* d_l2 = s.get<unsigned char>(N2);
-    int4* d_m = s.get<int4>(n);
-    int4* d_o = s.get<int4>(n);
-    unsigned char* d_lab = s.get<unsigned char>(n);
-    unsigned char* d_ol = s.get<unsigned char>(n);
-    int* d_cnt = s.get<int>(1);
-    if (!d_l1 || !d_l2 || !d_m || !d_o || !d_lab || !d_ol || !d_cnt) return 2;
-    ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(d_l1, labels1, N1, cudaMemcpyHostToDevice, nullptr));
-    ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(d_l2, labels2, N2, cudaMemcpyHostToDevice, nullptr));
-    ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(d_m, matches, (size_t)n * sizeof(int4), cudaMemcpyHostToDevice, nullptr));
-    k_match_valid<<<(n + 255) / 256, 256>>>(n, d_m, W1, H1, d_l1, W2, H2, d_l2, d_lab);
-    k_match_compact<<<1, 1024>>>(n, d_m, d_lab, d_o, d_ol, d_cnt);
-    int cnt = 0;
-    ARAP_CUDA_OR_RETURN(cudaMemcpy(&cnt, d_cnt, sizeof(int), cudaMemcpyDeviceToHost));
-    if (cnt > 0) {
-        ARAP_CUDA_OR_RETURN(cudaMemcpy(out_matches, d_o, (size_t)cnt * sizeof(int4), cudaMemcpyDeviceToHost));
-        if (out_labels) ARAP_CUDA_OR_RETURN(cudaMemcpy(out_labels, d_ol, (size_t)cnt, cudaMemcpyDeviceToHost));
-    }
-    *n_out = cnt;
-    return 0;
+    return guarded([&]() -> int {
+        const size_t N1 = (size_t)W1 * H1, N2 = (size_t)W2 * H2;
+        DevBuf<unsigned char> d_l1(N1), d_l2(N2), d_lab(n), d_ol(n);
+        DevBuf<int4> d_m(n), d_o(n);
+        DevBuf<int> d_cnt(1);
+        d_l1.up(labels1);
+        d_l2.up(labels2);
+        d_m.up((const int4*)matches);
+        k_match_valid<<<(n + 255) / 256, 256>>>(n, d_m.p, W1, H1, d_l1.p, W2, H2, d_l2.p, d_lab.p);
+        k_match_compact<<<1, 1024>>>(n, d_m.p, d_lab.p, d_o.p, d_ol.p, d_cnt.p);
+        int cnt = 0;
+        ARAP_CUDA_CHECK(cudaMemcpy(&cnt, d_cnt.p, sizeof(int), cudaMemcpyDeviceToHost));
+        if (cnt > 0) {
+            ARAP_CUDA_CHECK(cudaMemcpy(out_matches, d_o.p, (size_t)cnt * sizeof(int4), cudaMemcpyDeviceToHost));
+            if (out_labels) ARAP_CUDA_CHECK(cudaMemcpy(out_labels, d_ol.p, (size_t)cnt, cudaMemcpyDeviceToHost));
+        }
+        *n_out = cnt;
+        return 0;
+    });
 }
 
 extern "C" int arapb200_segment_mask(int W, int H, const uint8_t* labels, int segment, uint8_t* out_mask)
 {
     if (W <= 0 || H <= 0 || !labels || !out_mask || segment < 0 || segment > 255) return 1;
-    Scratch s;
-    const size_t N = (size_t)W * H;
-    unsigned char* d_l = s.get<unsigned char>(N);
-    unsigned char* d_o = s.get<unsigned char>(N);
-    if (!d_l || !d_o) return 2;
-    ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(d_l, labels, N, cudaMemcpyHostToDevice, nullptr));
-    k_segment_mask<<<(unsigned)((N + 255) / 256), 256>>>(N, d_l, segment, d_o);
-    ARAP_CUDA_OR_RETURN(cudaMemcpy(out_mask, d_o, N, cudaMemcpyDeviceToHost));
-    return 0;
+    return guarded([&]() -> int {
+        const size_t N = (size_t)W * H;
+        DevBuf<unsigned char> d_l(N), d_o(N);
+        d_l.up(labels);
+        k_segment_mask<<<(unsigned)((N + 255) / 256), 256>>>(N, d_l.p, segment, d_o.p);
+        ARAP_CUDA_CHECK(cudaMemcpy(out_mask, d_o.p, N, cudaMemcpyDeviceToHost));
+        return 0;
+    });
 }
 
 namespace {
-// One grow-only device arena per process, shared by the flatten and the composite (cudaMalloc / cudaFree of 15
-// multi-megabyte blocks per call cost far more than the kernel).  Callers hold arena_mu from arena_reserve until their
-// last copy out of it has returned.
-std::mutex arena_mu;
-unsigned char* arena = nullptr;
-size_t arena_bytes = 0;
-int arena_dev = -1;
-
-size_t al(size_t b) { return (b + 255) & ~(size_t)255; } // every block of the arena is 256-byte aligned
-
-// 0, or 2 on a CUDA failure
-int arena_reserve(size_t need)
-{
-    int dev = 0;
-    if (cudaGetDevice(&dev) != cudaSuccess) return 2;
-    if (need > arena_bytes || dev != arena_dev) {
-        if (arena) { cudaFree(arena); arena = nullptr; arena_bytes = 0; }
-        if (cudaMalloc(&arena, need) != cudaSuccess) return 2;
-        arena_bytes = need;
-        arena_dev = dev;
-    }
-    return 0;
-}
+// the flatten's and the composite's device workspace, used on the legacy default stream with synchronous copies out
+WorkspaceTable composite_workspaces;
 
 int flatten_common(int W, int H, int n_layers, const float* const* flows, const uint8_t* const* rgbs,
                    const uint8_t* const* masks, const uint8_t* background, const uint8_t* const* src_masks,
@@ -335,44 +295,46 @@ int flatten_common(int W, int H, int n_layers, const float* const* flows, const 
     if (out_occ && !src_masks) return 1;
     const bool ex = out_bflow || out_occ;
     const size_t N = (size_t)W * H;
-    Layers L{};
-    L.n = n_layers;
-    // arena: [layers: flow, rgb, mask (, bflow, src mask)][background][outputs]
-    std::lock_guard<std::mutex> lock(arena_mu);
-    const size_t per_layer = al(N * sizeof(float2)) + al(3 * N) + al(N) + (ex ? al(N * sizeof(float2)) + al(N) : 0);
-    const size_t need = (size_t)(n_layers + 1) * per_layer + al(3 * N);
-    int rc = arena_reserve(need);
-    unsigned char* cur = arena;
-    auto take = [&](size_t bytes) { unsigned char* p = cur; cur += al(bytes); return p; };
-    auto up = [&](const void* h, size_t bytes) -> void* {
-        void* d = take(bytes);
-        if (cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, nullptr) != cudaSuccess) rc = 2;
-        return d;
-    };
-    for (int s = 0; s < n_layers && !rc; ++s) {
-        L.flow[s] = (const float2*)up(flows[s], N * sizeof(float2));
-        L.rgb[s] = (const unsigned char*)up(rgbs[s], 3 * N);
-        L.mask[s] = (const unsigned char*)up(masks[s], N);
-        if (ex) L.bflow[s] = (const float2*)up(bflows[s], N * sizeof(float2));
-        if (out_occ) L.src[s] = (const unsigned char*)up(src_masks[s], N);
+    // workspace: [layers: flow, rgb, mask (, bflow)(, src mask)][background][outputs: flow, rgb, mask (, bflow)(, occ)]
+    struct { size_t flow, rgb, mask, bflow, src; } in[MAX_LAYERS];
+    Layout l;
+    for (int s = 0; s < n_layers; ++s) {
+        in[s].flow = l.take(8 * N);
+        in[s].rgb = l.take(3 * N);
+        in[s].mask = l.take(N);
+        in[s].bflow = l.take(ex ? 8 * N : 0);
+        in[s].src = l.take(out_occ ? N : 0);
     }
-    const unsigned char* d_bg = nullptr;
-    if (!rc && background) d_bg = (const unsigned char*)up(background, 3 * N);
-    if (!rc) {
-        float2* d_of = (float2*)take(N * sizeof(float2));
-        unsigned char* d_or = take(3 * N);
-        unsigned char* d_om = take(N);
-        float2* d_ob = out_bflow ? (float2*)take(N * sizeof(float2)) : nullptr;
-        unsigned char* d_oo = out_occ ? take(N) : nullptr;
-        k_flatten<<<(unsigned)((N + 255) / 256), 256>>>(W, H, L, d_bg, d_of, d_or, d_om, d_ob, d_oo);
-        if (cudaMemcpy(out_flow, d_of, N * sizeof(float2), cudaMemcpyDeviceToHost) ||
-            cudaMemcpy(out_rgb, d_or, 3 * N, cudaMemcpyDeviceToHost) || cudaMemcpy(out_mask, d_om, N, cudaMemcpyDeviceToHost) ||
-            (d_ob && cudaMemcpy(out_bflow, d_ob, N * sizeof(float2), cudaMemcpyDeviceToHost)) ||
-            (d_oo && cudaMemcpy(out_occ, d_oo, N, cudaMemcpyDeviceToHost)))
-            rc = 3;
-    }
-    if (rc) fprintf(stderr, "arapb200_flatten: CUDA failure (%s)\n", cudaGetErrorString(cudaGetLastError()));
-    return rc;
+    const size_t o_bg = l.take(background ? 3 * N : 0), o_flow = l.take(8 * N), o_rgb = l.take(3 * N),
+                 o_mask = l.take(N), o_bflow = l.take(out_bflow ? 8 * N : 0), o_occ = l.take(out_occ ? N : 0);
+    return guarded([&]() -> int {
+        Workspace& ws = composite_workspaces.current();
+        std::lock_guard<std::mutex> lock(ws.mu);
+        unsigned char* b = ws.buf.reserve(l.bytes());
+        auto up = [&](size_t at, const void* h, size_t bytes) {
+            ARAP_CUDA_CHECK(cudaMemcpyAsync(b + at, h, bytes, cudaMemcpyHostToDevice, nullptr));
+            return b + at;
+        };
+        Layers L{};
+        L.n = n_layers;
+        for (int s = 0; s < n_layers; ++s) {
+            L.flow[s] = (const float2*)up(in[s].flow, flows[s], 8 * N);
+            L.rgb[s] = up(in[s].rgb, rgbs[s], 3 * N);
+            L.mask[s] = up(in[s].mask, masks[s], N);
+            if (ex) L.bflow[s] = (const float2*)up(in[s].bflow, bflows[s], 8 * N);
+            if (out_occ) L.src[s] = up(in[s].src, src_masks[s], N);
+        }
+        const unsigned char* d_bg = background ? up(o_bg, background, 3 * N) : nullptr;
+        k_flatten<<<(unsigned)((N + 255) / 256), 256>>>(W, H, L, d_bg, (float2*)(b + o_flow), b + o_rgb, b + o_mask,
+                                                         out_bflow ? (float2*)(b + o_bflow) : nullptr,
+                                                         out_occ ? b + o_occ : nullptr);
+        ARAP_CUDA_CHECK(cudaMemcpy(out_flow, b + o_flow, 8 * N, cudaMemcpyDeviceToHost));
+        ARAP_CUDA_CHECK(cudaMemcpy(out_rgb, b + o_rgb, 3 * N, cudaMemcpyDeviceToHost));
+        ARAP_CUDA_CHECK(cudaMemcpy(out_mask, b + o_mask, N, cudaMemcpyDeviceToHost));
+        if (out_bflow) ARAP_CUDA_CHECK(cudaMemcpy(out_bflow, b + o_bflow, 8 * N, cudaMemcpyDeviceToHost));
+        if (out_occ) ARAP_CUDA_CHECK(cudaMemcpy(out_occ, b + o_occ, N, cudaMemcpyDeviceToHost));
+        return 0;
+    });
 }
 } // namespace
 
@@ -510,42 +472,44 @@ extern "C" int arapb200_composite(int W, int H, int n_layers, const float* const
     if (out_coeffs) std::copy(cf, cf + 18, out_coeffs);
 
     const size_t N = (size_t)W * H, NB = (size_t)bgW * bgH;
-    Layers L{};
-    L.n = n_layers;
-    // arena: [layers: flow, rgb, mask, src mask (, bflow)][background][outputs: flow, rgb, mask (, bflow)(, occ)]
-    std::lock_guard<std::mutex> lock(arena_mu);
-    const size_t per_layer = al(N * sizeof(float2)) + al(3 * N) + 2 * al(N) + (ex ? al(N * sizeof(float2)) : 0);
-    const size_t need = (size_t)n_layers * per_layer + al(3 * NB) + al(N * sizeof(float2)) + al(3 * N) + al(N) +
-                        (ex ? al(N * sizeof(float2)) : 0) + (out_occ ? al(N) : 0);
-    int rc = arena_reserve(need);
-    unsigned char* cur = arena;
-    auto take = [&](size_t bytes) { unsigned char* p = cur; cur += al(bytes); return p; };
-    auto up = [&](const void* h, size_t bytes) -> void* {
-        void* d = take(bytes);
-        if (cudaMemcpyAsync(d, h, bytes, cudaMemcpyHostToDevice, nullptr) != cudaSuccess) rc = 2;
-        return d;
-    };
-    for (int s = 0; s < n_layers && !rc; ++s) {
-        L.flow[s] = (const float2*)up(flows[s], N * sizeof(float2));
-        L.rgb[s] = (const unsigned char*)up(rgbs[s], 3 * N);
-        L.mask[s] = (const unsigned char*)up(masks[s], N);
-        L.src[s] = (const unsigned char*)up(src_masks[s], N);
-        if (ex) L.bflow[s] = (const float2*)up(bflows[s], N * sizeof(float2));
+    // workspace: [layers: flow, rgb, mask, src mask (, bflow)][background][outputs: flow, rgb, mask (, bflow)(, occ)];
+    // out_occ reads the whole frame-b bflow, so it has a block whenever either extra is asked for
+    struct { size_t flow, rgb, mask, src, bflow; } in[MAX_LAYERS];
+    Layout l;
+    for (int s = 0; s < n_layers; ++s) {
+        in[s].flow = l.take(8 * N);
+        in[s].rgb = l.take(3 * N);
+        in[s].mask = l.take(N);
+        in[s].src = l.take(N);
+        in[s].bflow = l.take(ex ? 8 * N : 0);
     }
-    const unsigned char* d_bg = rc ? nullptr : (const unsigned char*)up(background, 3 * NB);
-    if (!rc) {
-        float2* d_of = (float2*)take(N * sizeof(float2));
-        unsigned char* d_or = take(3 * N);
-        unsigned char* d_om = take(N);
-        float2* d_ob = ex ? (float2*)take(N * sizeof(float2)) : nullptr; // out_occ reads the whole frame-b bflow
-        unsigned char* d_oo = out_occ ? take(N) : nullptr;
-        enqueue_composite(W, H, L, false, d_bg, bgW, bgH, bg_x, bg_y, cf, d_of, d_or, d_om, d_ob, d_oo, nullptr);
-        if (cudaMemcpy(out_flow, d_of, N * sizeof(float2), cudaMemcpyDeviceToHost) ||
-            cudaMemcpy(out_rgb, d_or, 3 * N, cudaMemcpyDeviceToHost) || cudaMemcpy(out_mask, d_om, N, cudaMemcpyDeviceToHost) ||
-            (out_bflow && cudaMemcpy(out_bflow, d_ob, N * sizeof(float2), cudaMemcpyDeviceToHost)) ||
-            (d_oo && cudaMemcpy(out_occ, d_oo, N, cudaMemcpyDeviceToHost)))
-            rc = 3;
-    }
-    if (rc) fprintf(stderr, "arapb200_composite: CUDA failure (%s)\n", cudaGetErrorString(cudaGetLastError()));
-    return rc;
+    const size_t o_bg = l.take(3 * NB), o_flow = l.take(8 * N), o_rgb = l.take(3 * N), o_mask = l.take(N),
+                 o_bflow = l.take(ex ? 8 * N : 0), o_occ = l.take(out_occ ? N : 0);
+    return guarded([&]() -> int {
+        Workspace& ws = composite_workspaces.current();
+        std::lock_guard<std::mutex> lock(ws.mu);
+        unsigned char* b = ws.buf.reserve(l.bytes());
+        auto up = [&](size_t at, const void* h, size_t bytes) {
+            ARAP_CUDA_CHECK(cudaMemcpyAsync(b + at, h, bytes, cudaMemcpyHostToDevice, nullptr));
+            return b + at;
+        };
+        Layers L{};
+        L.n = n_layers;
+        for (int s = 0; s < n_layers; ++s) {
+            L.flow[s] = (const float2*)up(in[s].flow, flows[s], 8 * N);
+            L.rgb[s] = up(in[s].rgb, rgbs[s], 3 * N);
+            L.mask[s] = up(in[s].mask, masks[s], N);
+            L.src[s] = up(in[s].src, src_masks[s], N);
+            if (ex) L.bflow[s] = (const float2*)up(in[s].bflow, bflows[s], 8 * N);
+        }
+        const unsigned char* d_bg = up(o_bg, background, 3 * NB);
+        enqueue_composite(W, H, L, false, d_bg, bgW, bgH, bg_x, bg_y, cf, (float2*)(b + o_flow), b + o_rgb, b + o_mask,
+                          ex ? (float2*)(b + o_bflow) : nullptr, out_occ ? b + o_occ : nullptr, nullptr);
+        ARAP_CUDA_CHECK(cudaMemcpy(out_flow, b + o_flow, 8 * N, cudaMemcpyDeviceToHost));
+        ARAP_CUDA_CHECK(cudaMemcpy(out_rgb, b + o_rgb, 3 * N, cudaMemcpyDeviceToHost));
+        ARAP_CUDA_CHECK(cudaMemcpy(out_mask, b + o_mask, N, cudaMemcpyDeviceToHost));
+        if (out_bflow) ARAP_CUDA_CHECK(cudaMemcpy(out_bflow, b + o_bflow, 8 * N, cudaMemcpyDeviceToHost));
+        if (out_occ) ARAP_CUDA_CHECK(cudaMemcpy(out_occ, b + o_occ, N, cudaMemcpyDeviceToHost));
+        return 0;
+    });
 }

@@ -1,5 +1,5 @@
 // composite.cuh -- the layer composite over a moving background (composite.cu, DESIGN.md 4.5), enqueue-only, for the
-// callers that hold the layers on the device: arapb200_composite (the arena) and the batch's scenes (DESIGN.md 4.6).
+// callers that hold the layers on the device: arapb200_composite (its workspace) and the batch's scenes (DESIGN.md 4.6).
 #pragma once
 #include "common.cuh"
 

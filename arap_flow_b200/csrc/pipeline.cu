@@ -92,18 +92,18 @@ __global__ void k_copy_cost(const StreamScalars* __restrict__ sc, float* __restr
 // frames 1 .. K, so that each frame output leaves in one copy
 struct SceneLayout {
     size_t bg, rgb0, flow, rgb, mask, bflow, occ, bytes;
-    SceneLayout(const HostScene& sc)
+    explicit SceneLayout(const HostScene& sc)
     {
-        auto al = [](size_t b) { return (b + 255) & ~(size_t)255; };
         const size_t N = (size_t)sc.W * sc.H, F = N * (sc.maps.size() / 18);
-        bg = 0;
-        rgb0 = bg + al(3 * (size_t)sc.bgW * sc.bgH);
-        flow = rgb0 + (sc.out_rgb0 ? al(3 * N) : 0);
-        rgb = flow + al(8 * F);
-        mask = rgb + al(3 * F);
-        bflow = mask + al(F);
-        occ = bflow + al(8 * F);
-        bytes = occ + al(F);
+        Layout l;
+        bg = l.take(3 * (size_t)sc.bgW * sc.bgH);
+        rgb0 = l.take(sc.out_rgb0 ? 3 * N : 0);
+        flow = l.take(8 * F);
+        rgb = l.take(3 * F);
+        mask = l.take(F);
+        bflow = l.take(8 * F);
+        occ = l.take(F);
+        bytes = l.bytes();
     }
 };
 
@@ -140,20 +140,20 @@ BatchPipeline::BatchPipeline(int maxW, int maxH, int max_problems, int nCont, in
     dev_.resize(max_problems > 0 ? max_problems : 1);
     const size_t cbytes = (size_t)nCont * (nGN + 1) * sizeof(float);
     for (Dev& d : dev_) {
-        ARAP_CUDA_CHECK(cudaMalloc(&d.X, N * sizeof(float2)));
-        ARAP_CUDA_CHECK(cudaMalloc(&d.U, N * sizeof(float2)));
-        ARAP_CUDA_CHECK(cudaMalloc(&d.C, N * sizeof(float2)));
-        ARAP_CUDA_CHECK(cudaMalloc(&d.flow, N * sizeof(float2)));
-        ARAP_CUDA_CHECK(cudaMalloc(&d.A, N * sizeof(float)));
-        ARAP_CUDA_CHECK(cudaMalloc(&d.M, N * sizeof(float)));
-        ARAP_CUDA_CHECK(cudaMalloc(&d.costs, cbytes));
-        ARAP_CUDA_CHECK(cudaMalloc(&d.rgb, 3 * N));
-        ARAP_CUDA_CHECK(cudaMalloc(&d.mask, N));
-        ARAP_CUDA_CHECK(cudaMalloc(&d.orgb, 3 * N));
-        ARAP_CUDA_CHECK(cudaMalloc(&d.omask, N));
-        ARAP_CUDA_CHECK(cudaMalloc(&d.z, N * sizeof(unsigned)));
-        ARAP_CUDA_CHECK(cudaMallocHost(&d.h_in, 4 * N));
-        ARAP_CUDA_CHECK(cudaMallocHost(&d.h_out, 12 * N + cbytes));
+        d.X = DevBuf<float2>(N);
+        d.U = DevBuf<float2>(N);
+        d.C = DevBuf<float2>(N);
+        d.flow = DevBuf<float2>(N);
+        d.A = DevBuf<float>(N);
+        d.M = DevBuf<float>(N);
+        d.costs = DevBuf<float>((size_t)nCont * (nGN + 1));
+        d.rgb = DevBuf<unsigned char>(3 * N);
+        d.mask = DevBuf<unsigned char>(N);
+        d.orgb = DevBuf<unsigned char>(3 * N);
+        d.omask = DevBuf<unsigned char>(N);
+        d.z = DevBuf<unsigned>(N);
+        d.h_in.reserve(4 * N);
+        d.h_out.reserve(12 * N + cbytes);
     }
     if (backend_ != ARAPB200_BACKEND_STREAM) resident_ = new ResidentSolver(maxW, maxH, (int)dev_.size());
 }
@@ -164,23 +164,8 @@ BatchPipeline::~BatchPipeline()
     delete solver_;
     delete resident_;
     delete lm_;
-    for (Dev& d : dev_) {
-        cudaFree(d.X); cudaFree(d.U); cudaFree(d.C); cudaFree(d.flow); cudaFree(d.A); cudaFree(d.M);
-        cudaFree(d.costs); cudaFree(d.rgb); cudaFree(d.mask); cudaFree(d.orgb); cudaFree(d.omask);
-        cudaFree(d.z); cudaFree(d.matches); cudaFree(d.bflow); cudaFree(d.occ);
-        cudaFreeHost(d.h_in); cudaFreeHost(d.h_out); cudaFreeHost(d.h_extra);
-        free_seq(d);
-    }
-    for (SceneDev& sd : scene_dev_) cudaFree(sd.buf);
     for (auto& e : ev_) cudaEventDestroy(e);
     cudaStreamDestroy(stream_);
-}
-
-void BatchPipeline::free_seq(Dev& d)
-{
-    cudaFree(d.seq_pos); cudaFree(d.seq_z); cudaFree(d.seq.rgb); cudaFree(d.seq.mask); cudaFree(d.seq.flow);
-    cudaFree(d.seq.bflow); cudaFree(d.seq.occ); cudaFree(d.seq.flow0);
-    d.seq_pos = nullptr; d.seq_z = nullptr; d.seq = SeqOut{}; d.seq_cap = 0;
 }
 
 void BatchPipeline::snapshot(const HostProblem& hp, Dev& d, int t)
@@ -188,7 +173,7 @@ void BatchPipeline::snapshot(const HostProblem& hp, Dev& d, int t)
     const auto it = std::lower_bound(hp.steps.begin(), hp.steps.end(), t);
     if (it == hp.steps.end() || *it != t) return;
     const size_t N = (size_t)hp.W * hp.H;
-    ARAP_CUDA_CHECK(cudaMemcpyAsync(d.seq_pos + (size_t)(it - hp.steps.begin()) * N, d.X, N * sizeof(float2),
+    ARAP_CUDA_CHECK(cudaMemcpyAsync(d.seq_pos + (size_t)(it - hp.steps.begin()) * N, d.X.p, N * sizeof(float2),
                                     cudaMemcpyDeviceToDevice, stream_));
 }
 
@@ -207,16 +192,16 @@ void BatchPipeline::solve_streaming(const HostProblem& hp, Dev& d)
     const float wf = sqrtf(100.0f), wr = sqrtf(0.01f); // CombinedSolver.h:172-177
     solver_->set_pcg_rtol(pcg_rtol_);
     solver_->set_gn_rtol(gn_rtol_);
-    solver_->bind(d.X, d.A, d.U, d.C, d.M, wf, wr, stream_);
+    solver_->bind(d.X.p, d.A.p, d.U.p, d.C.p, d.M.p, wf, wr, stream_);
     for (int t = 0; t < nCont_; ++t) {
         const float alpha = (float)(t + 1) / (float)nCont_; // CombinedSolver.h:199-201
-        enqueue_constraint_image(W, H, d.matches, (int)d.recs.size(), alpha, d.C, stream_);
+        enqueue_constraint_image(W, H, d.recs_dev(), (int)d.recs.size(), alpha, d.C.p, stream_);
         launches_ += d.recs.empty() ? 1 : 2;
         solver_->enqueue_init(stream_);
-        k_copy_cost<<<1, 1, 0, stream_>>>(solver_->d_scalars(), d.costs + (size_t)t * (nGN_ + 1));
+        k_copy_cost<<<1, 1, 0, stream_>>>(solver_->d_scalars(), d.costs.p + (size_t)t * (nGN_ + 1));
         for (int g = 0; g < nGN_; ++g) {
             solver_->enqueue_gn_step(nPCG_, stream_);
-            k_copy_cost<<<1, 1, 0, stream_>>>(solver_->d_scalars(), d.costs + (size_t)t * (nGN_ + 1) + g + 1);
+            k_copy_cost<<<1, 1, 0, stream_>>>(solver_->d_scalars(), d.costs.p + (size_t)t * (nGN_ + 1) + g + 1);
         }
         launches_ += 1 + nGN_;
         snapshot(hp, d, t);
@@ -240,11 +225,11 @@ void BatchPipeline::solve_lm(const HostProblem& hp, Dev& d)
     }
     const long long l0 = lm_->launches();
     const float wf = sqrtf(100.0f), wr = sqrtf(0.01f); // CombinedSolver.h:172-177
-    lm_->bind(d.X, d.A, d.U, d.C, d.M, wf, wr);
+    lm_->bind(d.X.p, d.A.p, d.U.p, d.C.p, d.M.p, wf, wr);
     lm_costs_.assign((size_t)nCont_ * (nGN_ + 1), 0.0f);
     for (int t = 0; t < nCont_; ++t) {
         const float alpha = (float)(t + 1) / (float)nCont_; // CombinedSolver.h:199-201
-        enqueue_constraint_image(W, H, d.matches, (int)d.recs.size(), alpha, d.C, stream_);
+        enqueue_constraint_image(W, H, d.recs_dev(), (int)d.recs.size(), alpha, d.C.p, stream_);
         launches_ += d.recs.empty() ? 1 : 2;
         float* c = lm_costs_.data() + (size_t)t * (nGN_ + 1);
         float prev = lm_->init(stream_);
@@ -258,7 +243,7 @@ void BatchPipeline::solve_lm(const HostProblem& hp, Dev& d)
         for (int k = g + 1; k <= nGN_; ++k) c[k] = prev;
         snapshot(hp, d, t);
     }
-    ARAP_CUDA_CHECK(cudaMemcpyAsync(d.costs, lm_costs_.data(), lm_costs_.size() * sizeof(float), cudaMemcpyHostToDevice, stream_));
+    ARAP_CUDA_CHECK(cudaMemcpyAsync(d.costs.p, lm_costs_.data(), lm_costs_.size() * sizeof(float), cudaMemcpyHostToDevice, stream_));
     ARAP_CUDA_CHECK(cudaStreamSynchronize(stream_)); // lm_costs_ is reused by the next problem
     launches_ += lm_->launches() - l0;
 }
@@ -272,9 +257,9 @@ void BatchPipeline::solve_resident(const HostProblem* problems, int first, int c
         for (int j = 0; j < count; ++j) {
             Dev& dj = dev_[first + j];
             const HostProblem& hp = problems[first + j];
-            enqueue_target_image(hp.W, hp.H, dj.matches, (int)dj.recs.size(), dj.C, stream_);
+            enqueue_target_image(hp.W, hp.H, dj.recs_dev(), (int)dj.recs.size(), dj.C.p, stream_);
             launches_ += dj.recs.empty() ? 1 : 2;
-            resident_->set_problem(first + j, dj.X, dj.A, dj.C, 1, wf, wr, dj.costs, nullptr);
+            resident_->set_problem(first + j, dj.X.p, dj.A.p, dj.C.p, 1, wf, wr, dj.costs.p, nullptr);
         }
         if (cluster) resident_->enqueue_cluster(first, count, nCont_, nGN_, nPCG_, stream_);
         else resident_->enqueue_group(first, count, nCont_, nGN_, nPCG_, stream_);
@@ -287,9 +272,10 @@ void BatchPipeline::solve_resident(const HostProblem* problems, int first, int c
         for (int j = 0; j < count; ++j) {
             Dev& dj = dev_[first + j];
             const HostProblem& hp = problems[first + j];
-            enqueue_constraint_image(hp.W, hp.H, dj.matches, (int)dj.recs.size(), alpha, dj.C, stream_);
+            enqueue_constraint_image(hp.W, hp.H, dj.recs_dev(), (int)dj.recs.size(), alpha, dj.C.p, stream_);
             launches_ += dj.recs.empty() ? 1 : 2;
-            resident_->set_problem(first + j, dj.X, dj.A, dj.C, 0, wf, wr, dj.costs + (size_t)t * (nGN_ + 1), nullptr);
+            resident_->set_problem(first + j, dj.X.p, dj.A.p, dj.C.p, 0, wf, wr, dj.costs.p + (size_t)t * (nGN_ + 1),
+                                   nullptr);
         }
         if (cluster) resident_->enqueue_cluster(first, count, 1, nGN_, nPCG_, stream_);
         else resident_->enqueue_group(first, count, 1, nGN_, nPCG_, stream_);
@@ -309,14 +295,15 @@ void BatchPipeline::enqueue_scene(const HostScene& sc, unsigned char* buf)
     L.n = sc.n;
     for (int s = 0; s < sc.n; ++s) {
         const Dev& d = dev_[sc.first + s];
-        L.flow[s] = d.flow;
-        L.rgb[s] = d.orgb;
-        L.mask[s] = d.omask;
+        L.flow[s] = d.flow.p;
+        L.rgb[s] = d.orgb.p;
+        L.mask[s] = d.omask.p;
         L.bflow[s] = d.bflow;
-        L.src[s] = d.mask;
+        L.src[s] = d.mask.p;
     }
     if (sc.out_rgb0) {
-        enqueue_scene_input(sc.W, sc.H, L, dev_[sc.first].rgb, bg, sc.bgW, sc.bgH, sc.bg_x, sc.bg_y, buf + o.rgb0, stream_);
+        enqueue_scene_input(sc.W, sc.H, L, dev_[sc.first].rgb.p, bg, sc.bgW, sc.bgH, sc.bg_x, sc.bg_y, buf + o.rgb0,
+                            stream_);
         launches_ += 1;
     }
     for (int k = 0; k <= K; ++k) {
@@ -328,7 +315,7 @@ void BatchPipeline::enqueue_scene(const HostScene& sc, unsigned char* buf)
                 L.rgb[s] = q.rgb + 3 * f;
                 L.mask[s] = q.mask + f;
                 L.bflow[s] = q.bflow + f;
-                L.src[s] = k == 1 ? dev_[sc.first + s].mask : q.mask + f - N;
+                L.src[s] = k == 1 ? dev_[sc.first + s].mask.p : q.mask + f - N;
             }
         const size_t f = (size_t)k * N;
         enqueue_composite(sc.W, sc.H, L, k >= 2, bg, sc.bgW, sc.bgH, sc.bg_x, sc.bg_y, sc.maps.data() + 18 * k,
@@ -359,6 +346,9 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
     }
     const size_t cbytes = (size_t)nCont_ * (nGN_ + 1) * sizeof(float);
     const long long r0 = resident_ ? resident_->launches() : 0;
+    const size_t Nmax = (size_t)maxW_ * maxH_;
+    Layout xl; // a slot's opt-in extras, on the device and in pinned staging: [bflow | occ] of maxW x maxH
+    const size_t x_bflow = xl.take(8 * Nmax), x_occ = xl.take(Nmax);
     // ---- stage + upload every problem, reset its state (resetGPU), build its strip tables ----
     for (int i = 0; i < count; ++i) {
         const HostProblem& hp = problems[i];
@@ -369,68 +359,52 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
         }
         const size_t N = (size_t)hp.W * hp.H;
         build_match_records(hp.W, hp.H, hp.mask_red, hp.matches, hp.n_matches, d.recs);
-        if (d.recs.size() > d.matches_cap) {
-            cudaFree(d.matches);
-            d.matches_cap = d.recs.size() * 2 + 1024;
-            ARAP_CUDA_OR_RETURN(cudaMalloc(&d.matches, d.matches_cap * sizeof(MatchRec)));
+        if (d.recs.size() * sizeof(MatchRec) > d.matches.capacity())
+            d.matches.reserve((d.recs.size() * 2 + 1024) * sizeof(MatchRec));
+        if (hp.out_bflow || hp.out_occ || hp.scene) {
+            unsigned char* x = d.extras.reserve(xl.bytes());
+            d.bflow = (float2*)(x + x_bflow);
+            d.occ = x + x_occ;
         }
-        const size_t Nmax = (size_t)maxW_ * maxH_;
-        if ((hp.out_bflow || hp.out_occ || hp.scene) && !d.bflow) {
-            ARAP_CUDA_OR_RETURN(cudaMalloc(&d.bflow, Nmax * sizeof(float2)));
-            ARAP_CUDA_OR_RETURN(cudaMalloc(&d.occ, Nmax));
+        if (hp.out_bflow || hp.out_occ) d.h_extras.reserve(xl.bytes());
+        if (!hp.steps.empty()) { // [pos][z][rgb][mask][flow][bflow][occ][flow0]: z two z-buffers, the rest K frames each
+            const size_t F = Nmax * hp.steps.size();
+            Layout l;
+            const size_t pos = l.take(8 * F), z = l.take(2 * 4 * Nmax), rgb = l.take(3 * F), mask = l.take(F),
+                         flow = l.take(8 * F), bflow = l.take(8 * F), occ = l.take(F), flow0 = l.take(8 * F);
+            unsigned char* f = d.frames.reserve(l.bytes());
+            d.seq_pos = (float2*)(f + pos);
+            d.seq_z = (unsigned*)(f + z);
+            d.seq = SeqOut{f + rgb, f + mask, (float2*)(f + flow), (float2*)(f + bflow), f + occ, (float2*)(f + flow0)};
         }
-        if ((hp.out_bflow || hp.out_occ) && !d.h_extra) ARAP_CUDA_OR_RETURN(cudaMallocHost(&d.h_extra, 9 * Nmax));
-        if ((int)hp.steps.size() > d.seq_cap) {
-            free_seq(d);
-            const size_t F = (size_t)maxW_ * maxH_ * hp.steps.size(); // pixels of all frames
-            ARAP_CUDA_OR_RETURN(cudaMalloc(&d.seq_pos, F * sizeof(float2)));
-            ARAP_CUDA_OR_RETURN(cudaMalloc(&d.seq_z, 2 * (size_t)maxW_ * maxH_ * sizeof(unsigned)));
-            ARAP_CUDA_OR_RETURN(cudaMalloc(&d.seq.rgb, 3 * F));
-            ARAP_CUDA_OR_RETURN(cudaMalloc(&d.seq.mask, F));
-            ARAP_CUDA_OR_RETURN(cudaMalloc(&d.seq.flow, F * sizeof(float2)));
-            ARAP_CUDA_OR_RETURN(cudaMalloc(&d.seq.bflow, F * sizeof(float2)));
-            ARAP_CUDA_OR_RETURN(cudaMalloc(&d.seq.occ, F));
-            ARAP_CUDA_OR_RETURN(cudaMalloc(&d.seq.flow0, F * sizeof(float2)));
-            d.seq_cap = (int)hp.steps.size();
-        }
-        memcpy(d.h_in, hp.rgb, 3 * N);
-        memcpy(d.h_in + 3 * N, hp.mask_red, N);
+        memcpy(d.h_in.data(), hp.rgb, 3 * N);
+        memcpy(d.h_in.data() + 3 * N, hp.mask_red, N);
     }
     if (n_scenes > (int)scene_dev_.size()) scene_dev_.resize(n_scenes);
-    for (int j = 0; j < n_scenes; ++j) {
-        SceneDev& sd = scene_dev_[j];
-        const size_t need = SceneLayout(scenes[j]).bytes;
-        if (need > sd.cap) {
-            ARAP_CUDA_OR_RETURN(cudaFree(sd.buf));
-            sd.buf = nullptr;
-            sd.cap = 0;
-            ARAP_CUDA_OR_RETURN(cudaMalloc(&sd.buf, need));
-            sd.cap = need;
-        }
-    }
-    ARAP_CUDA_OR_RETURN(cudaEventRecord(ev_[0], stream_));
+    for (int j = 0; j < n_scenes; ++j) scene_dev_[j].reserve(SceneLayout(scenes[j]).bytes);
+    ARAP_CUDA_CHECK(cudaEventRecord(ev_[0], stream_));
     for (int i = 0; i < count; ++i) {
         const HostProblem& hp = problems[i];
         Dev& d = dev_[i];
         const size_t N = (size_t)hp.W * hp.H;
-        ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(d.rgb, d.h_in, 3 * N, cudaMemcpyHostToDevice, stream_));
-        ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(d.mask, d.h_in + 3 * N, N, cudaMemcpyHostToDevice, stream_));
+        ARAP_CUDA_CHECK(cudaMemcpyAsync(d.rgb.p, d.h_in.data(), 3 * N, cudaMemcpyHostToDevice, stream_));
+        ARAP_CUDA_CHECK(cudaMemcpyAsync(d.mask.p, d.h_in.data() + 3 * N, N, cudaMemcpyHostToDevice, stream_));
         if (!d.recs.empty())
-            ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(d.matches, d.recs.data(), d.recs.size() * sizeof(MatchRec),
-                                                cudaMemcpyHostToDevice, stream_));
-        enqueue_reset_state(hp.W, hp.H, d.mask, d.X, d.U, d.A, d.M, stream_);
+            ARAP_CUDA_CHECK(cudaMemcpyAsync(d.matches.data(), d.recs.data(), d.recs.size() * sizeof(MatchRec),
+                                            cudaMemcpyHostToDevice, stream_));
+        enqueue_reset_state(hp.W, hp.H, d.mask.p, d.X.p, d.U.p, d.A.p, d.M.p, stream_);
         launches_ += 1;
         d.resident = false;
-        if (resident_ && !lm_on_) resident_->prepare_enqueue(i, hp.W, hp.H, d.M, stream_);
+        if (resident_ && !lm_on_) resident_->prepare_enqueue(i, hp.W, hp.H, d.M.p, stream_);
     }
     for (int j = 0; j < n_scenes; ++j) {
         const HostScene& sc = scenes[j];
-        ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(scene_dev_[j].buf, sc.background, 3 * (size_t)sc.bgW * sc.bgH,
-                                            cudaMemcpyHostToDevice, stream_));
+        ARAP_CUDA_CHECK(cudaMemcpyAsync(scene_dev_[j].data(), sc.background, 3 * (size_t)sc.bgW * sc.bgH,
+                                        cudaMemcpyHostToDevice, stream_));
     }
     n_resident_ = 0;
     if (resident_ && !lm_on_) {
-        ARAP_CUDA_OR_RETURN(cudaStreamSynchronize(stream_)); // strip counts are needed to size the launches
+        ARAP_CUDA_CHECK(cudaStreamSynchronize(stream_)); // strip counts are needed to size the launches
         for (int i = 0; i < count; ++i) {
             dev_[i].resident = resident_->prepare_finish(i);
             if (!dev_[i].resident && backend_ == ARAPB200_BACKEND_RESIDENT) {
@@ -441,7 +415,7 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
             n_resident_ += dev_[i].resident ? 1 : 0;
         }
     }
-    ARAP_CUDA_OR_RETURN(cudaEventRecord(ev_[1], stream_));
+    ARAP_CUDA_CHECK(cudaEventRecord(ev_[1], stream_));
     // ---- solve.  Resident problems: whole continuation schedules, several problems per cooperative launch ----
     group_size_ = 0;
     for (int i = 0; i < count;) {
@@ -478,39 +452,42 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
         if (gsz > group_size_) group_size_ = gsz;
         i += gsz;
     }
-    ARAP_CUDA_OR_RETURN(cudaEventRecord(ev_[2], stream_));
+    ARAP_CUDA_CHECK(cudaEventRecord(ev_[2], stream_));
     // ---- flow extraction + forward warp + download ----
     for (int i = 0; i < count; ++i) {
         const HostProblem& hp = problems[i];
         Dev& d = dev_[i];
-        enqueue_pos_to_flow(hp.W, hp.H, d.X, d.flow, stream_);
+        enqueue_pos_to_flow(hp.W, hp.H, d.X.p, d.flow.p, stream_);
         const bool extras = hp.out_bflow || hp.out_occ || hp.scene;
-        enqueue_warp(hp.W, hp.H, d.X, d.rgb, d.mask, d.z, d.orgb, d.omask, stream_, extras ? d.bflow : nullptr);
+        enqueue_warp(hp.W, hp.H, d.X.p, d.rgb.p, d.mask.p, d.z.p, d.orgb.p, d.omask.p, stream_,
+                     extras ? d.bflow : nullptr);
         launches_ += 1 + warp_launches_per_call();
         if (extras) {
-            enqueue_occlusion(hp.W, hp.H, d.mask, d.flow, d.z, d.bflow, d.occ, stream_);
+            enqueue_occlusion(hp.W, hp.H, d.mask.p, d.flow.p, d.z.p, d.bflow, d.occ, stream_);
             launches_ += 1;
         }
         if (!hp.steps.empty())
-            launches_ += enqueue_warp_seq(hp.W, hp.H, (int)hp.steps.size(), d.seq_pos, d.rgb, d.mask, d.seq_z, d.seq, stream_);
+            launches_ += enqueue_warp_seq(hp.W, hp.H, (int)hp.steps.size(), d.seq_pos, d.rgb.p, d.mask.p, d.seq_z, d.seq,
+                                          stream_);
     }
-    for (int j = 0; j < n_scenes; ++j) enqueue_scene(scenes[j], scene_dev_[j].buf);
-    ARAP_CUDA_OR_RETURN(cudaEventRecord(ev_[3], stream_));
+    for (int j = 0; j < n_scenes; ++j) enqueue_scene(scenes[j], scene_dev_[j].data());
+    ARAP_CUDA_CHECK(cudaEventRecord(ev_[3], stream_));
     for (int i = 0; i < count; ++i) {
         const HostProblem& hp = problems[i];
         Dev& d = dev_[i];
         const size_t N = (size_t)hp.W * hp.H;
-        unsigned char* o = d.h_out;
+        unsigned char* o = d.h_out.data();
         if (!hp.scene) {
-            ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(o, d.flow, N * sizeof(float2), cudaMemcpyDeviceToHost, stream_));
-            ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(o + 8 * N, d.orgb, 3 * N, cudaMemcpyDeviceToHost, stream_));
-            ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(o + 11 * N, d.omask, N, cudaMemcpyDeviceToHost, stream_));
+            ARAP_CUDA_CHECK(cudaMemcpyAsync(o, d.flow.p, N * sizeof(float2), cudaMemcpyDeviceToHost, stream_));
+            ARAP_CUDA_CHECK(cudaMemcpyAsync(o + 8 * N, d.orgb.p, 3 * N, cudaMemcpyDeviceToHost, stream_));
+            ARAP_CUDA_CHECK(cudaMemcpyAsync(o + 11 * N, d.omask.p, N, cudaMemcpyDeviceToHost, stream_));
         }
         if (!hp.scene || hp.out_costs)
-            ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(o + 12 * N, d.costs, cbytes, cudaMemcpyDeviceToHost, stream_));
+            ARAP_CUDA_CHECK(cudaMemcpyAsync(o + 12 * N, d.costs.p, cbytes, cudaMemcpyDeviceToHost, stream_));
         if (hp.out_bflow || hp.out_occ) {
-            ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(d.h_extra, d.bflow, N * sizeof(float2), cudaMemcpyDeviceToHost, stream_));
-            ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(d.h_extra + 8 * N, d.occ, N, cudaMemcpyDeviceToHost, stream_));
+            unsigned char* h = d.h_extras.data();
+            ARAP_CUDA_CHECK(cudaMemcpyAsync(h + x_bflow, d.bflow, N * sizeof(float2), cudaMemcpyDeviceToHost, stream_));
+            ARAP_CUDA_CHECK(cudaMemcpyAsync(h + x_occ, d.occ, N, cudaMemcpyDeviceToHost, stream_));
         }
         // frames go straight to the caller's buffers: K of them would need K times the pinned staging
         const size_t F = N * hp.steps.size();
@@ -518,13 +495,13 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
             {hp.seq_rgb, d.seq.rgb, 3 * F}, {hp.seq_mask, d.seq.mask, F}, {hp.seq_flow, d.seq.flow, 8 * F},
             {hp.seq_bflow, d.seq.bflow, 8 * F}, {hp.seq_occ, d.seq.occ, F}, {hp.seq_flow0, d.seq.flow0, 8 * F}};
         for (const auto& c : seq)
-            if (c.dst && F) ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(c.dst, c.src, c.bytes, cudaMemcpyDeviceToHost, stream_));
+            if (c.dst && F) ARAP_CUDA_CHECK(cudaMemcpyAsync(c.dst, c.src, c.bytes, cudaMemcpyDeviceToHost, stream_));
     }
     // scene outputs go straight to the caller's buffers: the pair is frame index 0 of each block, frames 1 .. K follow
     for (int j = 0; j < n_scenes; ++j) {
         const HostScene& sc = scenes[j];
         const SceneLayout l(sc);
-        const unsigned char* b = scene_dev_[j].buf;
+        const unsigned char* b = scene_dev_[j].data();
         const size_t N = (size_t)sc.W * sc.H, F = N * (sc.maps.size() / 18 - 1);
         const struct { void* dst; size_t off, bytes; } out[] = {
             {sc.out_flow, l.flow, 8 * N}, {sc.out_rgb, l.rgb, 3 * N}, {sc.out_mask, l.mask, N},
@@ -533,9 +510,9 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
             {sc.seq_bflow, l.bflow + 8 * N, 8 * F}, {sc.seq_occ, l.occ + N, F}};
         for (const auto& c : out)
             if (c.dst && c.bytes)
-                ARAP_CUDA_OR_RETURN(cudaMemcpyAsync(c.dst, b + c.off, c.bytes, cudaMemcpyDeviceToHost, stream_));
+                ARAP_CUDA_CHECK(cudaMemcpyAsync(c.dst, b + c.off, c.bytes, cudaMemcpyDeviceToHost, stream_));
     }
-    ARAP_CUDA_OR_RETURN(cudaStreamSynchronize(stream_));
+    ARAP_CUDA_CHECK(cudaStreamSynchronize(stream_));
     if (resident_ && n_resident_ > 0) {
         if (int st = resident_->status(stream_)) {
             fprintf(stderr, "arapb200: resident solver aborted (watchdog, code %d)\n", st);
@@ -554,13 +531,13 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
         const HostProblem& hp = problems[i];
         Dev& d = dev_[i];
         const size_t N = (size_t)hp.W * hp.H;
-        const unsigned char* o = d.h_out;
+        const unsigned char* o = d.h_out.data();
         if (hp.out_flow) memcpy(hp.out_flow, o, N * sizeof(float2));
         if (hp.out_rgb) memcpy(hp.out_rgb, o + 8 * N, 3 * N);
         if (hp.out_mask) memcpy(hp.out_mask, o + 11 * N, N);
         if (hp.out_costs) memcpy(hp.out_costs, o + 12 * N, cbytes);
-        if (hp.out_bflow) memcpy(hp.out_bflow, d.h_extra, N * sizeof(float2));
-        if (hp.out_occ) memcpy(hp.out_occ, d.h_extra + 8 * N, N);
+        if (hp.out_bflow) memcpy(hp.out_bflow, d.h_extras.data() + x_bflow, N * sizeof(float2));
+        if (hp.out_occ) memcpy(hp.out_occ, d.h_extras.data() + x_occ, N);
     }
     if (resident_) launches_ += resident_->launches() - r0;
     cudaEventElapsedTime(&ms_total_, ev_[0], ev_[3]);

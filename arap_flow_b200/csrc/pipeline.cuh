@@ -3,6 +3,7 @@
 // CombinedSolverBase.h:99-120) do around the solver, for many independent (image, segment) problems at once,
 // with every host<->device hop removed except the upload of the inputs and the download of the outputs.
 #pragma once
+#include "devmem.cuh"
 #include "plan.cuh"
 #include "warp.cuh"
 #include <vector>
@@ -95,24 +96,25 @@ public:
 
 private:
     struct Dev { // device + pinned staging of one problem slot
-        float2 *X = nullptr, *U = nullptr, *C = nullptr, *flow = nullptr;
-        float *A = nullptr, *M = nullptr, *costs = nullptr;
-        unsigned char *rgb = nullptr, *mask = nullptr, *orgb = nullptr, *omask = nullptr;
-        unsigned* z = nullptr;
-        MatchRec* matches = nullptr;
-        size_t matches_cap = 0;
-        unsigned char *h_in = nullptr, *h_out = nullptr;
-        // opt-in extras, allocated the first time the slot asks for them: backward flow, occlusion, pinned [bflow | occ]
+        DevBuf<float2> X, U, C, flow;
+        DevBuf<float> A, M, costs;
+        DevBuf<unsigned char> rgb, mask, orgb, omask;
+        DevBuf<unsigned> z;
+        GrowBuf h_in{GrowBuf::Pinned}, h_out{GrowBuf::Pinned};
+        GrowBuf matches; // MatchRec[], grown with headroom for a longer list
+        // opt-in extras, allocated the first time the slot asks for them: [bflow | occ] on the device and pinned
+        GrowBuf extras, h_extras{GrowBuf::Pinned};
+        // opt-in frame sequence, allocated the first time the slot asks and regrown for a longer list
+        GrowBuf frames;
+        // placed in the buffers above for the current run
         float2* bflow = nullptr;
-        unsigned char *occ = nullptr, *h_extra = nullptr;
-        // opt-in frame sequence, allocated the first time the slot asks and regrown for a longer list: X after each
-        // requested continuation step, two z-buffers, the frames' outputs; seq_cap frames of maxW x maxH each
-        int seq_cap = 0;
-        float2* seq_pos = nullptr;
-        unsigned* seq_z = nullptr;
+        unsigned char* occ = nullptr;
+        float2* seq_pos = nullptr; // X after each requested continuation step
+        unsigned* seq_z = nullptr; // two z-buffers
         SeqOut seq{};
         std::vector<MatchRec> recs;
         bool resident = false;
+        const MatchRec* recs_dev() const { return (const MatchRec*)matches.data(); }
     };
     void solve_streaming(const HostProblem& hp, Dev& d);
     void solve_lm(const HostProblem& hp, Dev& d);
@@ -120,14 +122,9 @@ private:
     // continuation step when one of them asks for frames
     void solve_resident(const HostProblem* problems, int first, int count, bool cluster);
     void snapshot(const HostProblem& hp, Dev& d, int t); // X -> frame buffer if step t is one hp asks for
-    static void free_seq(Dev& d);
     // device buffer of the j-th scene of a run, allocated the first time and grown for a larger scene: the background,
     // frame 0 and the composited pair and frames (21 B/px each), laid out by SceneLayout (pipeline.cu)
-    struct SceneDev {
-        unsigned char* buf = nullptr;
-        size_t cap = 0;
-    };
-    std::vector<SceneDev> scene_dev_;
+    std::vector<GrowBuf> scene_dev_;
     void enqueue_scene(const HostScene& sc, unsigned char* buf); // the scene's kernels (DESIGN.md 4.6)
     LmSolver* lm_ = nullptr;
     int lmW_ = 0, lmH_ = 0;

@@ -50,7 +50,7 @@ def main():
             "composite_identity": lambda: lib.composite(*args, bg, I2),
             "composite_affine": lambda: lib.composite(*args, bg_big, A, origin=(m, m)),
         }
-        for f in arms.values():   # warm-up: module load, the arena at its largest size
+        for f in arms.values():   # warm-up: module load, the workspace at its largest size
             f()
         rec = {k: [] for k in arms}
         for _ in range(a.reps):
