@@ -30,54 +30,20 @@
 #include "solver_resident.cuh"
 #include "grid_math.cuh"
 #include "solver_stream.cuh" // FLAG_* bit layout
-#include "exact_limbs.cuh"
 #include <algorithm>
 
 namespace arapb200 {
 namespace {
 
 constexpr int TW = RS_STRIP_W + 2, TH = RS_STRIP_H + 2;
-constexpr int RS_THREADS_MAX = (RS_STRIP_H == 8) ? 384 : 512;
+constexpr int RS_THREADS_MAX = 384;
 constexpr int OB_LEFT = 64, OB_RIGHT = 64 + RS_STRIP_H;
-static_assert(RS_STRIP_H == 4 || RS_STRIP_H == 8, "strip height must be 4 or 8");
 constexpr long long LIMB_BIAS = 1ll << 36;
 constexpr int BAR_STRIDE = 128; // u64 words between barrier words (1 KiB): separate L2 slices, parallel atomics
 constexpr int S_MIN = -100, S_MAX = 100;
-// Measured alternatives of the barrier code (tools/build_variant.sh + tools/ab_sweep.sh, profiles/r2_barrier_ab.txt).
 // The barrier is ~55 % of a lone problem's PCG iteration, and its code is so latency-critical that harmless-looking
-// changes move C1 by several percent either way: every switch here is kept only with a measurement next to it.
-#ifndef ARAP_RS_HOIST
-#define ARAP_RS_HOIST 1 // the 168-register variants issue all shared-memory loads of phases 2 and 3 before the first store
-                        // (0: row by row everywhere, round 1).  The 128-register variants hoist in groups of ARAP_RS_HOIST_LEAN rows:
-                        // all eight at once spill there (C1s 28.4 -> 26.6, C2 6.04 -> 5.76, C3 6.00 -> 5.79 pairs/s)
-#endif
-#ifndef ARAP_RS_STAGE_V4
-#define ARAP_RS_STAGE_V4 0
-#endif
-#ifndef ARAP_RS_HOIST_LEAN
-#define ARAP_RS_HOIST_LEAN 4 // rows per hoisted group in the 128-register variants (0: not hoisted there; 8 spills: C1s -6 %;
-                             // 4: C1s / C2 / C3 +1.3 ... 1.9 %, 2: the same within noise)
-#endif
-#ifndef ARAP_RS_SUM_UNROLL4
-#define ARAP_RS_SUM_UNROLL4 2 // the CTA-level limb sum runs four warps per trip (its shared-memory loads overlap): 1 = in the
-                              // 168-register variants, 2 = everywhere, 0 = nowhere
-#endif
-#ifndef ARAP_RS_SUM_UNROLL
-#define ARAP_RS_SUM_UNROLL 0 // 1: the CTA-level sum over the warps' limb sums is unrolled (all shared-memory loads in flight)
-#endif
-#ifndef ARAP_RS_LEAN_CS_SMEM
-#define ARAP_RS_LEAN_CS_SMEM 0 // 1: the 128-register variants keep cos/sin of the own pixels in shared memory (the strip's `pre` array)
-                               // instead of 16 registers, and look the preconditioner up in a 15-entry table: on the pixel
-                               // grid it only depends on the number of valid neighbours and the fit flag
-#endif
-#ifndef ARAP_RS_DEFER_DELTA
-#define ARAP_RS_DEFER_DELTA 2 // delta += alpha p feeds no reduction: 1 = it is done AFTER the arrival at the second barrier, under the
-                              // barrier's latency, everywhere; 2 = in the 128-register variants only (fewer live values in
-                              // phase 2: C1s +1.4 %, C3 +1.3 %; at 168 registers it delays the poller: lone problem -1.4 %); 0 = never
-#endif
-#ifndef ARAP_RS_G1_LOCAL
-#define ARAP_RS_G1_LOCAL 0   // 1: a problem that runs in ONE CTA keeps its barrier in shared memory (no L2 round trip)
-#endif
+// changes move C1 by several percent either way.  Measure every alternative against this code (tools/build_variant.sh +
+// tools/ab_sweep.sh); profiles/r2_barrier_ab.txt and DESIGN.md 4.1 record what was tried and removed.
 
 struct __align__(16) StripSmem {
     float4 T[TH][TW];              // tile + ring: (p_x, p_y, sin*p_a, cos*p_a) or (X_x, X_y, cos, sin)
@@ -85,23 +51,18 @@ struct __align__(16) StripSmem {
     float2 rcs[RS_OUTBOX_ENTRIES]; // cos/sin of the ring pixels (remote sides only)
     float stage[RS_OUTBOX_ENTRIES][4]; // remote ring pixels: [0..2] fetched z (parked until beta is known), [3] their p_a
     float2 pre[RS_STRIP_H][32];        // (1/(1+sqrt(D_X))^2, 1/(1+sqrt(D_a))^2) per pixel, constant during a GN step
-                                       // (ARAP_RS_LEAN_CS_SMEM, 128-register variants: (cos, sin) of the pixel instead)
 };
 
 struct __align__(16) Ctl {
     int limb[RS_THREADS_MAX / 32][4];
     int ovf[RS_THREADS_MAX / 32];
     unsigned long long prev[2][4]; // totals last seen in each barrier buffer
-#if ARAP_RS_G1_LOCAL
-    unsigned long long local[4];   // G == 1: this CTA's contribution stays here, the barrier never leaves the SM
-#endif
     float bc;                      // broadcast result
     float stop;                    // opt-in early exit: leave the PCG loop once r.z <= stop (-1: never)
     float prev_cost;               // opt-in early exit of the Gauss-Newton loop: cost before the last step
     int bc_code;                   // 0 accept, 1 redo with bc_S
     int bc_S;
     int abort;
-    float preX[2][5], preA[5];     // ARAP_RS_LEAN_CS_SMEM: guarded-inverted diagonal by (fit, valid neighbours)
 };
 
 __device__ __forceinline__ unsigned long long ld_u64_volatile(const unsigned long long* p)
@@ -146,7 +107,7 @@ __device__ __forceinline__ void two_sum(double a, double b, double& s, double& e
 // L0*2^72 + L1*2^48 + L2*2^24 + L3 (|Lj| < 2^45, units 2^e_unit) -> binary32 with ONE rounding: the four terms
 // are exact doubles; they are added error-free (s + e), s + e is rounded to odd in binary64 (53 >= 24 + 2 bits)
 // and only then to binary32.
-__device__ __forceinline__ float limbs_to_float_rn_f64(const long long L[4], int e_unit, bool& is_zero)
+__device__ __forceinline__ float limbs_to_float_rn(const long long L[4], int e_unit, bool& is_zero)
 {
     const double a = __ll2double_rn(L[0]) * 4722366482869645213696.0; // 2^72
     const double b = __ll2double_rn(L[1]) * 281474976710656.0;        // 2^48
@@ -164,19 +125,6 @@ __device__ __forceinline__ float limbs_to_float_rn_f64(const long long L[4], int
     if (zd != zu) z = __longlong_as_double(__double_as_longlong(z) | 1ll);
     e_unit = max(-900, min(900, e_unit));
     return (float)(z * pow2_f64(e_unit)); // exact scaling (barring binary32 underflow), single rounding
-}
-
-// ARAP_RS_INT_FOLD == 2 (exact_limbs.cuh): a 64-bit integer fast path in front of the binary64 route
-__device__ __forceinline__ float limbs_to_float_rn(const long long L[4], int e_unit, bool& is_zero)
-{
-#if ARAP_RS_INT_FOLD == 2
-    float r;
-    if (limbs_to_float_i64(L, max(-900, min(900, e_unit)), is_zero, r)) return r;
-#elif ARAP_RS_INT_FOLD == 1
-    float r;
-    if (limbs_to_float_int(L, max(-900, min(900, e_unit)), is_zero, r)) return r;
-#endif
-    return limbs_to_float_rn_f64(L, e_unit, is_zero);
 }
 
 // Everything a warp needs to know about its strip
@@ -202,7 +150,6 @@ struct Cta {
     unsigned long long* bar; // = P->bar
     int* status;             // = P->status
     Ctl* ctl;
-    bool u4;                 // CTA-level limb sum four warps per trip (compile-time constant per kernel variant)
     struct ClusterCtl* xc;   // cluster-scope barrier only (null otherwise)
     int cta, G, lane, wid, nw;
     unsigned epoch;
@@ -234,7 +181,7 @@ __device__ __forceinline__ void limbs_to_smem(Cta& c, float g0, float g1, int S)
         const float v3 = (v2 - (float)l2) * 16777216.0f;
         l3 = __float2int_rn(v3);
     }
-    if (RS_STRIP_H == 8) {
+    {
         const float v = g1 * sc;
         const bool o1 = !(fabsf(v) < 16777216.0f);
         ovf = ovf || o1;
@@ -253,14 +200,10 @@ __device__ __forceinline__ void limbs_to_smem(Cta& c, float g0, float g1, int S)
     const int s3 = __reduce_add_sync(0xffffffffu, l3);
     const bool wovf = __any_sync(0xffffffffu, ovf);
     if (c.lane == 0) {
-#if ARAP_RS_STAGE_V4
-        *reinterpret_cast<int4*>(&ctl->limb[c.wid][0]) = make_int4(s0, s1, s2, s3);
-#else
         ctl->limb[c.wid][0] = s0;
         ctl->limb[c.wid][1] = s1;
         ctl->limb[c.wid][2] = s2;
         ctl->limb[c.wid][3] = s3;
-#endif
         ctl->ovf[c.wid] = wovf ? 1 : 0;
     }
     __syncthreads();
@@ -274,38 +217,16 @@ __device__ __forceinline__ void grid_arrive(Cta& c, float g0, float g1, int S, l
         unsigned long long* buf = c.bar + (size_t)(c.epoch & 1u) * 4 * BAR_STRIDE;
         long long sum = 0;
         int any = 0;
-#if ARAP_RS_SUM_UNROLL
-#pragma unroll
-        for (int w = 0; w < RS_THREADS_MAX / 32; ++w) {
-            const bool in = w < c.nw;
-            sum += in ? (long long)ctl->limb[w][c.lane] : 0ll;
-            any |= in ? ctl->ovf[w] : 0;
-        }
-#else
-        if (c.u4) {
+        // four warps per trip: their shared-memory loads overlap
 #pragma unroll 4
-            for (int w = 0; w < c.nw; ++w) {
-                sum += (long long)ctl->limb[w][c.lane];
-                any |= ctl->ovf[w];
-            }
-        } else {
-            for (int w = 0; w < c.nw; ++w) {
-                sum += (long long)ctl->limb[w][c.lane];
-                any |= ctl->ovf[w];
-            }
+        for (int w = 0; w < c.nw; ++w) {
+            sum += (long long)ctl->limb[w][c.lane];
+            any |= ctl->ovf[w];
         }
-#endif
         unsigned long long contrib = (1ull << 48) + (unsigned long long)(sum + LIMB_BIAS);
         if (c.lane == 0 && any) contrib += (1ull << 56);
-#if ARAP_RS_G1_LOCAL
-        if (c.G == 1) ctl->local[c.lane] = contrib;
-        else
-#endif
         red_add_u64(buf + (size_t)c.lane * BAR_STRIDE, contrib);
     }
-#if ARAP_RS_G1_LOCAL
-    __syncwarp(); // (G == 1) lane 0 reads ctl->local[0..3] in grid_wait
-#endif
     if (c.prof) t1 = clock64();
 }
 
@@ -320,12 +241,6 @@ __device__ __forceinline__ int grid_wait(Cta& c, int& S, bool& grown, float& res
         unsigned long long* prev = ctl->prev[c.epoch & 1u];
         unsigned long long d[4];
         unsigned spins = 0;
-#if ARAP_RS_G1_LOCAL
-        if (c.G == 1) {
-#pragma unroll
-            for (int j = 0; j < 4; ++j) d[j] = ctl->local[j]; // written by lanes 0..3 of this warp before the __syncwarp in grid_arrive
-        } else
-#endif
         for (;;) {
             bool done = true;
 #pragma unroll
@@ -348,9 +263,6 @@ __device__ __forceinline__ int grid_wait(Cta& c, int& S, bool& grown, float& res
         long long L[4];
 #pragma unroll
         for (int j = 0; j < 4; ++j) {
-#if ARAP_RS_G1_LOCAL
-            if (c.G != 1)
-#endif
             prev[j] += d[j];
             L[j] = (long long)(d[j] & ((1ull << 48) - 1)) - (long long)c.G * LIMB_BIAS;
         }
@@ -551,67 +463,13 @@ __device__ __forceinline__ int cl_wait(Cta& c, int& S, bool& grown, float& res, 
     return code;
 }
 
-// ARAP_RS_NOINLINE_BARRIER: one out-of-line copy of the arrival and of the wait instead of four / two inlined ones.  The
-// PCG loop of this kernel is ~50 KB of code shared by the warps of three co-resident problems that sit in different phases;
-// measurements (profiles/r2_barrier_ab.txt) show that its SIZE matters more than its instruction count.
-#ifndef ARAP_RS_NOINLINE_BARRIER
-#define ARAP_RS_NOINLINE_BARRIER 0
-#endif
-#if ARAP_RS_NOINLINE_BARRIER
-__device__ __noinline__ void grid_arrive_ni(Ctl* ctl, unsigned long long* bar, int G, unsigned epoch, float g0, float g1, int S)
-{
-    Cta c;
-    c.P = nullptr; c.bar = bar; c.status = nullptr; c.ctl = ctl; c.xc = nullptr; c.u4 = false; c.cta = 0; c.G = G;
-    c.lane = threadIdx.x & 31; c.wid = threadIdx.x >> 5; c.nw = blockDim.x >> 5; c.epoch = epoch; c.prof = false;
-    long long t0 = 0, t1 = 0;
-    grid_arrive(c, g0, g1, S, t0, t1);
-}
-// returns (result bits, 0 accept / 1 redo, new scale, bit 0: abort, bit 1: grown)
-__device__ __noinline__ int4 grid_wait_ni(Ctl* ctl, unsigned long long* bar, int* status, int G, unsigned epoch, int S, int grown)
-{
-    Cta c;
-    c.P = nullptr; c.bar = bar; c.status = status; c.ctl = ctl; c.xc = nullptr; c.u4 = false; c.cta = 0; c.G = G;
-    c.lane = threadIdx.x & 31; c.wid = threadIdx.x >> 5; c.nw = blockDim.x >> 5; c.epoch = epoch; c.prof = false;
-    bool gr = grown != 0, ok = true;
-    float res = 0.f;
-    const int code = grid_wait(c, S, gr, res, ok, 0, 0);
-    return make_int4(__float_as_int(res), code, S, (ok ? 0 : 1) | (gr ? 2 : 0));
-}
-__device__ __forceinline__ void arrive_x(Cta& c, float g0, float g1, int S, long long& t0, long long& t1)
-{
-    if (c.prof) t0 = clock64();
-    grid_arrive_ni(c.ctl, c.bar, c.G, c.epoch, g0, g1, S);
-    if (c.prof) t1 = clock64();
-}
-__device__ __forceinline__ int wait_x(Cta& c, int& S, bool& grown, float& res, bool& ok, long long t0, long long t1)
-{
-    const int4 w = grid_wait_ni(c.ctl, c.bar, c.status, c.G, c.epoch, S, grown ? 1 : 0);
-    if (c.prof && threadIdx.x == 0) {
-        c.acc[0] += (unsigned long long)(t1 - t0);
-        c.acc[1] += (unsigned long long)(clock64() - t1); // poll + decode + broadcast together
-    }
-    ++c.epoch;
-    res = __int_as_float(w.x);
-    S = w.z;
-    grown = (w.w & 2) != 0;
-    if (w.w & 1) { ok = false; res = 0.f; return 0; }
-    return w.y;
-}
-#else
-__device__ __forceinline__ void arrive_x(Cta& c, float g0, float g1, int S, long long& t0, long long& t1) { grid_arrive(c, g0, g1, S, t0, t1); }
-__device__ __forceinline__ int wait_x(Cta& c, int& S, bool& grown, float& res, bool& ok, long long t0, long long t1)
-{
-    return grid_wait(c, S, grown, res, ok, t0, t1);
-}
-#endif
-
 // arrive + wait (+ the rare redo with a corrected scale).  Returns the exact sum rounded once to binary32.
 // CL selects the cluster-scope barrier (a separate kernel instantiation: the L2 form compiles exactly as before).
 template <bool CL>
 __device__ __forceinline__ void arrive_t(Cta& c, float g0, float g1, int S, long long& t0, long long& t1)
 {
     if constexpr (CL) cl_arrive(c, g0, g1, S, t0, t1);
-    else arrive_x(c, g0, g1, S, t0, t1);
+    else grid_arrive(c, g0, g1, S, t0, t1);
 }
 template <bool CL>
 __device__ __forceinline__ float grid_finish(Cta& c, float g0, float g1, int& S, bool& ok, long long t0, long long t1)
@@ -621,7 +479,7 @@ __device__ __forceinline__ float grid_finish(Cta& c, float g0, float g1, int& S,
     for (;;) {
         int redo;
         if constexpr (CL) redo = cl_wait(c, S, grown, res, ok, t0, t1);
-        else redo = wait_x(c, S, grown, res, ok, t0, t1);
+        else redo = grid_wait(c, S, grown, res, ok, t0, t1);
         if (!redo) break;
         __syncthreads(); // everybody has read the broadcast before the redo overwrites it
         arrive_t<CL>(c, g0, g1, S, t0, t1);
@@ -745,9 +603,6 @@ __device__ __forceinline__ void ring_update(float4* cell, float* st, float beta,
 }
 
 // ring <- neighbours' new direction
-#ifndef ARAP_RS_HOIST_RING
-#define ARAP_RS_HOIST_RING 0 // 1: the (up to three) ring pixels of a lane are loaded together before the first is stored
-#endif
 template <bool FIRST>
 __device__ __forceinline__ void apply_p(const StripCtx& s, int lane, float beta)
 {
@@ -755,45 +610,10 @@ __device__ __forceinline__ void apply_p(const StripCtx& s, int lane, float beta)
     const int row = lft ? lane : lane - 8;
     const bool side = (lft && s.rem[2] >= 0) || (!lft && lane >= 8 && lane < 8 + RS_STRIP_H && s.rem[3] >= 0);
     const int slot = (lft ? OB_LEFT : OB_RIGHT) + row;
-#if ARAP_RS_HOIST_RING
-    // same arithmetic as ring_update, loads first (the stores of one ring pixel may alias the loads of the next as far as the
-    // compiler can tell, which would serialise three shared-memory round trips)
-    const bool top = s.rem[0] >= 0, bot = s.rem[1] >= 0;
-    float4* const ct = &s.own[0 * TW + lane + 1];
-    float4* const cb = &s.own[(TH - 1) * TW + lane + 1];
-    float4* const cd = &s.own[(row + 1) * TW + (lft ? 0 : TW - 1)];
-    float4* const st_t = reinterpret_cast<float4*>(s.stage + 4 * lane);
-    float4* const st_b = reinterpret_cast<float4*>(s.stage + 4 * (32 + lane));
-    float4* const st_d = reinterpret_cast<float4*>(s.stage + 4 * slot);
-    float4 vt = make_float4(0.f, 0.f, 0.f, 0.f), vb = vt, vd = vt, ot = vt, ob = vt, od = vt;
-    float2 rt = make_float2(0.f, 0.f), rb = rt, rd = rt;
-    if (top) { vt = *st_t; rt = s.rcs[lane]; if (!FIRST) ot = *ct; }
-    if (bot) { vb = *st_b; rb = s.rcs[32 + lane]; if (!FIRST) ob = *cb; }
-    if (side) { vd = *st_d; rd = s.rcs[slot]; if (!FIRST) od = *cd; }
-    if (top) {
-        float p0 = vt.x, p1 = vt.y, pa = vt.z;
-        if (!FIRST) { p0 = fmaf(beta, ot.x, p0); p1 = fmaf(beta, ot.y, p1); pa = fmaf(beta, vt.w, pa); }
-        s.stage[4 * lane + 3] = pa;
-        *ct = make_float4(p0, p1, rt.y * pa, rt.x * pa);
-    }
-    if (bot) {
-        float p0 = vb.x, p1 = vb.y, pa = vb.z;
-        if (!FIRST) { p0 = fmaf(beta, ob.x, p0); p1 = fmaf(beta, ob.y, p1); pa = fmaf(beta, vb.w, pa); }
-        s.stage[4 * (32 + lane) + 3] = pa;
-        *cb = make_float4(p0, p1, rb.y * pa, rb.x * pa);
-    }
-    if (side) {
-        float p0 = vd.x, p1 = vd.y, pa = vd.z;
-        if (!FIRST) { p0 = fmaf(beta, od.x, p0); p1 = fmaf(beta, od.y, p1); pa = fmaf(beta, vd.w, pa); }
-        s.stage[4 * slot + 3] = pa;
-        *cd = make_float4(p0, p1, rd.y * pa, rd.x * pa);
-    }
-#else
     if (s.rem[0] >= 0) ring_update<FIRST>(&s.own[0 * TW + lane + 1], s.stage + 4 * lane, beta, s.rcs[lane]);
     if (s.rem[1] >= 0) ring_update<FIRST>(&s.own[(TH - 1) * TW + lane + 1], s.stage + 4 * (32 + lane), beta, s.rcs[32 + lane]);
     // left column (lanes 0..H-1) and right column (lanes 8..8+H-1) in one predicated block
     if (side) ring_update<FIRST>(&s.own[(row + 1) * TW + (lft ? 0 : TW - 1)], s.stage + 4 * slot, beta, s.rcs[slot]);
-#endif
 }
 
 // constraint of a pixel for the current continuation weight (CombinedSolver.h:236-239)
@@ -836,12 +656,14 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
     StripSmem* S = reinterpret_cast<StripSmem*>(smem_raw);
 
     constexpr bool LEAN = (MINB >= 3);               // the 128-register variants
-    constexpr bool HOIST = ARAP_RS_HOIST && (!LEAN || ARAP_RS_HOIST_LEAN > 0);
-    constexpr bool CSM = LEAN && ARAP_RS_LEAN_CS_SMEM != 0;
-    constexpr bool DEFER = ARAP_RS_DEFER_DELTA == 1 || (ARAP_RS_DEFER_DELTA == 2 && LEAN);
-    constexpr int HG = (LEAN && ARAP_RS_HOIST_LEAN > 0) ? ARAP_RS_HOIST_LEAN : RS_STRIP_H; // rows whose loads are issued together
+    // Rows of phases 2 and 3 whose shared-memory loads are issued together: all eight in the 168-register variants.  All
+    // eight spill in the 128-register variants (C1s 28.4 -> 26.6, C2 6.04 -> 5.76, C3 6.00 -> 5.79 pairs/s); groups of
+    // four gain C1s / C2 / C3 1.3 ... 1.9 % over not hoisting there, groups of two the same within noise.
+    constexpr int HG = LEAN ? 4 : RS_STRIP_H;
+    // delta += alpha p after the arrival at the second barrier, under its latency, in the 128-register variants only:
+    // fewer live values in phase 2 there (C1s +1.4 %, C3 +1.3 %); at 168 registers it delays the poller (lone problem -1.4 %)
+    constexpr bool DEFER = LEAN;
     Cta c;
-    c.u4 = ARAP_RS_SUM_UNROLL4 && (ARAP_RS_SUM_UNROLL4 > 1 || !LEAN);
     c.P = &P; c.bar = P.bar; c.status = P.status; c.ctl = &ctl; c.xc = nullptr; c.cta = cta_in_problem; c.G = P.G;
     c.lane = threadIdx.x & 31; c.wid = threadIdx.x >> 5; c.nw = blockDim.x >> 5; c.epoch = 0;
     c.acc[0] = c.acc[1] = c.acc[2] = 0; c.prof = PROF && (P.prof != nullptr);
@@ -855,16 +677,6 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
 
     if (threadIdx.x == 0) ctl.abort = 0;
     if (threadIdx.x < 8) ctl.prev[threadIdx.x >> 2][threadIdx.x & 3] = 0ull; // the host zeroes P.bar before the launch
-    if constexpr (CSM) {
-        // jtf_finish's diagonal on the pixel grid: DX = (wr2 + wr2) * nv (+ wf2 with a constraint), DA = wr2 * nv
-        if (threadIdx.x < 15) {
-            const int nv = threadIdx.x % 5, which = threadIdx.x / 5;
-            float Dg = (which == 2) ? wr2 * (float)nv : (wr2 + wr2) * (float)nv;
-            if (which == 1) Dg = Dg + wf2;
-            const float v = guarded_invert(Dg);
-            if (which == 2) ctl.preA[nv] = v; else ctl.preX[which][nv] = v;
-        }
-    }
     if constexpr (CL) {
         // cluster launch: the problem IS the cluster (host: enqueue_cluster), rank in the cluster = CTA in the problem
         __shared__ ClusterCtl xc;
@@ -934,24 +746,9 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
     float q0[RS_STRIP_H], q1[RS_STRIP_H], qa[RS_STRIP_H];
 #pragma unroll
     for (int k = 0; k < RS_STRIP_H; ++k) { r0[k] = r1[k] = r2[k] = pa[k] = 0.f; cc[k] = 1.f; ss[k] = 0.f; q0[k] = q1[k] = qa[k] = 0.f; }
-    if constexpr (CSM) {
-#pragma unroll
-        for (int k = 0; k < RS_STRIP_H; ++k) s.pre[k * 32] = make_float2(1.f, 0.f); // (cos, sin) of a pixel that is never active
-    }
-    // (cos, sin) of own pixel k / its preconditioner entries (position, angle): registers + the per-pixel array, or --
-    // CSM -- the per-pixel array + a table lookup by (fit, number of valid neighbours)
-    auto cs_of = [&](int k) -> float2 {
-        if constexpr (CSM) return s.pre[k * 32];
-        else return make_float2(cc[k], ss[k]);
-    };
-    auto pre_of = [&](int k, unsigned f) -> float2 {
-        if constexpr (CSM) {
-            const int nv = __popc(f & 15u);
-            return make_float2(ctl.preX[(f & FLAG_FIT) ? 1 : 0][nv], ctl.preA[nv]);
-        } else {
-            return s.pre[k * 32];
-        }
-    };
+    // preconditioner entries (position, angle) of own pixel k.  Read through this lambda rather than as s.pre[k * 32] at
+    // each use: the plain reads compile to another register assignment of the kernel's set-up code.
+    auto pre_of = [&](int k) -> float2 { return s.pre[k * 32]; };
     // every tile cell must hold finite data (the masked stencil multiplies invalid neighbours by 0)
     for (int e = lane; e < TH * TW; e += 32) s.own[e] = make_float4(0.f, 0.f, 0.f, 0.f);
     int S_cost = 0, S_num = 0, S_den = 0, S_bnum = 0, S_sep = 8;
@@ -972,8 +769,7 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
                     const float2 X = P.X[i];
                     float sn, cs;
                     contract_sincos(P.A[i], sn, cs);
-                    if constexpr (CSM) s.pre[k * 32] = make_float2(cs, sn);
-                    else { cc[k] = cs; ss[k] = sn; }
+                    cc[k] = cs; ss[k] = sn;
                     e = make_float4(X.x, X.y, cs, sn);
                 }
                 s.own[(k + 1) * TW + lane + 1] = e;
@@ -1036,7 +832,7 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
                     unsigned f = flag_of(flo, fhi, k) & ~FLAG_FIT;
                     r0[k] = r1[k] = r2[k] = 0.f;
                     pa[k] = 0.f;
-                    if constexpr (!CSM) s.pre[k * 32] = make_float2(1.0f, 1.0f); // inactive pixels: r stays 0, any finite value works
+                    s.pre[k * 32] = make_float2(1.0f, 1.0f); // inactive pixels: r stays 0, any finite value works
                     s.D[(0 * RS_STRIP_H + k) * 32] = 0.f;
                     s.D[(1 * RS_STRIP_H + k) * 32] = 0.f;
                     s.D[(2 * RS_STRIP_H + k) * 32] = 0.f;
@@ -1055,7 +851,7 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
                         float g0, g1, ga, DX, DA;
                         jtf_finish(a, cur.x, cur.y, fit, ct.x, ct.y, wr2, wf2, g0, g1, ga, DX, DA);
                         const float pX = guarded_invert(DX), pA = guarded_invert(DA);
-                        if constexpr (!CSM) s.pre[k * 32] = make_float2(pX, pA);
+                        s.pre[k * 32] = make_float2(pX, pA);
                         r0[k] = -g0; r1[k] = -g1; r2[k] = -ga;
                         const float z0 = pX * r0[k], z1 = pX * r1[k], z2 = pA * r2[k];
                         const float term = dot3(r0[k], r1[k], r2[k], z0, z1, z2);
@@ -1071,7 +867,7 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
 #pragma unroll
                 for (int k = 0; k < RS_STRIP_H; ++k) {
                     if (any_rem) {
-                        const float2 pre = pre_of(k, flag_of(flo, fhi, k));
+                        const float2 pre = pre_of(k);
                         publish_rowcol(s, lane, k, seq, pre.x * r0[k], pre.x * r1[k], pre.y * r2[k], 0.f);
                     }
                 }
@@ -1083,12 +879,11 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
                 // p_0 = z_0 into the tile (all warps are past their J^T F reads: grid_sum synchronised)
 #pragma unroll
                 for (int k = 0; k < RS_STRIP_H; ++k) {
-                    const float2 pre = pre_of(k, flag_of(flo, fhi, k));
-                    const float2 csk = cs_of(k);
+                    const float2 pre = pre_of(k);
                     const float pX = pre.x, pA = pre.y;
                     const float p0 = pX * r0[k], p1 = pX * r1[k];
                     pa[k] = pA * r2[k];
-                    s.own[(k + 1) * TW + lane + 1] = make_float4(p0, p1, csk.y * pa[k], csk.x * pa[k]);
+                    s.own[(k + 1) * TW + lane + 1] = make_float4(p0, p1, ss[k] * pa[k], cc[k] * pa[k]);
                 }
                 if (any_rem) apply_p<true>(s, lane, 0.0f);
                 // N4 (opt-in, never on the parity path): relative tolerance on the preconditioned residual norm
@@ -1125,8 +920,7 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
                     jtj_nb_masked<1>(a, cur.x, cur.y, lf, m1);
                     jtj_nb_masked<2>(a, cur.x, cur.y, dn, m2);
                     jtj_nb_masked<3>(a, cur.x, cur.y, up, m3);
-                    const float2 csk = cs_of(k);
-                    jtj_finish(a, csk.x, csk.y, cur.x, cur.y, pa[k], (f & FLAG_FIT) != 0, wr2, wf2, q0[k], q1[k], qa[k]);
+                    jtj_finish(a, cc[k], ss[k], cur.x, cur.y, pa[k], (f & FLAG_FIT) != 0, wr2, wf2, q0[k], q1[k], qa[k]);
                     const float term = dot3(cur.x, cur.y, pa[k], q0[k], q1[k], qa[k]);
                     if (k < 4) gs0 = gs0 + term; else gs1 = gs1 + term;
                     up = cur;
@@ -1142,11 +936,9 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
                 gs0 = 0.f; gs1 = 0.f;
                 const bool pub = any_rem && (it + 1 < P.nPCG);
                 ++seq;
-                if constexpr (HOIST) {
                 // every shared-memory load of the phase first: the compiler cannot move a later row's loads above an earlier
                 // row's delta stores (it cannot prove that D, the tile and pre do not alias), so written row by row the phase
                 // pays the shared-memory latency eight times over
-                // (HG rows per group: all eight in the 168-register variants, fewer where registers are tight)
 #pragma unroll
                 for (int kb = 0; kb < RS_STRIP_H; kb += HG) {
                     float hx[HG], hy[HG], hd0[HG], hd1[HG], hd2[HG];
@@ -1160,7 +952,7 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
                             hx[j] = e.x; hy[j] = e.y;
                             hd0[j] = Dk[0 * RS_STRIP_H * 32]; hd1[j] = Dk[1 * RS_STRIP_H * 32]; hd2[j] = Dk[2 * RS_STRIP_H * 32];
                         }
-                        hpre[j] = pre_of(k, flag_of(flo, fhi, k));
+                        hpre[j] = pre_of(k);
                     }
 #pragma unroll
                     for (int j = 0; j < HG; ++j) {
@@ -1180,27 +972,6 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
                         if (k < 4) gs0 = gs0 + term; else gs1 = gs1 + term;
                         if (pub) publish_rowcol(s, lane, k, seq, z0, z1, z2, 0.f);
                     }
-                }
-                } else {
-#pragma unroll
-                for (int k = 0; k < RS_STRIP_H; ++k) {
-                    if constexpr (!DEFER) {
-                        const float4 e = s.own[(k + 1) * TW + lane + 1];
-                        float* Dk = s.D + k * 32;
-                        Dk[0 * RS_STRIP_H * 32] = fmaf(alpha, e.x, Dk[0 * RS_STRIP_H * 32]);
-                        Dk[1 * RS_STRIP_H * 32] = fmaf(alpha, e.y, Dk[1 * RS_STRIP_H * 32]);
-                        Dk[2 * RS_STRIP_H * 32] = fmaf(alpha, pa[k], Dk[2 * RS_STRIP_H * 32]);
-                    }
-                    r0[k] = fmaf(-alpha, q0[k], r0[k]);
-                    r1[k] = fmaf(-alpha, q1[k], r1[k]);
-                    r2[k] = fmaf(-alpha, qa[k], r2[k]);
-                    const float2 pre = pre_of(k, flag_of(flo, fhi, k));
-                    const float pX = pre.x, pA = pre.y;
-                    const float z0 = pX * r0[k], z1 = pX * r1[k], z2 = pA * r2[k];
-                    const float term = dot3(z0, z1, z2, r0[k], r1[k], r2[k]);
-                    if (k < 4) gs0 = gs0 + term; else gs1 = gs1 + term;
-                    if (pub) publish_rowcol(s, lane, k, seq, z0, z1, z2, 0.f);
-                }
                 }
                 RS_TICK(1);
                 long long tb0 = 0, tb1 = 0;
@@ -1243,40 +1014,25 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
                 if (bnum <= ctl.stop) { need_sep = true; break; } // early exit (every CTA decodes the same bnum: a uniform decision)
 
                 // ---- PCGStep3: p = z + beta p (own pixels, then the remote ring) ----
-                if constexpr (HOIST) {
 #pragma unroll
-                    for (int kb = 0; kb < RS_STRIP_H; kb += HG) {
-                        float hx[HG], hy[HG];
-                        float2 hpre[HG];
+                for (int kb = 0; kb < RS_STRIP_H; kb += HG) {
+                    float hx[HG], hy[HG];
+                    float2 hpre[HG];
 #pragma unroll
-                        for (int j = 0; j < HG; ++j) {
-                            const float4 e = s.own[(kb + j + 1) * TW + lane + 1];
-                            hx[j] = e.x; hy[j] = e.y;
-                            hpre[j] = pre_of(kb + j, flag_of(flo, fhi, kb + j));
-                        }
-#pragma unroll
-                        for (int j = 0; j < HG; ++j) {
-                            const int k = kb + j;
-                            const float pX = hpre[j].x, pA = hpre[j].y;
-                            const float p0 = fmaf(beta, hx[j], pX * r0[k]);
-                            const float p1 = fmaf(beta, hy[j], pX * r1[k]);
-                            pa[k] = fmaf(beta, pa[k], pA * r2[k]);
-                            const float2 csk = cs_of(k);
-                            s.own[(k + 1) * TW + lane + 1] = make_float4(p0, p1, csk.y * pa[k], csk.x * pa[k]);
-                        }
+                    for (int j = 0; j < HG; ++j) {
+                        const float4 e = s.own[(kb + j + 1) * TW + lane + 1];
+                        hx[j] = e.x; hy[j] = e.y;
+                        hpre[j] = pre_of(kb + j);
                     }
-                } else {
 #pragma unroll
-                for (int k = 0; k < RS_STRIP_H; ++k) {
-                    const float4 e = s.own[(k + 1) * TW + lane + 1];
-                    const float2 pre = pre_of(k, flag_of(flo, fhi, k));
-                    const float2 csk = cs_of(k);
-                    const float pX = pre.x, pA = pre.y;
-                    const float p0 = fmaf(beta, e.x, pX * r0[k]);
-                    const float p1 = fmaf(beta, e.y, pX * r1[k]);
-                    pa[k] = fmaf(beta, pa[k], pA * r2[k]);
-                    s.own[(k + 1) * TW + lane + 1] = make_float4(p0, p1, csk.y * pa[k], csk.x * pa[k]);
-                }
+                    for (int j = 0; j < HG; ++j) {
+                        const int k = kb + j;
+                        const float pX = hpre[j].x, pA = hpre[j].y;
+                        const float p0 = fmaf(beta, hx[j], pX * r0[k]);
+                        const float p1 = fmaf(beta, hy[j], pX * r1[k]);
+                        pa[k] = fmaf(beta, pa[k], pA * r2[k]);
+                        s.own[(k + 1) * TW + lane + 1] = make_float4(p0, p1, ss[k] * pa[k], cc[k] * pa[k]);
+                    }
                 }
                 if (any_rem) apply_p<false>(s, lane, beta);
                 __syncthreads();
@@ -1320,20 +1076,12 @@ struct KernelVariant {
     int max_threads, min_blocks;
     KernelFn fn, fn_prof;
 };
-#ifndef ARAP_RS_VARIANTS
-#if ARAP_RS_STRIP_H == 8
-#define ARAP_RS_VARIANTS {128, 4, k_resident_t<128, 4, false>, k_resident_t<128, 4, true>}, \
-                         {160, 3, k_resident_t<160, 3, false>, k_resident_t<160, 3, true>}, \
-                         {192, 2, k_resident_t<192, 2, false>, k_resident_t<192, 2, true>}, \
-                         {384, 1, k_resident_t<384, 1, false>, k_resident_t<384, 1, true>}
-#else
-#define ARAP_RS_VARIANTS {256, 4, k_resident_t<256, 4, false>, k_resident_t<256, 4, true>}, \
-                         {256, 3, k_resident_t<256, 3, false>, k_resident_t<256, 3, true>}, \
-                         {320, 3, k_resident_t<320, 3, false>, k_resident_t<320, 3, true>}, \
-                         {512, 1, k_resident_t<512, 1, false>, k_resident_t<512, 1, true>}
-#endif
-#endif
-const KernelVariant g_variants[] = {ARAP_RS_VARIANTS};
+const KernelVariant g_variants[] = {
+    {128, 4, k_resident_t<128, 4, false>, k_resident_t<128, 4, true>},
+    {160, 3, k_resident_t<160, 3, false>, k_resident_t<160, 3, true>},
+    {192, 2, k_resident_t<192, 2, false>, k_resident_t<192, 2, true>},
+    {384, 1, k_resident_t<384, 1, false>, k_resident_t<384, 1, true>},
+};
 constexpr int g_nvariants = sizeof(g_variants) / sizeof(g_variants[0]);
 // the cluster-scope instantiation: up to RS_THREADS_MAX / 32 strips per CTA, one CTA per SM
 const KernelFn g_cluster_fn = k_resident_t<RS_THREADS_MAX, 1, false, true>;
@@ -1443,7 +1191,6 @@ ResidentSolver::ResidentSolver(int maxW, int maxH, int max_slots) : maxW_(maxW),
         const int smem = (int)((RS_THREADS_MAX / 32) * sizeof(StripSmem));
         ARAP_CUDA_CHECK(cudaFuncSetAttribute((const void*)g_cluster_fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
         ARAP_CUDA_CHECK(cudaFuncSetAttribute((const void*)g_cluster_fn, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
-        if (const char* e = getenv("ARAP_RS_CLUSTER")) cluster_barrier_ = atoi(e) != 0;
     }
     for (int v = 0; v < g_nvariants; ++v) {
         const int smem = (int)((g_variants[v].max_threads / 32) * sizeof(StripSmem));
@@ -1495,11 +1242,6 @@ bool ResidentSolver::prepare_finish(int slot)
     sl.NW = (sl.n_strips + sm_count_ - 1) / sm_count_;
     if (sl.NW < 4) sl.NW = 4;
     if (sl.NW > max_warps) return false; // does not fit on chip
-#if ARAP_RS_G1_LOCAL
-    // a small problem (a DAVIS segment of a few percent of the frame, the 64x64 plumbing case) runs in ONE CTA: its two
-    // reductions per PCG iteration then never leave the SM
-    if (sl.n_strips <= max_warps) sl.NW = std::max(sl.n_strips, 4);
-#endif
     sl.G = (sl.n_strips + sl.NW - 1) / sl.NW;
     if (sl.G > sm_count_) sl.G = sm_count_;
     if (sl.G > RS_MAX_CTAS) return false;

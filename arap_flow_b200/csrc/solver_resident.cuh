@@ -9,11 +9,8 @@
 
 namespace arapb200 {
 
-#ifndef ARAP_RS_STRIP_H
-#define ARAP_RS_STRIP_H 8
-#endif
 constexpr int RS_STRIP_W = 32;   // a strip is 32 x RS_STRIP_H pixels: one warp, lane = column
-constexpr int RS_STRIP_H = ARAP_RS_STRIP_H; // 4 (one contract-C3 group per lane) or 8 (two)
+constexpr int RS_STRIP_H = 8;    // two contract-C3 groups per lane
 constexpr int RS_MAX_WARPS = 16; // strips per CTA
 constexpr int RS_MAX_CTAS = 160; // CTAs per problem (8-bit arrival count per barrier word)
 constexpr int RS_PROF_SLOTS = 16; // u64 per CTA of the optional cycle accounting (arapb200_debug_resident_profile)

@@ -16,14 +16,6 @@
 #include "solver_stream.cuh"
 #include "grid_math.cuh"
 
-// occupancy experiments (tools/build_variant.sh): minimum resident blocks per SM of the two PCG kernels; 0 = let ptxas choose
-#ifndef ARAP_ST_MINB_A
-#define ARAP_ST_MINB_A 0
-#endif
-#ifndef ARAP_ST_MINB_B
-#define ARAP_ST_MINB_B 0
-#endif
-
 namespace arapb200 {
 
 namespace {
@@ -218,13 +210,14 @@ __global__ void __launch_bounds__(ST_THREADS) k_init(const StreamDev* __restrict
 // Thread = one vertical quad of the tile (lane = column); threads 0..131 also own one pixel of the 1-pixel ring
 // around the tile, whose NEW direction they recompute (the neighbouring tile is writing it in this very kernel, so p is
 // ping-ponged).  Every global load of the block is issued before the first use; beta is decoded under them.
-// SUB = rows per block (32: one block per tile, 256 threads; 16: two blocks per tile, 128 threads -- shorter blocks leave
-// less idle time at the end of the grid).
 // RT (opt-in early exit, separate instantiation so that the default kernels compile exactly as before): once r.z of the
 // previous iteration is <= sc->stop, this launch and every later k_step_a / k_step_b of the Gauss-Newton step return at
 // once -- every block decodes the same scalar, so the decision is uniform; block 0 makes it sticky (sc->conv).
-template <bool FIRST, int SUB, bool RT = false>
-__global__ void __launch_bounds__(SUB * 8, ARAP_ST_MINB_A) k_step_a(const __grid_constant__ StreamPlanes pl,
+// SUB = rows per block, here and in k_step_b: two 128-thread blocks per tile beat one 256-thread block, because shorter
+// blocks leave less idle time at the end of the grid.
+constexpr int SUB = 16;
+template <bool FIRST, bool RT = false>
+__global__ void __launch_bounds__(SUB * 8) k_step_a(const __grid_constant__ StreamPlanes pl,
                                                     const StreamDev* __restrict__ dpp, int it)
 {
     constexpr int NSUB = ST_TILE / SUB, TSY = SUB + 2;
@@ -364,226 +357,11 @@ __global__ void __launch_bounds__(SUB * 8, ARAP_ST_MINB_A) k_step_a(const __grid
     publish(pl, ST_ACC_D0 + (it & 1), block_exact_sum(g, red));
 }
 
-// ---------------------------------------------------------------------------------------------
-// k_step_a with its inputs brought in by TMA bulk copies (VERDICT r1 item 7; opt-in: ARAP_STREAM_TMA=1).  Same block
-// shape as k_step_a<false, 16> (two 128-thread blocks per tile) and the same arithmetic; the difference is the way the
-// block's inputs arrive: warp 0 issues one cp.async.bulk per contiguous run -- ten 2 KB plane slabs (old direction, cos/sin,
-// preconditioner, residual), the 512 flag bytes, ten 128-byte rows above and below the slab and ten 64-byte runs of the
-// left / right neighbours' edge mirrors -- all completing on one mbarrier; beta is decoded while they are in flight and
-// every thread then reads its quad from shared memory.  35 KB of shared memory per block, so ptxas' six blocks per SM stay.
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void tma_load(void* dst, const void* src, unsigned bytes, unsigned long long* mbar, unsigned long long policy)
-{
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes.L2::cache_hint [%0], [%1], %2, [%3], %4;"
-                 ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(mbar)), "l"(policy) : "memory");
-}
-__device__ __forceinline__ int tma_plane(int k, int src) // the k-th staged plane
-{
-    return k < 3 ? src + k : k < 5 ? PL_CS + (k - 3) : k < 7 ? PL_PRE + (k - 5) : PL_R + (k - 7);
-}
-
-// RING_TMA = false: only the eleven large runs go through TMA, the ring pixels are loaded by their threads as in k_step_a
-template <bool RING_TMA>
-__global__ void __launch_bounds__(128) k_step_a_tma(const __grid_constant__ StreamPlanes pl, const StreamDev* __restrict__ dpp,
-                                                    int it)
-{
-    constexpr int SUB = 16, TSY = SUB + 2, NST = 10;
-    __shared__ __align__(128) float S[NST][SUB * ST_TILE];  // plane slabs of the block's 16 rows
-    __shared__ __align__(16) float RTB[2][NST][ST_TILE];    // row above / row below
-    __shared__ __align__(16) float RLR[2][NST][SUB];        // column left / column right (neighbours' edge mirrors)
-    __shared__ __align__(16) unsigned char SF[SUB * ST_TILE];
-    __shared__ float4 T[TSY][TS];
-    __shared__ double red[64];
-    __shared__ float s_beta;
-    __shared__ __align__(8) unsigned long long mbar;
-    const int tile = blockIdx.x >> 1, sub = blockIdx.x & 1;
-    const bool tile_on = pl.tile_active[tile] != 0;
-    if (!tile_on && blockIdx.x != 0) return;
-    const int W = pl.W, H = pl.H;
-    const int x0 = (tile % pl.tx) * ST_TILE, y0 = (tile / pl.tx) * ST_TILE + sub * SUB;
-    const int lx = threadIdx.x & 31, lyb = (threadIdx.x >> 5) * 4;
-    const int src = PL_P + 3 * ((it - 1) & 1), dst = PL_P + 3 * (it & 1);
-    float* const tb = tile_ptr(pl, tile);
-    const bool has_top = y0 > 0, has_bot = y0 + SUB < H, has_left = x0 > 0, has_right = x0 + ST_TILE < W;
-
-    if (threadIdx.x == 0) {
-        asm volatile("mbarrier.init.shared::cta.b64 [%0], 1;" ::"r"(smem_u32(&mbar)) : "memory");
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    }
-    __syncthreads();
-    long long raw = 0;
-    if (threadIdx.x < 32) {
-        unsigned long long pol_first, pol_last, pol_norm;
-        asm volatile("createpolicy.fractional.L2::evict_first.b64 %0, 1.0;" : "=l"(pol_first));
-        asm volatile("createpolicy.fractional.L2::evict_last.b64 %0, 1.0;" : "=l"(pol_last));
-        asm volatile("createpolicy.fractional.L2::evict_normal.b64 %0, 1.0;" : "=l"(pol_norm));
-        unsigned bytes = 0;
-        constexpr int NITEMS = RING_TMA ? 5 * NST : NST;
-        for (int item = threadIdx.x; item < 1 + NITEMS; item += 32) {
-            if (item == NITEMS) { // flags
-                tma_load(SF, reinterpret_cast<const unsigned char*>(tb + PL_FLAGS * ST_TILE_PX) + sub * SUB * ST_TILE,
-                         SUB * ST_TILE, &mbar, pol_last);
-                bytes += SUB * ST_TILE;
-                continue;
-            }
-            const int kind = item / NST, k = item % NST, plane = tma_plane(k, src);
-            // the old direction is dead after this kernel; cos/sin and the preconditioner are re-read by every PCG kernel
-            const unsigned long long pol = k < 3 ? pol_first : k < 7 ? pol_last : pol_norm;
-            if (kind == 0) {
-                tma_load(S[k], tb + plane * ST_TILE_PX + sub * SUB * ST_TILE, SUB * ST_TILE * 4, &mbar, pol);
-                bytes += SUB * ST_TILE * 4;
-            } else if (kind == 1 || kind == 2) {
-                const bool on = kind == 1 ? has_top : has_bot;
-                if (!on) continue;
-                const int hy = kind == 1 ? y0 - 1 : y0 + SUB;
-                tma_load(RTB[kind - 1][k], pl.planes + tiled_off(pl, x0, hy) + plane * ST_TILE_PX, ST_TILE * 4, &mbar, pol);
-                bytes += ST_TILE * 4;
-            } else {
-                const bool on = kind == 3 ? has_left : has_right;
-                if (!on) continue;
-                // left neighbour: its column 31 (mirror 1); right neighbour: its column 0 (mirror 0)
-                const float* nb = tile_ptr(pl, kind == 3 ? tile - 1 : tile + 1) + PL_EDGE * ST_TILE_PX +
-                                  (edge_slot(plane) * 2 + (kind == 3 ? 1 : 0)) * ST_TILE + (y0 & 31);
-                tma_load(RLR[kind - 3][k], nb, SUB * 4, &mbar, pol);
-                bytes += SUB * 4;
-            }
-        }
-#pragma unroll
-        for (int o = 16; o > 0; o >>= 1) bytes += __shfl_xor_sync(0xffffffffu, bytes, o);
-        if (threadIdx.x == 0)
-            asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(&mbar)), "r"(bytes) : "memory");
-        // ---- beta, while the copies are in flight ----
-        raw = fetch2(pl, bn_set(it - 1), bn_set(it - 2));
-        const float v = wide_round(raw);
-        const float bnum = __shfl_sync(0xffffffffu, v, 0), num = __shfl_sync(0xffffffffu, v, 16);
-        if (threadIdx.x == 0) {
-            s_beta = (num > 0.0f) ? bnum / num : 0.0f; // :544-547
-            if (blockIdx.x == 0 && dpp->trace) dpp->trace[3 * (it - 1) + 2] = bnum;
-        }
-    }
-    // ---- ring pixels by plain loads (RING_TMA = false), issued before anything is waited for ----
-    const int t = threadIdx.x;
-    float hv[NST];
-    bool hin = false;
-    if (!RING_TMA && t < 2 * TS + 2 * SUB) {
-        int hlx, hly;
-        if (t < TS) { hlx = t; hly = 0; }
-        else if (t < 2 * TS) { hlx = t - TS; hly = TSY - 1; }
-        else if (t < 2 * TS + SUB) { hlx = 0; hly = t - 2 * TS + 1; }
-        else { hlx = TS - 1; hly = t - 2 * TS - SUB + 1; }
-        const int hx = x0 + hlx - 1, hy = y0 + hly - 1;
-        hin = hx >= 0 && hx < W && hy >= 0 && hy < H;
-        const bool hedge = hin && (hlx == 0 || hlx == TS - 1);
-        const float* hpx = tb;
-        if (hin)
-            hpx = hedge ? tile_ptr(pl, (hy >> 5) * pl.tx + (hx >> 5)) + PL_EDGE * ST_TILE_PX + ((hx & 31) != 0 ? ST_TILE : 0) + (hy & 31)
-                        : pl.planes + tiled_off(pl, hx, hy);
-#pragma unroll
-        for (int k = 0; k < NST; ++k) {
-            const int plane = tma_plane(k, src);
-            hv[k] = hpx[hedge ? edge_slot(plane) * 2 * ST_TILE : plane * ST_TILE_PX];
-        }
-    }
-    const float wr2 = dpp->wr2, wf2 = dpp->wf2;
-    __syncthreads(); // s_beta
-    const float beta = s_beta;
-    {
-        unsigned done = 0;
-        while (!done)
-            asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], 0;\n\tselp.u32 %0, 1, 0, p;\n\t}"
-                         : "=r"(done) : "r"(smem_u32(&mbar)) : "memory");
-    }
-
-    float* const own = tb + (sub * SUB + lyb) * ST_TILE + lx;
-    float* const pd = own + dst * ST_TILE_PX;
-    float po[4][3], cs[4][2];
-    unsigned fl[4];
-    float4 ent[4];
-#pragma unroll
-    for (int r = 0; r < 4; ++r) {
-        const int loc = (lyb + r) * ST_TILE + lx;
-        cs[r][0] = S[3][loc]; cs[r][1] = S[4][loc];
-        const float pX = S[5][loc], pA = S[6][loc];
-        po[r][0] = fmaf(beta, S[0][loc], pX * S[7][loc]);
-        po[r][1] = fmaf(beta, S[1][loc], pX * S[8][loc]);
-        po[r][2] = fmaf(beta, S[2][loc], pA * S[9][loc]);
-        fl[r] = SF[loc];
-        if (tile_on) {
-            PLN(pd + r * ST_TILE, 0) = po[r][0]; PLN(pd + r * ST_TILE, 1) = po[r][1]; PLN(pd + r * ST_TILE, 2) = po[r][2];
-            edge_put(tb, dst, lx, sub * SUB + lyb + r, po[r][0]);
-            edge_put(tb, dst + 1, lx, sub * SUB + lyb + r, po[r][1]);
-            edge_put(tb, dst + 2, lx, sub * SUB + lyb + r, po[r][2]);
-        }
-        ent[r] = make_float4(po[r][0], po[r][1], cs[r][1] * po[r][2], cs[r][0] * po[r][2]);
-        T[lyb + r + 1][lx + 1] = ent[r];
-    }
-    // ---- ring: threads 0..99 recompute the new direction of one ring pixel (corners are never read) ----
-    if (!RING_TMA && t < 2 * TS + 2 * SUB) {
-        int hlx, hly;
-        if (t < TS) { hlx = t; hly = 0; }
-        else if (t < 2 * TS) { hlx = t - TS; hly = TSY - 1; }
-        else if (t < 2 * TS + SUB) { hlx = 0; hly = t - 2 * TS + 1; }
-        else { hlx = TS - 1; hly = t - 2 * TS - SUB + 1; }
-        float4 e = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (hin) {
-            const float h0 = fmaf(beta, hv[0], hv[5] * hv[7]);
-            const float h1 = fmaf(beta, hv[1], hv[5] * hv[8]);
-            const float h2 = fmaf(beta, hv[2], hv[6] * hv[9]);
-            e = make_float4(h0, h1, hv[4] * h2, hv[3] * h2);
-        }
-        T[hly][hlx] = e;
-    }
-    if (RING_TMA && t < 2 * TS + 2 * SUB) {
-        int hlx, hly;
-        const float* rp = nullptr; // staged plane 0 of the ring pixel, stride between planes in `rs`
-        int rs = 0;
-        if (t < 2 * TS) {
-            const int bot = t >= TS ? 1 : 0;
-            hlx = t - bot * TS; hly = bot ? TSY - 1 : 0;
-            if (hlx >= 1 && hlx <= ST_TILE && (bot ? has_bot : has_top) && x0 + hlx - 1 < W) { rp = &RTB[bot][0][hlx - 1]; rs = ST_TILE; }
-        } else {
-            const int rgt = t >= 2 * TS + SUB ? 1 : 0;
-            hlx = rgt ? TS - 1 : 0; hly = t - 2 * TS - rgt * SUB + 1;
-            if ((rgt ? has_right : has_left) && y0 + hly - 1 < H) { rp = &RLR[rgt][0][hly - 1]; rs = SUB; }
-        }
-        float4 e = make_float4(0.f, 0.f, 0.f, 0.f);
-        if (rp) {
-            const float pX = rp[5 * rs], pA = rp[6 * rs];
-            const float h0 = fmaf(beta, rp[0], pX * rp[7 * rs]);
-            const float h1 = fmaf(beta, rp[rs], pX * rp[8 * rs]);
-            const float h2 = fmaf(beta, rp[2 * rs], pA * rp[9 * rs]);
-            e = make_float4(h0, h1, rp[4 * rs] * h2, rp[3 * rs] * h2);
-        }
-        T[hly][hlx] = e;
-    }
-    __syncthreads();
-
-    float g = 0.0f;
-    float* const pq = own + PL_Q * ST_TILE_PX;
-#pragma unroll
-    for (int r = 0; r < 4; ++r) {
-        const unsigned f = fl[r];
-        if (!tile_on || !(f & FLAG_ACTIVE)) continue;
-        const int ly = lyb + r;
-        JtjAcc a;
-        jtj_zero(a);
-        jtj_nb_masked<0>(a, po[r][0], po[r][1], T[ly + 1][lx + 2], (f & 1u) ? 1.0f : 0.0f);
-        jtj_nb_masked<1>(a, po[r][0], po[r][1], T[ly + 1][lx], (f & 2u) ? 1.0f : 0.0f);
-        jtj_nb_masked<2>(a, po[r][0], po[r][1], r < 3 ? ent[r < 3 ? r + 1 : 3] : T[ly + 2][lx + 1], (f & 4u) ? 1.0f : 0.0f);
-        jtj_nb_masked<3>(a, po[r][0], po[r][1], r > 0 ? ent[r > 0 ? r - 1 : 0] : T[ly][lx + 1], (f & 8u) ? 1.0f : 0.0f);
-        float q0, q1, qa;
-        jtj_finish(a, cs[r][0], cs[r][1], po[r][0], po[r][1], po[r][2], (f & FLAG_FIT) != 0, wr2, wf2, q0, q1, qa);
-        PLN(pq + r * ST_TILE, 0) = q0; PLN(pq + r * ST_TILE, 1) = q1; PLN(pq + r * ST_TILE, 2) = qa;
-        g = g + dot3(po[r][0], po[r][1], po[r][2], q0, q1, qa);
-    }
-    publish(pl, ST_ACC_D0 + (it & 1), block_exact_sum(g, red));
-}
-
 // PCGStep2 (solverGPUGaussNewton.t:446-489).  Branch-free: the planes of inactive pixels hold zeros (they are
 // zero-initialised and never written), so they flow through as exact zeros and add +0 to the group term;
 // every load of the four rows is issued before the first use.
-template <int SUB, bool RT = false>
-__global__ void __launch_bounds__(SUB * 8, ARAP_ST_MINB_B) k_step_b(const __grid_constant__ StreamPlanes pl,
+template <bool RT = false>
+__global__ void __launch_bounds__(SUB * 8) k_step_b(const __grid_constant__ StreamPlanes pl,
                                                     const StreamDev* __restrict__ dpp, int it)
 {
     constexpr int NSUB = ST_TILE / SUB;
@@ -978,10 +756,6 @@ StreamSolver::StreamSolver(int W, int H)
     // behind it, and the branch-free kernels rely on "inactive pixels hold zeros": finish the clears here
     ARAP_CUDA_CHECK(cudaDeviceSynchronize());
     h_.trace = nullptr;
-    const char* e = getenv("ARAP_STREAM_SUB");
-    sub16_ = !(e && atoi(e) == 32);
-    e = getenv("ARAP_STREAM_TMA"); // opt-in A/B: k_step_a with TMA bulk copies (DESIGN.md 4.2)
-    tma_ = e ? atoi(e) : 0; // 1: everything through TMA; 2: the large runs only, ring pixels by plain loads
 }
 
 StreamSolver::~StreamSolver()
@@ -1076,31 +850,17 @@ void StreamSolver::launch_step_a(bool first, int it, cudaStream_t stream)
         else k_step_a_gen<false><<<h_.ntiles, ST_THREADS, 0, stream>>>(pl, d_, it);
     } else {
         const bool rt = this->rt(); // opt-in early exits: their own instantiations
-        if (sub16_) {
-            if (first) k_step_a<true, 16><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_, it);
-            else if (rt) k_step_a<false, 16, true><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_, it);
-            else if (tma_ == 1) k_step_a_tma<true><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_, it);
-            else if (tma_ == 2) k_step_a_tma<false><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_, it);
-            else k_step_a<false, 16><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_, it);
-        } else {
-            if (first) k_step_a<true, 32><<<h_.ntiles, 256, 0, stream>>>(pl, d_, it);
-            else if (rt) k_step_a<false, 32, true><<<h_.ntiles, 256, 0, stream>>>(pl, d_, it);
-            else k_step_a<false, 32><<<h_.ntiles, 256, 0, stream>>>(pl, d_, it);
-        }
+        if (first) k_step_a<true><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_, it);
+        else if (rt) k_step_a<false, true><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_, it);
+        else k_step_a<false><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_, it);
     }
 }
 
 void StreamSolver::launch_step_b(int it, cudaStream_t stream)
 {
     const StreamPlanes& pl = h_;
-    const bool rt = this->rt();
-    if (sub16_) {
-        if (rt) k_step_b<16, true><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_, it);
-        else k_step_b<16><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_, it);
-    } else {
-        if (rt) k_step_b<32, true><<<h_.ntiles, 256, 0, stream>>>(pl, d_, it);
-        else k_step_b<32><<<h_.ntiles, 256, 0, stream>>>(pl, d_, it);
-    }
+    if (rt()) k_step_b<true><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_, it);
+    else k_step_b<false><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_, it);
 }
 
 void StreamSolver::set_pcg_rtol(float rtol)

@@ -124,8 +124,6 @@ private:
     KernelTimer* timer_ = nullptr;
     float pcg_rtol_ = 0.0f, gn_rtol_ = 0.0f;
     bool rt() const { return (pcg_rtol_ > 0.0f || gn_rtol_ > 0.0f) && !general_; } // the early-exit kernel instantiations
-    int tma_ = 0;       // ARAP_STREAM_TMA=1 / 2: k_step_a_tma<true / false> instead of k_step_a<false, 16>
-    bool sub16_ = true; // two 128-thread blocks per tile in the PCG kernels (ARAP_STREAM_SUB=32: one 256-thread block)
     StreamDev h_{};
     StreamDev* d_ = nullptr;
     cudaGraphExec_t graph_ = nullptr;
