@@ -381,10 +381,7 @@ int arapb200_batch_set_option(arapb200_batch* b, const char* name, double value)
             b->pipe->set_pcg_rtol((float)value);
             return 0;
         }
-        if (strcmp(name, "cluster_barrier") == 0) { // 1: small problems use the cluster-scope barrier; 0 (default): always L2
-            b->pipe->set_cluster_barrier(value != 0.0);
-            return 0;
-        }
+        if (strcmp(name, "cluster_barrier") == 0) return 0; // no effect, accepted for compatibility (include/arapb200.h)
         if (strcmp(name, "gn_rtol") == 0) {
             if (!(value >= 0.0) || value >= 1.0) return 1;
             b->pipe->set_gn_rtol((float)value);

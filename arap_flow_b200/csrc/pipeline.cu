@@ -248,7 +248,7 @@ void BatchPipeline::solve_lm(const HostProblem& hp, Dev& d)
     launches_ += lm_->launches() - l0;
 }
 
-void BatchPipeline::solve_resident(const HostProblem* problems, int first, int count, bool cluster)
+void BatchPipeline::solve_resident(const HostProblem* problems, int first, int count)
 {
     const float wf = sqrtf(100.0f), wr = sqrtf(0.01f); // CombinedSolver.h:172-177
     bool frames = false;
@@ -261,8 +261,7 @@ void BatchPipeline::solve_resident(const HostProblem* problems, int first, int c
             launches_ += dj.recs.empty() ? 1 : 2;
             resident_->set_problem(first + j, dj.X.p, dj.A.p, dj.C.p, 1, wf, wr, dj.costs.p, nullptr);
         }
-        if (cluster) resident_->enqueue_cluster(first, count, nCont_, nGN_, nPCG_, stream_);
-        else resident_->enqueue_group(first, count, nCont_, nGN_, nPCG_, stream_);
+        resident_->enqueue_group(first, count, nCont_, nGN_, nPCG_, stream_);
         return;
     }
     // Frames need X after individual continuation steps: one launch per step, on the constraint image of that step as the
@@ -277,8 +276,7 @@ void BatchPipeline::solve_resident(const HostProblem* problems, int first, int c
             resident_->set_problem(first + j, dj.X.p, dj.A.p, dj.C.p, 0, wf, wr, dj.costs.p + (size_t)t * (nGN_ + 1),
                                    nullptr);
         }
-        if (cluster) resident_->enqueue_cluster(first, count, 1, nGN_, nPCG_, stream_);
-        else resident_->enqueue_group(first, count, 1, nGN_, nPCG_, stream_);
+        resident_->enqueue_group(first, count, 1, nGN_, nPCG_, stream_);
         for (int j = 0; j < count; ++j) snapshot(problems[first + j], dev_[first + j], t);
     }
 }
@@ -432,23 +430,12 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
         }
         int run_len = 0; // consecutive resident problems
         while (i + run_len < count && dev_[i + run_len].resident) ++run_len;
-        // small problems (each fits one thread-block cluster) share ONE launch, however many they are: their barriers run
-        // through distributed shared memory and the problems need not be co-resident
-        if (const int ncl = resident_->cluster_run(i, run_len)) {
-            solve_resident(problems, i, ncl, true);
-            if (ncl > group_size_) group_size_ = ncl;
-            i += ncl;
-            continue;
-        }
-        // the cluster-eligible problems further down this run get their own launch: stop the co-resident group before them
-        for (int j = 1; j < run_len; ++j)
-            if (resident_->cluster_run(i + j, 1)) { run_len = j; break; }
         int gsz = resident_->group_size(i, run_len);
         if (gsz < run_len) { // several launches: split the run evenly instead of one full launch and a small remainder
             const int ngroups = (run_len + gsz - 1) / gsz;
             gsz = std::min(gsz, (run_len + ngroups - 1) / ngroups);
         }
-        solve_resident(problems, i, gsz, false);
+        solve_resident(problems, i, gsz);
         if (gsz > group_size_) group_size_ = gsz;
         i += gsz;
     }

@@ -89,7 +89,6 @@ public:
     // opt-in early exits of the PCG loops / of the Gauss-Newton steps (both back-ends)
     void set_pcg_rtol(float rtol);
     void set_gn_rtol(float rtol);
-    void set_cluster_barrier(bool on) { if (resident_) resident_->set_cluster_barrier(on); }
     // opt-in: every Opt_ProblemSolve of the schedule runs the reference's other solver kind, "LMGPU" (solver_lm.cuh:
     // trust region + Q-based exit of the linear loops) with its default parameters, one problem at a time
     void set_lm(bool on) { lm_on_ = on; }
@@ -118,9 +117,9 @@ private:
     };
     void solve_streaming(const HostProblem& hp, Dev& d);
     void solve_lm(const HostProblem& hp, Dev& d);
-    // the resident problems first .. first + count - 1 in one cooperative (or cluster) launch per schedule, or per
-    // continuation step when one of them asks for frames
-    void solve_resident(const HostProblem* problems, int first, int count, bool cluster);
+    // the resident problems first .. first + count - 1 in one cooperative launch per schedule, or per continuation step
+    // when one of them asks for frames
+    void solve_resident(const HostProblem* problems, int first, int count);
     void snapshot(const HostProblem& hp, Dev& d, int t); // X -> frame buffer if step t is one hp asks for
     // device buffer of the j-th scene of a run, allocated the first time and grown for a larger scene: the background,
     // frame 0 and the composited pair and frames (21 B/px each), laid out by SceneLayout (pipeline.cu)

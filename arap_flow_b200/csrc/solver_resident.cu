@@ -150,7 +150,6 @@ struct Cta {
     unsigned long long* bar; // = P->bar
     int* status;             // = P->status
     Ctl* ctl;
-    struct ClusterCtl* xc;   // cluster-scope barrier only (null otherwise)
     int cta, G, lane, wid, nw;
     unsigned epoch;
     unsigned long long acc[3]; // optional cycle accounting (thread 0): reduce+arrive, poll, decode+broadcast
@@ -161,9 +160,10 @@ struct Cta {
 // Split in two so that independent work (the halo fetch) can sit between arrival and completion.
 // grid_arrive: this thread's group terms g0 (and g1 when a lane holds two groups) are converted to limbs
 // against the scale 2^S, summed over the CTA and added to the barrier words.
-__device__ __forceinline__ void limbs_to_smem(Cta& c, float g0, float g1, int S)
+__device__ __forceinline__ void grid_arrive(Cta& c, float g0, float g1, int S, long long& t0, long long& t1)
 {
     Ctl* ctl = c.ctl;
+    if (c.prof) t0 = clock64();
     // ---- thread -> four signed 24-bit limbs in units 2^(S-18), 2^(S-42), 2^(S-66), 2^(S-90) ----
     // (binary32 only: scaling by powers of two and the remainders are exact)
     const float sc = __int_as_float((127 + 18 - S) << 23);
@@ -207,12 +207,6 @@ __device__ __forceinline__ void limbs_to_smem(Cta& c, float g0, float g1, int S)
         ctl->ovf[c.wid] = wovf ? 1 : 0;
     }
     __syncthreads();
-}
-__device__ __forceinline__ void grid_arrive(Cta& c, float g0, float g1, int S, long long& t0, long long& t1)
-{
-    Ctl* ctl = c.ctl;
-    if (c.prof) t0 = clock64();
-    limbs_to_smem(c, g0, g1, S);
     if (c.wid == 0 && c.lane < 4) {
         unsigned long long* buf = c.bar + (size_t)(c.epoch & 1u) * 4 * BAR_STRIDE;
         long long sum = 0;
@@ -301,197 +295,24 @@ __device__ __forceinline__ int grid_wait(Cta& c, int& S, bool& grown, float& res
     return code;
 }
 
-// ---- cluster-scope barrier (problems of at most 16 CTAs) ---------------------------------------------------------
-// A problem that fits one thread-block cluster never touches L2 for its reductions: every CTA PUSHES its four limb sums
-// into the shared memory of every CTA of the cluster (st.async through distributed shared memory, completion counted in
-// bytes on the receiver's mbarrier), then waits on its OWN mbarrier and decodes locally.  One DSMEM hop (~200 cycles)
-// replaces red -> L2 -> poll (~1 700 cycles per barrier for a lone problem, profiles/r2_resident_cycle_accounting.txt).
-// Two buffers / two mbarriers alternate with the barrier's parity; a buffer is re-armed for its next use (two barriers
-// later) right after its wait completes, which is before this CTA arrives at the barrier in between -- and no peer can
-// send for the next use before it has passed that barrier.  Values are fresh per use (no running totals).
-constexpr int CL_MAX = 16; // CTAs per cluster (non-portable size, cudaFuncAttributeNonPortableClusterSizeAllowed)
-constexpr long long CL_BIAS = 1ll << 40;
-struct __align__(16) ClusterCtl {
-    unsigned long long x[2][CL_MAX][4]; // [buffer][sender rank][limb]: limb sum + CL_BIAS (bit 62 of limb 0: overflow)
-    unsigned long long mbar[2];
-};
-__device__ __forceinline__ unsigned smem_u32(const void* p) { return (unsigned)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long* b, unsigned count)
-{
-    asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(b)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_arm(unsigned long long* b, unsigned tx_bytes)
-{
-    asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(b)), "r"(tx_bytes) : "memory");
-}
-// (default .acquire.cta, the convention of CUTLASS's ClusterBarrier::wait for data that other CTAs of the cluster deliver
-// with complete_tx: the payload lands in THIS SM's shared memory and its arrival is what flips the phase.  The explicit
-// .acquire.cluster form compiles to an extra CCTL.IVALL + MEMBAR per wait.)
-__device__ __forceinline__ bool mbar_try_wait(unsigned long long* b, unsigned parity)
-{
-    unsigned ok;
-    asm volatile("{\n\t.reg .pred p;\n\t"
-                 "mbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\t"
-                 "selp.u32 %0, 1, 0, p;\n\t}"
-                 : "=r"(ok) : "r"(smem_u32(b)), "r"(parity) : "memory");
-    return ok != 0;
-}
-__device__ __forceinline__ void cluster_sync_all()
-{
-    asm volatile("barrier.cluster.arrive.release.aligned;\n\tbarrier.cluster.wait.acquire.aligned;" ::: "memory");
-}
-// remote (float data word, mbarrier) store: data lands in CTA `rank`'s copy of *dst and 8 bytes complete on its *mbar
-__device__ __forceinline__ void dsmem_push(unsigned long long* dst, unsigned long long* mbar, unsigned rank, unsigned long long v)
-{
-    unsigned rd, rm;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(rd) : "r"(smem_u32(dst)), "r"(rank));
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(rm) : "r"(smem_u32(mbar)), "r"(rank));
-    asm volatile("st.async.weak.shared::cluster.mbarrier::complete_tx::bytes.b64 [%0], %1, [%2];" ::"r"(rd), "l"(v), "r"(rm) : "memory");
-}
-__device__ __forceinline__ void cl_setup(Cta& c, ClusterCtl* xc)
-{
-    c.xc = xc;
-    if (threadIdx.x == 0) {
-        mbar_init(&xc->mbar[0], 1);
-        mbar_init(&xc->mbar[1], 1);
-        asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-        mbar_arm(&xc->mbar[0], (unsigned)c.G * 32u);
-        mbar_arm(&xc->mbar[1], (unsigned)c.G * 32u);
-    }
-    cluster_sync_all(); // nobody pushes before every peer's mbarriers exist
-}
-__device__ __forceinline__ void cl_arrive(Cta& c, float g0, float g1, int S, long long& t0, long long& t1)
-{
-    Ctl* ctl = c.ctl;
-    ClusterCtl* xc = c.xc;
-    if (c.prof) t0 = clock64();
-    limbs_to_smem(c, g0, g1, S);
-    if (c.wid == 0) {
-        // lanes 0..3 hold the CTA's limb sums, every lane then takes (peer = lane / 4 [+ 8], limb = lane % 4)
-        long long sum = 0;
-        int any = 0;
-        if (c.lane < 4)
-            for (int w = 0; w < c.nw; ++w) {
-                sum += (long long)ctl->limb[w][c.lane];
-                any |= ctl->ovf[w];
-            }
-        unsigned long long v = (unsigned long long)(sum + CL_BIAS);
-        if (c.lane == 0 && any) v |= 1ull << 62;
-        v = __shfl_sync(0xffffffffu, v, c.lane & 3);
-        const unsigned b = c.epoch & 1u;
-#pragma unroll
-        for (int half = 0; half < CL_MAX / 8; ++half) {
-            const int peer = (c.lane >> 2) + 8 * half;
-            if (peer < c.G) dsmem_push(&xc->x[b][c.cta][c.lane & 3], &xc->mbar[b], (unsigned)peer, v);
-        }
-    }
-    if (c.prof) t1 = clock64();
-}
-__device__ __forceinline__ int cl_wait(Cta& c, int& S, bool& grown, float& res, bool& ok, long long t0, long long t1)
-{
-    Ctl* ctl = c.ctl;
-    ClusterCtl* xc = c.xc;
-    long long t2 = 0;
-    if (c.wid == 0) {
-        const unsigned b = c.epoch & 1u, parity = (c.epoch >> 1) & 1u;
-        unsigned spins = 0;
-        bool aborted = false;
-        while (!mbar_try_wait(&xc->mbar[b], parity)) { // (a hardware-assisted sleep, not a busy poll)
-            if (++spins > (1u << 18) || ((spins & 0x3fu) == 0 && *(volatile int*)c.status)) { aborted = true; break; }
-        }
-        if (c.prof) t2 = clock64();
-        // sum the G senders' limbs: lane = 4 * sender + limb (senders 0..7), second half for senders 8..15
-        long long part = 0;
-        int fl = 0;
-#pragma unroll
-        for (int half = 0; half < CL_MAX / 8; ++half) {
-            const int sender = (c.lane >> 2) + 8 * half;
-            if (sender < c.G) {
-                const unsigned long long w = xc->x[b][sender][c.lane & 3];
-                fl |= (int)((w >> 62) & 1ull);
-                part += (long long)(w & ((1ull << 62) - 1ull)) - CL_BIAS;
-            }
-        }
-#pragma unroll
-        for (int o = 4; o < 32; o <<= 1) {
-            part += __shfl_xor_sync(0xffffffffu, part, o);
-            fl |= __shfl_xor_sync(0xffffffffu, fl, o);
-        }
-        long long L[4];
-#pragma unroll
-        for (int k = 0; k < 4; ++k) L[k] = __shfl_sync(0xffffffffu, part, k);
-        const int novf = __shfl_sync(0xffffffffu, fl, 0);
-        if (c.lane == 0) {
-            if (!aborted) mbar_arm(&xc->mbar[b], (unsigned)c.G * 32u); // for the use after next
-            bool T_is_zero;
-            const float r = limbs_to_float_rn(L, S - 90, T_is_zero);
-            int code = 0, newS = S;
-            if (novf) {
-                code = 1; newS = min(S + 24, S_MAX);
-                if (S >= S_MAX) code = 0;
-            } else if (T_is_zero) {
-                if (!grown && S > S_MIN) { code = 1; newS = max(S - 64, S_MIN); }
-            } else {
-                const int e = ilogb_f32(fabsf(r));
-                if (!grown && e < S - 24 && S > S_MIN) { code = 1; newS = max(e + 4, S_MIN); }
-                else newS = max(min(e + 4, S_MAX), S_MIN);
-            }
-            if (aborted) {
-                atomicExch(c.status, 1);
-                atomicCAS(c.status + 1, 0, 300 + (int)(c.epoch & 0xffff));
-                ctl->abort = 1;
-            }
-            ctl->bc = r;
-            ctl->bc_code = code;
-            ctl->bc_S = newS;
-        }
-    }
-    __syncthreads();
-    if (c.prof && threadIdx.x == 0) {
-        const long long t3 = clock64();
-        c.acc[0] += (unsigned long long)(t1 - t0);
-        c.acc[1] += (unsigned long long)(t2 - t1);
-        c.acc[2] += (unsigned long long)(t3 - t2);
-    }
-    ++c.epoch;
-    if (ctl->abort) { ok = false; res = 0.f; return 0; }
-    const int code = ctl->bc_code;
-    const int newS = ctl->bc_S;
-    res = ctl->bc;
-    if (newS > S) grown = true;
-    S = newS;
-    return code;
-}
-
 // arrive + wait (+ the rare redo with a corrected scale).  Returns the exact sum rounded once to binary32.
-// CL selects the cluster-scope barrier (a separate kernel instantiation: the L2 form compiles exactly as before).
-template <bool CL>
-__device__ __forceinline__ void arrive_t(Cta& c, float g0, float g1, int S, long long& t0, long long& t1)
-{
-    if constexpr (CL) cl_arrive(c, g0, g1, S, t0, t1);
-    else grid_arrive(c, g0, g1, S, t0, t1);
-}
-template <bool CL>
 __device__ __forceinline__ float grid_finish(Cta& c, float g0, float g1, int& S, bool& ok, long long t0, long long t1)
 {
     bool grown = false;
     float res;
     for (;;) {
-        int redo;
-        if constexpr (CL) redo = cl_wait(c, S, grown, res, ok, t0, t1);
-        else redo = grid_wait(c, S, grown, res, ok, t0, t1);
+        const int redo = grid_wait(c, S, grown, res, ok, t0, t1);
         if (!redo) break;
         __syncthreads(); // everybody has read the broadcast before the redo overwrites it
-        arrive_t<CL>(c, g0, g1, S, t0, t1);
+        grid_arrive(c, g0, g1, S, t0, t1);
     }
     return res;
 }
-template <bool CL>
 __device__ __forceinline__ float grid_sum(Cta& c, float g0, float g1, int& S, bool& ok)
 {
     long long t0 = 0, t1 = 0;
-    arrive_t<CL>(c, g0, g1, S, t0, t1);
-    return grid_finish<CL>(c, g0, g1, S, ok, t0, t1);
+    grid_arrive(c, g0, g1, S, t0, t1);
+    return grid_finish(c, g0, g1, S, ok, t0, t1);
 }
 
 // ---- halo publication / reception ----------------------------------------------------------------
@@ -635,7 +456,7 @@ __device__ __forceinline__ unsigned flag_of(unsigned flo, unsigned fhi, int k)
 }
 
 // =====================================================================================================
-template <int MAXT, int MINB, bool PROF, bool CL = false>
+template <int MAXT, int MINB, bool PROF>
 __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __restrict__ probs)
 {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -664,7 +485,7 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
     // fewer live values in phase 2 there (C1s +1.4 %, C3 +1.3 %); at 168 registers it delays the poller (lone problem -1.4 %)
     constexpr bool DEFER = LEAN;
     Cta c;
-    c.P = &P; c.bar = P.bar; c.status = P.status; c.ctl = &ctl; c.xc = nullptr; c.cta = cta_in_problem; c.G = P.G;
+    c.P = &P; c.bar = P.bar; c.status = P.status; c.ctl = &ctl; c.cta = cta_in_problem; c.G = P.G;
     c.lane = threadIdx.x & 31; c.wid = threadIdx.x >> 5; c.nw = blockDim.x >> 5; c.epoch = 0;
     c.acc[0] = c.acc[1] = c.acc[2] = 0; c.prof = PROF && (P.prof != nullptr);
     unsigned long long ph[4] = {0, 0, 0, 0}; // cycles in PCG phase 1, 2, 3 and everything else (thread 0)
@@ -677,11 +498,6 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
 
     if (threadIdx.x == 0) ctl.abort = 0;
     if (threadIdx.x < 8) ctl.prev[threadIdx.x >> 2][threadIdx.x & 3] = 0ull; // the host zeroes P.bar before the launch
-    if constexpr (CL) {
-        // cluster launch: the problem IS the cluster (host: enqueue_cluster), rank in the cluster = CTA in the problem
-        __shared__ ClusterCtl xc;
-        cl_setup(c, &xc);
-    }
 
     // ---- which strip is mine, who are my neighbours ----
     const int n = P.n_strips;
@@ -802,7 +618,7 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
                     up = cur;
                     cur = dn;
                 }
-                const float tot = grid_sum<CL>(c, gs0, gs1, S_cost, ok);
+                const float tot = grid_sum(c, gs0, gs1, S_cost, ok);
                 if (!ok) break;
                 if (c.cta == 0 && threadIdx.x == 0) P.costs[(size_t)t * (P.nGN + 1) + g] = 0.5f * tot;
                 if (P.gn_rtol > 0.0f) {
@@ -872,9 +688,9 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
                     }
                 }
                 long long ta0 = 0, ta1 = 0;
-                arrive_t<CL>(c, gs0, gs1, S_num, ta0, ta1);
+                grid_arrive(c, gs0, gs1, S_num, ta0, ta1);
                 if (any_rem) fetch_halo(P, &ctl, s, lane, seq, false); // overlaps the barrier latency
-                num = grid_finish<CL>(c, gs0, gs1, S_num, ok, ta0, ta1); // solverGPUGaussNewton.t:395 scanAlphaNumerator
+                num = grid_finish(c, gs0, gs1, S_num, ok, ta0, ta1); // solverGPUGaussNewton.t:395 scanAlphaNumerator
                 if (!ok) break;
                 // p_0 = z_0 into the tile (all warps are past their J^T F reads: grid_sum synchronised)
 #pragma unroll
@@ -927,7 +743,7 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
                     cur = dn;
                 }
                 RS_TICK(0);
-                const float den = grid_sum<CL>(c, gs0, gs1, S_den, ok);
+                const float den = grid_sum(c, gs0, gs1, S_den, ok);
                 RS_TOCK();
                 if (!ok) break;
                 const float alpha = (den > 0.0f) ? num / den : 0.0f; // :456-459
@@ -975,7 +791,7 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
                 }
                 RS_TICK(1);
                 long long tb0 = 0, tb1 = 0;
-                arrive_t<CL>(c, gs0, gs1, S_bnum, tb0, tb1);
+                grid_arrive(c, gs0, gs1, S_bnum, tb0, tb1);
                 if constexpr (DEFER) {
                     // delta += alpha p feeds no reduction: it runs here, under the latency of the barrier just arrived at
                     // (p -- the tile entries and pa -- does not change before phase 3)
@@ -1001,7 +817,7 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
                     }
                 }
                 if (pub) fetch_halo(P, &ctl, s, lane, seq, false); // overlaps the barrier latency
-                const float bnum = grid_finish<CL>(c, gs0, gs1, S_bnum, ok, tb0, tb1);
+                const float bnum = grid_finish(c, gs0, gs1, S_bnum, ok, tb0, tb1);
                 RS_TOCK();
                 if (!ok) break;
                 if (P.trace && c.cta == 0 && threadIdx.x == 0) {
@@ -1040,7 +856,7 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
             }
             if (!ok) break;
             if (need_sep) {
-                (void)grid_sum<CL>(c, threadIdx.x == 0 ? 1.0f : 0.0f, 0.0f, S_sep, ok); // sum = G: never zero, scale settles at once
+                (void)grid_sum(c, threadIdx.x == 0 ? 1.0f : 0.0f, 0.0f, S_sep, ok); // sum = G: never zero, scale settles at once
                 if (!ok) break;
             }
 
@@ -1064,7 +880,6 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
         o[0] = ph[0]; o[1] = ph[1]; o[2] = ph[2]; o[3] = ph[3];
         o[4] = c.acc[0]; o[5] = c.acc[1]; o[6] = c.acc[2]; o[7] = c.epoch;
     }
-    if constexpr (CL) cluster_sync_all(); // no CTA leaves while a peer may still push into its shared memory
 #undef RS_TICK
 #undef RS_TOCK
 }
@@ -1083,8 +898,6 @@ const KernelVariant g_variants[] = {
     {384, 1, k_resident_t<384, 1, false>, k_resident_t<384, 1, true>},
 };
 constexpr int g_nvariants = sizeof(g_variants) / sizeof(g_variants[0]);
-// the cluster-scope instantiation: up to RS_THREADS_MAX / 32 strips per CTA, one CTA per SM
-const KernelFn g_cluster_fn = k_resident_t<RS_THREADS_MAX, 1, false, true>;
 
 // ---- strip table construction -------------------------------------------------------------------------
 __global__ void __launch_bounds__(256) k_strip_active(int W, int H, int SX, int SY, const float* __restrict__ M,
@@ -1187,11 +1000,6 @@ ResidentSolver::ResidentSolver(int maxW, int maxH, int max_slots) : maxW_(maxW),
     // the memset ran on the legacy stream, all later work runs on non-blocking streams: finish it here
     ARAP_CUDA_CHECK(cudaDeviceSynchronize());
     ARAP_CUDA_CHECK(cudaMalloc(&d_probs_, slots_.size() * sizeof(ResProb)));
-    {
-        const int smem = (int)((RS_THREADS_MAX / 32) * sizeof(StripSmem));
-        ARAP_CUDA_CHECK(cudaFuncSetAttribute((const void*)g_cluster_fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
-        ARAP_CUDA_CHECK(cudaFuncSetAttribute((const void*)g_cluster_fn, cudaFuncAttributeNonPortableClusterSizeAllowed, 1));
-    }
     for (int v = 0; v < g_nvariants; ++v) {
         const int smem = (int)((g_variants[v].max_threads / 32) * sizeof(StripSmem));
         ARAP_CUDA_CHECK(cudaFuncSetAttribute((const void*)g_variants[v].fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
@@ -1232,13 +1040,7 @@ bool ResidentSolver::prepare_finish(int slot)
     if (h_counts_[slot] < 0) return false;
     sl.n_strips = h_counts_[slot];
     const int max_warps = RS_THREADS_MAX / 32;
-    sl.cluster_ctas = 0;
     if (sl.n_strips == 0) { sl.G = 1; sl.NW = 1; sl.fits = true; return true; }
-    // small problem: fits one thread-block cluster of at most CL_MAX CTAs x max_warps strips (cluster-scope barrier)
-    if (sl.n_strips <= CL_MAX * max_warps) {
-        const int cs = (sl.n_strips + max_warps - 1) / max_warps;
-        if (cluster_schedulable(cs)) sl.cluster_ctas = cs;
-    }
     sl.NW = (sl.n_strips + sm_count_ - 1) / sm_count_;
     if (sl.NW < 4) sl.NW = 4;
     if (sl.NW > max_warps) return false; // does not fit on chip
@@ -1328,88 +1130,11 @@ void ResidentSolver::enqueue_group(int first, int count, int nCont, int nGN, int
     launches_ += 1;
 }
 
-// can the device schedule a cluster of cs CTAs of the cluster kernel at full size?  (asked once per size)
-bool ResidentSolver::cluster_schedulable(int cs)
-{
-    if (cs < 1 || cs > CL_MAX) return false;
-    if (cluster_ok_[cs] == 0) {
-        cudaLaunchConfig_t cfg = {};
-        cfg.gridDim = dim3((unsigned)cs, 1, 1);
-        cfg.blockDim = dim3(RS_THREADS_MAX, 1, 1);
-        cfg.dynamicSmemBytes = (size_t)(RS_THREADS_MAX / 32) * sizeof(StripSmem);
-        cudaLaunchAttribute attr[1];
-        attr[0].id = cudaLaunchAttributeClusterDimension;
-        attr[0].val.clusterDim.x = (unsigned)cs; attr[0].val.clusterDim.y = 1; attr[0].val.clusterDim.z = 1;
-        cfg.attrs = attr; cfg.numAttrs = 1;
-        int n = 0;
-        const cudaError_t e = cudaOccupancyMaxActiveClusters(&n, (const void*)g_cluster_fn, &cfg);
-        if (e != cudaSuccess) (void)cudaGetLastError();
-        cluster_ok_[cs] = (e == cudaSuccess && n > 0) ? 1 : -1;
-    }
-    return cluster_ok_[cs] > 0;
-}
-
-// how many of the prepared slots first, first+1, ... (at most limit) can go into ONE cluster launch: 0 if the first
-// cannot.  Different problems of such a launch need not be co-resident (a cluster is scheduled as a unit, the problems do
-// not talk to each other), so the only limit is that a cluster must be schedulable at all.
-int ResidentSolver::cluster_run(int first, int limit) const
-{
-    if (!cluster_barrier_) return 0;
-    int n = 0;
-    while (n < limit && first + n < (int)slots_.size() && slots_[first + n].fits && slots_[first + n].cluster_ctas > 0) ++n;
-    return n;
-}
-
-void ResidentSolver::enqueue_cluster(int first, int count, int nCont, int nGN, int nPCG, cudaStream_t stream)
-{
-    const int max_warps = RS_THREADS_MAX / 32;
-    int cs = 1, nmax = 0;
-    for (int i = 0; i < count; ++i) {
-        cs = std::max(cs, slots_[first + i].cluster_ctas);
-        nmax = std::max(nmax, slots_[first + i].n_strips);
-    }
-    int nw = std::max(4, (nmax + cs - 1) / cs); // strips of the largest problem per CTA (balanced split)
-    if (nw > max_warps) arap_fail(1, "cluster launch: %d strips do not fit %d CTAs", nmax, cs);
-    std::vector<ResProb> host(count);
-    for (int i = 0; i < count; ++i) {
-        Slot& sl = slots_[first + i];
-        sl.prob.G = cs; // every problem of the launch spreads over the whole cluster
-        sl.prob.nCont = nCont; sl.prob.nGN = nGN; sl.prob.nPCG = nPCG;
-        sl.prob.pcg_rtol2 = pcg_rtol_ * pcg_rtol_;
-        sl.prob.gn_rtol = gn_rtol_;
-        sl.prob.prof = nullptr;
-        host[i] = sl.prob;
-        // halo tags start at 1, so a zeroed outbox is "nothing published yet" (the L2 barrier words are not used)
-        ARAP_CUDA_CHECK(cudaMemsetAsync(sl.d_outbox, 0,
-                                        (size_t)(sl.n_strips > 0 ? sl.n_strips : 1) * RS_OUTBOX_ENTRIES * 2 * sizeof(uint4), stream));
-    }
-    ARAP_CUDA_CHECK(cudaMemcpyAsync(d_probs_ + first, host.data(), count * sizeof(ResProb), cudaMemcpyHostToDevice, stream));
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = dim3((unsigned)(cs * count), 1, 1);
-    cfg.blockDim = dim3((unsigned)(nw * 32), 1, 1);
-    cfg.dynamicSmemBytes = (size_t)nw * sizeof(StripSmem);
-    cfg.stream = stream;
-    cudaLaunchAttribute attr[1];
-    attr[0].id = cudaLaunchAttributeClusterDimension;
-    attr[0].val.clusterDim.x = (unsigned)cs;
-    attr[0].val.clusterDim.y = 1;
-    attr[0].val.clusterDim.z = 1;
-    cfg.attrs = attr;
-    cfg.numAttrs = 1;
-    const ResProb* dp = d_probs_ + first;
-    last_variant_ = -1;
-    last_shape_[0] = RS_THREADS_MAX; last_shape_[1] = 0; // min CTAs/SM "0" marks the cluster kernel
-    last_shape_[2] = cs * count; last_shape_[3] = 1; last_shape_[4] = nw * 32;
-    ARAP_CUDA_CHECK(cudaLaunchKernelEx(&cfg, g_cluster_fn, dp));
-    launches_ += 1;
-}
-
 void ResidentSolver::enqueue(float2* X, float* A, const float2* C, int lerp_mode, float wf, float wr, int nCont, int nGN,
                              int nPCG, float* d_costs, float* d_trace, cudaStream_t stream)
 {
     set_problem(0, X, A, C, lerp_mode, wf, wr, d_costs, d_trace);
-    if (cluster_run(0, 1) == 1 && !d_prof_) enqueue_cluster(0, 1, nCont, nGN, nPCG, stream);
-    else enqueue_group(0, 1, nCont, nGN, nPCG, stream);
+    enqueue_group(0, 1, nCont, nGN, nPCG, stream);
 }
 
 int ResidentSolver::status(cudaStream_t stream)

@@ -65,12 +65,6 @@ public:
     // how many of the prepared slots first, first+1, ... can be co-resident in one launch (>= 1)
     int group_size(int first, int limit) const;
     void enqueue_group(int first, int count, int nCont, int nGN, int nPCG, cudaStream_t stream);
-    // small problems (each fits one thread-block cluster): cluster-scope barrier through distributed shared memory, any
-    // number of problems per launch.  cluster_run = how many consecutive prepared slots qualify (0: use enqueue_group).
-    int cluster_run(int first, int limit) const;
-    void enqueue_cluster(int first, int count, int nCont, int nGN, int nPCG, cudaStream_t stream);
-    void set_cluster_barrier(bool on) { cluster_barrier_ = on; }
-    int cluster_ctas(int slot = 0) const { return slots_[slot].cluster_ctas; }
 
     // after the stream has been synchronised: non-zero = the kernel bailed out (watchdog)
     int status(cudaStream_t stream);
@@ -91,7 +85,6 @@ public:
 private:
     struct Slot {
         int W = 0, H = 0, SX = 0, SY = 0, n_strips = 0, G = 0, NW = 0;
-        int cluster_ctas = 0; // > 0: the problem fits one cluster of that many CTAs
         bool fits = false;
         const float* d_M = nullptr;
         int2* d_strip_xy = nullptr;
@@ -113,9 +106,6 @@ private:
     int last_variant_ = -1;
     int last_shape_[5] = {0, 0, 0, 0, 0};
     float pcg_rtol_ = 0.0f, gn_rtol_ = 0.0f;
-    bool cluster_barrier_ = false; // measured slower than the L2 barrier with co-residency (DESIGN.md 4.1): opt-in
-    bool cluster_schedulable(int cs);
-    signed char cluster_ok_[17] = {0}; // per cluster size: 0 unknown, 1 yes, -1 no
 };
 
 } // namespace arapb200

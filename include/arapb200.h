@@ -216,9 +216,8 @@ ARAPB200_API int arapb200_batch_launch_info(arapb200_batch* b, int* info6);
  *   "gn_rtol": 0 <= value < 1.  > 0: the Gauss-Newton steps of a continuation step end as soon as one of them lowers
  *   the cost by less than value (relative) instead of always running nIterations steps; the skipped entries of
  *   out_costs repeat the last cost.  Same scope and caveats as "pcg_rtol" (both back-ends).
- *   "cluster_barrier": 1 = problems that fit one thread-block cluster (<= 16 CTAs of <= 12 strips) run with a cluster-scope
- *   barrier (limb sums pushed through distributed shared memory, mbarrier completion); 0 (default) = every resident
- *   problem uses the L2 barrier.  Same results bit for bit; measured slower on B200 (DESIGN.md 4.1), kept as an option.
+ *   "cluster_barrier": accepted for compatibility, any value, no effect: every resident problem uses the L2 barrier.  The
+ *   cluster-scope barrier it once selected gave the same bits and was slower on every workload (DESIGN.md 4.1).
  *   "lm": 1 = every Opt_ProblemSolve of the schedule is run by the reference's other solver kind, "LMGPU"
  *   (Levenberg-Marquardt trust region, Q-based exit of the linear loops, step acceptance / revert;
  *   ARAP/API/src/solverGPUGaussNewton.t with UsesLambda()) with its default solver parameters (:26-39), one problem at a

@@ -216,27 +216,26 @@ def energy_bound(E, E_start):
 
 
 # ---- the resident back-end's launch arithmetic, mirrored (solver_resident.cu: k_strip_active, prepare_finish) ----
-STRIP_W, STRIP_H, MAX_WARPS, CLUSTER_MAX_CTAS, MAX_CTAS = 32, 8, 12, 16, 160
+STRIP_W, STRIP_H, MAX_WARPS, MAX_CTAS = 32, 8, 12, 160
 
 
 def strip_count(mask, sms):
     """Strips (32x8 tiles with at least one object pixel), warps per CTA (NW), CTAs (G) and whether the problem fits on
-    chip on a device with `sms` SMs; `cluster` is the cluster size the cluster-scope barrier would use (0: too large).
-    Occupancy (pick_variant) is not mirrored: a problem that passes these checks can still be refused by it."""
+    chip on a device with `sms` SMs.  Occupancy (pick_variant) is not mirrored: a problem that passes these checks can
+    still be refused by it."""
     H, W = mask.shape
     SX, SY = -(-W // STRIP_W), -(-H // STRIP_H)
     act = np.zeros((SY * STRIP_H, SX * STRIP_W), bool)
     act[:H, :W] = mask == 0
     n = int(act.reshape(SY, STRIP_H, SX, STRIP_W).any(axis=(1, 3)).sum())
     if n == 0:
-        return dict(strips=0, NW=1, G=1, fits=True, cluster=0)
-    cluster = -(-n // MAX_WARPS) if n <= CLUSTER_MAX_CTAS * MAX_WARPS else 0
+        return dict(strips=0, NW=1, G=1, fits=True)
     NW = max(4, -(-n // sms))
     if NW > MAX_WARPS:
-        return dict(strips=n, NW=NW, G=0, fits=False, cluster=cluster)
+        return dict(strips=n, NW=NW, G=0, fits=False)
     G = min(-(-n // NW), sms)
     fits = G <= MAX_CTAS and -(-n // G) <= NW
-    return dict(strips=n, NW=NW, G=G, fits=fits, cluster=cluster)
+    return dict(strips=n, NW=NW, G=G, fits=fits)
 
 
 def epe(a, b, sel=None):

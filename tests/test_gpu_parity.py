@@ -559,10 +559,9 @@ def test_conditioning_bounds_the_gap_to_any_rounding_order():
     assert res["worst_mean_epe_px"] < 1e-4 and res["worst_rel_cost_diff"] < 1e-5, res
 
 
-def test_cluster_scope_barrier_equals_l2_barrier(oracle):
-    """Opt-in: small problems (each fits one thread-block cluster) run with a cluster-scope barrier -- limb sums pushed
-    through distributed shared memory, mbarrier completion -- instead of the L2 barrier.  Same bits as the L2 path and as the
-    oracle; any number of problems per launch; mixed with a large problem in one batch."""
+def test_cluster_barrier_option_is_a_no_op(oracle):
+    """The retired option "cluster_barrier" is still accepted and changes nothing: the same outputs and the same launch
+    with 1 as with 0, bit-exact against the oracle.  Then small problems in one batch with a problem of C1 size."""
     sps = [synth.synth(160, 120, 1, 2, 500 + i) for i in range(5)] + [synth.synth(320, 200, 2, 3, 600)]
     jobs = [(s, s.masks[0]) for s in sps] + [(sps[-1], sps[-1].masks[1])]
     kw = dict(nCont=2, nGN=2, nPCG=60)
@@ -572,22 +571,19 @@ def test_cluster_scope_barrier_equals_l2_barrier(oracle):
         b.set_option("cluster_barrier", mode)
         outs = [b.submit(i, s.rgb, m, s.matches) for i, (s, m) in enumerate(jobs)]
         b.run()
-        info = b.launch_info()
-        res[mode] = ([{k: v.copy() for k, v in o.items()} for o in outs], info)
-    assert res[1][1]["variant"][1] == 0 and res[1][1]["problems_per_launch"] == len(jobs), res[1][1]   # ONE cluster launch
-    assert res[0][1]["variant"][1] != 0, res[0][1]
+        res[mode] = ([{k: v.copy() for k, v in o.items()} for o in outs], b.launch_info(), b.resident_count())
+    assert res[1][1] == res[0][1] and res[1][2] == res[0][2] == len(jobs), (res[1][1:], res[0][1:])
     for a, c in zip(res[1][0], res[0][0]):
-        assert _eq(a["flow"], c["flow"]) and _eq(a["costs"], c["costs"]) and _eq(a["rgb"], c["rgb"])
-    for o, (s, m) in zip(res[1][0], jobs):
+        assert a.keys() == c.keys() and all(_eq(a[k], c[k]) for k in a)
+    for o, (s, m) in zip(res[0][0], jobs):
         Xo, Ao, co = oracle.solve(m, s.matches, **kw)
         assert _eq(o["flow"], oracle.flow(Xo)) and _eq(o["costs"], co)
     b.close()
-    # a batch that mixes small problems with one that needs the L2 barrier (C1 size)
+    # small problems in one batch with a problem of C1 size
     big = synth.config("C1")
     small = synth.synth(854, 480, 1, 1, 77, axes=(0.1, 0.1))
     kw = dict(nCont=1, nGN=1, nPCG=30)
     b = lib.Batch(854, 480, 3, **kw)
-    b.set_option("cluster_barrier", 1)
     outs = [b.submit(0, small.rgb, small.masks[0], small.matches), b.submit(1, big.rgb, big.masks[0], big.matches),
             b.submit(2, small.rgb, small.masks[0], small.matches)]
     b.run()

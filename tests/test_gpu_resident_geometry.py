@@ -1,7 +1,7 @@
 """The resident back-end on the mask geometries real segments produce (objects on the image border, holes, many
 components, one-pixel lines, isolated pixels, ragged masks, images smaller than one strip) and on the launch shapes they
-select (warps per CTA, co-resident variants, the on-chip limit, mixed batches, the cluster-scope barrier).  Every
-comparison is bit-exact against the CPU oracle, computed here from seeds."""
+select (warps per CTA, co-resident variants, the on-chip limit, mixed batches, tiny problems).  Every comparison is
+bit-exact against the CPU oracle, computed here from seeds."""
 import numpy as np
 import pytest
 
@@ -175,7 +175,7 @@ def test_on_chip_limit(oracle, sms):
     kw = dict(nCont=1, nGN=1, nPCG=20)
     job = _job(fit, 3)
     exp = strip_count(fit, sms)
-    assert exp == dict(strips=12 * sms, NW=12, G=sms, fits=True, cluster=0)
+    assert exp == dict(strips=12 * sms, NW=12, G=sms, fits=True)
     (o,), info, nres = _run([job], kw)
     assert nres == 1
     _expect_launch(info, exp)
@@ -234,18 +234,18 @@ def test_mixed_batch_streaming_between_resident(oracle, sms):
         _check_vs_oracle(oracle, o, j, kw)
 
 
-def test_cluster_barrier_tiny_and_border_problems(oracle, sms):
-    """Opt-in cluster-scope barrier: 1-strip problems spread over a cluster sized for the largest problem of the launch,
-    so most of their CTAs own no strip; border-touching problems in the same launch."""
+def test_tiny_and_border_problems_one_launch(oracle, sms):
+    """1-strip problems (one of them a 5x3 image) and border-touching ones share one launch: one CTA each for the tiny
+    problems, ragged CTA counts on the compact grid."""
     jobs = [_job(MASKS["single"](203, 77, 1), 1), _job(MASKS["full"](5, 3), 2), _job(MASKS["border_all"](203, 77, 3), 3),
             _job(MASKS["lines"](150, 97, 4), 4), _job(MASKS["pixels"](203, 77, 5), 5)]
     exps = [strip_count(j["mask"], sms) for j in jobs]
-    cs = max(e["cluster"] for e in exps)
-    nmax = max(e["strips"] for e in exps)
-    assert all(e["cluster"] > 0 for e in exps) and cs > 1
-    outs, info, nres = _run(jobs, SCHED, options=[("cluster_barrier", 1)], maxWH=(203, 97))
+    assert all(e["fits"] and e["NW"] == 4 for e in exps) and exps[0]["strips"] == exps[1]["strips"] == 1
+    Gs = [e["G"] for e in exps]
+    grid = (Gs[0], len(jobs)) if len(set(Gs)) == 1 else (sum(Gs), 1)
+    outs, info, nres = _run(jobs, SCHED, maxWH=(203, 97))
     assert nres == len(jobs)
-    _expect_launch(info, dict(NW=max(4, -(-nmax // cs))), problems=len(jobs), variant=(384, 0), grid=(cs * len(jobs), 1))
+    _expect_launch(info, dict(NW=4), problems=len(jobs), grid=grid)
     for o, j in zip(outs, jobs):
         _check_vs_oracle(oracle, o, j, SCHED)
 

@@ -166,9 +166,9 @@ def test_three_c2_scenes_and_plain_problems_in_one_run():
 
 
 # ------------------------------------------------------------------------------------- 6: solver paths
-@pytest.mark.parametrize("kind", ["stream", "lm", "cluster_barrier"])
+@pytest.mark.parametrize("kind", ["stream", "lm", "resident_small"])
 def test_solver_paths(kind):
-    sp = synth.synth(160, 120, 2, 2, 90) if kind != "cluster_barrier" else synth.synth(96, 80, 2, 2, 91)
+    sp = synth.synth(160, 120, 2, 2, 90) if kind != "resident_small" else synth.synth(96, 80, 2, 2, 91)
     matches = [sp.matches] * 2
     A, bg, origin = _moving(sp, 40)
     steps = [0, 3, 5]
@@ -176,13 +176,11 @@ def test_solver_paths(kind):
     b = lib.Batch(sp.W, sp.H, 2, backend=lib.BACKEND_STREAM if kind == "stream" else lib.BACKEND_AUTO, **KW)
     if kind == "lm":
         b.set_option("lm", 1)
-    if kind == "cluster_barrier":
-        b.set_option("cluster_barrier", 1)
     want = _host(b, sp.rgb, sp.masks, matches, bg, A, origin, steps, path)
     got = b.submit_scene(0, sp.rgb, sp.masks, matches, bg, A, origin=origin, frames=steps, frame_motions=path)
     b.run()
-    if kind == "cluster_barrier":
-        assert b.launch_info()["variant"][1] == 0 and b.resident_count() == 2   # min CTAs/SM 0: the cluster kernel
+    if kind == "resident_small":
+        assert b.resident_count() == 2
     else:
         assert b.resident_count() == 0
     b.close()

@@ -147,14 +147,13 @@ def test_batch_frames_c2_segments_compact_grid_and_flatten(oracle):
     b.close()
 
 
-def test_batch_frames_small_problems_cluster_barrier(oracle):
+def test_batch_frames_small_problems_one_launch(oracle):
     sps = [synth.synth(96, 80, 1, 2, 60 + i) for i in range(3)]
     b = lib.Batch(96, 80, 3, **KW)
-    b.set_option("cluster_barrier", 1)
     outs = [b.submit(i, s.rgb, s.masks[0], s.matches, frames=STEPS[i % 2]) for i, s in enumerate(sps)]
     b.run()
     info = b.launch_info()
-    assert info["variant"][1] == 0 and b.resident_count() == 3, info    # min CTAs/SM 0 marks the cluster kernel
+    assert info["problems_per_launch"] == 3 and b.resident_count() == 3, info
     for i, (o, s) in enumerate(zip(outs, sps)):
         _check_problem(o, s.rgb, s.masks[0], s.matches, STEPS[i % 2])
     b.close()
