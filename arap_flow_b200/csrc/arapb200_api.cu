@@ -4,6 +4,7 @@
 #include "devmem.cuh"
 #include "pipeline.cuh"
 
+#include <algorithm>
 #include <cmath>
 #include <cstring>
 #include <memory>
@@ -307,6 +308,8 @@ int arapb200_batch_submit_scene(arapb200_batch* b, int slot, int n_layers, int W
         sc.out_occ = out_occ; sc.out_rgb0 = out_rgb0;
         sc.seq_rgb = seq_rgb; sc.seq_mask = seq_mask; sc.seq_flow = seq_flow; sc.seq_bflow = seq_bflow;
         sc.seq_occ = seq_occ;
+        sc.motions.assign(motion, motion + 6);
+        if (n_frames > 0) sc.motions.insert(sc.motions.end(), frame_motions, frame_motions + 6 * (size_t)n_frames);
         const size_t cn = (size_t)b->nCont * (b->nGN + 1);
         for (int s = 0; s < n_layers; ++s) {
             HostProblem& hp = b->slots[slot + s];
@@ -322,6 +325,72 @@ int arapb200_batch_submit_scene(arapb200_batch* b, int slot, int n_layers, int W
         b->scenes.push_back(std::move(sc));
         return 0;
     });
+}
+
+int arapb200_batch_scene_blur(arapb200_batch* b, int slot, int n_samples, double shutter, uint8_t* blur_rgb,
+                              uint8_t* blur_rgb0, uint8_t* seq_blur_rgb)
+{
+    return guarded([&]() -> int {
+        // every rejection comes before the scene is changed
+        if (!b || slot < 0 || slot >= b->max_problems) return 1;
+        const int q = b->scene_of[slot];
+        if (q < 0 || b->scenes[q].first != slot) {
+            fprintf(stderr, "arapb200: batch_scene_blur: slot %d is not the first slot of a queued scene\n", slot);
+            return 1;
+        }
+        HostScene& sc = b->scenes[q];
+        const int K = (int)(sc.maps.size() / 18) - 1;
+        if (n_samples < 1 || n_samples > BLUR_MAX_SAMPLES || !(shutter >= 0.0 && shutter <= 1.0) || !blur_rgb ||
+            (blur_rgb0 && !sc.out_rgb0) || (seq_blur_rgb && K == 0)) {
+            fprintf(stderr, "arapb200: batch_scene_blur: bad request (%d samples, shutter %g, null blur_rgb, or a frame-0 "
+                    "or frame output the scene does not have)\n", n_samples, shutter);
+            return 1;
+        }
+        const std::vector<int>& steps = b->slots[slot].steps;
+        std::vector<BlurSub> tab((size_t)(K + 2) * n_samples);
+        for (int image = -1; image <= K; ++image) {
+            if ((image < 0 && !blur_rgb0) || (image > 0 && !seq_blur_rgb)) continue;
+            if (!blur_schedule(b->nCont, K, steps.data(), sc.motions.data(), sc.motions.data() + 6, n_samples, shutter,
+                               image, tab.data() + (size_t)(image + 1) * n_samples)) {
+                fprintf(stderr, "arapb200: batch_scene_blur: image %d has a non-finite or singular sub-frame motion\n",
+                        image);
+                return 1;
+            }
+        }
+        std::vector<int> states; // what the sub-frames read: j0 unless w == 1, j0 + 1 unless w == 0; never the grid
+        for (int image = -1; image <= K; ++image) {
+            if ((image < 0 && !blur_rgb0) || (image > 0 && !seq_blur_rgb)) continue;
+            for (int j = 0; j < n_samples; ++j) {
+                const BlurSub& e = tab[(size_t)(image + 1) * n_samples + j];
+                if (e.w != 1.f && e.j0 >= 0) states.push_back(e.j0);
+                if (e.w != 0.f) states.push_back(e.j0 + 1);
+            }
+        }
+        std::sort(states.begin(), states.end());
+        states.erase(std::unique(states.begin(), states.end()), states.end());
+        sc.blur_S = n_samples;
+        sc.blur.swap(tab);
+        sc.blur_states.swap(states);
+        sc.blur_rgb = blur_rgb;
+        sc.blur_rgb0 = blur_rgb0;
+        sc.seq_blur_rgb = seq_blur_rgb;
+        return 0;
+    });
+}
+
+int arapb200_blur_schedule(int nCont, int n_frames, const int* steps, const double* motion,
+                           const double* frame_motions, int n_samples, double shutter, int image, int* out_state,
+                           float* out_w, float* out_smap)
+{
+    if (!out_state || !out_w || !out_smap || n_samples < 1 || n_samples > BLUR_MAX_SAMPLES) return 1;
+    BlurSub tab[BLUR_MAX_SAMPLES];
+    if (!blur_schedule(nCont, n_frames, steps, motion, frame_motions, n_samples, shutter, image, tab)) return 1;
+    for (int j = 0; j < n_samples; ++j) {
+        out_state[j] = tab[j].j0;
+        out_w[j] = tab[j].w;
+        std::copy(tab[j].smap, tab[j].smap + 6, out_smap + 6 * j);
+    }
+    return 0;
 }
 
 int arapb200_batch_run(arapb200_batch* b)
@@ -341,7 +410,10 @@ int arapb200_batch_run(arapb200_batch* b)
         std::vector<HostScene> scenes;
         scenes.swap(b->scenes);
         b->scene_of.assign(b->max_problems, -1);
-        for (HostScene& sc : scenes) sc.first = at[sc.first]; // a scene's slots are consecutive and all pending
+        for (HostScene& sc : scenes) {
+            sc.first = at[sc.first]; // a scene's slots are consecutive and all pending
+            for (int s = 0; s < sc.n; ++s) b->todo[sc.first + s].blur_states = sc.blur_states;
+        }
         const int rc = b->pipe->run(b->todo.data(), (int)b->todo.size(), scenes.data(), (int)scenes.size());
         if (rc) return rc;
         b->ms[0] = b->pipe->last_ms_total();

@@ -61,35 +61,6 @@ __global__ void __launch_bounds__(256) k_flatten(int W, int H, Layers L, const u
 }
 
 // ---- background motion (DESIGN.md 4.5): the composite of the layers over an affinely moving background ----
-struct Affine {
-    float m00, m01, m02, m10, m11, m12;
-};
-
-__device__ __forceinline__ float2 affine_at(const Affine& M, int x, int y)
-{
-    const float fx = (float)x, fy = (float)y;
-    return make_float2(__fadd_rn(__fadd_rn(__fmul_rn(M.m00, fx), __fmul_rn(M.m01, fy)), M.m02),
-                       __fadd_rn(__fadd_rn(__fmul_rn(M.m10, fx), __fmul_rn(M.m11, fy)), M.m12));
-}
-
-// bilinear sample of the uint8x3 background at s, coordinates clamped to the image (NaN -> 0)
-__device__ __forceinline__ void sample_bg(const unsigned char* __restrict__ bg, int bgW, int bgH, float2 s,
-                                          unsigned char* __restrict__ out)
-{
-    const float sx = fminf(fmaxf(s.x, 0.f), (float)(bgW - 1)), sy = fminf(fmaxf(s.y, 0.f), (float)(bgH - 1));
-    const int x0 = (int)floorf(sx), y0 = (int)floorf(sy);
-    const int x1 = min(x0 + 1, bgW - 1), y1 = min(y0 + 1, bgH - 1);
-    const float fx = __fsub_rn(sx, (float)x0), fy = __fsub_rn(sy, (float)y0);
-    const float gx = __fsub_rn(1.f, fx), gy = __fsub_rn(1.f, fy);
-    const unsigned char* r0 = bg + 3 * (size_t)y0 * bgW;
-    const unsigned char* r1 = bg + 3 * (size_t)y1 * bgW;
-    for (int c = 0; c < 3; ++c) {
-        const float top = __fadd_rn(__fmul_rn((float)r0[3 * x0 + c], gx), __fmul_rn((float)r0[3 * x1 + c], fx));
-        const float bot = __fadd_rn(__fmul_rn((float)r1[3 * x0 + c], gx), __fmul_rn((float)r1[3 * x1 + c], fx));
-        out[c] = (unsigned char)min(255, __float2int_rn(__fadd_rn(__fmul_rn(top, gy), __fmul_rn(bot, fy))));
-    }
-}
-
 // frame-b pass: colour, mask and backward flow of the composite.  S: frame-b pixel -> background plane, B: frame-b
 // pixel -> frame a.  out_bflow may be null (no extras).
 __global__ void __launch_bounds__(256) k_composite_b(int W, int H, Layers L, const unsigned char* __restrict__ bg,
@@ -357,17 +328,11 @@ extern "C" int arapb200_flatten_ex(int W, int H, int n_layers, const float* cons
 
 namespace arapb200 {
 namespace {
-// 2x3 affine maps in binary64, row-major: (a00 a01 a02; a10 a11 a12).  The derivation of DESIGN.md 4.5, in its order;
-// fp-contract=off keeps a host compiler from fusing a product and a sum where the target has FMA.
+// 2x3 affine maps in binary64, row-major: (a00 a01 a02; a10 a11 a12).  The derivation of DESIGN.md 4.5, in its order
+// (ARAP_NO_CONTRACT, composite.cuh).
 struct Aff64 {
     double a[6];
 };
-
-#if defined(__GNUC__) && !defined(__clang__)
-#define ARAP_NO_CONTRACT __attribute__((optimize("fp-contract=off")))
-#else
-#define ARAP_NO_CONTRACT
-#endif
 
 ARAP_NO_CONTRACT Aff64 aff_inverse(const Aff64& A, double* det)
 {

@@ -3,6 +3,14 @@
 #pragma once
 #include "common.cuh"
 
+// fp-contract=off keeps a host compiler from fusing a product and a sum where the target has FMA: the host derivations
+// of the maps (DESIGN.md 4.5) and of the blur schedule (4.8) are binary64 in a documented order
+#if defined(__GNUC__) && !defined(__clang__)
+#define ARAP_NO_CONTRACT __attribute__((optimize("fp-contract=off")))
+#else
+#define ARAP_NO_CONTRACT
+#endif
+
 namespace arapb200 {
 
 constexpr int MAX_LAYERS = 32;
@@ -30,5 +38,37 @@ void enqueue_composite(int W, int H, const Layers& L, bool src_prev, const unsig
 // q + (bg_x, bg_y), coordinates clamped to the image as the composite clamps them
 void enqueue_scene_input(int W, int H, const Layers& L, const unsigned char* d_rgb, const unsigned char* d_bg, int bgW,
                          int bgH, int bg_x, int bg_y, unsigned char* d_out, cudaStream_t stream);
+
+#ifdef __CUDACC__
+// a 2x3 map rounded to binary32, shared by the composite and the motion blur (DESIGN.md 4.5, 4.8)
+struct Affine {
+    float m00, m01, m02, m10, m11, m12;
+};
+
+__device__ __forceinline__ float2 affine_at(const Affine& M, int x, int y)
+{
+    const float fx = (float)x, fy = (float)y;
+    return make_float2(__fadd_rn(__fadd_rn(__fmul_rn(M.m00, fx), __fmul_rn(M.m01, fy)), M.m02),
+                       __fadd_rn(__fadd_rn(__fmul_rn(M.m10, fx), __fmul_rn(M.m11, fy)), M.m12));
+}
+
+// bilinear sample of the uint8x3 background at s, coordinates clamped to the image (NaN -> 0)
+__device__ __forceinline__ void sample_bg(const unsigned char* __restrict__ bg, int bgW, int bgH, float2 s,
+                                          unsigned char* __restrict__ out)
+{
+    const float sx = fminf(fmaxf(s.x, 0.f), (float)(bgW - 1)), sy = fminf(fmaxf(s.y, 0.f), (float)(bgH - 1));
+    const int x0 = (int)floorf(sx), y0 = (int)floorf(sy);
+    const int x1 = min(x0 + 1, bgW - 1), y1 = min(y0 + 1, bgH - 1);
+    const float fx = __fsub_rn(sx, (float)x0), fy = __fsub_rn(sy, (float)y0);
+    const float gx = __fsub_rn(1.f, fx), gy = __fsub_rn(1.f, fy);
+    const unsigned char* r0 = bg + 3 * (size_t)y0 * bgW;
+    const unsigned char* r1 = bg + 3 * (size_t)y1 * bgW;
+    for (int c = 0; c < 3; ++c) {
+        const float top = __fadd_rn(__fmul_rn((float)r0[3 * x0 + c], gx), __fmul_rn((float)r0[3 * x1 + c], fx));
+        const float bot = __fadd_rn(__fmul_rn((float)r1[3 * x0 + c], gx), __fmul_rn((float)r1[3 * x1 + c], fx));
+        out[c] = (unsigned char)min(255, __float2int_rn(__fadd_rn(__fmul_rn(top, gy), __fmul_rn(bot, fy))));
+    }
+}
+#endif
 
 } // namespace arapb200

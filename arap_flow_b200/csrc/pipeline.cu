@@ -107,6 +107,23 @@ struct SceneLayout {
     }
 };
 
+// a blurred scene's scratch: [z: one z-buffer per layer][acc: ushort4 per pixel][rgb][rgb0][seq: K frames], the last
+// three the blurred images asked for (DESIGN.md 4.8)
+struct BlurLayout {
+    size_t z, acc, rgb, rgb0, seq, bytes;
+    explicit BlurLayout(const HostScene& sc)
+    {
+        const size_t N = (size_t)sc.W * sc.H, K = sc.maps.size() / 18 - 1;
+        Layout l;
+        z = l.take(4 * N * sc.n);
+        acc = l.take(sizeof(ushort4) * N);
+        rgb = l.take(3 * N);
+        rgb0 = l.take(sc.blur_rgb0 ? 3 * N : 0);
+        seq = l.take(sc.seq_blur_rgb ? 3 * N * K : 0);
+        bytes = l.bytes();
+    }
+};
+
 } // namespace
 
 void enqueue_reset_state(int W, int H, const unsigned char* d_mask_red, float2* d_X, float2* d_U, float* d_A,
@@ -170,11 +187,15 @@ BatchPipeline::~BatchPipeline()
 
 void BatchPipeline::snapshot(const HostProblem& hp, Dev& d, int t)
 {
-    const auto it = std::lower_bound(hp.steps.begin(), hp.steps.end(), t);
-    if (it == hp.steps.end() || *it != t) return;
     const size_t N = (size_t)hp.W * hp.H;
-    ARAP_CUDA_CHECK(cudaMemcpyAsync(d.seq_pos + (size_t)(it - hp.steps.begin()) * N, d.X.p, N * sizeof(float2),
-                                    cudaMemcpyDeviceToDevice, stream_));
+    auto copy = [&](const std::vector<int>& list, float2* dst) {
+        const auto it = std::lower_bound(list.begin(), list.end(), t);
+        if (it == list.end() || *it != t) return;
+        ARAP_CUDA_CHECK(cudaMemcpyAsync(dst + (size_t)(it - list.begin()) * N, d.X.p, N * sizeof(float2),
+                                        cudaMemcpyDeviceToDevice, stream_));
+    };
+    copy(hp.steps, d.seq_pos);
+    copy(hp.blur_states, d.blur_pos);
 }
 
 // the streaming back-end: one graph launch per Gauss-Newton step (problems too large for the chip)
@@ -252,7 +273,8 @@ void BatchPipeline::solve_resident(const HostProblem* problems, int first, int c
 {
     const float wf = sqrtf(100.0f), wr = sqrtf(0.01f); // CombinedSolver.h:172-177
     bool frames = false;
-    for (int j = 0; j < count; ++j) frames = frames || !problems[first + j].steps.empty();
+    for (int j = 0; j < count; ++j)
+        frames = frames || !problems[first + j].steps.empty() || !problems[first + j].blur_states.empty();
     if (!frames) { // the whole schedule in one launch; the kernel lerps the constraints itself (lerp_mode 1)
         for (int j = 0; j < count; ++j) {
             Dev& dj = dev_[first + j];
@@ -264,8 +286,8 @@ void BatchPipeline::solve_resident(const HostProblem* problems, int first, int c
         resident_->enqueue_group(first, count, nCont_, nGN_, nPCG_, stream_);
         return;
     }
-    // Frames need X after individual continuation steps: one launch per step, on the constraint image of that step as the
-    // streaming path builds it (lerp_mode 0), the same bits as the single launch (DESIGN.md 4.4)
+    // Frames and blur need X after individual continuation steps: one launch per step, on the constraint image of that
+    // step as the streaming path builds it (lerp_mode 0), the same bits as the single launch (DESIGN.md 4.4)
     for (int t = 0; t < nCont_; ++t) {
         const float alpha = (float)(t + 1) / (float)nCont_; // CombinedSolver.h:199-201
         for (int j = 0; j < count; ++j) {
@@ -323,6 +345,40 @@ void BatchPipeline::enqueue_scene(const HostScene& sc, unsigned char* buf)
     }
 }
 
+// per image asked for (frame 0, the pair, frames 1 .. K) its S sub-frames, each lerping every layer between two of its
+// blur snapshots (DESIGN.md 4.8); w == 0 and w == 1 read one state, which then stands for both
+void BatchPipeline::enqueue_scene_blur(const HostScene& sc, const unsigned char* scene_buf, unsigned char* buf)
+{
+    const BlurLayout o(sc);
+    const size_t N = (size_t)sc.W * sc.H;
+    const int K = (int)(sc.maps.size() / 18) - 1, S = sc.blur_S;
+    const unsigned char* bg = scene_buf + SceneLayout(sc).bg;
+    auto state = [&](int s, int t) -> const float2* { // null = the pixel grid
+        if (t < 0) return nullptr;
+        const auto it = std::lower_bound(sc.blur_states.begin(), sc.blur_states.end(), t);
+        return dev_[sc.first + s].blur_pos + (size_t)(it - sc.blur_states.begin()) * N;
+    };
+    BlurLayers L{};
+    L.n = sc.n;
+    for (int s = 0; s < sc.n; ++s) L.mask_red[s] = dev_[sc.first + s].mask.p;
+    for (int image = -1; image <= K; ++image) {
+        unsigned char* out = image < 0    ? (sc.blur_rgb0 ? buf + o.rgb0 : nullptr)
+                             : image == 0 ? buf + o.rgb
+                                          : (sc.seq_blur_rgb ? buf + o.seq + 3 * N * (image - 1) : nullptr);
+        if (!out) continue;
+        for (int j = 0; j < S; ++j) {
+            const BlurSub& b = sc.blur[(size_t)(image + 1) * S + j];
+            for (int s = 0; s < sc.n; ++s) {
+                L.qa[s] = b.w == 1.f ? state(s, b.j0 + 1) : state(s, b.j0);
+                L.qb[s] = b.w == 0.f ? L.qa[s] : state(s, b.j0 + 1);
+            }
+            launches_ += enqueue_blur_subframe(sc.W, sc.H, L, b.w, b.smap, dev_[sc.first].rgb.p, bg, sc.bgW, sc.bgH,
+                                               sc.bg_x, sc.bg_y, (unsigned*)(buf + o.z), (ushort4*)(buf + o.acc), j,
+                                               S, out, stream_);
+        }
+    }
+}
+
 void BatchPipeline::set_pcg_rtol(float rtol)
 {
     pcg_rtol_ = rtol > 0.0f ? rtol : 0.0f;
@@ -375,11 +431,15 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
             d.seq_z = (unsigned*)(f + z);
             d.seq = SeqOut{f + rgb, f + mask, (float2*)(f + flow), (float2*)(f + bflow), f + occ, (float2*)(f + flow0)};
         }
+        if (!hp.blur_states.empty()) d.blur_pos = (float2*)d.blur.reserve(8 * N * hp.blur_states.size());
         memcpy(d.h_in.data(), hp.rgb, 3 * N);
         memcpy(d.h_in.data() + 3 * N, hp.mask_red, N);
     }
     if (n_scenes > (int)scene_dev_.size()) scene_dev_.resize(n_scenes);
     for (int j = 0; j < n_scenes; ++j) scene_dev_[j].reserve(SceneLayout(scenes[j]).bytes);
+    if (n_scenes > (int)blur_dev_.size()) blur_dev_.resize(n_scenes);
+    for (int j = 0; j < n_scenes; ++j)
+        if (scenes[j].blur_S) blur_dev_[j].reserve(BlurLayout(scenes[j]).bytes);
     ARAP_CUDA_CHECK(cudaEventRecord(ev_[0], stream_));
     for (int i = 0; i < count; ++i) {
         const HostProblem& hp = problems[i];
@@ -457,7 +517,10 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
             launches_ += enqueue_warp_seq(hp.W, hp.H, (int)hp.steps.size(), d.seq_pos, d.rgb.p, d.mask.p, d.seq_z, d.seq,
                                           stream_);
     }
-    for (int j = 0; j < n_scenes; ++j) enqueue_scene(scenes[j], scene_dev_[j].data());
+    for (int j = 0; j < n_scenes; ++j) {
+        enqueue_scene(scenes[j], scene_dev_[j].data());
+        if (scenes[j].blur_S) enqueue_scene_blur(scenes[j], scene_dev_[j].data(), blur_dev_[j].data());
+    }
     ARAP_CUDA_CHECK(cudaEventRecord(ev_[3], stream_));
     for (int i = 0; i < count; ++i) {
         const HostProblem& hp = problems[i];
@@ -498,6 +561,14 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
         for (const auto& c : out)
             if (c.dst && c.bytes)
                 ARAP_CUDA_CHECK(cudaMemcpyAsync(c.dst, b + c.off, c.bytes, cudaMemcpyDeviceToHost, stream_));
+        if (!sc.blur_S) continue;
+        const BlurLayout bl(sc);
+        const unsigned char* bb = blur_dev_[j].data();
+        const struct { void* dst; size_t off, bytes; } blurred[] = {
+            {sc.blur_rgb, bl.rgb, 3 * N}, {sc.blur_rgb0, bl.rgb0, 3 * N}, {sc.seq_blur_rgb, bl.seq, 3 * F}};
+        for (const auto& c : blurred)
+            if (c.dst && c.bytes)
+                ARAP_CUDA_CHECK(cudaMemcpyAsync(c.dst, bb + c.off, c.bytes, cudaMemcpyDeviceToHost, stream_));
     }
     ARAP_CUDA_CHECK(cudaStreamSynchronize(stream_));
     if (resident_ && n_resident_ > 0) {

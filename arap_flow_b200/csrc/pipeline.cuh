@@ -3,6 +3,7 @@
 // CombinedSolverBase.h:99-120) do around the solver, for many independent (image, segment) problems at once,
 // with every host<->device hop removed except the upload of the inputs and the download of the outputs.
 #pragma once
+#include "blur.cuh"
 #include "devmem.cuh"
 #include "plan.cuh"
 #include "warp.cuh"
@@ -30,6 +31,8 @@ struct HostProblem {
     // a layer of a HostScene: backward flow, occlusion and frames are computed and stay on the device; of the outputs
     // above only out_costs is copied out
     bool scene = false;
+    // a layer of a blurred scene: the continuation steps whose X its sub-frames read (sorted; DESIGN.md 4.8)
+    std::vector<int> blur_states;
 };
 
 // A scene (DESIGN.md 4.6): problems first .. first + n - 1 of a run are its layers in segment order (same W x H and rgb),
@@ -46,6 +49,14 @@ struct HostScene {
     float* out_bflow = nullptr;
     unsigned char *seq_rgb = nullptr, *seq_mask = nullptr, *seq_occ = nullptr;
     float *seq_flow = nullptr, *seq_bflow = nullptr;
+    std::vector<double> motions; // [1 + K][6]: A, then A_1 .. A_K, as submitted
+    // opt-in motion blur (DESIGN.md 4.8, arapb200_batch_scene_blur): blur_S sub-frames per image (0 = none); blur[(image
+    // + 1) * blur_S + j] is sub-frame j of image -1 (frame 0), 0 (the pair) or k (frame k), filled for the images asked
+    // for; blur_states: the continuation steps those sub-frames read, sorted
+    int blur_S = 0;
+    std::vector<BlurSub> blur;
+    std::vector<int> blur_states;
+    unsigned char *blur_rgb = nullptr, *blur_rgb0 = nullptr, *seq_blur_rgb = nullptr;
 };
 
 // compact constraint record: source pixel index and the match, after the reference's filtering
@@ -105,10 +116,13 @@ private:
         GrowBuf extras, h_extras{GrowBuf::Pinned};
         // opt-in frame sequence, allocated the first time the slot asks and regrown for a longer list
         GrowBuf frames;
+        // X after each of the blur states of a blurred scene's layer (8 B/px per state), regrown for a longer list
+        GrowBuf blur;
         // placed in the buffers above for the current run
         float2* bflow = nullptr;
         unsigned char* occ = nullptr;
         float2* seq_pos = nullptr; // X after each requested continuation step
+        float2* blur_pos = nullptr; // X after each blur state
         unsigned* seq_z = nullptr; // two z-buffers
         SeqOut seq{};
         std::vector<MatchRec> recs;
@@ -118,13 +132,19 @@ private:
     void solve_streaming(const HostProblem& hp, Dev& d);
     void solve_lm(const HostProblem& hp, Dev& d);
     // the resident problems first .. first + count - 1 in one cooperative launch per schedule, or per continuation step
-    // when one of them asks for frames
+    // when one of them asks for frames or blur states
     void solve_resident(const HostProblem* problems, int first, int count);
-    void snapshot(const HostProblem& hp, Dev& d, int t); // X -> frame buffer if step t is one hp asks for
+    // X -> frame buffer if step t is one of hp's frames, and -> blur buffer if it is one of its blur states
+    void snapshot(const HostProblem& hp, Dev& d, int t);
     // device buffer of the j-th scene of a run, allocated the first time and grown for a larger scene: the background,
     // frame 0 and the composited pair and frames (21 B/px each), laid out by SceneLayout (pipeline.cu)
     std::vector<GrowBuf> scene_dev_;
     void enqueue_scene(const HostScene& sc, unsigned char* buf); // the scene's kernels (DESIGN.md 4.6)
+    // the blurred scene at the j-th scene position, its scratch allocated the first time and grown for a larger scene:
+    // the layers' z-buffers (4 B/px each), the accumulator (8 B/px) and the blurred images (3 B/px each), laid out by
+    // BlurLayout (pipeline.cu)
+    std::vector<GrowBuf> blur_dev_;
+    void enqueue_scene_blur(const HostScene& sc, const unsigned char* scene_buf, unsigned char* buf); // DESIGN.md 4.8
     LmSolver* lm_ = nullptr;
     int lmW_ = 0, lmH_ = 0;
     bool lm_on_ = false;

@@ -30,6 +30,7 @@ ARAP_SYMBOLS = [
     "arapb200_batch_set_option", "arapb200_batch_resident_count", "arapb200_debug_wide_sum", "arapb200_plan_error", "arapb200_plan_lm_info", "arapb200_plan_timing_report",
     "arapb200_batch_launch_info", "arapb200_warp_ex", "arapb200_batch_submit_ex", "arapb200_flatten_ex",
     "arapb200_warp_seq", "arapb200_batch_submit_seq", "arapb200_composite", "arapb200_batch_submit_scene",
+    "arapb200_batch_scene_blur", "arapb200_blur_schedule",
 ]
 
 
@@ -299,6 +300,30 @@ def composite_seq(seqs, src_masks, background, motions, origin=(0, 0)):
     return {key: np.stack([f[key] for f in frames]) for key in frames[0]}
 
 
+BLUR_SCHEDULE_ARGTYPES = [C.c_int] * 2 + [C.c_void_p] * 3 + [C.c_int, C.c_double, C.c_int] + [C.c_void_p] * 3
+
+
+def blur_schedule(nCont, steps, motion, frame_motions, n_samples, shutter, image):
+    """The sub-frame table of one blurred image of a scene (arapb200_blur_schedule, DESIGN.md 4.8): image -1 = frame 0,
+    0 = the pair, k = frame k of the frames at `steps` (None or empty: no frames) with motions frame_motions (A_1 ..
+    A_K); motion is the pair's A.  Returns (state int32[S], the lower continuation state of each sub-frame's lerp, -1 =
+    the pixel grid; w float32[S], its weight; smap float32[S,2,3], the map from the frame to the background plane)."""
+    st = np.ascontiguousarray([] if steps is None else steps, np.int32).reshape(-1)
+    K = len(st)
+    fm = np.ascontiguousarray(np.asarray(frame_motions, np.float64).reshape(-1, 2, 3)) if K else None
+    if K and len(fm) != K:
+        raise ValueError(f"{len(fm)} frame motions for {K} frames")
+    A = _motion(motion)
+    S = int(n_samples)
+    state, w, smap = np.zeros(max(S, 1), np.int32), np.zeros(max(S, 1), np.float32), np.zeros((max(S, 1), 2, 3), np.float32)
+    L = load()
+    L.arapb200_blur_schedule.argtypes = BLUR_SCHEDULE_ARGTYPES
+    _check(L.arapb200_blur_schedule(int(nCont), K, st.ctypes.data if K else None, A.ctypes.data,
+                                    fm.ctypes.data if K else None, S, float(shutter), int(image), state.ctypes.data,
+                                    w.ctypes.data, smap.ctypes.data), "arapb200_blur_schedule")
+    return state, w, smap
+
+
 def filter_matches(matches, labels1, labels2):
     """N3: keep the matches para_gen.valid_cnstr keeps (para_gen.py:216-223, 468-482), in order.
     Returns (matches int32[k,4], labels uint8[k])."""
@@ -386,7 +411,7 @@ class Batch:
     SCENE_KEYS = ("flow", "rgb", "mask", "bflow", "occ")
 
     def submit_scene(self, slot, rgb, masks, matches, background, motion, origin=(0, 0), frames=None, frame_motions=None,
-                     input_frame=False, out=None):
+                     input_frame=False, out=None, blur=None):
         """Queue a scene (arapb200_batch_submit_scene, DESIGN.md 4.6): one image rgb, its segments' masks (0 = object, in
         segment order) with one match list each, and a background uint8[bgH,bgW,3] that moves by the 2x3 float64 map
         `motion` (frame pixel q of a still background shows background[q + origin]).  The layers take slots
@@ -396,7 +421,12 @@ class Batch:
         input_frame=True rgb0[H,W,3] (frame 0: rgb on the objects, the background crop elsewhere), and with frames (a
         strictly increasing list of continuation steps) and frame_motions (A_1 .. A_K, e.g. synth.motion_path) "seq",
         stacked like composite_seq()'s result.  `out` may be the dict a previous submit_scene() of the same shape returned:
-        its arrays are then written in place."""
+        its arrays are then written in place.
+        blur=(n_samples, shutter): motion blur (arapb200_batch_scene_blur, DESIGN.md 4.8) adds blur_rgb[H,W,3], with
+        input_frame blur_rgb0[H,W,3], and with frames seq["blur_rgb"][K,H,W,3]: each image averaged over n_samples
+        sub-frames of a trailing shutter open for the fraction `shutter` of the interval before it.  The sub-frame table
+        of every image to blur is checked (lib.blur_schedule) before anything is queued, so a request the library would
+        refuse raises with no scene queued."""
         n = len(masks)
         H, W = masks[0].shape
         rgb = _c(rgb, np.uint8)
@@ -415,6 +445,9 @@ class Batch:
             fm = np.ascontiguousarray(np.asarray(frame_motions, np.float64).reshape(-1, 2, 3))
             if len(fm) != K:   # the library reads one motion per frame
                 raise ValueError(f"{len(fm)} frame motions for {K} frames")
+        if blur is not None:
+            for image in ([-1] if input_frame else []) + list(range(K + 1)):
+                blur_schedule(self.nCont, steps, A, fm, blur[0], blur[1], image)
         if out is None or out["flow"].shape != (H, W, 2) or out["costs"].shape[0] != n:
             out = dict(flow=np.zeros((H, W, 2), np.float32), rgb=np.zeros((H, W, 3), np.uint8),
                        mask=np.zeros((H, W), np.uint8), bflow=np.zeros((H, W, 2), np.float32),
@@ -433,6 +466,19 @@ class Batch:
         ptrs = (P(*[m.ctypes.data for m in mk]), P(*[m.ctypes.data for m in mt]), (C.c_int * n)(*[len(m) for m in mt]))
         self._keep[slot] = (rgb, mk, mt, bg, A, steps, fm, ptrs, out)
         seq = out.get("seq")
+        if blur is not None:
+            out.setdefault("blur_rgb", np.zeros((H, W, 3), np.uint8))
+            if input_frame:
+                out.setdefault("blur_rgb0", np.zeros((H, W, 3), np.uint8))
+            else:
+                out.pop("blur_rgb0", None)
+            if K:
+                seq.setdefault("blur_rgb", np.zeros((K, H, W, 3), np.uint8))
+        else:
+            out.pop("blur_rgb", None)
+            out.pop("blur_rgb0", None)
+            if seq is not None:
+                seq.pop("blur_rgb", None)
         self.L.arapb200_batch_submit_scene.argtypes = ([C.c_void_p] + [C.c_int] * 4 + [C.c_void_p] * 4 + [C.c_int] * 2 +
                                                        [C.c_void_p] + [C.c_int] * 2 + [C.c_void_p, C.c_int] +
                                                        [C.c_void_p] * 14)
@@ -443,6 +489,13 @@ class Batch:
             out["rgb0"].ctypes.data if input_frame else None, out["costs"].ctypes.data,
             *[None if seq is None else seq[k].ctypes.data for k in ("rgb", "mask", "flow", "bflow", "occ")]),
             "arapb200_batch_submit_scene")
+        if blur is not None:
+            n_samples, shutter = blur
+            self.L.arapb200_batch_scene_blur.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_double] + [C.c_void_p] * 3
+            _check(self.L.arapb200_batch_scene_blur(
+                self.h, slot, int(n_samples), float(shutter), out["blur_rgb"].ctypes.data,
+                out["blur_rgb0"].ctypes.data if input_frame else None, seq["blur_rgb"].ctypes.data if K else None),
+                "arapb200_batch_scene_blur")
         return out
 
     def run(self):

@@ -193,6 +193,39 @@ ARAPB200_API int arapb200_batch_submit_scene(arapb200_batch* b, int slot, int n_
                                              uint8_t* out_mask, float* out_bflow, uint8_t* out_occ, uint8_t* out_rgb0,
                                              float* out_costs, uint8_t* seq_rgb, uint8_t* seq_mask, float* seq_flow,
                                              float* seq_bflow, uint8_t* seq_occ);
+/* Motion blur of a queued scene (DESIGN.md 4.8): the "final pass" next to the scene's sharp images.  Each blurred image
+ * is the mean, per pixel and channel (sum + S/2) / S in integers, of n_samples = S sub-frame renders over a trailing
+ * shutter that is open for the fraction `shutter` of the interval before the image's time: the layers splatted at
+ * positions lerped between the continuation states, over the background at the lerped motion.  Masks, flows, backward
+ * flows and occlusion stay as they are (defined at the frame times).  slot is the scene's first slot.
+ * blur_rgb uint8x3[W*H], required: the blurred pair.  blur_rgb0 uint8x3[W*H], may be NULL: the blurred frame 0, which
+ * extrapolates backwards at the first interval's velocity; it needs a scene that asked for out_rgb0.  seq_blur_rgb
+ * uint8x3[n_frames][W*H], may be NULL: the blurred frames; it needs a scene with frames.  With n_samples = 1 or shutter
+ * = 0 the blurred images are the sharp ones (frame 0: where the layers' warp at the grid covers the pixel or no layer has
+ * it on its object).  Applies to the next run only; a second call replaces the first.  The sub-frames need the layers'
+ * states after individual continuation steps, so a resident group holding a blurred layer runs one launch per step
+ * (same results bit for bit).  Per blurred image the run launches 2 * n_samples more kernels, counted in
+ * arapb200_batch_launches and in the warp span of arapb200_batch_timing; the scene keeps a second device buffer of
+ * 4 B/px per layer + 8 B/px + 3 B/px per blurred image, and each layer 8 B/px per continuation state its sub-frames read.
+ * Returns non-zero, and changes nothing, for: a NULL batch; a slot that is not the first slot of a scene queued for the
+ * next run; n_samples outside [1, 64]; a shutter that is NaN or outside [0, 1]; a NULL blur_rgb; a blur_rgb0 for a
+ * scene without out_rgb0; a seq_blur_rgb for a scene without frames; and a sub-frame motion of an image asked for that
+ * is non-finite or singular or whose maps are non-finite (arapb200_blur_schedule; frame 0's extrapolation can produce
+ * one). */
+ARAPB200_API int arapb200_batch_scene_blur(arapb200_batch* b, int slot, int n_samples, double shutter, uint8_t* blur_rgb,
+                                           uint8_t* blur_rgb0, uint8_t* seq_blur_rgb);
+/* The sub-frame table a blurred scene uses for one image (DESIGN.md 4.8); host only, no CUDA call.  nCont, the frames'
+ * steps and motions as arapb200_batch_submit_scene takes them (n_frames 0: steps and frame_motions may be NULL);
+ * image -1 = frame 0, 0 = the pair, k = frame k.  Per sub-frame j < n_samples: out_state[j] = j0, the lower continuation
+ * state of the lerp (-1 = the pixel grid), out_w[j] = its weight w (the positions are state j0 + w * (state j0+1 - state
+ * j0)), out_smap[6 j .. 6 j + 5] = the binary32 map from the frame to the background plane (row-major 2x3).  Returns
+ * non-zero, and writes nothing, for: NULL outputs; nCont < 1; n_frames < 0; a NULL motion; frames without steps or
+ * frame_motions; a step list that is not strictly increasing within [0, nCont - 1]; n_samples outside [1, 64]; a
+ * shutter that is NaN or outside [0, 1]; image outside [-1, n_frames]; and a sub-frame motion that is non-finite or
+ * singular or whose maps are non-finite. */
+ARAPB200_API int arapb200_blur_schedule(int nCont, int n_frames, const int* steps, const double* motion,
+                                        const double* frame_motions, int n_samples, double shutter, int image,
+                                        int* out_state, float* out_w, float* out_smap);
 /* run everything submitted since the last run; returns after all outputs are in host memory */
 ARAPB200_API int arapb200_batch_run(arapb200_batch* b);
 /* device milliseconds of the last run: [0] total, [1] solve kernels only, [2] warp kernels only (with the scenes'
