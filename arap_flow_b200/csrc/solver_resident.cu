@@ -7,8 +7,8 @@
 //
 // Decomposition: the active part of the image is cut into 32x8-pixel strips; a warp owns one strip, a lane
 // one column of 8 pixels (two contract-C3 groups).  r, p_angle, cos/sin and the neighbour flags live in
-// registers for the whole PCG loop, delta in shared memory; (p_x, p_y, sin*p_a, cos*p_a) of every pixel sits
-// in a shared-memory tile with a one-pixel ring.  Strips of the same CTA read each other's tiles directly;
+// registers for the whole PCG loop, delta and q = J^T J p in shared memory; (p_x, p_y, sin*p_a, cos*p_a) of every
+// pixel sits in a shared-memory tile with a one-pixel ring.  Strips of the same CTA read each other's tiles directly;
 // strips of other CTAs exchange their boundary through a small global "outbox" per strip.
 //
 // Everything that crosses CTAs is FENCE-FREE (a __threadfence is MEMBAR.SC + CCTL.IVALL, > 1 us here):
@@ -50,7 +50,8 @@ struct __align__(16) StripSmem {
     float D[3][RS_STRIP_H][32];    // delta
     float2 rcs[RS_OUTBOX_ENTRIES]; // cos/sin of the ring pixels (remote sides only)
     float stage[RS_OUTBOX_ENTRIES][4]; // remote ring pixels: [0..2] fetched z (parked until beta is known), [3] their p_a
-    float2 pre[RS_STRIP_H][32];        // (1/(1+sqrt(D_X))^2, 1/(1+sqrt(D_a))^2) per pixel, constant during a GN step
+    float2 qxy[RS_STRIP_H][32];        // q = J^T J p of the own pixels (position; angle in qa): written in phase 1, read in
+    float qa[RS_STRIP_H][32];          // phase 2 -- in shared memory rather than 24 registers live across the den barrier
 };
 
 struct __align__(16) Ctl {
@@ -63,6 +64,9 @@ struct __align__(16) Ctl {
     int bc_code;                   // 0 accept, 1 redo with bc_S
     int bc_S;
     int abort;
+    // (1/(1+sqrt(D_X))^2, 1/(1+sqrt(D_a))^2) by [valid neighbours + 5 * fit]: on the pixel grid the diagonal of J^T J only
+    // depends on the number of valid neighbours and the fit flag (jtf_finish), so the problem has ten preconditioner pairs
+    float2 pre_tab[10];
 };
 
 __device__ __forceinline__ unsigned long long ld_u64_volatile(const unsigned long long* p)
@@ -139,7 +143,8 @@ struct StripCtx {
     float* D;               // &D[0][0][lane]
     float2* rcs;
     float* stage;           // &stage[0][0]
-    float2* pre;            // &pre[0][lane]
+    float2* qxy;            // &qxy[0][lane]
+    float* qa;              // &qa[0][lane]
     int rem[4];             // remote neighbour strip id per side (0 up, 1 down, 2 left, 3 right) or -1
     uint4* outbox;          // own outbox: [RS_OUTBOX_ENTRIES][3]
     uint4* side_out;        // lane 0 / lane 31: where the left / right column entries of row 0 go (null: nothing to publish)
@@ -479,7 +484,8 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
     constexpr bool LEAN = (MINB >= 3);               // the 128-register variants
     // Rows of phases 2 and 3 whose shared-memory loads are issued together: all eight in the 168-register variants.  All
     // eight spill in the 128-register variants (C1s 28.4 -> 26.6, C2 6.04 -> 5.76, C3 6.00 -> 5.79 pairs/s); groups of
-    // four gain C1s / C2 / C3 1.3 ... 1.9 % over not hoisting there, groups of two the same within noise.
+    // four gain C1s / C2 / C3 1.3 ... 1.9 % over not hoisting there, groups of two the same within noise.  With q in shared
+    // memory eight still spill there (72 B of stack; C1 8.97 against 9.14 pairs/s for groups of four).
     constexpr int HG = LEAN ? 4 : RS_STRIP_H;
     // delta += alpha p after the arrival at the second barrier, under its latency, in the 128-register variants only:
     // fewer live values in phase 2 there (C1s +1.4 %, C3 +1.3 %); at 168 registers it delays the poller (lone problem -1.4 %)
@@ -498,6 +504,15 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
 
     if (threadIdx.x == 0) ctl.abort = 0;
     if (threadIdx.x < 8) ctl.prev[threadIdx.x >> 2][threadIdx.x & 3] = 0ull; // the host zeroes P.bar before the launch
+    if (threadIdx.x < 10) {
+        // jtf_finish + guarded_invert with nv = nd = the number of valid neighbours (a sum of 1.0f: exact); entry 0 (no
+        // valid neighbour, no constraint) is guarded_invert(0) = 1, which is also what inactive pixels look up
+        const float nv = (float)(threadIdx.x % 5);
+        float DX = (wr2 + wr2) * nv;
+        if (threadIdx.x >= 5) DX = DX + wf2;
+        const float DA = wr2 * nv;
+        ctl.pre_tab[threadIdx.x] = make_float2(guarded_invert(DX), guarded_invert(DA));
+    }
 
     // ---- which strip is mine, who are my neighbours ----
     const int n = P.n_strips;
@@ -509,7 +524,8 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
     s.D = &S[wid].D[0][0][lane];
     s.rcs = S[wid].rcs;
     s.stage = &S[wid].stage[0][0];
-    s.pre = &S[wid].pre[0][lane];
+    s.qxy = &S[wid].qxy[0][lane];
+    s.qa = &S[wid].qa[0][lane];
     s.up_row = s.own + 0 * TW + 1;
     s.down_row = s.own + (TH - 1) * TW + 1;
     s.lptr = s.own + 1 * TW + lane;
@@ -559,12 +575,11 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
     // registers that live across the PCG loop
     float r0[RS_STRIP_H], r1[RS_STRIP_H], r2[RS_STRIP_H];
     float pa[RS_STRIP_H], cc[RS_STRIP_H], ss[RS_STRIP_H];
-    float q0[RS_STRIP_H], q1[RS_STRIP_H], qa[RS_STRIP_H];
+    unsigned pidx = 0; // 4 bits per own pixel k: its entry of ctl.pre_tab (0 for inactive pixels), set in PCGInit1
 #pragma unroll
-    for (int k = 0; k < RS_STRIP_H; ++k) { r0[k] = r1[k] = r2[k] = pa[k] = 0.f; cc[k] = 1.f; ss[k] = 0.f; q0[k] = q1[k] = qa[k] = 0.f; }
-    // preconditioner entries (position, angle) of own pixel k.  Read through this lambda rather than as s.pre[k * 32] at
-    // each use: the plain reads compile to another register assignment of the kernel's set-up code.
-    auto pre_of = [&](int k) -> float2 { return s.pre[k * 32]; };
+    for (int k = 0; k < RS_STRIP_H; ++k) { r0[k] = r1[k] = r2[k] = pa[k] = 0.f; cc[k] = 1.f; ss[k] = 0.f; }
+    // preconditioner entries (position, angle) of own pixel k
+    auto pre_of = [&](int k) -> float2 { return ctl.pre_tab[(pidx >> (4 * k)) & 15u]; };
     // every tile cell must hold finite data (the masked stencil multiplies invalid neighbours by 0)
     for (int e = lane; e < TH * TW; e += 32) s.own[e] = make_float4(0.f, 0.f, 0.f, 0.f);
     int S_cost = 0, S_num = 0, S_den = 0, S_bnum = 0, S_sep = 8;
@@ -641,14 +656,13 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
             {
                 float gs0 = 0.f, gs1 = 0.f;
                 float4 up = s.up_row[lane], cur = s.own[1 * TW + lane + 1];
-                unsigned nflo = 0, nfhi = 0;
+                unsigned nflo = 0, nfhi = 0, npidx = 0;
 #pragma unroll
                 for (int k = 0; k < RS_STRIP_H; ++k) {
                     const float4 dn = (k < RS_STRIP_H - 1) ? s.own[(k + 2) * TW + lane + 1] : s.down_row[lane];
                     unsigned f = flag_of(flo, fhi, k) & ~FLAG_FIT;
                     r0[k] = r1[k] = r2[k] = 0.f;
                     pa[k] = 0.f;
-                    s.pre[k * 32] = make_float2(1.0f, 1.0f); // inactive pixels: r stays 0, any finite value works
                     s.D[(0 * RS_STRIP_H + k) * 32] = 0.f;
                     s.D[(1 * RS_STRIP_H + k) * 32] = 0.f;
                     s.D[(2 * RS_STRIP_H + k) * 32] = 0.f;
@@ -666,18 +680,18 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
                         if (fit) f |= FLAG_FIT;
                         float g0, g1, ga, DX, DA;
                         jtf_finish(a, cur.x, cur.y, fit, ct.x, ct.y, wr2, wf2, g0, g1, ga, DX, DA);
-                        const float pX = guarded_invert(DX), pA = guarded_invert(DA);
-                        s.pre[k * 32] = make_float2(pX, pA);
+                        const float pX = guarded_invert(DX), pA = guarded_invert(DA); // == ctl.pre_tab[its index]
                         r0[k] = -g0; r1[k] = -g1; r2[k] = -ga;
                         const float z0 = pX * r0[k], z1 = pX * r1[k], z2 = pA * r2[k];
                         const float term = dot3(r0[k], r1[k], r2[k], z0, z1, z2);
                         if (k < 4) gs0 = gs0 + term; else gs1 = gs1 + term;
                     }
                     if (k < 4) nflo |= f << (8 * k); else nfhi |= f << (8 * (k - 4));
+                    npidx |= ((unsigned)__popc(f & 15u) + ((f & FLAG_FIT) ? 5u : 0u)) << (4 * k);
                     up = cur;
                     cur = dn;
                 }
-                flo = nflo; fhi = nfhi;
+                flo = nflo; fhi = nfhi; pidx = npidx;
                 // publish (z = p_0, p_old = 0) of the boundary so that neighbours rebuild p_0 with beta = 0
                 ++seq;
 #pragma unroll
@@ -716,6 +730,11 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
             // barrier before the next prologue publishes again -- those two paths run one extra barrier.
             bool need_sep = (P.nPCG == 0);
             for (int it = 0; it < P.nPCG; ++it) {
+                // The flag words do not change inside the PCG loop, so the compiler hoists what it derives from them (the 0/1
+                // neighbour multipliers, fit selects and table offsets of all eight rows) out of the loop, and at 128 registers
+                // spills those values and reloads them from local memory in every iteration.  Passing the words through an
+                // empty asm makes them new values each iteration: each row's masks are rebuilt next to their use instead.
+                asm volatile("" : "+r"(flo), "+r"(fhi), "+r"(pidx));
                 // ---- PCGStep1: q = J^T J p, den = sum p.q.  Inactive pixels hold zeros throughout.
                 float gs0 = 0.f, gs1 = 0.f;
                 // One code path for every strip: 0/1-masked FMAs (bit-identical to skipping invalid neighbours).  A
@@ -736,8 +755,11 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
                     jtj_nb_masked<1>(a, cur.x, cur.y, lf, m1);
                     jtj_nb_masked<2>(a, cur.x, cur.y, dn, m2);
                     jtj_nb_masked<3>(a, cur.x, cur.y, up, m3);
-                    jtj_finish(a, cc[k], ss[k], cur.x, cur.y, pa[k], (f & FLAG_FIT) != 0, wr2, wf2, q0[k], q1[k], qa[k]);
-                    const float term = dot3(cur.x, cur.y, pa[k], q0[k], q1[k], qa[k]);
+                    float q0, q1, qa;
+                    jtj_finish(a, cc[k], ss[k], cur.x, cur.y, pa[k], (f & FLAG_FIT) != 0, wr2, wf2, q0, q1, qa);
+                    s.qxy[k * 32] = make_float2(q0, q1); // warp-private, read back in phase 2 after the den barrier
+                    s.qa[k * 32] = qa;
+                    const float term = dot3(cur.x, cur.y, pa[k], q0, q1, qa);
                     if (k < 4) gs0 = gs0 + term; else gs1 = gs1 + term;
                     up = cur;
                     cur = dn;
@@ -753,15 +775,17 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
                 const bool pub = any_rem && (it + 1 < P.nPCG);
                 ++seq;
                 // every shared-memory load of the phase first: the compiler cannot move a later row's loads above an earlier
-                // row's delta stores (it cannot prove that D, the tile and pre do not alias), so written row by row the phase
+                // row's delta stores (it cannot prove that D, the tile and q do not alias), so written row by row the phase
                 // pays the shared-memory latency eight times over
 #pragma unroll
                 for (int kb = 0; kb < RS_STRIP_H; kb += HG) {
-                    float hx[HG], hy[HG], hd0[HG], hd1[HG], hd2[HG];
-                    float2 hpre[HG];
+                    float hx[HG], hy[HG], hd0[HG], hd1[HG], hd2[HG], hqa[HG];
+                    float2 hpre[HG], hq[HG];
 #pragma unroll
                     for (int j = 0; j < HG; ++j) {
                         const int k = kb + j;
+                        hq[j] = s.qxy[k * 32];
+                        hqa[j] = s.qa[k * 32];
                         if constexpr (!DEFER) {
                             const float4 e = s.own[(k + 1) * TW + lane + 1];
                             const float* Dk = s.D + k * 32;
@@ -779,9 +803,9 @@ __global__ void __launch_bounds__(MAXT, MINB) k_resident_t(const ResProb* __rest
                             Dk[1 * RS_STRIP_H * 32] = fmaf(alpha, hy[j], hd1[j]);
                             Dk[2 * RS_STRIP_H * 32] = fmaf(alpha, pa[k], hd2[j]);
                         }
-                        r0[k] = fmaf(-alpha, q0[k], r0[k]);
-                        r1[k] = fmaf(-alpha, q1[k], r1[k]);
-                        r2[k] = fmaf(-alpha, qa[k], r2[k]);
+                        r0[k] = fmaf(-alpha, hq[j].x, r0[k]);
+                        r1[k] = fmaf(-alpha, hq[j].y, r1[k]);
+                        r2[k] = fmaf(-alpha, hqa[j], r2[k]);
                         const float pX = hpre[j].x, pA = hpre[j].y;
                         const float z0 = pX * r0[k], z1 = pX * r1[k], z2 = pA * r2[k];
                         const float term = dot3(z0, z1, z2, r0[k], r1[k], r2[k]);
