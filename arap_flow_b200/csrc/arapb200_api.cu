@@ -32,8 +32,7 @@ int warp_common(int W, int H, const float* pos_or_flow, bool is_flow, const uint
     Workspace& ws = warp_workspaces.current();
     std::lock_guard<std::mutex> g(ws.mu);
     unsigned char* b = ws.buf.reserve(l.bytes());
-    if (!ws.stream) ARAP_CUDA_CHECK(cudaStreamCreateWithFlags(&ws.stream, cudaStreamNonBlocking));
-    cudaStream_t s = ws.stream;
+    cudaStream_t s = ws.stream();
     float2* d_in = (float2*)(b + o_in);
     float2* d_pos = (float2*)(b + o_pos);
     unsigned* d_z = (unsigned*)(b + o_z);
@@ -629,16 +628,12 @@ int arapb200_debug_resident_profile(int W, int H, const uint8_t* mask_red, const
         ResidentSolver rs(W, H);
         if (!rs.prepare(W, H, dM.p, nullptr)) return 3;
         rs.set_profile(dprof.p);
-        cudaEvent_t e0, e1;
-        cudaEventCreate(&e0);
-        cudaEventCreate(&e1);
-        cudaEventRecord(e0, nullptr);
+        const EventHandle e0 = make_event(), e1 = make_event();
+        cudaEventRecord(e0.get(), nullptr);
         rs.enqueue(dX.p, dA.p, dC.p, 1, sqrtf(100.f), sqrtf(0.01f), nCont, nGN, nPCG, dcost.p, nullptr, nullptr);
-        cudaEventRecord(e1, nullptr);
+        cudaEventRecord(e1.get(), nullptr);
         ARAP_CUDA_OR_RETURN(cudaDeviceSynchronize());
-        if (ms) cudaEventElapsedTime(ms, e0, e1);
-        cudaEventDestroy(e0);
-        cudaEventDestroy(e1);
+        if (ms) cudaEventElapsedTime(ms, e0.get(), e1.get());
         if (int st = rs.status(nullptr)) return 100 + st;
         dprof.down(prof);
         ARAP_CUDA_OR_RETURN(cudaDeviceSynchronize());
@@ -685,16 +680,12 @@ int arapb200_debug_resident_profile_group(int W, int H, const uint8_t* mask_red,
         }
         if (rs.group_size(0, copies) < copies) return 4; // they must share ONE launch
         rs.set_profile(dprof.p);
-        cudaEvent_t e0, e1;
-        cudaEventCreate(&e0);
-        cudaEventCreate(&e1);
-        cudaEventRecord(e0, nullptr);
+        const EventHandle e0 = make_event(), e1 = make_event();
+        cudaEventRecord(e0.get(), nullptr);
         rs.enqueue_group(0, copies, nCont, nGN, nPCG, nullptr);
-        cudaEventRecord(e1, nullptr);
+        cudaEventRecord(e1.get(), nullptr);
         ARAP_CUDA_OR_RETURN(cudaDeviceSynchronize());
-        if (ms) cudaEventElapsedTime(ms, e0, e1);
-        cudaEventDestroy(e0);
-        cudaEventDestroy(e1);
+        if (ms) cudaEventElapsedTime(ms, e0.get(), e1.get());
         if (int st = rs.status(nullptr)) return 100 + st;
         dprof.down(prof);
         ARAP_CUDA_OR_RETURN(cudaDeviceSynchronize());

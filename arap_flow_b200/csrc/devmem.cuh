@@ -1,6 +1,8 @@
-// devmem.cuh -- who owns host-side device memory (DESIGN.md 4.7): DevBuf, one exact-size device array; GrowBuf, one
-// grow-only block of device or pinned host memory; Workspace, a GrowBuf per device shared by the stand-alone calls;
-// Layout, the 256-byte-aligned carve of one block into many.  And guarded, which turns a failure into a return code.
+// devmem.cuh -- who owns host-side CUDA resources (DESIGN.md 4.7): GrowBuf, one grow-only block of device or pinned
+// host memory; DevBuf, one exact-size device or pinned array; StreamHandle, EventHandle, GraphHandle and
+// GraphExecHandle, owning handles made by make_stream, make_event, capture and instantiate; Workspace, a GrowBuf and a
+// stream per device shared by the stand-alone calls; Layout, the 256-byte-aligned carve of one block into many.  And
+// guarded, which turns a failure into a return code.
 //
 // Layout is plain integer arithmetic and compiles without CUDA (tests/devmem_host.cpp); the rest needs nvcc.
 #pragma once
@@ -30,38 +32,12 @@ private:
 #ifdef __CUDACC__
 #include "common.cuh"
 #include <exception>
+#include <memory>
 #include <mutex>
+#include <type_traits>
 #include <utility>
 
 namespace arapb200 {
-
-// count elements of device memory (at least one, so that p is never null), freed by the destructor
-template <class T>
-struct DevBuf {
-    T* p = nullptr;
-    size_t n = 0;
-    DevBuf() = default;
-    explicit DevBuf(size_t count) : n(count) { ARAP_CUDA_CHECK(cudaMalloc(&p, (count ? count : 1) * sizeof(T))); }
-    ~DevBuf()
-    {
-        if (p) cudaFree(p);
-    }
-    DevBuf(DevBuf&& o) noexcept : p(std::exchange(o.p, nullptr)), n(std::exchange(o.n, 0)) {}
-    DevBuf& operator=(DevBuf&& o) noexcept
-    {
-        std::swap(p, o.p);
-        std::swap(n, o.n);
-        return *this;
-    }
-    void up(const T* h, cudaStream_t s = nullptr)
-    {
-        ARAP_CUDA_CHECK(cudaMemcpyAsync(p, h, n * sizeof(T), cudaMemcpyHostToDevice, s));
-    }
-    void down(T* h, cudaStream_t s = nullptr)
-    {
-        ARAP_CUDA_CHECK(cudaMemcpyAsync(h, p, n * sizeof(T), cudaMemcpyDeviceToHost, s));
-    }
-};
 
 // A block of device (cudaMalloc) or pinned host (cudaMallocHost) memory that only grows.  reserve() keeps the block
 // when it is large enough; otherwise it frees it and leaves the buffer empty (null, capacity 0) before it allocates, so
@@ -107,13 +83,110 @@ private:
     size_t cap_ = 0;
 };
 
+// count elements (at least one, so that p is never null) of device memory, or of pinned host memory for a small block
+// the host reads back; the block is a GrowBuf sized once
+template <class T>
+struct DevBuf {
+    T* p = nullptr;
+    size_t n = 0;
+    DevBuf() = default;
+    explicit DevBuf(size_t count, GrowBuf::Kind kind = GrowBuf::Device) : n(count), mem_(kind)
+    {
+        p = (T*)mem_.reserve((count ? count : 1) * sizeof(T));
+    }
+    DevBuf(DevBuf&& o) noexcept : p(std::exchange(o.p, nullptr)), n(std::exchange(o.n, 0)), mem_(std::move(o.mem_)) {}
+    DevBuf& operator=(DevBuf&& o) noexcept
+    {
+        std::swap(p, o.p);
+        std::swap(n, o.n);
+        std::swap(mem_, o.mem_);
+        return *this;
+    }
+    void up(const T* h, cudaStream_t s = nullptr)
+    {
+        ARAP_CUDA_CHECK(cudaMemcpyAsync(p, h, n * sizeof(T), cudaMemcpyHostToDevice, s));
+    }
+    void down(T* h, cudaStream_t s = nullptr)
+    {
+        ARAP_CUDA_CHECK(cudaMemcpyAsync(h, p, n * sizeof(T), cudaMemcpyDeviceToHost, s));
+    }
+
+private:
+    GrowBuf mem_;
+};
+
+// Owning handles of streams, events, graphs and executable graphs: a unique_ptr that destroys what it holds.  Each
+// make_* / capture / instantiate wraps what it creates before anything else can fail.
+struct CudaDestroy {
+    void operator()(cudaStream_t s) const { cudaStreamDestroy(s); }
+    void operator()(cudaEvent_t e) const { cudaEventDestroy(e); }
+    void operator()(cudaGraph_t g) const { cudaGraphDestroy(g); }
+    void operator()(cudaGraphExec_t g) const { cudaGraphExecDestroy(g); }
+};
+template <class H>
+using CudaHandle = std::unique_ptr<std::remove_pointer_t<H>, CudaDestroy>;
+using StreamHandle = CudaHandle<cudaStream_t>;
+using EventHandle = CudaHandle<cudaEvent_t>;
+using GraphHandle = CudaHandle<cudaGraph_t>;
+using GraphExecHandle = CudaHandle<cudaGraphExec_t>;
+
+// a non-blocking stream: it does not order behind the legacy default stream
+inline StreamHandle make_stream()
+{
+    cudaStream_t s = nullptr;
+    ARAP_CUDA_CHECK(cudaStreamCreateWithFlags(&s, cudaStreamNonBlocking));
+    return StreamHandle(s);
+}
+
+inline EventHandle make_event()
+{
+    cudaEvent_t e = nullptr;
+    ARAP_CUDA_CHECK(cudaEventCreate(&e));
+    return EventHandle(e);
+}
+
+// The graph of what body enqueues on s.  The capture is ended on every path: when body throws, what was recorded is
+// released and the exception goes on, and s is no longer capturing.
+template <class F>
+GraphHandle capture(cudaStream_t s, F&& body)
+{
+    ARAP_CUDA_CHECK(cudaStreamBeginCapture(s, cudaStreamCaptureModeThreadLocal));
+    cudaGraph_t g = nullptr;
+    try {
+        body();
+    } catch (...) {
+        cudaStreamEndCapture(s, &g);
+        GraphHandle partial(g);
+        throw;
+    }
+    const cudaError_t e = cudaStreamEndCapture(s, &g);
+    GraphHandle graph(g);
+    ARAP_CUDA_CHECK(e);
+    return graph;
+}
+
+inline GraphExecHandle instantiate(const GraphHandle& g)
+{
+    cudaGraphExec_t x = nullptr;
+    ARAP_CUDA_CHECK(cudaGraphInstantiate(&x, g.get(), 0));
+    return GraphExecHandle(x);
+}
+
 // Device workspace of a stand-alone call, kept for the life of the process: a cudaMalloc / cudaFree per call costs more
 // than the kernels, and cudaFree synchronises the device.  A caller holds mu until its last copy out of buf has
-// returned.  stream: a non-blocking stream of the workspace's own, for a caller that creates and uses one.
+// returned, and calls stream() under mu.
 struct Workspace {
     std::mutex mu;
     GrowBuf buf;
-    cudaStream_t stream = nullptr;
+    // a non-blocking stream of the workspace's own, created on first use and, like the workspace, never destroyed
+    cudaStream_t stream()
+    {
+        if (!stream_) ARAP_CUDA_CHECK(cudaStreamCreateWithFlags(&stream_, cudaStreamNonBlocking));
+        return stream_;
+    }
+
+private:
+    cudaStream_t stream_ = nullptr;
 };
 
 // One Workspace per device ordinal, created on first use and never freed: it outlives the CUDA context teardown at

@@ -3,7 +3,7 @@
 // util.t:828-840) and printed when verbosityLevel > 0.  One CUDA event pair per launch, aggregated by kernel name in
 // first-seen order at the end of a solve; same table layout and the same two summary lines.
 #pragma once
-#include "common.cuh"
+#include "devmem.cuh"
 #include <string>
 #include <vector>
 
@@ -11,21 +11,20 @@ namespace arapb200 {
 
 class KernelTimer {
 public:
-    ~KernelTimer() { clear(); }
     // returns the index of the new event pair (for stop_at)
     size_t start(const char* name, cudaStream_t s)
     {
         Ev e;
         e.name = name;
-        ARAP_CUDA_CHECK(cudaEventCreate(&e.a));
-        ARAP_CUDA_CHECK(cudaEventCreate(&e.b));
-        ARAP_CUDA_CHECK(cudaEventRecord(e.a, s));
-        ev_.push_back(e);
+        e.a = make_event();
+        e.b = make_event();
+        ARAP_CUDA_CHECK(cudaEventRecord(e.a.get(), s));
+        ev_.push_back(std::move(e));
         return ev_.size() - 1;
     }
     void stop_at(size_t idx, cudaStream_t s)
     {
-        if (idx < ev_.size()) { ARAP_CUDA_CHECK(cudaEventRecord(ev_[idx].b, s)); ev_[idx].ended = true; }
+        if (idx < ev_.size()) { ARAP_CUDA_CHECK(cudaEventRecord(ev_[idx].b.get(), s)); ev_[idx].ended = true; }
     }
     void stop(cudaStream_t s) { stop_at(ev_.size() - 1, s); }
     bool empty() const { return ev_.empty(); }
@@ -42,8 +41,8 @@ public:
         for (Ev& e : ev_) {
             if (!e.ended) continue;
             float ms = 0.f;
-            ARAP_CUDA_CHECK(cudaEventSynchronize(e.b));
-            ARAP_CUDA_CHECK(cudaEventElapsedTime(&ms, e.a, e.b));
+            ARAP_CUDA_CHECK(cudaEventSynchronize(e.b.get()));
+            ARAP_CUDA_CHECK(cudaEventElapsedTime(&ms, e.a.get(), e.b.get()));
             size_t i = 0;
             for (; i < rows.size(); ++i)
                 if (rows[i].name == e.name) break;
@@ -51,7 +50,7 @@ public:
             rows[i].count += 1;
             rows[i].total_ms += ms;
         }
-        clear();
+        ev_.clear();
         return rows;
     }
     // the reference's table + "TIMING" + "Per-iter times" lines (util.t:469-508)
@@ -93,15 +92,10 @@ public:
 
 private:
     struct Ev {
-        cudaEvent_t a = nullptr, b = nullptr;
+        EventHandle a, b;
         const char* name = "";
         bool ended = false;
     };
-    void clear()
-    {
-        for (Ev& e : ev_) { cudaEventDestroy(e.a); cudaEventDestroy(e.b); }
-        ev_.clear();
-    }
     std::vector<Ev> ev_;
 };
 

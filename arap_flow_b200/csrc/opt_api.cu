@@ -8,6 +8,7 @@
 #include "plan.cuh"
 
 #include <cstring>
+#include <memory>
 #include <string>
 
 using namespace arapb200;
@@ -22,7 +23,7 @@ struct Opt_Problem {
 };
 
 struct Opt_Plan {
-    GnPlan* plan;
+    std::unique_ptr<GnPlan> plan;
 };
 
 // These three have no error return in the ABI.  A failure (CUDA error, watchdog) is printed, recorded on the plan
@@ -102,22 +103,16 @@ Opt_Plan* Opt_ProblemPlan(Opt_State* state, Opt_Problem* problem, unsigned int* 
     }
     // failure => NULL, which the reference caller asserts on (ARAP/shared/OptSolver.h:54-56)
     try {
-        Opt_Plan* pl = new Opt_Plan;
-        pl->plan = new GnPlan((int)W, (int)H, state->params.verbosityLevel, ARAPB200_BACKEND_AUTO, problem->lm,
-                              state->params.collectPerKernelTimingInfo != 0);
-        return pl;
+        std::unique_ptr<GnPlan> plan(new GnPlan((int)W, (int)H, state->params.verbosityLevel, ARAPB200_BACKEND_AUTO,
+                                                problem->lm, state->params.collectPerKernelTimingInfo != 0));
+        return new Opt_Plan{std::move(plan)};
     } catch (...) {
         fprintf(stderr, "arapb200: Opt_ProblemPlan failed for %u x %u\n", W, H);
         return nullptr;
     }
 }
 
-void Opt_PlanFree(Opt_State*, Opt_Plan* plan)
-{
-    if (!plan) return;
-    delete plan->plan;
-    delete plan;
-}
+void Opt_PlanFree(Opt_State*, Opt_Plan* plan) { delete plan; }
 
 void Opt_SetSolverParameter(Opt_State* state, Opt_Plan* plan, const char* name, void* value)
 {

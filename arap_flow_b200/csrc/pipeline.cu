@@ -152,8 +152,8 @@ BatchPipeline::BatchPipeline(int maxW, int maxH, int max_problems, int nCont, in
     : maxW_(maxW), maxH_(maxH), nCont_(nCont), nGN_(nGN), nPCG_(nPCG), backend_(backend)
 {
     const size_t N = (size_t)maxW * maxH;
-    ARAP_CUDA_CHECK(cudaStreamCreateWithFlags(&stream_, cudaStreamNonBlocking));
-    for (auto& e : ev_) ARAP_CUDA_CHECK(cudaEventCreate(&e));
+    stream_ = make_stream();
+    for (auto& e : ev_) e = make_event();
     dev_.resize(max_problems > 0 ? max_problems : 1);
     const size_t cbytes = (size_t)nCont * (nGN + 1) * sizeof(float);
     for (Dev& d : dev_) {
@@ -172,17 +172,12 @@ BatchPipeline::BatchPipeline(int maxW, int maxH, int max_problems, int nCont, in
         d.h_in.reserve(4 * N);
         d.h_out.reserve(12 * N + cbytes);
     }
-    if (backend_ != ARAPB200_BACKEND_STREAM) resident_ = new ResidentSolver(maxW, maxH, (int)dev_.size());
+    if (backend_ != ARAPB200_BACKEND_STREAM) resident_.reset(new ResidentSolver(maxW, maxH, (int)dev_.size()));
 }
 
 BatchPipeline::~BatchPipeline()
 {
-    cudaStreamSynchronize(stream_);
-    delete solver_;
-    delete resident_;
-    delete lm_;
-    for (auto& e : ev_) cudaEventDestroy(e);
-    cudaStreamDestroy(stream_);
+    cudaStreamSynchronize(stream_.get());
 }
 
 void BatchPipeline::snapshot(const HostProblem& hp, Dev& d, int t)
@@ -192,7 +187,7 @@ void BatchPipeline::snapshot(const HostProblem& hp, Dev& d, int t)
         const auto it = std::lower_bound(list.begin(), list.end(), t);
         if (it == list.end() || *it != t) return;
         ARAP_CUDA_CHECK(cudaMemcpyAsync(dst + (size_t)(it - list.begin()) * N, d.X.p, N * sizeof(float2),
-                                        cudaMemcpyDeviceToDevice, stream_));
+                                        cudaMemcpyDeviceToDevice, stream_.get()));
     };
     copy(hp.steps, d.seq_pos);
     copy(hp.blur_states, d.blur_pos);
@@ -204,8 +199,8 @@ void BatchPipeline::solve_streaming(const HostProblem& hp, Dev& d)
     const int W = hp.W, H = hp.H;
     if (!solver_ || solverW_ != W || solverH_ != H) { // re-plan on a size change (CombinedSolver.h:149-160)
         if (solver_) launches_ += solver_->launches();
-        delete solver_;
-        solver_ = new StreamSolver(W, H);
+        solver_.reset(); // the old solver's memory is freed before the new one allocates
+        solver_.reset(new StreamSolver(W, H));
         solverW_ = W;
         solverH_ = H;
     }
@@ -213,16 +208,16 @@ void BatchPipeline::solve_streaming(const HostProblem& hp, Dev& d)
     const float wf = sqrtf(100.0f), wr = sqrtf(0.01f); // CombinedSolver.h:172-177
     solver_->set_pcg_rtol(pcg_rtol_);
     solver_->set_gn_rtol(gn_rtol_);
-    solver_->bind(d.X.p, d.A.p, d.U.p, d.C.p, d.M.p, wf, wr, stream_);
+    solver_->bind(d.X.p, d.A.p, d.U.p, d.C.p, d.M.p, wf, wr, stream_.get());
     for (int t = 0; t < nCont_; ++t) {
         const float alpha = (float)(t + 1) / (float)nCont_; // CombinedSolver.h:199-201
-        enqueue_constraint_image(W, H, d.recs_dev(), (int)d.recs.size(), alpha, d.C.p, stream_);
+        enqueue_constraint_image(W, H, d.recs_dev(), (int)d.recs.size(), alpha, d.C.p, stream_.get());
         launches_ += d.recs.empty() ? 1 : 2;
-        solver_->enqueue_init(stream_);
-        k_copy_cost<<<1, 1, 0, stream_>>>(solver_->d_scalars(), d.costs.p + (size_t)t * (nGN_ + 1));
+        solver_->enqueue_init(stream_.get());
+        k_copy_cost<<<1, 1, 0, stream_.get()>>>(solver_->d_scalars(), d.costs.p + (size_t)t * (nGN_ + 1));
         for (int g = 0; g < nGN_; ++g) {
-            solver_->enqueue_gn_step(nPCG_, stream_);
-            k_copy_cost<<<1, 1, 0, stream_>>>(solver_->d_scalars(), d.costs.p + (size_t)t * (nGN_ + 1) + g + 1);
+            solver_->enqueue_gn_step(nPCG_, stream_.get());
+            k_copy_cost<<<1, 1, 0, stream_.get()>>>(solver_->d_scalars(), d.costs.p + (size_t)t * (nGN_ + 1) + g + 1);
         }
         launches_ += 1 + nGN_;
         snapshot(hp, d, t);
@@ -238,9 +233,8 @@ void BatchPipeline::solve_lm(const HostProblem& hp, Dev& d)
     const int W = hp.W, H = hp.H;
     if (!lm_ || lmW_ != W || lmH_ != H) {
         if (lm_) launches_ += lm_->launches();
-        delete lm_;
-        lm_ = nullptr;
-        lm_ = new LmSolver(W, H);
+        lm_.reset();
+        lm_.reset(new LmSolver(W, H));
         lmW_ = W;
         lmH_ = H;
     }
@@ -250,22 +244,22 @@ void BatchPipeline::solve_lm(const HostProblem& hp, Dev& d)
     lm_costs_.assign((size_t)nCont_ * (nGN_ + 1), 0.0f);
     for (int t = 0; t < nCont_; ++t) {
         const float alpha = (float)(t + 1) / (float)nCont_; // CombinedSolver.h:199-201
-        enqueue_constraint_image(W, H, d.recs_dev(), (int)d.recs.size(), alpha, d.C.p, stream_);
+        enqueue_constraint_image(W, H, d.recs_dev(), (int)d.recs.size(), alpha, d.C.p, stream_.get());
         launches_ += d.recs.empty() ? 1 : 2;
         float* c = lm_costs_.data() + (size_t)t * (nGN_ + 1);
-        float prev = lm_->init(stream_);
+        float prev = lm_->init(stream_.get());
         c[0] = prev;
         int g = 0;
         while (g < nGN_) {
-            const int more = lm_->step(nPCG_, stream_, &prev);
+            const int more = lm_->step(nPCG_, stream_.get(), &prev);
             c[++g] = prev;
             if (!more) break;
         }
         for (int k = g + 1; k <= nGN_; ++k) c[k] = prev;
         snapshot(hp, d, t);
     }
-    ARAP_CUDA_CHECK(cudaMemcpyAsync(d.costs.p, lm_costs_.data(), lm_costs_.size() * sizeof(float), cudaMemcpyHostToDevice, stream_));
-    ARAP_CUDA_CHECK(cudaStreamSynchronize(stream_)); // lm_costs_ is reused by the next problem
+    ARAP_CUDA_CHECK(cudaMemcpyAsync(d.costs.p, lm_costs_.data(), lm_costs_.size() * sizeof(float), cudaMemcpyHostToDevice, stream_.get()));
+    ARAP_CUDA_CHECK(cudaStreamSynchronize(stream_.get())); // lm_costs_ is reused by the next problem
     launches_ += lm_->launches() - l0;
 }
 
@@ -279,11 +273,11 @@ void BatchPipeline::solve_resident(const HostProblem* problems, int first, int c
         for (int j = 0; j < count; ++j) {
             Dev& dj = dev_[first + j];
             const HostProblem& hp = problems[first + j];
-            enqueue_target_image(hp.W, hp.H, dj.recs_dev(), (int)dj.recs.size(), dj.C.p, stream_);
+            enqueue_target_image(hp.W, hp.H, dj.recs_dev(), (int)dj.recs.size(), dj.C.p, stream_.get());
             launches_ += dj.recs.empty() ? 1 : 2;
             resident_->set_problem(first + j, dj.X.p, dj.A.p, dj.C.p, 1, wf, wr, dj.costs.p, nullptr);
         }
-        resident_->enqueue_group(first, count, nCont_, nGN_, nPCG_, stream_);
+        resident_->enqueue_group(first, count, nCont_, nGN_, nPCG_, stream_.get());
         return;
     }
     // Frames and blur need X after individual continuation steps: one launch per step, on the constraint image of that
@@ -293,12 +287,12 @@ void BatchPipeline::solve_resident(const HostProblem* problems, int first, int c
         for (int j = 0; j < count; ++j) {
             Dev& dj = dev_[first + j];
             const HostProblem& hp = problems[first + j];
-            enqueue_constraint_image(hp.W, hp.H, dj.recs_dev(), (int)dj.recs.size(), alpha, dj.C.p, stream_);
+            enqueue_constraint_image(hp.W, hp.H, dj.recs_dev(), (int)dj.recs.size(), alpha, dj.C.p, stream_.get());
             launches_ += dj.recs.empty() ? 1 : 2;
             resident_->set_problem(first + j, dj.X.p, dj.A.p, dj.C.p, 0, wf, wr, dj.costs.p + (size_t)t * (nGN_ + 1),
                                    nullptr);
         }
-        resident_->enqueue_group(first, count, 1, nGN_, nPCG_, stream_);
+        resident_->enqueue_group(first, count, 1, nGN_, nPCG_, stream_.get());
         for (int j = 0; j < count; ++j) snapshot(problems[first + j], dev_[first + j], t);
     }
 }
@@ -323,7 +317,7 @@ void BatchPipeline::enqueue_scene(const HostScene& sc, unsigned char* buf)
     }
     if (sc.out_rgb0) {
         enqueue_scene_input(sc.W, sc.H, L, dev_[sc.first].rgb.p, bg, sc.bgW, sc.bgH, sc.bg_x, sc.bg_y, buf + o.rgb0,
-                            stream_);
+                            stream_.get());
         launches_ += 1;
     }
     for (int k = 0; k <= K; ++k) {
@@ -340,7 +334,7 @@ void BatchPipeline::enqueue_scene(const HostScene& sc, unsigned char* buf)
         const size_t f = (size_t)k * N;
         enqueue_composite(sc.W, sc.H, L, k >= 2, bg, sc.bgW, sc.bgH, sc.bg_x, sc.bg_y, sc.maps.data() + 18 * k,
                           (float2*)(buf + o.flow) + f, buf + o.rgb + 3 * f, buf + o.mask + f,
-                          (float2*)(buf + o.bflow) + f, buf + o.occ + f, stream_);
+                          (float2*)(buf + o.bflow) + f, buf + o.occ + f, stream_.get());
         launches_ += 2;
     }
 }
@@ -374,7 +368,7 @@ void BatchPipeline::enqueue_scene_blur(const HostScene& sc, const unsigned char*
             }
             launches_ += enqueue_blur_subframe(sc.W, sc.H, L, b.w, b.smap, dev_[sc.first].rgb.p, bg, sc.bgW, sc.bgH,
                                                sc.bg_x, sc.bg_y, (unsigned*)(buf + o.z), (ushort4*)(buf + o.acc), j,
-                                               S, out, stream_);
+                                               S, out, stream_.get());
         }
     }
 }
@@ -440,29 +434,29 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
     if (n_scenes > (int)blur_dev_.size()) blur_dev_.resize(n_scenes);
     for (int j = 0; j < n_scenes; ++j)
         if (scenes[j].blur_S) blur_dev_[j].reserve(BlurLayout(scenes[j]).bytes);
-    ARAP_CUDA_CHECK(cudaEventRecord(ev_[0], stream_));
+    ARAP_CUDA_CHECK(cudaEventRecord(ev_[0].get(), stream_.get()));
     for (int i = 0; i < count; ++i) {
         const HostProblem& hp = problems[i];
         Dev& d = dev_[i];
         const size_t N = (size_t)hp.W * hp.H;
-        ARAP_CUDA_CHECK(cudaMemcpyAsync(d.rgb.p, d.h_in.data(), 3 * N, cudaMemcpyHostToDevice, stream_));
-        ARAP_CUDA_CHECK(cudaMemcpyAsync(d.mask.p, d.h_in.data() + 3 * N, N, cudaMemcpyHostToDevice, stream_));
+        ARAP_CUDA_CHECK(cudaMemcpyAsync(d.rgb.p, d.h_in.data(), 3 * N, cudaMemcpyHostToDevice, stream_.get()));
+        ARAP_CUDA_CHECK(cudaMemcpyAsync(d.mask.p, d.h_in.data() + 3 * N, N, cudaMemcpyHostToDevice, stream_.get()));
         if (!d.recs.empty())
             ARAP_CUDA_CHECK(cudaMemcpyAsync(d.matches.data(), d.recs.data(), d.recs.size() * sizeof(MatchRec),
-                                            cudaMemcpyHostToDevice, stream_));
-        enqueue_reset_state(hp.W, hp.H, d.mask.p, d.X.p, d.U.p, d.A.p, d.M.p, stream_);
+                                            cudaMemcpyHostToDevice, stream_.get()));
+        enqueue_reset_state(hp.W, hp.H, d.mask.p, d.X.p, d.U.p, d.A.p, d.M.p, stream_.get());
         launches_ += 1;
         d.resident = false;
-        if (resident_ && !lm_on_) resident_->prepare_enqueue(i, hp.W, hp.H, d.M.p, stream_);
+        if (resident_ && !lm_on_) resident_->prepare_enqueue(i, hp.W, hp.H, d.M.p, stream_.get());
     }
     for (int j = 0; j < n_scenes; ++j) {
         const HostScene& sc = scenes[j];
         ARAP_CUDA_CHECK(cudaMemcpyAsync(scene_dev_[j].data(), sc.background, 3 * (size_t)sc.bgW * sc.bgH,
-                                        cudaMemcpyHostToDevice, stream_));
+                                        cudaMemcpyHostToDevice, stream_.get()));
     }
     n_resident_ = 0;
     if (resident_ && !lm_on_) {
-        ARAP_CUDA_CHECK(cudaStreamSynchronize(stream_)); // strip counts are needed to size the launches
+        ARAP_CUDA_CHECK(cudaStreamSynchronize(stream_.get())); // strip counts are needed to size the launches
         for (int i = 0; i < count; ++i) {
             dev_[i].resident = resident_->prepare_finish(i);
             if (!dev_[i].resident && backend_ == ARAPB200_BACKEND_RESIDENT) {
@@ -473,7 +467,7 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
             n_resident_ += dev_[i].resident ? 1 : 0;
         }
     }
-    ARAP_CUDA_CHECK(cudaEventRecord(ev_[1], stream_));
+    ARAP_CUDA_CHECK(cudaEventRecord(ev_[1].get(), stream_.get()));
     // ---- solve.  Resident problems: whole continuation schedules, several problems per cooperative launch ----
     group_size_ = 0;
     for (int i = 0; i < count;) {
@@ -499,45 +493,45 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
         if (gsz > group_size_) group_size_ = gsz;
         i += gsz;
     }
-    ARAP_CUDA_CHECK(cudaEventRecord(ev_[2], stream_));
+    ARAP_CUDA_CHECK(cudaEventRecord(ev_[2].get(), stream_.get()));
     // ---- flow extraction + forward warp + download ----
     for (int i = 0; i < count; ++i) {
         const HostProblem& hp = problems[i];
         Dev& d = dev_[i];
-        enqueue_pos_to_flow(hp.W, hp.H, d.X.p, d.flow.p, stream_);
+        enqueue_pos_to_flow(hp.W, hp.H, d.X.p, d.flow.p, stream_.get());
         const bool extras = hp.out_bflow || hp.out_occ || hp.scene;
-        enqueue_warp(hp.W, hp.H, d.X.p, d.rgb.p, d.mask.p, d.z.p, d.orgb.p, d.omask.p, stream_,
+        enqueue_warp(hp.W, hp.H, d.X.p, d.rgb.p, d.mask.p, d.z.p, d.orgb.p, d.omask.p, stream_.get(),
                      extras ? d.bflow : nullptr);
         launches_ += 1 + warp_launches_per_call();
         if (extras) {
-            enqueue_occlusion(hp.W, hp.H, d.mask.p, d.flow.p, d.z.p, d.bflow, d.occ, stream_);
+            enqueue_occlusion(hp.W, hp.H, d.mask.p, d.flow.p, d.z.p, d.bflow, d.occ, stream_.get());
             launches_ += 1;
         }
         if (!hp.steps.empty())
             launches_ += enqueue_warp_seq(hp.W, hp.H, (int)hp.steps.size(), d.seq_pos, d.rgb.p, d.mask.p, d.seq_z, d.seq,
-                                          stream_);
+                                          stream_.get());
     }
     for (int j = 0; j < n_scenes; ++j) {
         enqueue_scene(scenes[j], scene_dev_[j].data());
         if (scenes[j].blur_S) enqueue_scene_blur(scenes[j], scene_dev_[j].data(), blur_dev_[j].data());
     }
-    ARAP_CUDA_CHECK(cudaEventRecord(ev_[3], stream_));
+    ARAP_CUDA_CHECK(cudaEventRecord(ev_[3].get(), stream_.get()));
     for (int i = 0; i < count; ++i) {
         const HostProblem& hp = problems[i];
         Dev& d = dev_[i];
         const size_t N = (size_t)hp.W * hp.H;
         unsigned char* o = d.h_out.data();
         if (!hp.scene) {
-            ARAP_CUDA_CHECK(cudaMemcpyAsync(o, d.flow.p, N * sizeof(float2), cudaMemcpyDeviceToHost, stream_));
-            ARAP_CUDA_CHECK(cudaMemcpyAsync(o + 8 * N, d.orgb.p, 3 * N, cudaMemcpyDeviceToHost, stream_));
-            ARAP_CUDA_CHECK(cudaMemcpyAsync(o + 11 * N, d.omask.p, N, cudaMemcpyDeviceToHost, stream_));
+            ARAP_CUDA_CHECK(cudaMemcpyAsync(o, d.flow.p, N * sizeof(float2), cudaMemcpyDeviceToHost, stream_.get()));
+            ARAP_CUDA_CHECK(cudaMemcpyAsync(o + 8 * N, d.orgb.p, 3 * N, cudaMemcpyDeviceToHost, stream_.get()));
+            ARAP_CUDA_CHECK(cudaMemcpyAsync(o + 11 * N, d.omask.p, N, cudaMemcpyDeviceToHost, stream_.get()));
         }
         if (!hp.scene || hp.out_costs)
-            ARAP_CUDA_CHECK(cudaMemcpyAsync(o + 12 * N, d.costs.p, cbytes, cudaMemcpyDeviceToHost, stream_));
+            ARAP_CUDA_CHECK(cudaMemcpyAsync(o + 12 * N, d.costs.p, cbytes, cudaMemcpyDeviceToHost, stream_.get()));
         if (hp.out_bflow || hp.out_occ) {
             unsigned char* h = d.h_extras.data();
-            ARAP_CUDA_CHECK(cudaMemcpyAsync(h + x_bflow, d.bflow, N * sizeof(float2), cudaMemcpyDeviceToHost, stream_));
-            ARAP_CUDA_CHECK(cudaMemcpyAsync(h + x_occ, d.occ, N, cudaMemcpyDeviceToHost, stream_));
+            ARAP_CUDA_CHECK(cudaMemcpyAsync(h + x_bflow, d.bflow, N * sizeof(float2), cudaMemcpyDeviceToHost, stream_.get()));
+            ARAP_CUDA_CHECK(cudaMemcpyAsync(h + x_occ, d.occ, N, cudaMemcpyDeviceToHost, stream_.get()));
         }
         // frames go straight to the caller's buffers: K of them would need K times the pinned staging
         const size_t F = N * hp.steps.size();
@@ -545,7 +539,7 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
             {hp.seq_rgb, d.seq.rgb, 3 * F}, {hp.seq_mask, d.seq.mask, F}, {hp.seq_flow, d.seq.flow, 8 * F},
             {hp.seq_bflow, d.seq.bflow, 8 * F}, {hp.seq_occ, d.seq.occ, F}, {hp.seq_flow0, d.seq.flow0, 8 * F}};
         for (const auto& c : seq)
-            if (c.dst && F) ARAP_CUDA_CHECK(cudaMemcpyAsync(c.dst, c.src, c.bytes, cudaMemcpyDeviceToHost, stream_));
+            if (c.dst && F) ARAP_CUDA_CHECK(cudaMemcpyAsync(c.dst, c.src, c.bytes, cudaMemcpyDeviceToHost, stream_.get()));
     }
     // scene outputs go straight to the caller's buffers: the pair is frame index 0 of each block, frames 1 .. K follow
     for (int j = 0; j < n_scenes; ++j) {
@@ -560,7 +554,7 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
             {sc.seq_bflow, l.bflow + 8 * N, 8 * F}, {sc.seq_occ, l.occ + N, F}};
         for (const auto& c : out)
             if (c.dst && c.bytes)
-                ARAP_CUDA_CHECK(cudaMemcpyAsync(c.dst, b + c.off, c.bytes, cudaMemcpyDeviceToHost, stream_));
+                ARAP_CUDA_CHECK(cudaMemcpyAsync(c.dst, b + c.off, c.bytes, cudaMemcpyDeviceToHost, stream_.get()));
         if (!sc.blur_S) continue;
         const BlurLayout bl(sc);
         const unsigned char* bb = blur_dev_[j].data();
@@ -568,18 +562,18 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
             {sc.blur_rgb, bl.rgb, 3 * N}, {sc.blur_rgb0, bl.rgb0, 3 * N}, {sc.seq_blur_rgb, bl.seq, 3 * F}};
         for (const auto& c : blurred)
             if (c.dst && c.bytes)
-                ARAP_CUDA_CHECK(cudaMemcpyAsync(c.dst, bb + c.off, c.bytes, cudaMemcpyDeviceToHost, stream_));
+                ARAP_CUDA_CHECK(cudaMemcpyAsync(c.dst, bb + c.off, c.bytes, cudaMemcpyDeviceToHost, stream_.get()));
     }
-    ARAP_CUDA_CHECK(cudaStreamSynchronize(stream_));
+    ARAP_CUDA_CHECK(cudaStreamSynchronize(stream_.get()));
     if (resident_ && n_resident_ > 0) {
-        if (int st = resident_->status(stream_)) {
+        if (int st = resident_->status(stream_.get())) {
             fprintf(stderr, "arapb200: resident solver aborted (watchdog, code %d)\n", st);
             return 4;
         }
     }
     if (solver_ && n_resident_ < count) {
         unsigned bad = 0;
-        solver_->read_back(stream_, nullptr, &bad);
+        solver_->read_back(stream_.get(), nullptr, &bad);
         if (bad) {
             fprintf(stderr, "arapb200: internal error: UrShape check failed\n");
             return 2;
@@ -598,9 +592,9 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
         if (hp.out_occ) memcpy(hp.out_occ, d.h_extras.data() + x_occ, N);
     }
     if (resident_) launches_ += resident_->launches() - r0;
-    cudaEventElapsedTime(&ms_total_, ev_[0], ev_[3]);
-    cudaEventElapsedTime(&ms_solve_, ev_[1], ev_[2]);
-    cudaEventElapsedTime(&ms_warp_, ev_[2], ev_[3]);
+    cudaEventElapsedTime(&ms_total_, ev_[0].get(), ev_[3].get());
+    cudaEventElapsedTime(&ms_solve_, ev_[1].get(), ev_[2].get());
+    cudaEventElapsedTime(&ms_warp_, ev_[2].get(), ev_[3].get());
     return 0;
 }
 

@@ -7,6 +7,7 @@
 #include "devmem.cuh"
 #include "plan.cuh"
 #include "warp.cuh"
+#include <memory>
 #include <vector>
 
 namespace arapb200 {
@@ -105,6 +106,8 @@ public:
     void set_lm(bool on) { lm_on_ = on; }
 
 private:
+    StreamHandle stream_; // declared first: destroyed after everything that enqueues work on it
+    EventHandle ev_[4];
     struct Dev { // device + pinned staging of one problem slot
         DevBuf<float2> X, U, C, flow;
         DevBuf<float> A, M, costs;
@@ -145,17 +148,15 @@ private:
     // BlurLayout (pipeline.cu)
     std::vector<GrowBuf> blur_dev_;
     void enqueue_scene_blur(const HostScene& sc, const unsigned char* scene_buf, unsigned char* buf); // DESIGN.md 4.8
-    LmSolver* lm_ = nullptr;
+    std::unique_ptr<LmSolver> lm_;
     int lmW_ = 0, lmH_ = 0;
     bool lm_on_ = false;
     std::vector<float> lm_costs_;
     int maxW_, maxH_, nCont_, nGN_, nPCG_, backend_;
     std::vector<Dev> dev_;
-    StreamSolver* solver_ = nullptr;
+    std::unique_ptr<StreamSolver> solver_;
     int solverW_ = 0, solverH_ = 0;
-    ResidentSolver* resident_ = nullptr;
-    cudaStream_t stream_ = nullptr;
-    cudaEvent_t ev_[4] = {nullptr, nullptr, nullptr, nullptr};
+    std::unique_ptr<ResidentSolver> resident_;
     long long launches_ = 0;
     float ms_total_ = 0, ms_solve_ = 0, ms_warp_ = 0;
     int n_resident_ = 0, group_size_ = 0;

@@ -45,10 +45,10 @@ GnPlan::GnPlan(int W, int H, int verbosity, int backend, bool lm, bool collect_t
     : W_(W), H_(H), verbosity_(verbosity), backend_(backend), collect_timing_(collect_timing)
 {
     if (lm) lm_.reset(new LmSolver(W, H));
-    ARAP_CUDA_CHECK(cudaStreamCreateWithFlags(&stream_h_, cudaStreamNonBlocking));
-    ARAP_CUDA_CHECK(cudaMalloc(&d_costs_, kMaxCostLog * sizeof(float)));
-    ARAP_CUDA_CHECK(cudaMalloc(&d_check_, 3 * sizeof(unsigned long long)));
-    ARAP_CUDA_CHECK(cudaMallocHost(&h_check_, 3 * sizeof(unsigned long long)));
+    stream_h_ = make_stream();
+    d_costs_ = DevBuf<float>(kMaxCostLog);
+    d_check_ = DevBuf<unsigned long long>(3);
+    h_check_ = DevBuf<unsigned long long>(3, GrowBuf::Pinned);
 }
 
 // The caller works on the default stream (the reference host: cudaMemset of Angle on the legacy stream,
@@ -69,13 +69,7 @@ long long GnPlan::launches() const
 
 GnPlan::~GnPlan()
 {
-    if (stream_h_) {
-        cudaStreamSynchronize(stream_h_);
-        cudaStreamDestroy(stream_h_);
-    }
-    cudaFree(d_costs_);
-    cudaFree(d_check_);
-    cudaFreeHost(h_check_);
+    cudaStreamSynchronize(stream_h_.get());
 }
 
 bool GnPlan::set_parameter(const char* name, const void* value)
@@ -111,21 +105,23 @@ void GnPlan::choose_backend(void** pp)
 {
     order_after_caller();
     const size_t N = (size_t)W_ * H_;
-    ARAP_CUDA_CHECK(cudaMemsetAsync(d_check_, 0, 3 * sizeof(unsigned long long), stream_h_));
-    k_check_grid<<<(unsigned)((N + 255) / 256), 256, 0, stream_h_>>>(W_, H_, (const float2*)pp[2], (const float*)pp[4],
-                                                                     d_check_);
-    ARAP_CUDA_CHECK(cudaMemcpyAsync(h_check_, d_check_, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, stream_h_));
-    ARAP_CUDA_CHECK(cudaStreamSynchronize(stream_h_));
-    general_ = h_check_[0] != 0;
-    const bool same_mask = have_mask_key_ && mask_ptr_ == pp[4] && mask_key_[0] == h_check_[1] && mask_key_[1] == h_check_[2];
-    mask_ptr_ = pp[4]; mask_key_[0] = h_check_[1]; mask_key_[1] = h_check_[2]; have_mask_key_ = true;
+    cudaStream_t s = stream_h_.get();
+    ARAP_CUDA_CHECK(cudaMemsetAsync(d_check_.p, 0, 3 * sizeof(unsigned long long), s));
+    k_check_grid<<<(unsigned)((N + 255) / 256), 256, 0, s>>>(W_, H_, (const float2*)pp[2], (const float*)pp[4],
+                                                             d_check_.p);
+    ARAP_CUDA_CHECK(cudaMemcpyAsync(h_check_.p, d_check_.p, 3 * sizeof(unsigned long long), cudaMemcpyDeviceToHost, s));
+    ARAP_CUDA_CHECK(cudaStreamSynchronize(s));
+    const unsigned long long* chk = h_check_.p;
+    general_ = chk[0] != 0;
+    const bool same_mask = have_mask_key_ && mask_ptr_ == pp[4] && mask_key_[0] == chk[1] && mask_key_[1] == chk[2];
+    mask_ptr_ = pp[4]; mask_key_[0] = chk[1]; mask_key_[1] = chk[2]; have_mask_key_ = true;
     const bool was_resident = use_resident_;
     use_resident_ = false;
     // per-kernel timing needs kernels to time: the streaming back-end (same results bit for bit), launched eagerly
     if (backend_ != ARAPB200_BACKEND_STREAM && !general_ && !collect_timing_) {
         if (!resident_) resident_.reset(new ResidentSolver(W_, H_));
         // same Mask image as the previous call: the strip tables are still valid
-        use_resident_ = (same_mask && was_resident) ? true : resident_->prepare(W_, H_, (const float*)pp[4], stream_h_);
+        use_resident_ = (same_mask && was_resident) ? true : resident_->prepare(W_, H_, (const float*)pp[4], s);
         if (!use_resident_ && backend_ == ARAPB200_BACKEND_RESIDENT)
             arap_fail(1, "problem %dx%d (%d strips) does not fit the resident back-end", W_, H_, resident_->n_strips());
     }
@@ -150,11 +146,11 @@ float GnPlan::run_resident(void** pp, int nGN, float* trace)
     resident_->set_pcg_rtol(pcg_rtol_);
     resident_->set_gn_rtol(gn_rtol_);
     resident_->enqueue((float2*)pp[0], (float*)pp[1], (const float2*)pp[3], 0, *(const float*)pp[5],
-                       *(const float*)pp[6], 1, nGN, l_iterations_, d_costs_, trace, stream_h_);
+                       *(const float*)pp[6], 1, nGN, l_iterations_, d_costs_.p, trace, stream_h_.get());
     float c = 0.f;
-    ARAP_CUDA_CHECK(cudaMemcpyAsync(&c, d_costs_ + nGN, sizeof(float), cudaMemcpyDeviceToHost, stream_h_));
-    ARAP_CUDA_CHECK(cudaStreamSynchronize(stream_h_));
-    if (int st = resident_->status(stream_h_)) arap_fail(3, "resident solver aborted (watchdog, code %d)", st);
+    ARAP_CUDA_CHECK(cudaMemcpyAsync(&c, d_costs_.p + nGN, sizeof(float), cudaMemcpyDeviceToHost, stream_h_.get()));
+    ARAP_CUDA_CHECK(cudaStreamSynchronize(stream_h_.get()));
+    if (int st = resident_->status(stream_h_.get())) arap_fail(3, "resident solver aborted (watchdog, code %d)", st);
     return c;
 }
 
@@ -163,7 +159,7 @@ void GnPlan::bind(void** pp)
     // arap_plan.t:2-8: Offset, Angle, UrShape, Constraints, Mask, w_fitSqrt, w_regSqrt
     // (scalars are dereferenced on the host at init AND at every step: util.t:664-692)
     stream_->bind((float2*)pp[0], (float*)pp[1], (const float2*)pp[2], (const float2*)pp[3], (const float*)pp[4],
-                  *(const float*)pp[5], *(const float*)pp[6], stream_h_);
+                  *(const float*)pp[5], *(const float*)pp[6], stream_h_.get());
 }
 
 void GnPlan::timer_begin()
@@ -171,7 +167,7 @@ void GnPlan::timer_begin()
     timer_.reset();
     if (verbosity_ > 0 || collect_timing_) {
         timer_.reset(new KernelTimer);
-        overall_idx_ = timer_->start("overall", stream_h_);
+        overall_idx_ = timer_->start("overall", stream_h_.get());
     }
     if (lm_) lm_->set_timer(collect_timing_ ? timer_.get() : nullptr);
 }
@@ -181,7 +177,7 @@ void GnPlan::cleanup()
 {
     if (verbosity_ > 0) printf("final cost=%f\n", prev_cost_);
     if (!timer_) return;
-    timer_->stop_at(overall_idx_, stream_h_);
+    timer_->stop_at(overall_idx_, stream_h_.get());
     timing_report_ = KernelTimer::format(timer_->aggregate());
     if (verbosity_ > 0) fputs(timing_report_.c_str(), stdout); // Timer:evaluate prints under verbosity only (util.t:452)
     if (stream_) stream_->set_timer(nullptr);
@@ -202,7 +198,7 @@ void GnPlan::init(void** pp)
         order_after_caller();
         lm_bind(pp);
         n_iter_ = 0;
-        prev_cost_ = lm_->init(stream_h_);
+        prev_cost_ = lm_->init(stream_h_.get());
         return;
     }
     choose_backend(pp);
@@ -212,8 +208,8 @@ void GnPlan::init(void** pp)
         return;
     }
     bind(pp);
-    stream_->enqueue_init(stream_h_);
-    stream_->read_back(stream_h_, &prev_cost_, nullptr);
+    stream_->enqueue_init(stream_h_.get());
+    stream_->read_back(stream_h_.get(), &prev_cost_, nullptr);
 }
 
 int GnPlan::step(void** pp)
@@ -223,7 +219,7 @@ int GnPlan::step(void** pp)
     if (lm_) {
         lm_bind(pp);
         const float before = prev_cost_;
-        const int more = lm_->step(l_iterations_, stream_h_, &prev_cost_);
+        const int more = lm_->step(l_iterations_, stream_h_.get(), &prev_cost_);
         if (verbosity_ > 0) {
             const LmStepInfo& st = lm_->last_step();
             printf("cost: %f -> %f (model %f, %d linear iterations, %s, trust_region_radius=%f)\n", before, st.new_cost,
@@ -242,8 +238,8 @@ int GnPlan::step(void** pp)
         c = run_resident(pp, 1, tr);
     } else {
         bind(pp);
-        stream_->enqueue_gn_step(l_iterations_, stream_h_, tr);
-        stream_->read_back(stream_h_, &c, nullptr);
+        stream_->enqueue_gn_step(l_iterations_, stream_h_.get(), tr);
+        stream_->read_back(stream_h_.get(), &c, nullptr);
     }
     if (verbosity_ > 0) printf("cost: %f -> %f\n", prev_cost_, c); // :1158-1163
     prev_cost_ = c;
@@ -266,12 +262,12 @@ void GnPlan::solve(void** pp)
         return;
     }
     bind(pp);
-    stream_->enqueue_init(stream_h_);
+    stream_->enqueue_init(stream_h_.get());
     for (; n_iter_ < n_iterations_; ++n_iter_) {
         float* tr = d_trace_ ? d_trace_ + (size_t)3 * l_iterations_ * n_iter_ : nullptr;
-        stream_->enqueue_gn_step(l_iterations_, stream_h_, tr);
+        stream_->enqueue_gn_step(l_iterations_, stream_h_.get(), tr);
     }
-    stream_->read_back(stream_h_, &prev_cost_, nullptr);
+    stream_->read_back(stream_h_.get(), &prev_cost_, nullptr);
 }
 
 } // namespace arapb200

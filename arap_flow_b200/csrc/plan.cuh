@@ -45,7 +45,7 @@ private:
     int n_iter_ = 0;
     int error_ = 0;
     float prev_cost_ = 0.f;
-    cudaStream_t stream_h_ = nullptr;
+    StreamHandle stream_h_;                     // declared before the solvers: destroyed after them
     std::unique_ptr<StreamSolver> stream_;      // created on first use
     std::unique_ptr<ResidentSolver> resident_;  // created on first use
     std::unique_ptr<LmSolver> lm_;              // "LMGPU" plans only
@@ -59,9 +59,9 @@ private:
     bool use_resident_ = false;
     bool general_ = false;                      // UrShape is not the pixel grid
     void** last_params_ = nullptr;
-    float* d_costs_ = nullptr;                  // resident: cost log of the current launch
-    unsigned long long* d_check_ = nullptr;     // [0] non-grid UrShape count, [1..2] fingerprint of the active set
-    unsigned long long* h_check_ = nullptr;     // pinned copy
+    DevBuf<float> d_costs_;                     // resident: cost log of the current launch
+    DevBuf<unsigned long long> d_check_;        // [0] non-grid UrShape count, [1..2] fingerprint of the active set
+    DevBuf<unsigned long long> h_check_;        // pinned copy
     const void* mask_ptr_ = nullptr;            // Mask image + fingerprint the resident strip tables were built for
     unsigned long long mask_key_[2] = {0, 0};
     bool have_mask_key_ = false;

@@ -11,26 +11,11 @@
 
 namespace arapb200 {
 
-struct LmSolver::Dev {
-    int W, H;
-    size_t N;
-    float2* X;
-    float* A;
-    const float2* U;
-    const float2* C;
-    const float* M;
-    float wf, wr, wf2, wr2;
-    float* pl;
-    unsigned char* flags;
-    unsigned long long* acc;
-    LmScalars* sc;
-};
-
 namespace {
 using Dev = LmSolver::Dev;
 
 constexpr int LM_THREADS = 128;
-constexpr int LM_RING = 64; // PCG iterations whose accumulators are live at a time (solver_lm.cu: ensure_acc)
+constexpr int LM_RING = 64; // PCG iterations whose accumulators are live at a time (accumulator sets: LmSolver::LmSolver)
 // planes of N floats each
 enum : int {
     L_CS = 0,    // cos, sin of the angle the current linearisation uses
@@ -439,43 +424,21 @@ __global__ void __launch_bounds__(32) k_lm_finish(const Dev d, int set_model, in
 LmSolver::LmSolver(int W, int H) : W_(W), H_(H)
 {
     const size_t N = (size_t)W * H;
-    d_ = new Dev;
-    memset(d_, 0, sizeof(Dev));
-    d_->W = W; d_->H = H; d_->N = N;
-    ARAP_CUDA_CHECK(cudaMalloc(&planes_, (size_t)L_PLANES * N * sizeof(float)));
-    ARAP_CUDA_CHECK(cudaMemset(planes_, 0, (size_t)L_PLANES * N * sizeof(float)));
-    ARAP_CUDA_CHECK(cudaMalloc(&flags_, N));
-    ARAP_CUDA_CHECK(cudaMemset(flags_, 0, N));
-    ARAP_CUDA_CHECK(cudaMalloc(&sc_, sizeof(LmScalars)));
-    ARAP_CUDA_CHECK(cudaMemset(sc_, 0, sizeof(LmScalars)));
-    ARAP_CUDA_CHECK(cudaMallocHost(&h_sc_, sizeof(LmScalars)));
+    d_.W = W; d_.H = H; d_.N = N;
+    planes_ = DevBuf<float>((size_t)L_PLANES * N);
+    ARAP_CUDA_CHECK(cudaMemset(planes_.p, 0, (size_t)L_PLANES * N * sizeof(float)));
+    flags_ = DevBuf<unsigned char>(N);
+    ARAP_CUDA_CHECK(cudaMemset(flags_.p, 0, N));
+    sc_ = DevBuf<LmScalars>(1);
+    ARAP_CUDA_CHECK(cudaMemset(sc_.p, 0, sizeof(LmScalars)));
+    h_sc_ = DevBuf<LmScalars>(1, GrowBuf::Pinned);
     ARAP_CUDA_CHECK(cudaDeviceSynchronize()); // the memsets ran on the legacy stream; the solver runs on its own
-    d_->pl = planes_; d_->flags = flags_; d_->sc = sc_;
-    ensure_acc(10);
-}
-
-LmSolver::~LmSolver()
-{
-    cudaFree(planes_);
-    cudaFree(flags_);
-    cudaFree(acc_);
-    cudaFree(sc_);
-    cudaFreeHost(h_sc_);
-    delete d_;
-}
-
-// Accumulator sets: 0 / 1 = r.z and Q of PCGInit, then a ring of LM_RING iterations x (p.q, r.z, Q), then model cost and
-// cost.  A ring slot is cleared (stream-ordered memset) before its second use, so the footprint does not grow with
-// lIterations.
-void LmSolver::ensure_acc(int)
-{
-    const int need = 2 + 3 * LM_RING + 2;
-    if (need <= acc_sets_) return;
-    if (acc_) ARAP_CUDA_CHECK(cudaFree(acc_)); // cudaFree waits for the device
-    acc_ = nullptr;
-    ARAP_CUDA_CHECK(cudaMalloc(&acc_, (size_t)need * WA_WORDS * sizeof(unsigned long long)));
-    acc_sets_ = need;
-    d_->acc = acc_;
+    d_.pl = planes_.p; d_.flags = flags_.p; d_.sc = sc_.p;
+    // Accumulator sets: 0 / 1 = r.z and Q of PCGInit, then a ring of LM_RING iterations x (p.q, r.z, Q), then model cost
+    // and cost.  A ring slot is cleared (stream-ordered memset) before its second use, so the footprint does not grow
+    // with lIterations.
+    acc_ = DevBuf<unsigned long long>((size_t)(2 + 3 * LM_RING + 2) * WA_WORDS);
+    d_.acc = acc_.p;
 }
 
 bool LmSolver::set_parameter(const char* name, const void* value)
@@ -503,16 +466,16 @@ bool LmSolver::set_parameter(const char* name, const void* value)
 
 void LmSolver::bind(float2* X, float* A, const float2* U, const float2* C, const float* M, float wf, float wr)
 {
-    d_->X = X; d_->A = A; d_->U = U; d_->C = C; d_->M = M;
-    d_->wf = wf; d_->wr = wr; d_->wf2 = wf * wf; d_->wr2 = wr * wr;
+    d_.X = X; d_.A = A; d_.U = U; d_.C = C; d_.M = M;
+    d_.wf = wf; d_.wr = wr; d_.wf2 = wf * wf; d_.wr2 = wr * wr;
 }
 
 void LmSolver::enqueue_cost(cudaStream_t s, int acc)
 {
-    const unsigned nb = (unsigned)((d_->N + 255) / 256);
+    const unsigned nb = (unsigned)((d_.N + 255) / 256);
     const dim3 grid((W_ + 31) / 32, (H_ + 15) / 16);
-    ARAP_TIMED(timer_, "precompute", s, (k_lm_cs<<<nb, 256, 0, s>>>(*d_)));
-    ARAP_TIMED(timer_, "computeCost", s, (k_lm_cost<<<grid, LM_THREADS, 0, s>>>(*d_, acc)));
+    ARAP_TIMED(timer_, "precompute", s, (k_lm_cs<<<nb, 256, 0, s>>>(d_)));
+    ARAP_TIMED(timer_, "computeCost", s, (k_lm_cost<<<grid, LM_THREADS, 0, s>>>(d_, acc)));
     launches_ += 2;
 }
 
@@ -524,27 +487,26 @@ float LmSolver::init(cudaStream_t s)
     min_diag_ = sp_.min_lm_diagonal;
     max_diag_ = sp_.max_lm_diagonal;
     first_ = true;
-    const unsigned nb = (unsigned)((d_->N + 255) / 256);
-    ARAP_CUDA_CHECK(cudaMemsetAsync(acc_, 0, (size_t)2 * WA_WORDS * sizeof(unsigned long long), s));
-    k_lm_flags<<<nb, 256, 0, s>>>(*d_);
+    const unsigned nb = (unsigned)((d_.N + 255) / 256);
+    ARAP_CUDA_CHECK(cudaMemsetAsync(acc_.p, 0, (size_t)2 * WA_WORDS * sizeof(unsigned long long), s));
+    k_lm_flags<<<nb, 256, 0, s>>>(d_);
     enqueue_cost(s, 1);
-    k_lm_finish<<<1, 32, 0, s>>>(*d_, 0, 1);
+    k_lm_finish<<<1, 32, 0, s>>>(d_, 0, 1);
     launches_ += 2;
     ARAP_CUDA_CHECK(cudaGetLastError());
-    ARAP_CUDA_CHECK(cudaMemcpyAsync(h_sc_, sc_, sizeof(LmScalars), cudaMemcpyDeviceToHost, s));
+    ARAP_CUDA_CHECK(cudaMemcpyAsync(h_sc_.p, sc_.p, sizeof(LmScalars), cudaMemcpyDeviceToHost, s));
     ARAP_CUDA_CHECK(cudaStreamSynchronize(s));
-    return h_sc_->cost;
+    return h_sc_.p->cost;
 }
 
 int LmSolver::step(int L, cudaStream_t s, float* prev_cost)
 {
     if (L < 0) L = 0;
-    ensure_acc(L);
-    const Dev& d = *d_;
+    const Dev& d = d_;
     const unsigned nb = (unsigned)((d.N + 255) / 256);
     const dim3 grid((W_ + 31) / 32, (H_ + 15) / 16);
     const int set_model = 2 + 3 * LM_RING, set_cost = set_model + 1;
-    ARAP_CUDA_CHECK(cudaMemsetAsync(acc_, 0, (size_t)(set_cost + 1) * WA_WORDS * sizeof(unsigned long long), s));
+    ARAP_CUDA_CHECK(cudaMemsetAsync(acc_.p, 0, (size_t)(set_cost + 1) * WA_WORDS * sizeof(unsigned long long), s));
     k_lm_flags<<<nb, 256, 0, s>>>(d);
     ARAP_TIMED(timer_, "precompute", s, (k_lm_cs<<<nb, 256, 0, s>>>(d)));
     // PCGInit1 + PCGSaveSSq + PCGComputeCtC + PCGFinalizeDiagonal in one kernel
@@ -556,7 +518,7 @@ int LmSolver::step(int L, cudaStream_t s, float* prev_cost)
     for (int it = 0; it < L; ++it) {
         const int base = 2 + 3 * (it % LM_RING);
         if (it > 0 && it % LM_RING == 0) // the ring wraps: every consumer of these sets is behind us in the stream
-            ARAP_CUDA_CHECK(cudaMemsetAsync(acc_ + (size_t)2 * WA_WORDS, 0, (size_t)3 * LM_RING * WA_WORDS * sizeof(unsigned long long), s));
+            ARAP_CUDA_CHECK(cudaMemsetAsync(acc_.p + (size_t)2 * WA_WORDS, 0, (size_t)3 * LM_RING * WA_WORDS * sizeof(unsigned long long), s));
         ARAP_TIMED(timer_, "PCGStep1", s, (k_lm_apply<0><<<grid, LM_THREADS, 0, s>>>(d, base)));
         k_lm_alpha<<<1, 32, 0, s>>>(d, base);
         if (((it + 1) % sp_.residual_reset_period) == 0) { // :1077-1086
@@ -571,9 +533,9 @@ int LmSolver::step(int L, cudaStream_t s, float* prev_cost)
         ARAP_TIMED(timer_, "PCGStep3", s, (k_lm_step3<<<nb, 256, 0, s>>>(d)));
         launches_ += 5;
         if ((it & 15) == 15 && it + 1 < L) { // has the Q test ended the loop?  (the remaining launches would be no-ops)
-            ARAP_CUDA_CHECK(cudaMemcpyAsync(&h_sc_->conv, &sc_->conv, sizeof(unsigned), cudaMemcpyDeviceToHost, s));
+            ARAP_CUDA_CHECK(cudaMemcpyAsync(&h_sc_.p->conv, &sc_.p->conv, sizeof(unsigned), cudaMemcpyDeviceToHost, s));
             ARAP_CUDA_CHECK(cudaStreamSynchronize(s));
-            if (h_sc_->conv) break;
+            if (h_sc_.p->conv) break;
         }
     }
     ARAP_TIMED(timer_, "computeModelCost", s, (k_lm_model<<<grid, LM_THREADS, 0, s>>>(d, set_model))); // before the update (:1106-1112)
@@ -582,19 +544,19 @@ int LmSolver::step(int L, cudaStream_t s, float* prev_cost)
     k_lm_finish<<<1, 32, 0, s>>>(d, set_model, set_cost);
     launches_ += 3;
     ARAP_CUDA_CHECK(cudaGetLastError());
-    ARAP_CUDA_CHECK(cudaMemcpyAsync(h_sc_, sc_, sizeof(LmScalars), cudaMemcpyDeviceToHost, s));
+    ARAP_CUDA_CHECK(cudaMemcpyAsync(h_sc_.p, sc_.p, sizeof(LmScalars), cudaMemcpyDeviceToHost, s));
     ARAP_CUDA_CHECK(cudaStreamSynchronize(s));
 
     // the trust-region bookkeeping of :1106-1170, in the reference's types (binary32 fields, binary64 literals)
     const float prevCost = *prev_cost;
-    const float model_cost = h_sc_->model, newCost = h_sc_->cost;
+    const float model_cost = h_sc_.p->model, newCost = h_sc_.p->cost;
     const float model_cost_change = prevCost - model_cost;
     const float cost_change = prevCost - newCost;
     const float relative_decrease = cost_change / model_cost_change;
-    info_.pcg_iterations = h_sc_->iters;
+    info_.pcg_iterations = h_sc_.p->iters;
     info_.model_cost = model_cost;
     info_.new_cost = newCost;
-    info_.q_last = h_sc_->q_last;
+    info_.q_last = h_sc_.p->q_last;
     int more = 1;
     if (cost_change >= 0.0f && relative_decrease > sp_.min_relative_decrease) {
         const float absolute_function_tolerance = prevCost * sp_.function_tolerance;

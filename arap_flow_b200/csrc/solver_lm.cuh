@@ -6,6 +6,7 @@
 // bit for bit against oracle/arap_oracle.c (arap_oracle_lm_solve).
 #pragma once
 #include "common.cuh"
+#include "devmem.cuh"
 #include "kernel_timer.cuh"
 
 namespace arapb200 {
@@ -43,7 +44,6 @@ struct LmStepInfo {
 class LmSolver {
 public:
     LmSolver(int W, int H);
-    ~LmSolver();
     LmSolver(const LmSolver&) = delete;
     LmSolver& operator=(const LmSolver&) = delete;
 
@@ -57,23 +57,34 @@ public:
     const LmStepInfo& last_step() const { return info_; }
     long long launches() const { return launches_; }
     void set_timer(KernelTimer* t) { timer_ = t; } // per-kernel timing under the reference's kernel names; null = off
-    struct Dev; // the kernels' argument block (solver_lm.cu)
+    struct Dev { // the argument block of the kernels in solver_lm.cu
+        int W, H;
+        size_t N;
+        float2* X;
+        float* A;
+        const float2* U;
+        const float2* C;
+        const float* M;
+        float wf, wr, wf2, wr2;
+        float* pl;
+        unsigned char* flags;
+        unsigned long long* acc;
+        LmScalars* sc;
+    };
 
 private:
     void enqueue_cost(cudaStream_t s, int acc);
-    void ensure_acc(int lIterations);
     int W_, H_;
     LmParameters sp_;                       // solver parameters (what set_parameter writes)
     float radius_ = 0.f, decrease_ = 0.f;   // pd.parameters.trust_region_radius / radius_decrease_factor (run time)
     float min_diag_ = 0.f, max_diag_ = 0.f;
     bool first_ = true;                     // nIter == 0: save the Jacobi scaling (ONCE_PER_SOLVE)
-    Dev* d_ = nullptr;                      // host copy of the kernel argument block
-    float* planes_ = nullptr;
-    unsigned char* flags_ = nullptr;
-    unsigned long long* acc_ = nullptr;
-    int acc_sets_ = 0;
-    LmScalars* sc_ = nullptr;
-    LmScalars* h_sc_ = nullptr;             // pinned
+    Dev d_{};                               // host copy of the kernel argument block
+    DevBuf<float> planes_;
+    DevBuf<unsigned char> flags_;
+    DevBuf<unsigned long long> acc_;
+    DevBuf<LmScalars> sc_;
+    DevBuf<LmScalars> h_sc_;                // pinned
     LmStepInfo info_{};
     long long launches_ = 0;
     KernelTimer* timer_ = nullptr;

@@ -1010,34 +1010,25 @@ ResidentSolver::ResidentSolver(int maxW, int maxH, int max_slots) : maxW_(maxW),
     strip_cap_ = (size_t)SX * SY;
     slots_.resize(max_slots > 0 ? max_slots : 1);
     for (Slot& sl : slots_) {
-        ARAP_CUDA_CHECK(cudaMalloc(&sl.d_strip_xy, strip_cap_ * sizeof(int2)));
-        ARAP_CUDA_CHECK(cudaMalloc(&sl.d_slot_of_strip, strip_cap_ * sizeof(int) + strip_cap_)); // + the active bytes
-        ARAP_CUDA_CHECK(cudaMalloc(&sl.d_count, sizeof(int)));
+        sl.d_strip_xy = DevBuf<int2>(strip_cap_);
+        sl.d_slot_of_strip = DevBuf<int>(strip_cap_ + (strip_cap_ + 3) / 4); // + the active bytes
+        sl.d_count = DevBuf<int>(1);
         // the outbox only has to hold what can be resident: at most sm_count * max warps strips
         const size_t ob = std::min(strip_cap_, (size_t)sm_count_ * (RS_THREADS_MAX / 32));
-        ARAP_CUDA_CHECK(cudaMalloc(&sl.d_outbox, ob * RS_OUTBOX_ENTRIES * 2 * sizeof(uint4)));
-        ARAP_CUDA_CHECK(cudaMalloc(&sl.d_bar, 8 * BAR_STRIDE * sizeof(unsigned long long)));
+        sl.d_outbox = DevBuf<uint4>(ob * RS_OUTBOX_ENTRIES * 2);
+        sl.d_bar = DevBuf<unsigned long long>(8 * BAR_STRIDE);
     }
-    ARAP_CUDA_CHECK(cudaMallocHost(&h_counts_, slots_.size() * sizeof(int)));
-    ARAP_CUDA_CHECK(cudaMalloc(&d_status_, 2 * sizeof(int)));
-    ARAP_CUDA_CHECK(cudaMemset(d_status_, 0, 2 * sizeof(int)));
+    h_counts_ = DevBuf<int>(slots_.size(), GrowBuf::Pinned);
+    d_status_ = DevBuf<int>(2);
+    ARAP_CUDA_CHECK(cudaMemset(d_status_.p, 0, 2 * sizeof(int)));
     // the memset ran on the legacy stream, all later work runs on non-blocking streams: finish it here
     ARAP_CUDA_CHECK(cudaDeviceSynchronize());
-    ARAP_CUDA_CHECK(cudaMalloc(&d_probs_, slots_.size() * sizeof(ResProb)));
+    d_probs_ = DevBuf<ResProb>(slots_.size());
     for (int v = 0; v < g_nvariants; ++v) {
         const int smem = (int)((g_variants[v].max_threads / 32) * sizeof(StripSmem));
         ARAP_CUDA_CHECK(cudaFuncSetAttribute((const void*)g_variants[v].fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
         ARAP_CUDA_CHECK(cudaFuncSetAttribute((const void*)g_variants[v].fn_prof, cudaFuncAttributeMaxDynamicSharedMemorySize, smem));
     }
-}
-
-ResidentSolver::~ResidentSolver()
-{
-    for (Slot& sl : slots_) {
-        cudaFree(sl.d_strip_xy); cudaFree(sl.d_slot_of_strip); cudaFree(sl.d_count); cudaFree(sl.d_outbox); cudaFree(sl.d_bar);
-    }
-    cudaFreeHost(h_counts_);
-    cudaFree(d_status_); cudaFree(d_probs_);
 }
 
 void ResidentSolver::prepare_enqueue(int slot, int W, int H, const float* d_M, cudaStream_t stream)
@@ -1049,20 +1040,20 @@ void ResidentSolver::prepare_enqueue(int slot, int W, int H, const float* d_M, c
     sl.d_M = d_M;
     sl.fits = false;
     sl.n_strips = 0;
-    if ((size_t)W * H > (size_t)maxW_ * maxH_ || (size_t)sl.SX * sl.SY > strip_cap_) { h_counts_[slot] = -1; return; }
-    unsigned char* d_active = reinterpret_cast<unsigned char*>(sl.d_slot_of_strip + (size_t)sl.SX * sl.SY);
+    if ((size_t)W * H > (size_t)maxW_ * maxH_ || (size_t)sl.SX * sl.SY > strip_cap_) { h_counts_.p[slot] = -1; return; }
+    unsigned char* d_active = reinterpret_cast<unsigned char*>(sl.d_slot_of_strip.p + (size_t)sl.SX * sl.SY);
     k_strip_active<<<(sl.SX * sl.SY + 7) / 8, 256, 0, stream>>>(W, H, sl.SX, sl.SY, d_M, d_active);
-    k_strip_compact<<<1, 1024, 0, stream>>>(sl.SX, sl.SY, d_active, sl.d_strip_xy, sl.d_slot_of_strip, sl.d_count);
+    k_strip_compact<<<1, 1024, 0, stream>>>(sl.SX, sl.SY, d_active, sl.d_strip_xy.p, sl.d_slot_of_strip.p, sl.d_count.p);
     launches_ += 2;
-    ARAP_CUDA_CHECK(cudaMemcpyAsync(&h_counts_[slot], sl.d_count, sizeof(int), cudaMemcpyDeviceToHost, stream));
+    ARAP_CUDA_CHECK(cudaMemcpyAsync(&h_counts_.p[slot], sl.d_count.p, sizeof(int), cudaMemcpyDeviceToHost, stream));
 }
 
 bool ResidentSolver::prepare_finish(int slot)
 {
     Slot& sl = slots_[slot];
     sl.fits = false;
-    if (h_counts_[slot] < 0) return false;
-    sl.n_strips = h_counts_[slot];
+    if (h_counts_.p[slot] < 0) return false;
+    sl.n_strips = h_counts_.p[slot];
     const int max_warps = RS_THREADS_MAX / 32;
     if (sl.n_strips == 0) { sl.G = 1; sl.NW = 1; sl.fits = true; return true; }
     sl.NW = (sl.n_strips + sm_count_ - 1) / sm_count_;
@@ -1093,8 +1084,8 @@ void ResidentSolver::set_problem(int slot, float2* X, float* A, const float2* C,
     p.W = sl.W; p.H = sl.H; p.SX = sl.SX; p.SY = sl.SY; p.n_strips = sl.n_strips; p.G = sl.G;
     p.X = X; p.A = A; p.C = C; p.M = sl.d_M; p.lerp_mode = lerp_mode;
     p.wf = wf; p.wr = wr; p.wf2 = wf * wf; p.wr2 = wr * wr;
-    p.strip_xy = sl.d_strip_xy; p.slot_of_strip = sl.d_slot_of_strip;
-    p.outbox = sl.d_outbox; p.bar = sl.d_bar; p.costs = d_costs; p.trace = d_trace; p.status = d_status_;
+    p.strip_xy = sl.d_strip_xy.p; p.slot_of_strip = sl.d_slot_of_strip.p;
+    p.outbox = sl.d_outbox.p; p.bar = sl.d_bar.p; p.costs = d_costs; p.trace = d_trace; p.status = d_status_.p;
 }
 
 int ResidentSolver::group_size(int first, int limit) const
@@ -1128,18 +1119,18 @@ void ResidentSolver::enqueue_group(int first, int count, int nCont, int nGN, int
         ctas += sl.G;
         nwmax = std::max(nwmax, sl.NW);
         // barrier words start at zero; halo tags start at 1, so a zeroed outbox is "nothing published yet"
-        ARAP_CUDA_CHECK(cudaMemsetAsync(sl.d_bar, 0, 8 * BAR_STRIDE * sizeof(unsigned long long), stream));
-        ARAP_CUDA_CHECK(cudaMemsetAsync(sl.d_outbox, 0,
+        ARAP_CUDA_CHECK(cudaMemsetAsync(sl.d_bar.p, 0, 8 * BAR_STRIDE * sizeof(unsigned long long), stream));
+        ARAP_CUDA_CHECK(cudaMemsetAsync(sl.d_outbox.p, 0,
                                           (size_t)(sl.n_strips > 0 ? sl.n_strips : 1) * RS_OUTBOX_ENTRIES * 2 * sizeof(uint4), stream));
     }
-    ARAP_CUDA_CHECK(cudaMemcpyAsync(d_probs_ + first, host.data(), count * sizeof(ResProb), cudaMemcpyHostToDevice, stream));
+    ARAP_CUDA_CHECK(cudaMemcpyAsync(d_probs_.p + first, host.data(), count * sizeof(ResProb), cudaMemcpyHostToDevice, stream));
     // the live CTAs of all problems form one 1-D grid; the variant with the most registers that keeps them co-resident
     const int v = pick_variant(nwmax, ctas, sm_count_);
     if (v < 0) arap_fail(1, "resident kernel cannot be co-resident (%lld CTAs of %d warps)", ctas, nwmax);
     last_variant_ = v;
     const int threads = nwmax * 32;
     const size_t smem = (size_t)nwmax * sizeof(StripSmem);
-    const ResProb* dp = d_probs_ + first;
+    const ResProb* dp = d_probs_.p + first;
     void* args[] = {(void*)&dp};
     const void* fn = d_prof_ ? (const void*)g_variants[v].fn_prof : (const void*)g_variants[v].fn;
     // equal-sized problems keep the 2-D shape (measured 4 % faster on C1: the hardware's placement of a 2-D grid mixes the
@@ -1164,10 +1155,10 @@ void ResidentSolver::enqueue(float2* X, float* A, const float2* C, int lerp_mode
 int ResidentSolver::status(cudaStream_t stream)
 {
     int st[2] = {0, 0};
-    ARAP_CUDA_CHECK(cudaMemcpyAsync(st, d_status_, sizeof(st), cudaMemcpyDeviceToHost, stream));
+    ARAP_CUDA_CHECK(cudaMemcpyAsync(st, d_status_.p, sizeof(st), cudaMemcpyDeviceToHost, stream));
     ARAP_CUDA_CHECK(cudaStreamSynchronize(stream));
     if (st[0]) {
-        ARAP_CUDA_CHECK(cudaMemsetAsync(d_status_, 0, sizeof(st), stream));
+        ARAP_CUDA_CHECK(cudaMemsetAsync(d_status_.p, 0, sizeof(st), stream));
         return st[1] ? st[1] : 1;
     }
     return 0;

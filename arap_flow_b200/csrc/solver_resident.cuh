@@ -5,6 +5,7 @@
 // See DESIGN.md section 4 for the decomposition, the barrier and the halo protocol.
 #pragma once
 #include "common.cuh"
+#include "devmem.cuh"
 #include <vector>
 
 namespace arapb200 {
@@ -44,7 +45,6 @@ class ResidentSolver {
 public:
     // capacity: largest image handled, number of problem slots that can be prepared / launched together
     explicit ResidentSolver(int maxW, int maxH, int max_slots = 1);
-    ~ResidentSolver();
     ResidentSolver(const ResidentSolver&) = delete;
     ResidentSolver& operator=(const ResidentSolver&) = delete;
 
@@ -87,19 +87,19 @@ private:
         int W = 0, H = 0, SX = 0, SY = 0, n_strips = 0, G = 0, NW = 0;
         bool fits = false;
         const float* d_M = nullptr;
-        int2* d_strip_xy = nullptr;
-        int* d_slot_of_strip = nullptr;
-        int* d_count = nullptr;
-        uint4* d_outbox = nullptr;
-        unsigned long long* d_bar = nullptr;
+        DevBuf<int2> d_strip_xy;
+        DevBuf<int> d_slot_of_strip; // then the strips' active bytes
+        DevBuf<int> d_count;
+        DevBuf<uint4> d_outbox;
+        DevBuf<unsigned long long> d_bar;
         ResProb prob{};
     };
     int maxW_, maxH_;
     size_t strip_cap_ = 0;
     std::vector<Slot> slots_;
-    int* h_counts_ = nullptr;   // pinned
-    int* d_status_ = nullptr;   // shared by all slots
-    ResProb* d_probs_ = nullptr;
+    DevBuf<int> h_counts_;      // pinned
+    DevBuf<int> d_status_;      // shared by all slots
+    DevBuf<ResProb> d_probs_;
     int sm_count_ = 0;
     long long launches_ = 0;
     unsigned long long* d_prof_ = nullptr;

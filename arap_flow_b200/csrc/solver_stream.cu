@@ -743,29 +743,23 @@ StreamSolver::StreamSolver(int W, int H)
     h_.ty = (H + ST_TILE - 1) / ST_TILE;
     h_.ntiles = h_.tx * h_.ty;
     const size_t bytes = (size_t)h_.ntiles * ST_TILE_FLOATS * sizeof(float);
-    ARAP_CUDA_CHECK(cudaMalloc(&h_.planes, bytes));
+    planes_ = DevBuf<float>((size_t)h_.ntiles * ST_TILE_FLOATS);
+    h_.planes = planes_.p;
     ARAP_CUDA_CHECK(cudaMemset(h_.planes, 0, bytes));
-    ARAP_CUDA_CHECK(cudaMalloc(&h_.tile_active, (size_t)h_.ntiles));
+    tile_active_ = DevBuf<unsigned char>((size_t)h_.ntiles);
+    h_.tile_active = tile_active_.p;
     ARAP_CUDA_CHECK(cudaMemset(h_.tile_active, 1, (size_t)h_.ntiles));
-    ARAP_CUDA_CHECK(cudaMalloc(&h_.acc, ACC_BYTES));
+    acc_ = DevBuf<unsigned long long>((size_t)ST_ACC_SETS * WA_WORDS);
+    h_.acc = acc_.p;
     ARAP_CUDA_CHECK(cudaMemset(h_.acc, 0, ACC_BYTES));
-    ARAP_CUDA_CHECK(cudaMalloc(&h_.sc, sizeof(StreamScalars)));
+    sc_ = DevBuf<StreamScalars>(1);
+    h_.sc = sc_.p;
     ARAP_CUDA_CHECK(cudaMemset(h_.sc, 0, sizeof(StreamScalars)));
-    ARAP_CUDA_CHECK(cudaMalloc(&d_, sizeof(StreamDev)));
+    d_ = DevBuf<StreamDev>(1);
     // the memsets above ran on the legacy stream; the solver's kernels run on non-blocking streams that do not order
     // behind it, and the branch-free kernels rely on "inactive pixels hold zeros": finish the clears here
     ARAP_CUDA_CHECK(cudaDeviceSynchronize());
     h_.trace = nullptr;
-}
-
-StreamSolver::~StreamSolver()
-{
-    if (graph_) cudaGraphExecDestroy(graph_);
-    cudaFree(h_.planes);
-    cudaFree(h_.tile_active);
-    cudaFree(h_.acc);
-    cudaFree(h_.sc);
-    cudaFree(d_);
 }
 
 // ---- debug access: row-major host image <-> one tile-interleaved plane ----
@@ -814,7 +808,7 @@ void StreamSolver::download_flags(unsigned char* dst) const
 
 void StreamSolver::upload(cudaStream_t stream)
 {
-    ARAP_CUDA_CHECK(cudaMemcpyAsync(d_, &h_, sizeof(StreamDev), cudaMemcpyHostToDevice, stream));
+    d_.up(&h_, stream);
 }
 
 void StreamSolver::bind(float2* X, float* A, const float2* U, const float2* C, const float* M, float wf,
@@ -831,14 +825,14 @@ void StreamSolver::bind(float2* X, float* A, const float2* U, const float2* C, c
 void StreamSolver::enqueue_prep(cudaStream_t stream)
 {
     ARAP_CUDA_CHECK(cudaMemsetAsync(h_.acc, 0, ACC_BYTES, stream));
-    k_prep<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_);
+    k_prep<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_.p);
     ++launches_;
 }
 
 void StreamSolver::enqueue_pcg_init(cudaStream_t stream)
 {
-    if (general_) k_init_gen<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_);
-    else k_init<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_);
+    if (general_) k_init_gen<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_.p);
+    else k_init<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_.p);
     ++launches_;
 }
 
@@ -846,21 +840,21 @@ void StreamSolver::launch_step_a(bool first, int it, cudaStream_t stream)
 {
     const StreamPlanes& pl = h_;
     if (general_) {
-        if (first) k_step_a_gen<true><<<h_.ntiles, ST_THREADS, 0, stream>>>(pl, d_, it);
-        else k_step_a_gen<false><<<h_.ntiles, ST_THREADS, 0, stream>>>(pl, d_, it);
+        if (first) k_step_a_gen<true><<<h_.ntiles, ST_THREADS, 0, stream>>>(pl, d_.p, it);
+        else k_step_a_gen<false><<<h_.ntiles, ST_THREADS, 0, stream>>>(pl, d_.p, it);
     } else {
         const bool rt = this->rt(); // opt-in early exits: their own instantiations
-        if (first) k_step_a<true><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_, it);
-        else if (rt) k_step_a<false, true><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_, it);
-        else k_step_a<false><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_, it);
+        if (first) k_step_a<true><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_.p, it);
+        else if (rt) k_step_a<false, true><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_.p, it);
+        else k_step_a<false><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_.p, it);
     }
 }
 
 void StreamSolver::launch_step_b(int it, cudaStream_t stream)
 {
     const StreamPlanes& pl = h_;
-    if (rt()) k_step_b<true><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_, it);
-    else k_step_b<false><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_, it);
+    if (rt()) k_step_b<true><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_.p, it);
+    else k_step_b<false><<<2 * h_.ntiles, 128, 0, stream>>>(pl, d_.p, it);
 }
 
 void StreamSolver::set_pcg_rtol(float rtol)
@@ -868,9 +862,7 @@ void StreamSolver::set_pcg_rtol(float rtol)
     rtol = rtol > 0.0f ? rtol : 0.0f;
     const bool was = rt();
     pcg_rtol_ = rtol;
-    if (rt() != was && graph_) { // other kernel instantiations: re-capture
-        cudaGraphExecDestroy(graph_); graph_ = nullptr; graph_npcg_ = -1;
-    }
+    if (rt() != was) drop_graph(); // other kernel instantiations
 }
 
 void StreamSolver::set_gn_rtol(float rtol)
@@ -878,16 +870,20 @@ void StreamSolver::set_gn_rtol(float rtol)
     rtol = rtol > 0.0f ? rtol : 0.0f;
     const bool was = rt();
     gn_rtol_ = rtol;
-    if (rt() != was && graph_) {
-        cudaGraphExecDestroy(graph_); graph_ = nullptr; graph_npcg_ = -1;
-    }
+    if (rt() != was) drop_graph();
 }
 
 void StreamSolver::set_general(bool general)
 {
     if (general == general_) return;
     general_ = general;
-    if (graph_) { cudaGraphExecDestroy(graph_); graph_ = nullptr; graph_npcg_ = -1; } // other kernels: re-capture
+    drop_graph(); // other kernels
+}
+
+void StreamSolver::drop_graph()
+{
+    graph_.reset();
+    graph_npcg_ = -1;
 }
 
 void StreamSolver::enqueue_step_a(bool first, int it, cudaStream_t stream)
@@ -903,9 +899,9 @@ void StreamSolver::enqueue_init(cudaStream_t stream)
     const StreamPlanes& pl = h_;
     ARAP_CUDA_CHECK(cudaMemsetAsync(&h_.sc->bad_u, 0, sizeof(unsigned), stream));
     ARAP_TIMED(timer_, "precompute", stream, enqueue_prep(stream));
-    if (general_) ARAP_TIMED(timer_, "computeCost", stream, (k_cost_gen<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_)));
-    else ARAP_TIMED(timer_, "computeCost", stream, (k_cost<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_)));
-    k_finish<<<1, 32, 0, stream>>>(pl, d_, -1, 1);
+    if (general_) ARAP_TIMED(timer_, "computeCost", stream, (k_cost_gen<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_.p)));
+    else ARAP_TIMED(timer_, "computeCost", stream, (k_cost<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_.p)));
+    k_finish<<<1, 32, 0, stream>>>(pl, d_.p, -1, 1);
     launches_ += 2;
     ARAP_CUDA_CHECK(cudaGetLastError());
 }
@@ -916,18 +912,18 @@ void StreamSolver::launch_gn_body(int nPCG, cudaStream_t stream, bool tracing)
     KernelTimer* const tm = tracing ? timer_ : nullptr; // never inside a graph capture
     ARAP_CUDA_CHECK(cudaMemsetAsync(h_.acc, 0, ACC_BYTES, stream));
     // the caller may have changed the constraint image / mask between steps (Opt.h:58-60): refresh flags
-    ARAP_TIMED(tm, "precompute", stream, (k_prep<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_)));
-    if (general_) ARAP_TIMED(tm, "PCGInit1", stream, (k_init_gen<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_)));
-    else ARAP_TIMED(tm, "PCGInit1", stream, (k_init<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_)));
+    ARAP_TIMED(tm, "precompute", stream, (k_prep<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_.p)));
+    if (general_) ARAP_TIMED(tm, "PCGInit1", stream, (k_init_gen<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_.p)));
+    else ARAP_TIMED(tm, "PCGInit1", stream, (k_init<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_.p)));
     for (int it = 0; it < nPCG; ++it) {
         // PCGStep3 of the previous iteration is fused into this kernel (k_step_a)
         ARAP_TIMED(tm, "PCGStep1", stream, launch_step_a(it == 0, it, stream));
         ARAP_TIMED(tm, "PCGStep2", stream, launch_step_b(it, stream));
     }
-    ARAP_TIMED(tm, "PCGLinearUpdate", stream, (k_update<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_)));
-    if (general_) ARAP_TIMED(tm, "computeCost", stream, (k_cost_gen<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_)));
-    else ARAP_TIMED(tm, "computeCost", stream, (k_cost<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_)));
-    k_finish<<<1, 32, 0, stream>>>(pl, d_, nPCG - 1, 0);
+    ARAP_TIMED(tm, "PCGLinearUpdate", stream, (k_update<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_.p)));
+    if (general_) ARAP_TIMED(tm, "computeCost", stream, (k_cost_gen<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_.p)));
+    else ARAP_TIMED(tm, "computeCost", stream, (k_cost<<<h_.ntiles, ST_THREADS, 0, stream>>>(d_.p)));
+    k_finish<<<1, 32, 0, stream>>>(pl, d_.p, nPCG - 1, 0);
 }
 
 void StreamSolver::enqueue_gn_step(int nPCG, cudaStream_t stream, float* d_trace)
@@ -950,20 +946,14 @@ void StreamSolver::enqueue_gn_step(int nPCG, cudaStream_t stream, float* d_trace
         return;
     }
     if (!graph_ || graph_npcg_ != nPCG) {
-        if (graph_) { cudaGraphExecDestroy(graph_); graph_ = nullptr; }
-        cudaStream_t cap;
-        ARAP_CUDA_CHECK(cudaStreamCreateWithFlags(&cap, cudaStreamNonBlocking));
-        cudaGraph_t g;
-        ARAP_CUDA_CHECK(cudaStreamBeginCapture(cap, cudaStreamCaptureModeThreadLocal));
-        launch_gn_body(nPCG, cap, false);
-        ARAP_CUDA_CHECK(cudaStreamEndCapture(cap, &g));
-        ARAP_CUDA_CHECK(cudaGraphInstantiate(&graph_, g, 0));
-        ARAP_CUDA_CHECK(cudaGraphDestroy(g));
-        ARAP_CUDA_CHECK(cudaStreamDestroy(cap));
+        drop_graph();
+        const StreamHandle cap = make_stream();
+        const GraphHandle g = capture(cap.get(), [&] { launch_gn_body(nPCG, cap.get(), false); });
+        graph_ = instantiate(g);
         graph_npcg_ = nPCG;
         graph_nodes_ = nodes;
     }
-    ARAP_CUDA_CHECK(cudaGraphLaunch(graph_, stream));
+    ARAP_CUDA_CHECK(cudaGraphLaunch(graph_.get(), stream));
     launches_ += graph_nodes_;
 }
 

@@ -3,6 +3,7 @@
 // does not fit on chip (1920x1080, SURVEY.md C4) and as the general-size path behind Opt.h.
 #pragma once
 #include "common.cuh"
+#include "devmem.cuh"
 #include "kernel_timer.cuh"
 #include <vector>
 
@@ -78,7 +79,6 @@ struct StreamDev : StreamPlanes {
 class StreamSolver {
 public:
     StreamSolver(int W, int H);
-    ~StreamSolver();
     StreamSolver(const StreamSolver&) = delete;
     StreamSolver& operator=(const StreamSolver&) = delete;
 
@@ -120,13 +120,19 @@ private:
     void launch_gn_body(int nPCG, cudaStream_t stream, bool tracing);
     void launch_step_a(bool first, int it, cudaStream_t stream);
     void launch_step_b(int it, cudaStream_t stream);
+    void drop_graph(); // the next graph step re-captures
     bool general_ = false;
     KernelTimer* timer_ = nullptr;
     float pcg_rtol_ = 0.0f, gn_rtol_ = 0.0f;
     bool rt() const { return (pcg_rtol_ > 0.0f || gn_rtol_ > 0.0f) && !general_; } // the early-exit kernel instantiations
     StreamDev h_{};
-    StreamDev* d_ = nullptr;
-    cudaGraphExec_t graph_ = nullptr;
+    // what h_ points to, and its device copy
+    DevBuf<float> planes_;
+    DevBuf<unsigned char> tile_active_;
+    DevBuf<unsigned long long> acc_;
+    DevBuf<StreamScalars> sc_;
+    DevBuf<StreamDev> d_;
+    GraphExecHandle graph_;
     int graph_npcg_ = -1;
     long long graph_nodes_ = 0;
     long long launches_ = 0;

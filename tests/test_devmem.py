@@ -1,7 +1,8 @@
-"""Who owns device memory (arap_flow_b200/csrc/devmem.cuh, DESIGN.md 4.7).  CPU only.
+"""Who owns CUDA resources (arap_flow_b200/csrc/devmem.cuh, DESIGN.md 4.7).  CPU only.
 
-Only devmem.cuh and the solvers' and the plan's fixed-size constructors allocate.  Every carve the library makes with
-Layout (tests/devmem_host.cpp, built with g++ against the header's CUDA-free part) puts each block at the offset the
+Only devmem.cuh allocates or frees memory, or creates or destroys a stream, an event or a graph.  Only the C ABI
+functions that free a handle contain a delete expression.  Every carve the library makes with Layout
+(tests/devmem_host.cpp, built with g++ against the header's CUDA-free part) puts each block at the offset the
 hand-chained 256-byte arithmetic it replaced gave it, and keeps each block's byte count."""
 import ctypes as C
 import os
@@ -13,9 +14,18 @@ import pytest
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
 
-# allocation owners: the RAII types, and objects whose buffers are fixed-size and owned by constructor and destructor
-OWNERS = {"devmem.cuh", "solver_stream.cu", "solver_resident.cu", "solver_lm.cu", "plan.cu"}
-ALLOC = re.compile(r"\bcuda(?:Malloc|Free)(?:Host)?\s*\(")
+CSRC = os.path.join(ROOT, "arap_flow_b200", "csrc")
+SOURCES = (".cu", ".cuh", ".cpp", ".h")
+
+# the owners: DevBuf, GrowBuf, the stream / event / graph handles and the workspace's stream
+OWNERS = {"devmem.cuh"}
+ALLOC = re.compile(r"\bcuda(?:(?:Malloc|Free)(?:Host)?|StreamCreate\w*|StreamDestroy|EventCreate\w*|EventDestroy"
+                   r"|GraphInstantiate\w*|GraphDestroy|GraphExecDestroy)\s*\(")
+# the functions that free a C ABI handle: the only places a delete expression may stand
+C_ABI_FREES = {"arapb200_api.cu": {"arapb200_batch_create", "arapb200_batch_destroy"},
+               "opt_api.cu": {"Opt_ProblemDelete", "Opt_PlanFree"}}
+# a definition starting in column 0: its name is the last identifier before the first parenthesis
+DEFINITION = re.compile(r"^[A-Za-z_][\w\s*&:<>,]*?\b(\w+)\s*\(", re.M)
 
 C1 = 854 * 480  # C1 and C2 frames
 SIZES = (6, 1021 * 7, C1)
@@ -30,13 +40,40 @@ def test_only_the_owners_allocate():
     for top in ("arap_flow_b200", "include"):
         for d, _, files in os.walk(os.path.join(ROOT, top)):
             for f in files:
-                if not f.endswith((".cu", ".cuh", ".cpp", ".h")):
+                if not f.endswith(SOURCES):
                     continue
                 with open(os.path.join(d, f), encoding="utf-8") as fh:
                     if ALLOC.search(fh.read()):
                         found.add(f)
     assert "devmem.cuh" in found
     assert found <= OWNERS, sorted(found - OWNERS)
+
+
+def _code(text):
+    """text with comments and string literals blanked (line numbers kept)"""
+    return re.sub(r'//[^\n]*|/\*.*?\*/|"(?:\\.|[^"\\\n])*"', lambda m: re.sub(r"[^\n]", " ", m.group()), text,
+                  flags=re.S)
+
+
+def test_only_the_c_abi_frees_delete():
+    stray, frees = [], set()
+    for d, _, files in os.walk(CSRC):
+        for f in files:
+            if not f.endswith(SOURCES):
+                continue
+            with open(os.path.join(d, f), encoding="utf-8") as fh:
+                code = _code(fh.read())
+            defs = [(m.start(), m.group(1)) for m in DEFINITION.finditer(code)]
+            for m in re.finditer(r"\bdelete\b", code):
+                if code[:m.start()].rstrip().endswith("="):  # a deleted function
+                    continue
+                fn = max(((at, name) for at, name in defs if at < m.start()), default=(0, None))[1]
+                if fn in C_ABI_FREES.get(f, ()):
+                    frees.add(fn)
+                else:
+                    stray.append(f"{f}:{code.count(chr(10), 0, m.start()) + 1} in {fn}")
+    assert not stray, stray
+    assert frees == set().union(*C_ABI_FREES.values())  # the scan sees the deletes that are allowed
 
 
 @pytest.fixture(scope="module")
