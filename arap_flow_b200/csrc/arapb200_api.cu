@@ -63,6 +63,17 @@ int warp_common(int W, int H, const float* pos_or_flow, bool is_flow, const uint
     return 0;
 }
 
+// forget a slot's tracks request (DESIGN.md 4.9)
+void drop_tracks(HostProblem& hp)
+{
+    hp.tracks = false;
+    hp.trk_flow0 = hp.trk_bflow0 = nullptr;
+    hp.trk_occ0 = nullptr;
+    hp.queries.clear();
+    hp.query_pos = nullptr;
+    hp.query_occ = nullptr;
+}
+
 } // namespace
 
 struct arapb200_batch {
@@ -144,6 +155,28 @@ int arapb200_warp_seq(int W, int H, int K, const float* pos, const uint8_t* rgb,
         if (out_bflow) d_bflow.down((float2*)out_bflow);
         if (out_occ) d_occ.down(out_occ);
         if (out_flow0) d_flow0.down((float2*)out_flow0);
+        ARAP_CUDA_OR_RETURN(cudaDeviceSynchronize());
+        return 0;
+    });
+}
+
+int arapb200_warp_tracks(int W, int H, int K, const float* pos, const uint8_t* mask_red, float* out_bflow0,
+                         uint8_t* out_occ0)
+{
+    return guarded([&]() -> int {
+        if (W <= 0 || H <= 0 || K <= 0 || !pos || !mask_red) return 1;
+        // the batch's kernels: enqueue_warp_seq with the tracks of DESIGN.md 4.9 (colours are not asked for: black rgb)
+        const size_t N = (size_t)W * H, F = N * K;
+        DevBuf<float2> d_pos(F), d_flow(F), d_bflow(F), d_flow0(F), d_bflow0(F);
+        DevBuf<unsigned char> d_rgb(3 * N), d_mask(N), d_orgb(3 * F), d_omask(F), d_occ(F), d_occ0(F);
+        DevBuf<unsigned> d_z(2 * N);
+        d_pos.up((const float2*)pos);
+        d_mask.up(mask_red);
+        ARAP_CUDA_OR_RETURN(cudaMemsetAsync(d_rgb.p, 0, 3 * N, nullptr));
+        const SeqOut o{d_orgb.p, d_omask.p, d_flow.p, d_bflow.p, d_occ.p, d_flow0.p, d_bflow0.p, d_occ0.p};
+        enqueue_warp_seq(W, H, K, d_pos.p, d_rgb.p, d_mask.p, d_z.p, o, nullptr);
+        if (out_bflow0) d_bflow0.down((float2*)out_bflow0);
+        if (out_occ0) d_occ0.down(out_occ0);
         ARAP_CUDA_OR_RETURN(cudaDeviceSynchronize());
         return 0;
     });
@@ -240,6 +273,7 @@ int arapb200_batch_submit_seq(arapb200_batch* b, int slot, int W, int H, const u
         hp.seq_rgb = seq_rgb; hp.seq_mask = seq_mask; hp.seq_flow = seq_flow; hp.seq_bflow = seq_bflow;
         hp.seq_occ = seq_occ; hp.seq_flow0 = seq_flow0;
         hp.scene = false; // the slot may have been a scene layer in an earlier run
+        drop_tracks(hp); // a new problem drops an earlier tracks request
         b->pending[slot] = 1;
         return 0;
     });
@@ -377,6 +411,53 @@ int arapb200_batch_scene_blur(arapb200_batch* b, int slot, int n_samples, double
     });
 }
 
+int arapb200_batch_tracks(arapb200_batch* b, int slot, float* flow0, float* bflow0, uint8_t* occ0, int n_queries,
+                          const int32_t* queries, float* query_pos, uint8_t* query_occ)
+{
+    return guarded([&]() -> int {
+        // every rejection comes before anything is changed
+        if (!b || slot < 0 || slot >= b->max_problems) return 1;
+        const int q = b->scene_of[slot];
+        HostScene* sc = q >= 0 && b->scenes[q].first == slot ? &b->scenes[q] : nullptr;
+        HostProblem& hp = b->slots[slot];
+        const bool plain = q < 0 && b->pending[slot] && !hp.scene;
+        const int K = sc ? (int)(sc->maps.size() / 18) - 1 : plain ? (int)hp.steps.size() : 0;
+        if (K == 0) {
+            fprintf(stderr, "arapb200: batch_tracks: slot %d holds no problem or scene queued with frames\n", slot);
+            return 1;
+        }
+        const int W = sc ? sc->W : hp.W, H = sc ? sc->H : hp.H;
+        bool ok = n_queries >= 0 && (flow0 || bflow0 || occ0 || n_queries > 0) &&
+                  (n_queries == 0 ? !query_pos && !query_occ : queries && query_pos);
+        for (int i = 0; ok && i < n_queries; ++i)
+            ok = queries[2 * i] >= 0 && queries[2 * i] < W && queries[2 * i + 1] >= 0 && queries[2 * i + 1] < H;
+        if (!ok) {
+            fprintf(stderr, "arapb200: batch_tracks: bad request (nothing asked for, %d queries, null queries or "
+                    "query_pos, query outputs without queries, or a query outside the %dx%d frame)\n", n_queries, W, H);
+            return 1;
+        }
+        std::vector<float> maps(sc ? 18 * (size_t)K : 0);
+        for (int k = 1; sc && k <= K; ++k) // frame 0 -> frame k of the background: composite_coeffs(NULL, A_k)
+            if (!composite_coeffs(nullptr, sc->motions.data() + 6 * k, maps.data() + 18 * (k - 1))) {
+                fprintf(stderr, "arapb200: batch_tracks: frame %d's motion gives non-finite maps\n", k);
+                return 1;
+            }
+        auto attach = [&](auto& t) {
+            t.tracks = true;
+            t.trk_flow0 = flow0; t.trk_bflow0 = bflow0; t.trk_occ0 = occ0;
+            t.queries.assign(queries, queries + 2 * (size_t)n_queries);
+            t.query_pos = query_pos; t.query_occ = query_occ;
+        };
+        if (sc) {
+            attach(*sc);
+            sc->track_maps.swap(maps);
+        } else {
+            attach(hp);
+        }
+        return 0;
+    });
+}
+
 int arapb200_blur_schedule(int nCont, int n_frames, const int* steps, const double* motion,
                            const double* frame_motions, int n_samples, double shutter, int image, int* out_state,
                            float* out_w, float* out_smap)
@@ -411,8 +492,12 @@ int arapb200_batch_run(arapb200_batch* b)
         b->scene_of.assign(b->max_problems, -1);
         for (HostScene& sc : scenes) {
             sc.first = at[sc.first]; // a scene's slots are consecutive and all pending
-            for (int s = 0; s < sc.n; ++s) b->todo[sc.first + s].blur_states = sc.blur_states;
+            for (int s = 0; s < sc.n; ++s) {
+                b->todo[sc.first + s].blur_states = sc.blur_states;
+                b->todo[sc.first + s].tracks = sc.tracks; // a tracked scene's layers keep their frame k -> 0 flows
+            }
         }
+        for (HostProblem& hp : b->slots) drop_tracks(hp); // the run drops the tracks requests, as it drops the scenes
         const int rc = b->pipe->run(b->todo.data(), (int)b->todo.size(), scenes.data(), (int)scenes.size());
         if (rc) return rc;
         b->ms[0] = b->pipe->last_ms_total();

@@ -94,23 +94,26 @@ __global__ void __launch_bounds__(256) k_composite_b(int W, int H, Layers L, con
 // frame b; bflow_b: the frame-b backward flow k_composite_b wrote (read only for out_occ).  kSrcPrev: L.src are the
 // warped masks of frame k-1 of a sequence, p being on layer s where one is 255 -- the "255 - mask" of the flatten recipe
 // (DESIGN.md 4.4) read in place.
-template <bool kSrcPrev>
-__global__ void __launch_bounds__(256) k_composite_a(int W, int H, Layers L, Affine F,
-                                                      const float2* __restrict__ bflow_b, float2* __restrict__ out_flow,
-                                                      unsigned char* __restrict__ out_occ)
+// kOwnerFlow: the flow of p's own surface on object pixels instead of the flatten's selection (tracks, DESIGN.md 4.9)
+template <bool kSrcPrev, bool kOwnerFlow>
+__device__ __forceinline__ void composite_a_at(int W, int H, const Layers& L, const Affine& F,
+                                               const float2* __restrict__ bflow_b, float2* __restrict__ out_flow,
+                                               unsigned char* __restrict__ out_occ, size_t i)
 {
-    const size_t N = (size_t)W * H;
-    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (i >= N) return;
     const int px = (int)(i % W), py = (int)(i / W);
     int seg = L.n; // p's surface: the (last) layer whose input mask has p on the object, else the background
     for (int s = L.n - 1; s >= 0; --s)
         if (kSrcPrev ? L.src[s][i] == 255 : L.src[s][i] == 0) { seg = s; break; }
     float2 f;
     if (seg < L.n) {
-        const int front = front_layer(L, i);
-        out_flow[i] = L.flow[front < 0 ? 0 : front][i]; // the flatten's own selection
-        f = L.flow[seg][i];
+        if (kOwnerFlow) {
+            f = L.flow[seg][i];
+            out_flow[i] = f;
+        } else {
+            const int front = front_layer(L, i);
+            out_flow[i] = L.flow[front < 0 ? 0 : front][i]; // the flatten's own selection
+            f = L.flow[seg][i];
+        }
     } else {
         const float2 a = affine_at(F, px, py);
         f = make_float2(__fsub_rn(a.x, (float)px), __fsub_rn(a.y, (float)py));
@@ -121,6 +124,44 @@ __global__ void __launch_bounds__(256) k_composite_a(int W, int H, Layers L, Aff
             const int s = front_layer(L, q);
             return s < 0 ? L.n : s;
         });
+}
+
+template <bool kSrcPrev>
+__global__ void __launch_bounds__(256) k_composite_a(int W, int H, Layers L, Affine F,
+                                                      const float2* __restrict__ bflow_b, float2* __restrict__ out_flow,
+                                                      unsigned char* __restrict__ out_occ)
+{
+    const size_t N = (size_t)W * H;
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= N) return;
+    composite_a_at<kSrcPrev, false>(W, H, L, F, bflow_b, out_flow, out_occ, i);
+}
+
+// ---- tracks (DESIGN.md 4.9): frame 0 to frame k of a scene ----
+// frame-k pass: k_composite_b's backward flow alone (L.bflow the layers' frame k -> 0 flows, B: frame k -> frame 0)
+__global__ void __launch_bounds__(256) k_track_b(int W, int H, Layers L, Affine B, float2* __restrict__ out_bflow)
+{
+    const size_t N = (size_t)W * H;
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= N) return;
+    const int qx = (int)(i % W), qy = (int)(i / W);
+    const int front = front_layer(L, i);
+    if (front >= 0) {
+        out_bflow[i] = L.bflow[front][i];
+        return;
+    }
+    const float2 b = affine_at(B, qx, qy);
+    out_bflow[i] = make_float2(__fsub_rn(b.x, (float)qx), __fsub_rn(b.y, (float)qy));
+}
+
+// frame-0 pass: k_composite_a<false> with the owner's flow (L.flow the layers' frame 0 -> k flows, F: frame 0 -> frame k)
+__global__ void __launch_bounds__(256) k_track_a(int W, int H, Layers L, Affine F, const float2* __restrict__ bflow_b,
+                                                  float2* __restrict__ out_flow, unsigned char* __restrict__ out_occ)
+{
+    const size_t N = (size_t)W * H;
+    const size_t i = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (i >= N) return;
+    composite_a_at<false, true>(W, H, L, F, bflow_b, out_flow, out_occ, i);
 }
 
 // frame 0 of a scene: the input image where any layer's input mask is 0 (the object), the background crop elsewhere
@@ -398,6 +439,14 @@ void enqueue_composite(int W, int H, const Layers& L, bool src_prev, const unsig
                                               d_rgb, d_mask, d_bflow);
     if (src_prev) k_composite_a<true><<<blocks, 256, 0, stream>>>(W, H, L, affine_of(c), d_bflow, d_flow, d_occ);
     else k_composite_a<false><<<blocks, 256, 0, stream>>>(W, H, L, affine_of(c), d_bflow, d_flow, d_occ);
+}
+
+void enqueue_composite_tracks(int W, int H, const Layers& L, const float c[18], float2* d_flow0, float2* d_bflow0,
+                              unsigned char* d_occ0, cudaStream_t stream)
+{
+    const unsigned blocks = (unsigned)(((size_t)W * H + 255) / 256);
+    k_track_b<<<blocks, 256, 0, stream>>>(W, H, L, affine_of(c + 6), d_bflow0);
+    k_track_a<<<blocks, 256, 0, stream>>>(W, H, L, affine_of(c), d_bflow0, d_flow0, d_occ0);
 }
 
 void enqueue_scene_input(int W, int H, const Layers& L, const unsigned char* d_rgb, const unsigned char* d_bg, int bgW,

@@ -34,6 +34,11 @@ void enqueue_composite(int W, int H, const Layers& L, bool src_prev, const unsig
                        int bg_x, int bg_y, const float c[18], float2* d_flow, unsigned char* d_rgb,
                        unsigned char* d_mask, float2* d_bflow, unsigned char* d_occ, cudaStream_t stream);
 
+// the tracks of frame k of a scene (DESIGN.md 4.9) with c = composite_coeffs(NULL, A_k): k_track_b (bflow0, frame k) then
+// k_track_a (flow0 and occ0, frame 0).  L: the layers' flow0, warped mask and bflow0 of frame k and their input masks.
+void enqueue_composite_tracks(int W, int H, const Layers& L, const float c[18], float2* d_flow0, float2* d_bflow0,
+                              unsigned char* d_occ0, cudaStream_t stream);
+
 // frame 0 of a scene (k_scene_input): d_rgb where any layer's input mask L.src is 0, else the background at
 // q + (bg_x, bg_y), coordinates clamped to the image as the composite clamps them
 void enqueue_scene_input(int W, int H, const Layers& L, const unsigned char* d_rgb, const unsigned char* d_bg, int bgW,

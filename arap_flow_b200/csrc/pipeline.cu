@@ -89,12 +89,14 @@ __global__ void __launch_bounds__(256) k_scatter_t(const MatchRec* __restrict__ 
 __global__ void k_copy_cost(const StreamScalars* __restrict__ sc, float* __restrict__ dst) { *dst = sc->cost; }
 
 // a scene's device buffer: [background][rgb0][flow][rgb][mask][bflow][occ], the last five holding the pair (index 0) and
-// frames 1 .. K, so that each frame output leaves in one copy
+// frames 1 .. K, so that each frame output leaves in one copy; with tracks then [flow0][bflow0][occ0] of frames 1 .. K
+// and [queries][query_pos][query_occ] (DESIGN.md 4.9)
 struct SceneLayout {
-    size_t bg, rgb0, flow, rgb, mask, bflow, occ, bytes;
+    size_t bg, rgb0, flow, rgb, mask, bflow, occ, flow0, bflow0, occ0, queries, query_pos, query_occ, bytes;
     explicit SceneLayout(const HostScene& sc)
     {
         const size_t N = (size_t)sc.W * sc.H, F = N * (sc.maps.size() / 18);
+        const size_t T = sc.tracks ? F - N : 0, n = sc.queries.size() / 2, Q = n * (sc.maps.size() / 18 - 1);
         Layout l;
         bg = l.take(3 * (size_t)sc.bgW * sc.bgH);
         rgb0 = l.take(sc.out_rgb0 ? 3 * N : 0);
@@ -103,6 +105,12 @@ struct SceneLayout {
         mask = l.take(F);
         bflow = l.take(8 * F);
         occ = l.take(F);
+        flow0 = l.take(8 * T);
+        bflow0 = l.take(8 * T);
+        occ0 = l.take(T);
+        queries = l.take(8 * n);
+        query_pos = l.take(8 * Q);
+        query_occ = l.take(Q);
         bytes = l.bytes();
     }
 };
@@ -337,6 +345,29 @@ void BatchPipeline::enqueue_scene(const HostScene& sc, unsigned char* buf)
                           (float2*)(buf + o.bflow) + f, buf + o.occ + f, stream_.get());
         launches_ += 2;
     }
+    if (!sc.tracks) return;
+    // tracks (DESIGN.md 4.9): frame k's layers with their frame 0 -> k flows and frame k -> 0 backward flows, and the
+    // input masks as source masks, composited against the background's motion from frame 0
+    for (int k = 1; k <= K; ++k) {
+        const size_t f = (size_t)(k - 1) * N;
+        for (int s = 0; s < sc.n; ++s) {
+            const Dev& d = dev_[sc.first + s];
+            L.flow[s] = d.seq.flow0 + f;
+            L.rgb[s] = d.seq.rgb + 3 * f;
+            L.mask[s] = d.seq.mask + f;
+            L.bflow[s] = d.seq.bflow0 + f;
+            L.src[s] = d.mask.p;
+        }
+        enqueue_composite_tracks(sc.W, sc.H, L, sc.track_maps.data() + 18 * (k - 1), (float2*)(buf + o.flow0) + f,
+                                 (float2*)(buf + o.bflow0) + f, buf + o.occ0 + f, stream_.get());
+        launches_ += 2;
+    }
+    if (!sc.queries.empty()) {
+        enqueue_track_queries(sc.W, sc.H, K, (int)(sc.queries.size() / 2), (const int2*)(buf + o.queries),
+                              (const float2*)(buf + o.flow0), buf + o.occ0, (float2*)(buf + o.query_pos),
+                              buf + o.query_occ, stream_.get());
+        launches_ += 1;
+    }
 }
 
 // per image asked for (frame 0, the pair, frames 1 .. K) its S sub-frames, each lerping every layer between two of its
@@ -415,15 +446,23 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
             d.occ = x + x_occ;
         }
         if (hp.out_bflow || hp.out_occ) d.h_extras.reserve(xl.bytes());
-        if (!hp.steps.empty()) { // [pos][z][rgb][mask][flow][bflow][occ][flow0]: z two z-buffers, the rest K frames each
-            const size_t F = Nmax * hp.steps.size();
+        if (!hp.steps.empty()) { // [pos][z][rgb][mask][flow][bflow][occ][flow0]: z two z-buffers, the rest K frames each;
+            // with tracks then [bflow0][occ0] (K frames each, a scene layer no occ0) and [queries][query_pos][query_occ]
+            const size_t F = Nmax * hp.steps.size(), Q = hp.queries.size() / 2 * hp.steps.size();
+            const bool occ0 = hp.tracks && !hp.scene;
             Layout l;
             const size_t pos = l.take(8 * F), z = l.take(2 * 4 * Nmax), rgb = l.take(3 * F), mask = l.take(F),
-                         flow = l.take(8 * F), bflow = l.take(8 * F), occ = l.take(F), flow0 = l.take(8 * F);
+                         flow = l.take(8 * F), bflow = l.take(8 * F), occ = l.take(F), flow0 = l.take(8 * F),
+                         t_bflow0 = l.take(hp.tracks ? 8 * F : 0), t_occ0 = l.take(occ0 ? F : 0),
+                         queries = l.take(4 * hp.queries.size()), qpos = l.take(8 * Q), qocc = l.take(Q);
             unsigned char* f = d.frames.reserve(l.bytes());
             d.seq_pos = (float2*)(f + pos);
             d.seq_z = (unsigned*)(f + z);
-            d.seq = SeqOut{f + rgb, f + mask, (float2*)(f + flow), (float2*)(f + bflow), f + occ, (float2*)(f + flow0)};
+            d.seq = SeqOut{f + rgb, f + mask, (float2*)(f + flow), (float2*)(f + bflow), f + occ, (float2*)(f + flow0),
+                           hp.tracks ? (float2*)(f + t_bflow0) : nullptr, occ0 ? f + t_occ0 : nullptr};
+            d.queries = (int2*)(f + queries);
+            d.query_pos = (float2*)(f + qpos);
+            d.query_occ = f + qocc;
         }
         if (!hp.blur_states.empty()) d.blur_pos = (float2*)d.blur.reserve(8 * N * hp.blur_states.size());
         memcpy(d.h_in.data(), hp.rgb, 3 * N);
@@ -444,6 +483,9 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
         if (!d.recs.empty())
             ARAP_CUDA_CHECK(cudaMemcpyAsync(d.matches.data(), d.recs.data(), d.recs.size() * sizeof(MatchRec),
                                             cudaMemcpyHostToDevice, stream_.get()));
+        if (!hp.queries.empty())
+            ARAP_CUDA_CHECK(cudaMemcpyAsync(d.queries, hp.queries.data(), hp.queries.size() * sizeof(int),
+                                            cudaMemcpyHostToDevice, stream_.get()));
         enqueue_reset_state(hp.W, hp.H, d.mask.p, d.X.p, d.U.p, d.A.p, d.M.p, stream_.get());
         launches_ += 1;
         d.resident = false;
@@ -453,6 +495,9 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
         const HostScene& sc = scenes[j];
         ARAP_CUDA_CHECK(cudaMemcpyAsync(scene_dev_[j].data(), sc.background, 3 * (size_t)sc.bgW * sc.bgH,
                                         cudaMemcpyHostToDevice, stream_.get()));
+        if (!sc.queries.empty())
+            ARAP_CUDA_CHECK(cudaMemcpyAsync(scene_dev_[j].data() + SceneLayout(sc).queries, sc.queries.data(),
+                                            sc.queries.size() * sizeof(int), cudaMemcpyHostToDevice, stream_.get()));
     }
     n_resident_ = 0;
     if (resident_ && !lm_on_) {
@@ -510,6 +555,11 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
         if (!hp.steps.empty())
             launches_ += enqueue_warp_seq(hp.W, hp.H, (int)hp.steps.size(), d.seq_pos, d.rgb.p, d.mask.p, d.seq_z, d.seq,
                                           stream_.get());
+        if (!hp.scene && !hp.queries.empty()) {
+            enqueue_track_queries(hp.W, hp.H, (int)hp.steps.size(), (int)(hp.queries.size() / 2), d.queries, d.seq.flow0,
+                                  d.seq.occ0, d.query_pos, d.query_occ, stream_.get());
+            launches_ += 1;
+        }
     }
     for (int j = 0; j < n_scenes; ++j) {
         enqueue_scene(scenes[j], scene_dev_[j].data());
@@ -537,7 +587,10 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
         const size_t F = N * hp.steps.size();
         const struct { void* dst; const void* src; size_t bytes; } seq[] = {
             {hp.seq_rgb, d.seq.rgb, 3 * F}, {hp.seq_mask, d.seq.mask, F}, {hp.seq_flow, d.seq.flow, 8 * F},
-            {hp.seq_bflow, d.seq.bflow, 8 * F}, {hp.seq_occ, d.seq.occ, F}, {hp.seq_flow0, d.seq.flow0, 8 * F}};
+            {hp.seq_bflow, d.seq.bflow, 8 * F}, {hp.seq_occ, d.seq.occ, F}, {hp.seq_flow0, d.seq.flow0, 8 * F},
+            {hp.trk_flow0, d.seq.flow0, 8 * F}, {hp.trk_bflow0, d.seq.bflow0, 8 * F}, {hp.trk_occ0, d.seq.occ0, F},
+            {hp.query_pos, d.query_pos, 4 * hp.queries.size() * hp.steps.size()},
+            {hp.query_occ, d.query_occ, hp.queries.size() / 2 * hp.steps.size()}};
         for (const auto& c : seq)
             if (c.dst && F) ARAP_CUDA_CHECK(cudaMemcpyAsync(c.dst, c.src, c.bytes, cudaMemcpyDeviceToHost, stream_.get()));
     }
@@ -551,7 +604,10 @@ int BatchPipeline::run(const HostProblem* problems, int count, const HostScene* 
             {sc.out_flow, l.flow, 8 * N}, {sc.out_rgb, l.rgb, 3 * N}, {sc.out_mask, l.mask, N},
             {sc.out_bflow, l.bflow, 8 * N}, {sc.out_occ, l.occ, N}, {sc.out_rgb0, l.rgb0, 3 * N},
             {sc.seq_flow, l.flow + 8 * N, 8 * F}, {sc.seq_rgb, l.rgb + 3 * N, 3 * F}, {sc.seq_mask, l.mask + N, F},
-            {sc.seq_bflow, l.bflow + 8 * N, 8 * F}, {sc.seq_occ, l.occ + N, F}};
+            {sc.seq_bflow, l.bflow + 8 * N, 8 * F}, {sc.seq_occ, l.occ + N, F}, {sc.trk_flow0, l.flow0, 8 * F},
+            {sc.trk_bflow0, l.bflow0, 8 * F}, {sc.trk_occ0, l.occ0, F},
+            {sc.query_pos, l.query_pos, 4 * sc.queries.size() * (F / N)},
+            {sc.query_occ, l.query_occ, sc.queries.size() / 2 * (F / N)}};
         for (const auto& c : out)
             if (c.dst && c.bytes)
                 ARAP_CUDA_CHECK(cudaMemcpyAsync(c.dst, b + c.off, c.bytes, cudaMemcpyDeviceToHost, stream_.get()));

@@ -34,6 +34,15 @@ struct HostProblem {
     bool scene = false;
     // a layer of a blurred scene: the continuation steps whose X its sub-frames read (sorted; DESIGN.md 4.8)
     std::vector<int> blur_states;
+    // opt-in tracks from frame 0 to every frame (DESIGN.md 4.9, arapb200_batch_tracks; needs steps): bflow0 and occ0 of
+    // every frame on the device (a scene layer: bflow0 only, the scene composites the rest), and per frame the outputs
+    // [K][N][...] (trk_flow0 the same bits as seq_flow0) and the query gather [K][n][...], each may be null
+    bool tracks = false;
+    float *trk_flow0 = nullptr, *trk_bflow0 = nullptr;
+    unsigned char* trk_occ0 = nullptr;
+    std::vector<int> queries; // (x, y) frame-0 pixels
+    float* query_pos = nullptr;
+    unsigned char* query_occ = nullptr;
 };
 
 // A scene (DESIGN.md 4.6): problems first .. first + n - 1 of a run are its layers in segment order (same W x H and rgb),
@@ -58,6 +67,15 @@ struct HostScene {
     std::vector<BlurSub> blur;
     std::vector<int> blur_states;
     unsigned char *blur_rgb = nullptr, *blur_rgb0 = nullptr, *seq_blur_rgb = nullptr;
+    // opt-in tracks (DESIGN.md 4.9, arapb200_batch_tracks), as HostProblem's; track_maps [K][18]: composite_coeffs(NULL,
+    // A_k) of frame k = 1 .. K
+    bool tracks = false;
+    std::vector<float> track_maps;
+    float *trk_flow0 = nullptr, *trk_bflow0 = nullptr;
+    unsigned char* trk_occ0 = nullptr;
+    std::vector<int> queries;
+    float* query_pos = nullptr;
+    unsigned char* query_occ = nullptr;
 };
 
 // compact constraint record: source pixel index and the match, after the reference's filtering
@@ -128,6 +146,9 @@ private:
         float2* blur_pos = nullptr; // X after each blur state
         unsigned* seq_z = nullptr; // two z-buffers
         SeqOut seq{};
+        int2* queries = nullptr; // a tracked problem's queries and their gather (DESIGN.md 4.9)
+        float2* query_pos = nullptr;
+        unsigned char* query_occ = nullptr;
         std::vector<MatchRec> recs;
         bool resident = false;
         const MatchRec* recs_dev() const { return (const MatchRec*)matches.data(); }
@@ -140,7 +161,8 @@ private:
     // X -> frame buffer if step t is one of hp's frames, and -> blur buffer if it is one of its blur states
     void snapshot(const HostProblem& hp, Dev& d, int t);
     // device buffer of the j-th scene of a run, allocated the first time and grown for a larger scene: the background,
-    // frame 0 and the composited pair and frames (21 B/px each), laid out by SceneLayout (pipeline.cu)
+    // frame 0 and the composited pair and frames (21 B/px each), with tracks 17 B/px per frame and the queries, laid out
+    // by SceneLayout (pipeline.cu)
     std::vector<GrowBuf> scene_dev_;
     void enqueue_scene(const HostScene& sc, unsigned char* buf); // the scene's kernels (DESIGN.md 4.6)
     // the blurred scene at the j-th scene position, its scratch allocated the first time and grown for a larger scene:

@@ -43,6 +43,16 @@ __device__ __forceinline__ float2 interp_minus_q(const Bary& w, const Tri& tr, V
     return make_float2(__fsub_rn(sx, (float)qx), __fsub_rn(sy, (float)qy));
 }
 
+// The pixel grid as a vertex source: vertex i at its undeformed position.  The backward flow of frame 1 (k_resolve<true>)
+// and the backward flow of frame k to frame 0 (k_interp_grid, DESIGN.md 4.9) both use it, so the two agree bit for bit.
+struct GridVert {
+    int W;
+    __device__ __forceinline__ float2 operator()(size_t i) const
+    {
+        return make_float2((float)(int)(i % W), (float)(int)(i / W));
+    }
+};
+
 // pass 2: one thread per output pixel.  BFLOW: also the backward flow -- the winning triangle's barycentrics applied to
 // its undeformed vertex coordinates give the exact frame-1 source point of the pixel (DESIGN.md 4.3).
 template <bool BFLOW>
@@ -76,9 +86,7 @@ __global__ void __launch_bounds__(256) k_resolve(int W, int H, const float2* __r
         c2 = (unsigned char)__float2int_rz(v[2]);
         m = 255;
         if (BFLOW)
-            bf = interp_minus_q(w, Tri{ia, ib, ic}, [W](size_t i) {
-                return make_float2((float)(int)(i % W), (float)(int)(i / W));
-            }, x, y);
+            bf = interp_minus_q(w, Tri{ia, ib, ic}, GridVert{W}, x, y);
     }
     out_rgb[3 * o] = c0;
     out_rgb[3 * o + 1] = c1;
@@ -104,13 +112,10 @@ __global__ void __launch_bounds__(256) k_occlusion(int W, int H, const unsigned 
 // interp(z_a, P_a, V)[q] = the weights of q's winning triangle in frame a (lk against P_a) applied to that triangle's
 // vertices in V, minus q; (0, 0) where nothing landed (z_a[q] == 0).  (z_{k-1}, P_{k-1}, P_k) is the flow from frame
 // k - 1 to frame k, (z_k, P_k, P_{k-1}) the backward flow from frame k to frame k - 1 (DESIGN.md 4.4).
-__global__ void __launch_bounds__(256) k_interp(int W, int H, const unsigned* __restrict__ z_a,
-                                                 const float2* __restrict__ P_a, const float2* __restrict__ V,
-                                                 float2* __restrict__ out)
+template <class Vert>
+__device__ __forceinline__ float2 interp_at(int W, const unsigned* __restrict__ z_a, const float2* __restrict__ P_a,
+                                            Vert vert, size_t q)
 {
-    const size_t N = (size_t)W * H;
-    const size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
-    if (q >= N) return;
     const unsigned id = z_a[q];
     float2 r = make_float2(0.f, 0.f);
     if (id) {
@@ -118,9 +123,44 @@ __global__ void __launch_bounds__(256) k_interp(int W, int H, const unsigned* __
         const float2 a = P_a[tr.ia], b = P_a[tr.ib], c = P_a[tr.ic];
         const int x = (int)(q % W), y = (int)(q / W);
         const Bary w = lk(a.x, a.y, b.x, b.y, c.x, c.y, (float)x, (float)y);
-        r = interp_minus_q(w, tr, [V](size_t i) { return V[i]; }, x, y);
+        r = interp_minus_q(w, tr, vert, x, y);
     }
-    out[q] = r;
+    return r;
+}
+
+__global__ void __launch_bounds__(256) k_interp(int W, int H, const unsigned* __restrict__ z_a,
+                                                 const float2* __restrict__ P_a, const float2* __restrict__ V,
+                                                 float2* __restrict__ out)
+{
+    const size_t N = (size_t)W * H;
+    const size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= N) return;
+    out[q] = interp_at(W, z_a, P_a, [V](size_t i) { return V[i]; }, q);
+}
+
+// interp(z_k, P_k, grid): the backward flow of frame k to frame 0 (DESIGN.md 4.9), k_resolve<true>'s for k = 1
+__global__ void __launch_bounds__(256) k_interp_grid(int W, int H, const unsigned* __restrict__ z_a,
+                                                      const float2* __restrict__ P_a, float2* __restrict__ out)
+{
+    const size_t N = (size_t)W * H;
+    const size_t q = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (q >= N) return;
+    out[q] = interp_at(W, z_a, P_a, GridVert{W}, q);
+}
+
+// query i of frame k: its frame-0 pixel p plus flow0[k][p], and occ0[k][p] (DESIGN.md 4.9); one thread per (k, i)
+__global__ void __launch_bounds__(256) k_track_queries(int W, int H, int K, int n, const int2* __restrict__ queries,
+                                                        const float2* __restrict__ flow0,
+                                                        const unsigned char* __restrict__ occ0,
+                                                        float2* __restrict__ pos, unsigned char* __restrict__ qocc)
+{
+    const size_t t = (size_t)blockIdx.x * blockDim.x + threadIdx.x;
+    if (t >= (size_t)K * n) return;
+    const int2 c = queries[t % n];
+    const size_t p = (t / n) * ((size_t)W * H) + (size_t)c.y * W + c.x;
+    const float2 f = flow0[p];
+    pos[t] = make_float2(__fadd_rn((float)c.x, f.x), __fadd_rn((float)c.y, f.y));
+    qocc[t] = occ0[p];
 }
 
 // occlusion of frame k - 1 >= 1 in frame k: k_occlusion with p's surface taken from frame k - 1's z-buffer instead of
@@ -209,10 +249,31 @@ int enqueue_warp_seq(int W, int H, int K, const float2* d_pos, const unsigned ch
             k_interp<<<g, 256, 0, stream>>>(W, H, z, P, P - N, bflow);
             k_occlusion_z<<<g, 256, 0, stream>>>(W, H, zp, flow, z, bflow, o.occ + N * k);
         }
-        ARAP_CUDA_CHECK(cudaGetLastError());
         launches += warp_launches_per_call() + (k == 0 ? 3 : 4);
+        // tracks (DESIGN.md 4.9) while z_k is live; frame 1 is the consecutive pair, whose outputs are already there
+        if (o.bflow0) {
+            float2* bflow0 = o.bflow0 + (size_t)k * N;
+            unsigned char* occ0 = o.occ0 ? o.occ0 + (size_t)k * N : nullptr;
+            if (k == 0) {
+                ARAP_CUDA_CHECK(cudaMemcpyAsync(bflow0, bflow, N * sizeof(float2), cudaMemcpyDeviceToDevice, stream));
+                if (occ0) ARAP_CUDA_CHECK(cudaMemcpyAsync(occ0, o.occ, N, cudaMemcpyDeviceToDevice, stream));
+            } else {
+                k_interp_grid<<<g, 256, 0, stream>>>(W, H, z, P, bflow0);
+                if (occ0) k_occlusion<<<g, 256, 0, stream>>>(W, H, d_mask_red, o.flow0 + (size_t)k * N, z, bflow0, occ0);
+                launches += occ0 ? 2 : 1;
+            }
+        }
+        ARAP_CUDA_CHECK(cudaGetLastError());
     }
     return launches;
+}
+
+void enqueue_track_queries(int W, int H, int K, int n, const int2* d_queries, const float2* d_flow0,
+                           const unsigned char* d_occ0, float2* d_pos, unsigned char* d_occ, cudaStream_t stream)
+{
+    const size_t T = (size_t)K * n;
+    k_track_queries<<<(unsigned)((T + 255) / 256), 256, 0, stream>>>(W, H, K, n, d_queries, d_flow0, d_occ0, d_pos, d_occ);
+    ARAP_CUDA_CHECK(cudaGetLastError());
 }
 
 void enqueue_flow_to_pos(int W, int H, const float2* d_flow, float2* d_pos, cudaStream_t stream)

@@ -19,11 +19,19 @@ struct SeqOut {
     float2 *flow, *bflow;      // frame k - 1 -> k on the frame k - 1 grid; frame k -> k - 1 on the frame k grid
     unsigned char* occ;        // occlusion of frame k - 1 in frame k (0 visible, 255 not)
     float2* flow0;             // P_k - grid
+    // opt-in tracks (DESIGN.md 4.9), null = none: interp(z_k, P_k, grid) on the frame k grid, and the occlusion of frame 0
+    // in frame k (k_occlusion with flow0); occ0 needs bflow0.  Frame 1 is copied from bflow and occ.
+    float2* bflow0 = nullptr;
+    unsigned char* occ0 = nullptr;
 };
 // d_pos: the K position fields P_1 .. P_K (frame 0 is the grid); d_z2: uint32[2][W*H] scratch (the z-buffers of two
 // consecutive frames).  Frames are rendered in order.  Returns the number of kernels launched.
 int enqueue_warp_seq(int W, int H, int K, const float2* d_pos, const unsigned char* d_rgb,
                      const unsigned char* d_mask_red, unsigned* d_z2, const SeqOut& out, cudaStream_t stream);
+// the query gather of DESIGN.md 4.9: d_queries int2[n] frame-0 pixels, d_flow0 / d_occ0 [K][W*H]; d_pos float2[K][n] and
+// d_occ uint8[K][n] frame-major.  One launch.
+void enqueue_track_queries(int W, int H, int K, int n, const int2* d_queries, const float2* d_flow0,
+                           const unsigned char* d_occ0, float2* d_pos, unsigned char* d_occ, cudaStream_t stream);
 void enqueue_flow_to_pos(int W, int H, const float2* d_flow, float2* d_pos, cudaStream_t stream);
 void enqueue_pos_to_flow(int W, int H, const float2* d_pos, float2* d_flow, cudaStream_t stream);
 int warp_launches_per_call();

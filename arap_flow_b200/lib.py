@@ -30,7 +30,7 @@ ARAP_SYMBOLS = [
     "arapb200_batch_set_option", "arapb200_batch_resident_count", "arapb200_debug_wide_sum", "arapb200_plan_error", "arapb200_plan_lm_info", "arapb200_plan_timing_report",
     "arapb200_batch_launch_info", "arapb200_warp_ex", "arapb200_batch_submit_ex", "arapb200_flatten_ex",
     "arapb200_warp_seq", "arapb200_batch_submit_seq", "arapb200_composite", "arapb200_batch_submit_scene",
-    "arapb200_batch_scene_blur", "arapb200_blur_schedule",
+    "arapb200_batch_scene_blur", "arapb200_blur_schedule", "arapb200_warp_tracks", "arapb200_batch_tracks",
 ]
 
 
@@ -181,6 +181,62 @@ def warp_seq(positions, rgb, mask_red):
     _check(L.arapb200_warp_seq(W, H, K, pos, _c(rgb, np.uint8), _c(mask_red, np.uint8),
                                *[out[k].ctypes.data for k in SEQ_KEYS]), "arapb200_warp_seq")
     return out
+
+
+def warp_tracks(positions, mask_red):
+    """Tracks from frame 0 of the frame sequence warp_seq renders from the same positions (include/arapb200.h
+    arapb200_warp_tracks, DESIGN.md 4.9).  Returns a dict with a leading K axis, index k - 1 holding frame k: bflow0[K,H,W,2]
+    f32 (frame k -> 0 on the frame k grid) and occ0[K,H,W] u8 (occlusion of frame 0 in frame k, 0 visible, 255 not).
+    The forward flow from frame 0 is warp_seq's flow0."""
+    H, W = mask_red.shape
+    pos = _c(positions, np.float32)
+    K = pos.shape[0]
+    assert pos.shape == (K, H, W, 2), pos.shape
+    out = dict(bflow0=np.zeros((K, H, W, 2), np.float32), occ0=np.zeros((K, H, W), np.uint8))
+    L = load()
+    L.arapb200_warp_tracks.argtypes = [C.c_int, C.c_int, C.c_int, _f32p, _u8p, C.c_void_p, C.c_void_p]
+    _check(L.arapb200_warp_tracks(W, H, K, pos, _c(mask_red, np.uint8), out["bflow0"].ctypes.data,
+                                  out["occ0"].ctypes.data), "arapb200_warp_tracks")
+    return out
+
+
+def _track_queries(queries, W, H):
+    """queries as int32[n, 2] (x, y) pixels of a W x H frame 0, or None for none; raises for anything the library would
+    refuse, so that a bad list queues nothing."""
+    if queries is None:
+        return None
+    q = np.ascontiguousarray(np.asarray(queries).reshape(-1, 2), np.int32)
+    if not len(q):
+        return None
+    if not np.array_equal(q, np.asarray(queries).reshape(-1, 2)):
+        raise ValueError("queries are integer (x, y) pixels")
+    if (q[:, 0] < 0).any() or (q[:, 0] >= W).any() or (q[:, 1] < 0).any() or (q[:, 1] >= H).any():
+        raise ValueError(f"a query lies outside the {W}x{H} frame")
+    return q
+
+
+def _track_arrays(out, tracks, q, K, H, W):
+    """out["tracks"]: flow0, bflow0, occ0 [K,H,W,...] with tracks, query_pos[K,n,2] and query_occ[K,n] with queries;
+    arrays of a previous call are reused where their shapes fit."""
+    want = {}
+    if tracks:
+        want.update(flow0=((K, H, W, 2), np.float32), bflow0=((K, H, W, 2), np.float32), occ0=((K, H, W), np.uint8))
+    if q is not None:
+        want.update(query_pos=((K, len(q), 2), np.float32), query_occ=((K, len(q)), np.uint8))
+    if not want:
+        out.pop("tracks", None)
+        return None
+    old = out.get("tracks", {})
+    out["tracks"] = {k: old[k] if k in old and old[k].shape == shp else np.zeros(shp, dt) for k, (shp, dt) in want.items()}
+    return out["tracks"]
+
+
+def _attach_tracks(L, h, slot, t, q):
+    L.arapb200_batch_tracks.argtypes = [C.c_void_p, C.c_int] + [C.c_void_p] * 3 + [C.c_int] + [C.c_void_p] * 3
+    ptr = lambda k: t[k].ctypes.data if k in t else None  # noqa: E731
+    _check(L.arapb200_batch_tracks(h, slot, ptr("flow0"), ptr("bflow0"), ptr("occ0"), 0 if q is None else len(q),
+                                   None if q is None else q.ctypes.data, ptr("query_pos"), ptr("query_occ")),
+           "arapb200_batch_tracks")
 
 
 def deform(rgb, mask_red, matches, nCont=19, nGN=8, nPCG=400, backend=BACKEND_AUTO):
@@ -369,14 +425,22 @@ class Batch:
         self.L.arapb200_batch_set_option.argtypes = [C.c_void_p, C.c_char_p, C.c_double]
         _check(self.L.arapb200_batch_set_option(self.h, name.encode(), float(value)), "arapb200_batch_set_option")
 
-    def submit(self, slot, rgb, mask_red, matches, out=None, extras=False, frames=None):
+    def submit(self, slot, rgb, mask_red, matches, out=None, extras=False, frames=None, tracks=False, queries=None):
         """Queue one problem.  `out` may be the dict a previous submit() of the same image size returned: its arrays are
         then written in place instead of allocating fresh ones (what a caller looping over many pairs does).
         extras=True: the dict also gets bflow[H,W,2] f32 (backward flow) and occ[H,W] u8 (occlusion of frame 1, 0 visible,
         255 not), as lib.warp_ex computes them on the solved positions (arapb200_batch_submit_ex).
         frames: a strictly increasing list of continuation steps in [0, nCont-1]; the dict then also gets "seq", the
-        dict lib.warp_seq returns for the solver's states after those steps (arapb200_batch_submit_seq)."""
+        dict lib.warp_seq returns for the solver's states after those steps (arapb200_batch_submit_seq).
+        tracks=True (needs frames): the dict also gets "tracks" with flow0[K,H,W,2] (frame 0 -> k, the bits of
+        seq["flow0"]), bflow0[K,H,W,2] (frame k -> 0) and occ0[K,H,W] (occlusion of frame 0 in frame k), as lib.warp_tracks
+        computes them (arapb200_batch_tracks, DESIGN.md 4.9).  queries (needs frames): int (x, y) pixels of frame 0,
+        shape [n, 2]; "tracks" then also gets query_pos[K,n,2] and query_occ[K,n], flow0 and occ0 gathered there.  Raises
+        before anything is queued for tracks or queries without frames and for a query outside the frame."""
         H, W = mask_red.shape
+        q = _track_queries(queries, W, H)
+        if (tracks or q is not None) and (frames is None or len(frames) == 0):
+            raise ValueError("tracks and queries need frames")
         rgb = _c(rgb, np.uint8)
         mask_red = _c(mask_red, np.uint8)
         m = _c(matches, np.int32).reshape(-1, 4)
@@ -400,18 +464,24 @@ class Batch:
             _check(self.L.arapb200_batch_submit_seq(
                 *args, out["bflow"].ctypes.data if extras else None, out["occ"].ctypes.data if extras else None,
                 len(steps), steps.ctypes.data, *[seq[k].ctypes.data for k in SEQ_KEYS]), "arapb200_batch_submit_seq")
+            t = _track_arrays(out, tracks, q, len(steps), H, W)
+            if t is not None:
+                self._keep[slot] += (q,)
+                _attach_tracks(self.L, self.h, slot, t, q)
         elif extras:
             self.L.arapb200_batch_submit_ex.argtypes = self.L.arapb200_batch_submit.argtypes + [C.c_void_p, C.c_void_p]
             _check(self.L.arapb200_batch_submit_ex(*args, out["bflow"].ctypes.data, out["occ"].ctypes.data),
                    "arapb200_batch_submit_ex")
         else:
             _check(self.L.arapb200_batch_submit(*args), "arapb200_batch_submit")
+        if steps is None:
+            out.pop("tracks", None)
         return out
 
     SCENE_KEYS = ("flow", "rgb", "mask", "bflow", "occ")
 
     def submit_scene(self, slot, rgb, masks, matches, background, motion, origin=(0, 0), frames=None, frame_motions=None,
-                     input_frame=False, out=None, blur=None):
+                     input_frame=False, out=None, blur=None, tracks=False, queries=None):
         """Queue a scene (arapb200_batch_submit_scene, DESIGN.md 4.6): one image rgb, its segments' masks (0 = object, in
         segment order) with one match list each, and a background uint8[bgH,bgW,3] that moves by the 2x3 float64 map
         `motion` (frame pixel q of a still background shows background[q + origin]).  The layers take slots
@@ -426,9 +496,17 @@ class Batch:
         input_frame blur_rgb0[H,W,3], and with frames seq["blur_rgb"][K,H,W,3]: each image averaged over n_samples
         sub-frames of a trailing shutter open for the fraction `shutter` of the interval before it.  The sub-frame table
         of every image to blur is checked (lib.blur_schedule) before anything is queued, so a request the library would
-        refuse raises with no scene queued."""
+        refuse raises with no scene queued.
+        tracks=True / queries (both need frames): "tracks" as in submit(), for the scene (arapb200_batch_tracks, DESIGN.md
+        4.9): flow0 takes the flow of the layer that owns the frame-0 pixel (its input mask is 0 there), else the
+        background's; bflow0 and occ0 are what composite() gives for bflow and occ with motion_from=None, motion=A_k and
+        the layers' frame-k masks, frame 0 -> k flows and frame k -> 0 backward flows.  Raises before anything is queued
+        for tracks or queries without frames and for a query outside the frame."""
         n = len(masks)
         H, W = masks[0].shape
+        q = _track_queries(queries, W, H)
+        if (tracks or q is not None) and (frames is None or len(frames) == 0):
+            raise ValueError("tracks and queries need frames")
         rgb = _c(rgb, np.uint8)
         mk = [_c(m, np.uint8) for m in masks]
         mt = [_c(m, np.int32).reshape(-1, 4) for m in matches]
@@ -496,6 +574,10 @@ class Batch:
                 self.h, slot, int(n_samples), float(shutter), out["blur_rgb"].ctypes.data,
                 out["blur_rgb0"].ctypes.data if input_frame else None, seq["blur_rgb"].ctypes.data if K else None),
                 "arapb200_batch_scene_blur")
+        t = _track_arrays(out, tracks, q, K, H, W)
+        if t is not None:
+            self._keep[slot] += (q,)
+            _attach_tracks(self.L, self.h, slot, t, q)
         return out
 
     def run(self):

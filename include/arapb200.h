@@ -59,6 +59,15 @@ ARAPB200_API int arapb200_warp_ex(int W, int H, const float* pos_or_flow, int is
 ARAPB200_API int arapb200_warp_seq(int W, int H, int K, const float* pos, const uint8_t* rgb, const uint8_t* mask_red,
                                    uint8_t* out_rgb, uint8_t* out_mask, float* out_flow, float* out_bflow,
                                    uint8_t* out_occ, float* out_flow0);
+/* Tracks from frame 0 (DESIGN.md 4.9) of the frame sequence arapb200_warp_seq renders from the same pos and mask_red:
+ * out_bflow0 float2[K][W*H], frame k -> frame 0 on the frame k grid (at every pixel something landed on in frame k, the
+ * weights of its winning triangle applied to that triangle's vertices on the pixel grid, minus the pixel; (0, 0)
+ * elsewhere); out_occ0 uint8[K][W*H], the occlusion of frame 0 in frame k (0 visible, 255 not: arapb200_warp_ex's rule
+ * with the forward flow P_k - grid, frame k's z-buffer and out_bflow0).  Index k - 1 holds frame k; frame 1 is
+ * arapb200_warp_seq's out_bflow and out_occ.  The same bits as arapb200_batch_tracks.  Either output may be NULL.
+ * Returns non-zero for W, H or K <= 0 and a NULL pos or mask_red. */
+ARAPB200_API int arapb200_warp_tracks(int W, int H, int K, const float* pos, const uint8_t* mask_red, float* out_bflow0,
+                                      uint8_t* out_occ0);
 
 /* ---- one image / segment, end to end (replaces deformSingle, deformation/src/main.cpp:140-160:
  * border pins :130-136, resetGPU + continuation CombinedSolver.h:172-242, solve, warp, flow :352-366).
@@ -214,6 +223,30 @@ ARAPB200_API int arapb200_batch_submit_scene(arapb200_batch* b, int slot, int n_
  * one). */
 ARAPB200_API int arapb200_batch_scene_blur(arapb200_batch* b, int slot, int n_samples, double shutter, uint8_t* blur_rgb,
                                            uint8_t* blur_rgb0, uint8_t* seq_blur_rgb);
+/* Tracks from frame 0 to every frame (DESIGN.md 4.9) for the next run: slot holds a problem queued with frames
+ * (arapb200_batch_submit_seq, n_frames > 0) or is the first slot of a scene queued with frames.  Every output is
+ * frame-major, index k - 1 holding frame k; each dense one may be NULL.
+ * flow0 float2[K][W*H], frame 0 -> k on the frame 0 grid: P_k - grid for a problem (the bits of its seq_flow0), and for a
+ * scene the flow of the layer whose input mask has the pixel on its object (the last one), else the background's A_k(p)
+ * - p.  bflow0 float2[K][W*H], frame k -> 0 on the frame k grid: arapb200_warp_tracks's out_bflow0 for a problem; for a
+ * scene the front layer's (the last one whose frame-k warped mask is non-zero), else inv(A_k)(q) - q.  occ0 uint8[K][W*H]:
+ * the occlusion of frame 0 in frame k (0 visible, 255 not), the rule of arapb200_warp_ex for a problem and of
+ * arapb200_composite (motion_from = NULL, motion_to = A_k) for a scene.  Frame 1's bflow0 and occ0 are the sequence's
+ * frame-1 bflow and occ.
+ * queries int32[n_queries][2]: (x, y) pixels of frame 0, copied; query_pos float2[K][n_queries] = (x, y) + flow0[k] at
+ * the query, query_occ uint8[K][n_queries] = occ0[k] there (may be NULL), gathered on the device.
+ * The run computes the dense outputs on the device whichever are asked for: a problem's slot keeps 9 B/px per frame more,
+ * a scene's layers 8 B/px per frame each and the scene's buffer 17 B/px per frame and 9 B per query and frame; outputs
+ * are copied straight into the caller's buffers.  The kernels count in arapb200_batch_launches and in the warp span of
+ * arapb200_batch_timing: per frame k >= 2, two for a problem and one per scene layer; per frame two for a scene; one
+ * gather with queries.  Applies to the next run only; a second call replaces the first, and a new submit into the
+ * problem's slot drops it.
+ * Returns non-zero, and changes nothing, for: a NULL batch; a slot that holds no problem queued with frames and is not
+ * the first slot of a scene queued with frames; nothing asked for (every dense output NULL and n_queries == 0);
+ * n_queries < 0; queries without a queries array or without query_pos (query_occ may be NULL); query_pos or query_occ
+ * without queries; a query outside the W x H frame; and, for a scene, a frame motion A_k whose maps are non-finite. */
+ARAPB200_API int arapb200_batch_tracks(arapb200_batch* b, int slot, float* flow0, float* bflow0, uint8_t* occ0,
+                                       int n_queries, const int32_t* queries, float* query_pos, uint8_t* query_occ);
 /* The sub-frame table a blurred scene uses for one image (DESIGN.md 4.8); host only, no CUDA call.  nCont, the frames'
  * steps and motions as arapb200_batch_submit_scene takes them (n_frames 0: steps and frame_motions may be NULL);
  * image -1 = frame 0, 0 = the pair, k = frame k.  Per sub-frame j < n_samples: out_state[j] = j0, the lower continuation
@@ -231,7 +264,7 @@ ARAPB200_API int arapb200_batch_run(arapb200_batch* b);
 /* device milliseconds of the last run: [0] total, [1] solve kernels only, [2] warp kernels only (with the scenes'
  * composite kernels) */
 ARAPB200_API int arapb200_batch_timing(arapb200_batch* b, float* ms3);
-/* number of kernel launches issued by the last run (the scenes' composite kernels included) */
+/* number of kernel launches issued by the last run (the scenes' composite kernels and the tracks' kernels included) */
 ARAPB200_API long long arapb200_batch_launches(arapb200_batch* b);
 
 /* how many problems of the last run were solved by the resident (on-chip) back-end; the rest took the streaming one */
